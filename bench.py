@@ -2,6 +2,7 @@
 """Throughput benchmark of the catfish inference hot path (contract in the task statement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--legs main,probs,python,job,configs,cpu,check]
+                    [--dump-outputs DIR]
 
 Workload of the headline line (BASELINE.json configs[3], the configuration the metric is quoted on):
 ResNetRNN with the shipped checkpoint over synthetic raw-signal reads of ragged length
@@ -33,6 +34,10 @@ Further legs, extra keys on the same JSON line:
 
 --impl reference times the CPU restatement (TensorFlow itself is not installable offline; see DESIGN.md)
 on bounded samples of the same workload.
+
+--dump-outputs DIR writes what the last timed step of `value` returned to its caller (rank 0's batch, which the
+seeds make the same from run to run and for every --gpus) as float64 .npy files, so that two builds can be
+compared output for output; see dump_outputs.
 """
 import argparse
 import ctypes
@@ -49,6 +54,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree, which may be read-only
 
 METRIC = "raw_signal_samples_per_sec_resnetrnn_infer"
 UNIT = "samples/s"
@@ -56,6 +62,7 @@ LEN_LO, LEN_HI = 50_000, 200_000
 JOB_READS = 16384
 JOB_POOL = 4096
 JOB_SEED = 20_000
+DUMP_BYTES = 64 << 20
 
 # algorithmic work per real sample (SURVEY.md section 8d / BASELINE.md section 4)
 BYTES_PER_SAMPLE = {"k1_stats": 2.0, "k6_intervals": 4.0, "k1_window_table": 0.0}
@@ -92,7 +99,14 @@ def parse_args():
     ap.add_argument("--legs", default=None,
                     help="comma list of main,probs,python,job,configs,cpu,check (default: all at N=1; main,job at N>1)")
     ap.add_argument("--job-reads", type=int, default=JOB_READS)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 def load_peaks():
@@ -169,6 +183,22 @@ def make_batch(n_reads, seed):
     lengths = synth.ragged_lengths(n_reads, LEN_LO, LEN_HI, seed=seed)
     reads = synth.synth_reads(lengths, base_seed=seed * 1_000_003)
     return synth.concat_reads(reads)
+
+
+def dump_outputs(out_dir, iv, ioff):
+    """Write one cf_infer_reads result (intervals int64 [n, 2], CSR offsets int64 [reads + 1]) as float64, which
+    holds these integers exactly: intervals.npy [n, 2], interval_offsets.npy [reads + 1] and read_ids.npy [reads],
+    the batch index of each read written.  A result above DUMP_BYTES is cut to a fixed seeded sample of whole reads."""
+    counts = np.diff(ioff)
+    order = np.random.default_rng(0).permutation(len(counts))
+    fits = np.cumsum(16 * counts[order] + 16) <= DUMP_BYTES - 4096           # 16 B per interval, 16 B per read
+    reads = np.sort(order[:int(np.count_nonzero(fits))])
+    rows = np.concatenate([np.arange(ioff[r], ioff[r + 1]) for r in reads] + [np.zeros(0, np.int64)])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "intervals.npy"), iv[rows].reshape(-1, 2).astype(np.float64))
+    np.save(os.path.join(out_dir, "interval_offsets.npy"),
+            np.concatenate([[0], np.cumsum(counts[reads])]).astype(np.float64))
+    np.save(os.path.join(out_dir, "read_ids.npy"), reads.astype(np.float64))
 
 
 def workload_config(reads_per_step, engine):
@@ -419,6 +449,10 @@ def run_b200(args):
     launches = _cabi.launch_count() - launches0
     prof = _cabi.profile_read(handle)
     _cabi.profile_enable(handle, False)
+    if args.dump_outputs and rank == 0:
+        # the last timed step ran batch (steps - 1) % 2; its result is still in iv_dev / ioff_dev
+        ioff_last = ioff_dev.cpu().numpy()
+        dump_outputs(args.dump_outputs, iv_dev[:int(ioff_last[-1])].cpu().numpy(), ioff_last)
 
     # ---- timed region 2: host buffers through the public C-ABI call
     for i in range(2):
@@ -610,7 +644,7 @@ def configs_leg(args, resnetrnn, peaks):
     lib = _cabi.load_library()
     stream = torch.cuda.current_stream()
     sp = stream.cuda_stream
-    steps = 3
+    steps = args.steps
     out = {}
 
     def measure(model, kind, step_fn, samples_per_step, reads_per_step, describe, flops_of=None):
