@@ -75,7 +75,6 @@ SIGNATURES = {
     "cf_vote_events": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int64, c_i64_p, ctypes.c_int64, ctypes.c_int64,
                                       ctypes.c_int64, c_void, c_i64_p, c_i64_p, c_i64_p, ctypes.POINTER(ctypes.c_int32),
                                       c_void]),
-    "cf_selftest_xproj": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int64, ctypes.c_int32, c_void, c_void, c_void, c_void]),
     "cf_selftest_f16e5": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int32, ctypes.c_int32, c_void, ctypes.c_int32, c_void, c_void]),
     "cf_launch_count": (ctypes.c_int64, []),
 }

@@ -584,14 +584,6 @@ int cf_split_raw(int32_t device, const int16_t* raw_dev, const int64_t* offsets_
     return s;
 }
 
-int cf_selftest_xproj(int32_t device, const float* a_dev, int64_t n_blocks, int32_t k, const float* wx_host,
-                      const float* bias_host, float* out_dev, void* stream) {
-    if (!a_dev || !wx_host || !bias_host || !out_dev || n_blocks <= 0) { cf::set_error("cf_selftest_xproj: bad argument"); return CF_ERR_BAD_ARG; }
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(device));
-    return cf::tc_selftest_xproj(a_dev, n_blocks, k, wx_host, bias_host, out_dev, static_cast<cudaStream_t>(stream));
-}
-
 int cf_selftest_f16e5(int32_t device, const float* a_dev, int32_t k, int32_t n, const float* w_host, int32_t mode,
                       float* out_dev, void* stream) {
     if (!a_dev || !w_host || !out_dev) { cf::set_error("cf_selftest_f16e5: bad argument"); return CF_ERR_BAD_ARG; }

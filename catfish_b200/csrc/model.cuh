@@ -71,7 +71,5 @@ int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const doubl
                cudaStream_t stream, Profiler* prof, bool want_logits = false, const LabelBits* bits = nullptr);
 
 int tc_selftest_f16e5(const float* a_dev, int K, int N, const float* w_host, int mode, float* out_dev, cudaStream_t stream);
-int tc_selftest_xproj(const float* a_dev, int64_t n_blocks, int K, const float* wx_host, const float* bias_host,
-                      float* out_dev, cudaStream_t stream);
 
 }  // namespace cf

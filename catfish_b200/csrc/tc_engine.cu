@@ -13,19 +13,16 @@
 //   TK4G  tc_gru_fused2_kernel   one GRU layer (input projection + recurrence), two tiles per CTA
 //   TK5   tc_head_kernel         dense 128 -> 1 + sigmoid from the partial dots of the last layer
 // (the conv stack and the GRU layer it feeds use bf16x3, the 128-wide GRU layers f16e5).
-// Other shapes / cross-checks: tc_conv2_kernel (networks with ONE residual block), and the unfused pair
-//   TK3   tc_xproj_kernel  GRU input projection  xp = y W_x + b   (rnn_class.py:146,170: the
-//         x rows of gates/kernel and candidate/kernel, hoisted out of the time loop)
-//   TK4   tc_gru_kernel    GRU recurrence over the 35 steps of a window tile, both directions
-//         as two independent chains per CTA (rnn_class.py:142-175)
-// (CF_TC_UNFUSED=1 only; layer 0 of RNN-only networks, whose input is 1 wide, is the KX = 1 form of TK4G:
-// no x MMAs, the rank-1 update x_t * w_row is added in the epilogue).
+// Other shapes: tc_conv2_kernel (networks with ONE residual block), tc_head_conv_kernel (ResNet-only
+// networks with one residual block), tc_pack_a_kernel (conv stacks of more than two blocks run on the
+// CUDA-core engine; their output is packed into the first GRU layer's operand form).  Layer 0 of
+// RNN-only networks, whose input is 1 wide, is the KX = 1 form of TK4G: no x MMAs, the rank-1 update
+// x_t * w_row is added in the epilogue.
 //
 // Data layout: a tile is 128 windows (= 128 TMEM lanes = UMMA M); a block is (tile, t), one of
 // the 35 positions of those windows.  Activations that feed an MMA live in global memory as
 // ready-made UMMA operands: per block plane 0 then plane 1, each [K/8][128][16 bytes], so a
-// block is one contiguous cp.async.bulk (TMA) copy.  xp is stored per block as [384][128] fp32
-// (column-major), which makes both its producer (TMEM lane = window) and its consumer coalesced.
+// block is one contiguous cp.async.bulk (TMA) copy.
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
@@ -47,14 +44,6 @@ constexpr float kGateScale = -1.4426950408889634f;    // -log2(e)
 constexpr float kCandScale = 2.8853900817779268f;     // 2 log2(e)
 
 constexpr int kFmtBf16x3 = 0, kFmtF16E5 = 1;   // operand formats, see "operand formats" below
-
-// Sensitivity experiments on TK4G, BUILD-TIME ONLY (-DCF_EXP=<bits>, tools/ab_exp.sh builds variant libraries;
-// the shipped library is always built with 0 and contains none of this): 1 = no x traffic, 2 = no correction
-// MMAs, 4 = no layer-output stores, 8 = no MUFU in the epilogue.  Results of such builds are wrong by design.
-#ifndef CF_EXP
-#define CF_EXP 0
-#endif
-constexpr int kExp = CF_EXP;
 
 struct ConvParams {                    // byte offsets inside the parameter block
     static constexpr int kFloats = 10 * 32;              // a_sc b_sc a1 b1 | b2 b3 b4 b5 b6 b7
@@ -112,11 +101,7 @@ static void pack_b_operand_f16e5(const float* w, int K, int N, int ldw, int col0
 
 struct TcLayer {
     int in = 0;                       // input features of this GRU layer (1, 32 or 128)
-    __nv_bfloat16* wx = nullptr;      // [dir][plane][in/8][192][8]          (in >= 32)
-    float* wx_f32 = nullptr;          // [in][384] fp32                       (in == 1)
-    float* bx = nullptr;              // [384]
-    __nv_bfloat16* wh = nullptr;      // [dir]{Wg hi, Wg lo [8][128][8]; Wc hi, Wc lo [8][64][8]}
-    uint8_t* wfused = nullptr;        // [dir]{Wgx, Wcx, Wgh, Wch} as in GruFusedCfg (in = 32 or 128), exponent domain
+    uint8_t* wfused = nullptr;        // [dir]{Wgx, Wcx, Wgh, Wch} as in GruF2Cfg (no Wgx, Wcx for in = 1), exponent domain
     int fmt = 0;                      // operand format of wfused / of this layer's x and state operands
     float* bz = nullptr;              // [384] biases in the exponent domain
     float* wxz = nullptr;             // [384] the single x row of gates / candidate kernels, exponent domain (in == 1)
@@ -133,12 +118,13 @@ struct TcEngine {
     DevBuf ws;
     int n_sms = 148;
     bool attr_done = false;
+#ifdef CF_TRACE_PROBES
     bool trace_done = false;
     const char* trace_path = nullptr; // CF_TC_TRACE=<file>: in-kernel timeline of one TK4G launch (debug; results unaffected)
-    bool use_fused = true;            // CF_TC_UNFUSED=1 selects the xp + recurrence pair (TK3 + TK4)
-    int fmt = kFmtBf16x3;             // operand format of the 128-wide fused GRU layers (kFmtF16E5 unless CF_TC_FMT=0 or a
-                                      // cross-check variant / a network the default kernels do not cover is selected); the
-                                      // conv stack and the first GRU layer (input = conv output) always run bf16x3
+#endif
+    int fmt = kFmtBf16x3;             // operand format of the 128-wide GRU layers (kFmtF16E5 unless the network is not
+                                      // covered by f16e5 kernels or its weights are out of fp16 range); the conv stack
+                                      // and the first GRU layer (input = conv output) always run bf16x3
 };
 
 bool tc_supported(const HostModel& hm) {
@@ -164,14 +150,14 @@ TcEngine* tc_create(const HostModel& hm) {
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&e->n_sms, cudaDevAttrMultiProcessorCount, dev);
     e->simt = simt_create(hm);
-    if (const char* env = getenv("CF_TC_UNFUSED")) e->use_fused = !(env[0] == '1');
+#ifdef CF_TRACE_PROBES
     e->trace_path = getenv("CF_TC_TRACE");
+#endif
     {
         // fp16 + e5m2 operands need every tensor-core kernel of the pass to speak the format: the default
         // conv stack (two residual blocks) followed by fused GRU layers only
-        const bool covered = e->use_fused && ((hm.desc.network_type == CF_NET_RESNET_RNN && hm.n_res() == 2 && hm.conv_channels() == kC) ||
-                                              hm.desc.network_type == CF_NET_RNN);
-        const char* env = getenv("CF_TC_FMT");
+        const bool covered = (hm.desc.network_type == CF_NET_RESNET_RNN && hm.n_res() == 2 && hm.conv_channels() == kC) ||
+                             hm.desc.network_type == CF_NET_RNN;
         float wmax = 0.f;                             // the fp16 weight plane is stored times S = 64
         for (const GruDir& g : hm.gru) {
             for (float v : g.wx) wmax = std::max(wmax, std::fabs(v));
@@ -179,18 +165,17 @@ TcEngine* tc_create(const HostModel& hm) {
             for (float v : g.wch) wmax = std::max(wmax, std::fabs(v));
         }
         const bool in_range = wmax * kCandScale * kCorrScale < 60000.f;
-        e->fmt = covered && in_range && !(env && env[0] == '0') ? kFmtF16E5 : kFmtBf16x3;
+        e->fmt = covered && in_range ? kFmtF16E5 : kFmtBf16x3;
     }
     if (hm.n_res() >= 1 && hm.n_res() <= 2 && hm.conv_channels() == kC) {
-        // TK2 parameter block: fp32 vectors, then the B operands in the given format (see ConvParams)
-        auto build_conv_block = [&](int fmt) {
+        // TK2 parameter block: fp32 vectors, then the B operands, split bf16 (see ConvParams)
         std::vector<uint8_t> blk(ConvParams::kBytes, 0);
         float* fp = reinterpret_cast<float*>(blk.data());
         auto put = [&](int slot, const std::vector<float>& v) { memcpy(fp + 32 * slot, v.data(), 32 * sizeof(float)); };
         put(0, hm.convs[0].w); put(1, hm.convs[0].b);          // shortcut of block 0: [1][1][32]
         put(2, hm.convs[1].w); put(3, hm.convs[1].b);
         put(4, hm.convs[2].b); put(5, hm.convs[3].b);
-        auto put_w_bf16 = [&](int off, const float* w, int n, int ldw, int col0, int dst_col0, int n_total) {
+        auto put_w = [&](int off, const float* w, int n, int ldw, int col0, int dst_col0, int n_total) {
             // pack a [32][n] matrix into columns [dst_col0, dst_col0 + n) of a {hi, lo} x [4][n_total][8] operand
             __nv_bfloat16* hi = reinterpret_cast<__nv_bfloat16*>(blk.data() + off);
             __nv_bfloat16* lo = hi + 32 * n_total;
@@ -203,26 +188,6 @@ TcEngine* tc_create(const HostModel& hm) {
                     lo[idx] = __float2bfloat16_rn(v - __bfloat162float(h));
                 }
         };
-        auto& put_w_bf = put_w_bf16;
-        auto put_w_e5 = [&](int off, const float* w, int n, int ldw, int col0, int dst_col0, int n_total) {
-            // the same [32][n] matrix in the f16e5 format: fp16 plane, then e5m2 [4][n_total][16]
-            uint16_t* mn = reinterpret_cast<uint16_t*>(blk.data() + off);
-            uint8_t* cr = blk.data() + off + 32 * n_total * 2;
-            for (int k = 0; k < 32; ++k)
-                for (int j = 0; j < n; ++j) {
-                    const float v = w[(size_t)k * ldw + col0 + j];
-                    const __half h = __float2half_rn(v);
-                    const float hf = __half2float(h);
-                    mn[((size_t)(k / 8) * n_total + dst_col0 + j) * 8 + (k % 8)] = *reinterpret_cast<const uint16_t*>(&h);
-                    const int c = k / 16, kc = k % 16;
-                    cr[((size_t)(2 * c) * n_total + dst_col0 + j) * 16 + kc] = (uint8_t)__nv_cvt_float_to_fp8(hf / kCorrScale, __NV_SATFINITE, __NV_E5M2);
-                    cr[((size_t)(2 * c + 1) * n_total + dst_col0 + j) * 16 + kc] = (uint8_t)__nv_cvt_float_to_fp8((v - hf) * kCorrScale, __NV_SATFINITE, __NV_E5M2);
-                }
-        };
-        auto put_w = [&](int off, const float* w, int n, int ldw, int col0, int dst_col0, int n_total) {
-            if (fmt == kFmtF16E5) put_w_e5(off, w, n, ldw, col0, dst_col0, n_total);
-            else put_w_bf(off, w, n, ldw, col0, dst_col0, n_total);
-        };
         for (int tap = 0; tap < 3; ++tap) put_w(ConvParams::kW2 + tap * 4096, hm.convs[2].w.data() + tap * 32 * 32, 32, 32, 0, 0, 32);
         put_w(ConvParams::kW3, hm.convs[3].w.data(), 32, 32, 0, 0, 32);
         if (hm.n_res() == 2) {
@@ -232,73 +197,40 @@ TcEngine* tc_create(const HostModel& hm) {
             for (int tap = 0; tap < 3; ++tap) put_w(ConvParams::kW6 + tap * 4096, hm.convs[6].w.data() + tap * 32 * 32, 32, 32, 0, 0, 32);
             put_w(ConvParams::kW7, hm.convs[7].w.data(), 32, 32, 0, 0, 32);
         }
-        return blk;
-        };
-        e->conv_params = tc_upload(e, build_conv_block(kFmtBf16x3));    // the conv stack is bf16x3 throughout
+        e->conv_params = tc_upload(e, blk);
         e->conv_nres = hm.n_res();
     }
     for (int l = 0; l < hm.n_rnn(); ++l) {
         TcLayer L;
-        const GruDir& f = hm.gru[2 * l];
-        const GruDir& b = hm.gru[2 * l + 1];
-        L.in = f.in;
-        std::vector<float> bx(2 * kNX);
-        for (int j = 0; j < kNX; ++j) { bx[j] = f.bx[j]; bx[kNX + j] = b.bx[j]; }
-        L.bx = tc_upload(e, bx);
-        if (L.in % 16 == 0) {
-            std::vector<__nv_bfloat16> wx;
-            pack_b_operand(f.wx.data(), L.in, kNX, kNX, 0, &wx);
-            pack_b_operand(b.wx.data(), L.in, kNX, kNX, 0, &wx);
-            L.wx = tc_upload(e, wx);
-        } else {
-            std::vector<float> wx((size_t)L.in * 2 * kNX);
-            for (int k = 0; k < L.in; ++k)
-                for (int j = 0; j < kNX; ++j) {
-                    wx[(size_t)k * 2 * kNX + j] = f.wx[(size_t)k * kNX + j];
-                    wx[(size_t)k * 2 * kNX + kNX + j] = b.wx[(size_t)k * kNX + j];
-                }
-            L.wx_f32 = tc_upload(e, wx);
-        }
-        std::vector<__nv_bfloat16> wh;
+        L.in = hm.gru[2 * l].in;
+        // The layer fed by the conv stack stays bf16x3: it contributes nearly all of f16e5's extra error
+        // (emulation: 5.8e-5 of 6.1e-5; conv activations span 2^-10 .. 60 and would need an fp16 range
+        // guard) and its K = 32 input part is too small to gain from the cheaper passes.
+        L.fmt = L.in == kC ? kFmtBf16x3 : e->fmt;
+        std::vector<__nv_bfloat16> wf;
         for (int d = 0; d < 2; ++d) {
             const GruDir& g = hm.gru[2 * l + d];
-            pack_b_operand(g.wgh.data(), kH, 2 * kH, 2 * kH, 0, &wh);
-            pack_b_operand(g.wch.data(), kH, kH, kH, 0, &wh);
+            // exponent domain: gates scaled by -log2(e), candidate by 2 log2(e) (see sigmoid4_z / tanh4_z)
+            // x rows of gates/kernel and candidate/kernel side by side: one N = 192 operand
+            auto pack = L.fmt == kFmtF16E5 ? pack_b_operand_f16e5 : pack_b_operand;
+            if (L.in > 1) pack(g.wx.data(), L.in, kNX, kNX, 0, &wf, kGateScale, 2 * kH, kCandScale);
+            pack(g.wgh.data(), kH, 2 * kH, 2 * kH, 0, &wf, kGateScale, 1 << 30, 1.f);
+            pack(g.wch.data(), kH, kH, kH, 0, &wf, kCandScale, 1 << 30, 1.f);
         }
-        L.wh = tc_upload(e, wh);
-        if (L.in == kC || L.in == 2 * kH || L.in == 1) {
-            auto build_fused = [&](int fmt) {
-                std::vector<__nv_bfloat16> wf;
-                for (int d = 0; d < 2; ++d) {
-                    const GruDir& g = hm.gru[2 * l + d];
-                    // exponent domain: gates scaled by -log2(e), candidate by 2 log2(e) (see sigmoid4_z / tanh4_z)
-                    // x rows of gates/kernel and candidate/kernel side by side: one N = 192 operand
-                    auto pack = fmt == kFmtF16E5 ? pack_b_operand_f16e5 : pack_b_operand;
-                    if (L.in > 1) pack(g.wx.data(), L.in, kNX, kNX, 0, &wf, kGateScale, 2 * kH, kCandScale);
-                    pack(g.wgh.data(), kH, 2 * kH, 2 * kH, 0, &wf, kGateScale, 1 << 30, 1.f);
-                    pack(g.wch.data(), kH, kH, kH, 0, &wf, kCandScale, 1 << 30, 1.f);
-                }
-                return wf;
-            };
-            // The layer fed by the conv stack stays bf16x3: it contributes nearly all of f16e5's extra error
-            // (emulation: 5.8e-5 of 6.1e-5; conv activations span 2^-10 .. 60 and would need an fp16 range
-            // guard) and its K = 32 input part is too small to gain from the cheaper passes.
-            L.fmt = L.in == kC ? kFmtBf16x3 : e->fmt;
-            L.wfused = reinterpret_cast<uint8_t*>(tc_upload(e, build_fused(L.fmt)));
-            std::vector<float> bz(2 * kNX);
+        L.wfused = reinterpret_cast<uint8_t*>(tc_upload(e, wf));
+        std::vector<float> bz(2 * kNX);
+        for (int d = 0; d < 2; ++d)
+            for (int j = 0; j < kNX; ++j)
+                bz[d * kNX + j] = hm.gru[2 * l + d].bx[j] * (j < 2 * kH ? kGateScale : kCandScale);
+        L.bz = tc_upload(e, bz);
+        if (L.in == 1) {
+            // RNN-only layer 0 (neural_network.py:17-18): the x part of concat([x, h]) W is a rank-1 update
+            // x_t * w_row, added to the bias in the epilogue of the fused kernel - no MMA
+            std::vector<float> wxz(2 * kNX);
             for (int d = 0; d < 2; ++d)
                 for (int j = 0; j < kNX; ++j)
-                    bz[d * kNX + j] = hm.gru[2 * l + d].bx[j] * (j < 2 * kH ? kGateScale : kCandScale);
-            L.bz = tc_upload(e, bz);
-            if (L.in == 1) {
-                // RNN-only layer 0 (neural_network.py:17-18): the x part of concat([x, h]) W is a rank-1 update
-                // x_t * w_row, added to the bias in the epilogue of the fused kernel - no MMA, no projection buffer
-                std::vector<float> wxz(2 * kNX);
-                for (int d = 0; d < 2; ++d)
-                    for (int j = 0; j < kNX; ++j)
-                        wxz[d * kNX + j] = hm.gru[2 * l + d].wx[j] * (j < 2 * kH ? kGateScale : kCandScale);
-                L.wxz = tc_upload(e, wxz);
-            }
+                    wxz[d * kNX + j] = hm.gru[2 * l + d].wx[j] * (j < 2 * kH ? kGateScale : kCandScale);
+            L.wxz = tc_upload(e, wxz);
         }
         e->layers.push_back(L);
     }
@@ -347,26 +279,19 @@ __global__ void tc_pack_a_kernel(const float* __restrict__ in, int K, int64_t n_
 // t, so the k = 3 taps are whole 128-row operand slices of t-1, t, t+1 and the "same" padding at
 // the window edges is simply a skipped MMA.
 //
-// Time-skewed schedule over u = 0..37 (block-1 stages only when NRES == 2):
-//   phase 1  o1[u]    = relu(x a1 + b1)                     CUDA cores      -> O1[u % 3]
-//   round 1  o2[u-1]  = relu(conv3(o1) + b2)  ;  p2[u-3] = relu(conv3(p1) + b6)
-//   round 2  o3[u-1] -> y0 = relu(relu(o3 + b3) + sc0)  ;  p3[u-3] -> y1 = relu(relu(p3 + b7) + sc1)
-//   round 3  [sc1 | p1][u-1] = y0 [W4 | W5]   (sc1 stays in TMEM until y1 needs it)
-// Each round is: operands to smem -> one thread issues the MMAs -> commit -> all threads run the
-// TMEM epilogue for their own window (thread = TMEM lane = window).
 constexpr uint32_t kSliceBytes = 2u * 128 * kC * 2;       // one position of a tile as A operand: 16 KB
 constexpr uint32_t kConvSmem = ConvParams::kBytes + 10 * kSliceBytes + 35 * 128 * 4 + 256;   // tc_conv2: O1 ring of 4
 
-// ====================================================================== TK2 v2: deeper skew, one round per position
-// The residual stack with every operand slice in shared memory; the five MMA stages of the two residual
-// blocks are skewed over time so that ALL of them are issued in one batch per iteration u:
-//   o2[u-1], o3[u-2], [sc1|p1][u-3], p2[u-5], p3[u-6]
-// followed by ONE epilogue pass that consumes the five accumulators (all TMEM loads in flight at
-// once), writes the next operands, and computes o1[u+1] on CUDA cores.  One commit + one
-// "operands ready" barrier per iteration instead of three block-wide rounds.
+// ====================================================================== TK2, one residual block
+// Every operand slice in shared memory; the two MMA stages of the block are skewed over time so that
+// both are issued in one batch per iteration u = 0..36:
+//   o2[u-1] = relu(conv3(o1) + b2)                  TMEM 0
+//   o3[u-2] -> y0 = relu(relu(o3 + b3) + sc0)       TMEM 32; y0 is the kernel's output
+// followed by ONE epilogue pass that consumes both accumulators (all TMEM loads in flight at once),
+// writes the next operand, and computes o1[u+2] = relu(x a1 + b1) on CUDA cores (ring of 4 slices).
+// One commit + one "operands ready" barrier per iteration.
 //   warps 0-7 : epilogue; thread = (window, 16 of the 32 channels)
 //   warp 8    : MMA issuer (warp-converged issue, elected lane)
-// TMEM: o2 0, o3 32, p2 64, p3 96, [sc1|p1] ring of 4 at 128 + 64 k (sc1 is read 3 iterations later).
 __device__ __forceinline__ void store_a_row16(uint8_t* slice, int row, int c0, const float* v) {
 #pragma unroll
     for (int g = 0; g < 2; ++g) {
@@ -393,7 +318,6 @@ __device__ __forceinline__ void conv_mma_pred(uint32_t tmem_d, uint32_t a_slice,
     }
 }
 
-template <int NRES>
 __global__ void __launch_bounds__(288, 1)
 tc_conv2_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ raw, const double* __restrict__ stats,
                 const float* __restrict__ xwin, const int64_t* __restrict__ src, const int32_t* __restrict__ valid,
@@ -427,20 +351,20 @@ tc_conv2_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
     __syncthreads();
     tc_fence_after_sync();
     const uint32_t tmem = *tmem_slot;
-    constexpr int kLastU = NRES == 2 ? kWindow + 5 : kWindow + 1;      // p3[34] at u = 40, o3[34] at u = 36
+    constexpr int kLastU = kWindow + 1;               // o3[34] at u = 36
     mbar_wait(bar_prm, 0);
 
     if (warp == 8) {
         // ------------------------------------------------------------ issuer (all lanes converged)
         const uint32_t elected = elect_one();
         const uint32_t prm_u = smem_u32(prm);
-        const uint32_t o1_u = smem_u32(o1), o2_u = smem_u32(o2), y0_u = smem_u32(y0), p1_u = smem_u32(p1), p2_u = smem_u32(p2);
+        const uint32_t o1_u = smem_u32(o1), o2_u = smem_u32(o2);
         uint32_t it = 0;
         for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
             for (int u = 0; u <= kLastU; ++u, ++it) {
                 mbar_wait(bar_ready, it & 1);
                 tc_fence_after_sync();
-                const int t1 = u - 1, t2 = u - 2, t3 = u - 3, t4 = u - 5, t5 = u - 6;
+                const int t1 = u - 1, t2 = u - 2;
                 if (t1 >= 0 && t1 < kWindow) {
                     bool first = true;
 #pragma unroll
@@ -452,21 +376,6 @@ tc_conv2_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                     }
                 }
                 if (t2 >= 0 && t2 < kWindow) conv_mma_pred<32>(tmem + 32, o2_u, prm_u + ConvParams::kW3, true, elected);
-                if (NRES == 2) {
-                    if (t3 >= 0 && t3 < kWindow)
-                        conv_mma_pred<64>(tmem + 128 + (t3 & 3) * 64, y0_u, prm_u + ConvParams::kW45, true, elected);
-                    if (t4 >= 0 && t4 < kWindow) {
-                        bool first = true;
-#pragma unroll
-                        for (int tap = 0; tap < 3; ++tap) {
-                            const int tt = t4 + tap - 1;
-                            if (tt < 0 || tt >= kWindow) continue;
-                            conv_mma_pred<32>(tmem + 64, p1_u + (tt % 3) * kSliceBytes, prm_u + ConvParams::kW6 + tap * 4096, first, elected);
-                            first = false;
-                        }
-                    }
-                    if (t5 >= 0 && t5 < kWindow) conv_mma_pred<32>(tmem + 96, p2_u, prm_u + ConvParams::kW7, true, elected);
-                }
                 umma_commit_pred(bar_mma, elected);
             }
         }
@@ -518,21 +427,13 @@ tc_conv2_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_ready);
             for (int u = 0; u <= kLastU; ++u, ++it) {
-                const int t1 = u - 1, t2 = u - 2, t3 = u - 3, t4 = u - 5, t5 = u - 6;
+                const int t1 = u - 1, t2 = u - 2;
                 const bool h1 = t1 >= 0 && t1 < kWindow, h2 = t2 >= 0 && t2 < kWindow;
-                const bool h3 = NRES == 2 && t3 >= 0 && t3 < kWindow, h4 = NRES == 2 && t4 >= 0 && t4 < kWindow;
-                const bool h5 = NRES == 2 && t5 >= 0 && t5 < kWindow;
                 mbar_wait(bar_mma, it & 1);
                 tc_fence_after_sync();
-                uint32_t r1[16], r2[16], r3[16], r4[16], r5[16], rs[16];
+                uint32_t r1[16], r2[16];
                 if (h1) tmem_ld16_nowait(t_lane + 0, r1);
                 if (h2) tmem_ld16_nowait(t_lane + 32, r2);
-                if (h3) tmem_ld16_nowait(t_lane + 128 + (t3 & 3) * 64 + 32, r3);
-                if (h4) tmem_ld16_nowait(t_lane + 64, r4);
-                if (h5) {
-                    tmem_ld16_nowait(t_lane + 96, r5);
-                    tmem_ld16_nowait(t_lane + 128 + (t5 & 3) * 64, rs);
-                }
                 tmem_ld_wait();
                 tc_fence_before_sync();
                 float v[16];
@@ -542,23 +443,14 @@ tc_conv2_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                     const float x = xs[t2 * 128 + row];
 #pragma unroll
                     for (int i = 0; i < 16; ++i) v[i] = fmaxf(v[i] + fmaf(x, fp[c0 + i], fp[32 + c0 + i]), 0.f);   // + shortcut
-                    if (NRES == 2) store_a_row16(y0, row, c0, v);
-                    else store_a_row16(reinterpret_cast<uint8_t*>(y_out) + ((size_t)tile * kWindow + t2) * kSliceBytes, row, c0, v);
+                    store_a_row16(reinterpret_cast<uint8_t*>(y_out) + ((size_t)tile * kWindow + t2) * kSliceBytes, row, c0, v);
                 }
-                if (h3) { relu_bias(r3, 7, v); store_a_row16(p1 + (t3 % 3) * kSliceBytes, row, c0, v); }   // b5
-                if (h4) { relu_bias(r4, 8, v); store_a_row16(p2, row, c0, v); }                  // b6
-                // operands of the next MMA batch are complete: hand over, then finish the work the
-                // issuer does not wait for (block output y1[u-6], o1 two positions ahead)
+                // operands of the next MMA batch are complete: hand over, then make o1 two positions ahead,
+                // which that batch does not read
                 if (u < kLastU) {
                     fence_proxy_async_smem();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(bar_ready);
-                }
-                if (h5) {
-                    relu_bias(r5, 9, v);                                                         // b7
-#pragma unroll
-                    for (int i = 0; i < 16; ++i) v[i] = fmaxf(v[i] + (__uint_as_float(rs[i]) + fp[192 + c0 + i]), 0.f);   // + sc1 + b4
-                    store_a_row16(reinterpret_cast<uint8_t*>(y_out) + ((size_t)tile * kWindow + t5) * kSliceBytes, row, c0, v);
                 }
                 if (u + 2 < kWindow) make_o1(u + 2);
             }
@@ -613,23 +505,6 @@ __device__ __forceinline__ void store_a_tmem16_f(uint32_t t_slot, const float* v
     tmem_st8_u32(t_slot + 16, s8);
 }
 
-// All MMAs of one K = 32 operand slice against one [32 x N] weight matrix ({plane 0, plane 1}).
-template <int N, int FMT>
-__device__ __forceinline__ void conv_mma_f(uint32_t tmem_d, uint32_t a_slice, uint32_t w_mat, bool first, uint32_t elected) {
-    if (FMT == kFmtBf16x3) {
-        conv_mma_pred<N>(tmem_d, a_slice, w_mat, first, elected);
-    } else {
-        constexpr uint32_t id16 = make_idesc_f16(128, N), id8 = make_idesc_e5m2(128, N);
-#pragma unroll
-        for (int kk = 0; kk < 2; ++kk) {
-            umma_bf16_pred(tmem_d, make_smem_desc(a_slice + kk * 4096, 2048, 128),
-                           make_smem_desc(w_mat + kk * 2 * (N * 16), N * 16, 128), id16, !(first && kk == 0), elected);
-            umma_f8_pred(tmem_d, make_smem_desc(a_slice + 8192 + kk * 4096, 2048, 128),
-                         make_smem_desc(w_mat + kC * N * 2 + kk * 2 * (N * 16), N * 16, 128), id8, 1, elected);
-        }
-    }
-}
-
 // ====================================================================== TK2 v4: two chains, k = 3 operands in tensor memory
 // The two residual blocks as two independently clocked chains, with the A operands of both k = 3 convolutions (the o1 and p1 rings) and y0 held in
 // TENSOR MEMORY: an N = 32 MMA that reads its 4 KB A operand from shared memory is bound by that
@@ -641,19 +516,9 @@ __device__ __forceinline__ void conv_mma_f(uint32_t tmem_d, uint32_t a_slice, ui
 // 288 + 32 k | p1 ring of 3 at 416 + 32 k.  Operand slot: hi K 0-15 | hi K 16-31 | lo K 0-15 | lo K 16-31.
 constexpr uint32_t kConv4Smem = ConvParams::kBytes + 2 * kSliceBytes + 4 * (32 * 128 * 4) + 35 * 128 * 4 + 256;
 
-template <int N, int FMT>
+// conv_mma_pred with the A operand in tensor memory (".ts" form)
+template <int N>
 __device__ __forceinline__ void conv_mma_ts_pred(uint32_t tmem_d, uint32_t tmem_a, uint32_t w_mat, bool first, uint32_t elected) {
-    if (FMT == kFmtF16E5) {
-        constexpr uint32_t id16 = make_idesc_f16(128, N), id8 = make_idesc_e5m2(128, N);
-#pragma unroll
-        for (int kk = 0; kk < 2; ++kk) {
-            umma_bf16_ts_pred(tmem_d, tmem_a + kk * 8, make_smem_desc(w_mat + kk * 2 * (N * 16), N * 16, 128), id16,
-                              !(first && kk == 0), elected);
-            umma_f8_ts_pred(tmem_d, tmem_a + 16 + kk * 8, make_smem_desc(w_mat + kC * N * 2 + kk * 2 * (N * 16), N * 16, 128),
-                            id8, 1, elected);
-        }
-        return;
-    }
     constexpr uint32_t idesc = make_idesc_bf16(128, N);
 #pragma unroll
     for (int pass = 0; pass < 3; ++pass) {
@@ -666,7 +531,6 @@ __device__ __forceinline__ void conv_mma_ts_pred(uint32_t tmem_d, uint32_t tmem_
     }
 }
 
-template <int FMT>
 __global__ void __launch_bounds__(576, 1)
 tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ raw, const double* __restrict__ stats,
                 const float* __restrict__ xwin, const int64_t* __restrict__ src, const int32_t* __restrict__ valid,
@@ -675,10 +539,9 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
     // head_w != nullptr (ResNet-only network, resnet_class.py:23): the dense 32 -> 1 layer is taken in this epilogue -
     // every thread writes the partial dot of its 16 channels to head_part[(block * 2 + half) * 128 + window] and the
     // 128 B/sample operand block is never stored; tc_head_kernel adds the two halves.
-    // FMT is the format of the OUTPUT (the first GRU layer's x operand; the engine uses bf16x3); inside the
-    // stack every operand is split bf16 - the epilogue, not the tensor pipe, bounds this kernel and the bf16
-    // split is the cheaper one.
-    constexpr int kInt = kFmtBf16x3;
+    // Every operand, the output (the first GRU layer's x operand) included, is split bf16: the epilogue, not the
+    // tensor pipe, bounds this kernel and the bf16 split is the cheaper one.
+    constexpr int kFmt = kFmtBf16x3;
     extern __shared__ __align__(128) uint8_t smem[];
     uint8_t* prm = smem;
     uint8_t* o2 = smem + ConvParams::kBytes;
@@ -734,11 +597,11 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                     for (int tap = 0; tap < 3; ++tap) {
                         const int tt = t1 + tap - 1;
                         if (tt < 0 || tt >= kWindow) continue;
-                        conv_mma_ts_pred<32, kInt>(tmem + 0, tmem + kTmO1 + (tt & 3) * 32, prm_u + ConvParams::kW2 + tap * 4096, first, elected);
+                        conv_mma_ts_pred<32>(tmem + 0, tmem + kTmO1 + (tt & 3) * 32, prm_u + ConvParams::kW2 + tap * 4096, first, elected);
                         first = false;
                     }
                 }
-                if (t2 >= 0 && t2 < kWindow) conv_mma_f<32, kInt>(tmem + 32, o2_u, prm_u + ConvParams::kW3, true, elected);
+                if (t2 >= 0 && t2 < kWindow) conv_mma_pred<32>(tmem + 32, o2_u, prm_u + ConvParams::kW3, true, elected);
                 umma_commit_pred(bar_mma_x, elected);
             }
         }
@@ -755,7 +618,7 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                 if (t3 < kWindow) {
                     mbar_wait(&bar_y0_full[ny_slot], ny_par);
                     tc_fence_after_sync();
-                    conv_mma_ts_pred<64, kInt>(tmem + kTmScp1, tmem + kTmY0 + ny_slot * 32, prm_u + ConvParams::kW45, true, elected);
+                    conv_mma_ts_pred<64>(tmem + kTmScp1, tmem + kTmY0 + ny_slot * 32, prm_u + ConvParams::kW45, true, elected);
                     umma_commit_pred(&bar_y0_empty[ny_slot], elected);
                     ++ny;
                     if (++ny_slot == 3) { ny_slot = 0; ny_par ^= 1; }
@@ -766,11 +629,11 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                     for (int tap = 0; tap < 3; ++tap) {
                         const int tt = t4 + tap - 1;
                         if (tt < 0 || tt >= kWindow) continue;
-                        conv_mma_ts_pred<32, kInt>(tmem + 64, tmem + kTmP1 + (tt % 3) * 32, prm_u + ConvParams::kW6 + tap * 4096, first, elected);
+                        conv_mma_ts_pred<32>(tmem + 64, tmem + kTmP1 + (tt % 3) * 32, prm_u + ConvParams::kW6 + tap * 4096, first, elected);
                         first = false;
                     }
                 }
-                if (t5 >= 0 && t5 < kWindow) conv_mma_f<32, kInt>(tmem + 96, p2_u, prm_u + ConvParams::kW7, true, elected);
+                if (t5 >= 0 && t5 < kWindow) conv_mma_pred<32>(tmem + 96, p2_u, prm_u + ConvParams::kW7, true, elected);
                 umma_commit_pred(bar_mma_y, elected);
             }
         }
@@ -805,7 +668,7 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                     v[i] = fmaxf(o.x, 0.f);
                     v[i + 1] = fmaxf(o.y, 0.f);
                 }
-                store_a_tmem16_f<kInt>(t_opnd + kTmO1 + (t & 3) * 32, v);
+                store_a_tmem16_f<kFmt>(t_opnd + kTmO1 + (t & 3) * 32, v);
             };
             uint32_t it = 0, ny = 0, ny_slot = 0, ny_par = 1;      // empty-barrier parity of the previous use
             for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -842,7 +705,7 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                     if (h2) tmem_ld16_nowait(t_lane + 32, r2);
                     tmem_ld_wait();
                     float v[16];
-                    if (h1) { relu_bias(r1, 4, v); store_a_row16_f<kInt>(o2, row, c0, v); }              // b2
+                    if (h1) { relu_bias(r1, 4, v); store_a_row16_f<kFmt>(o2, row, c0, v); }              // b2
                     // o2 and o1[u+1] (made one iteration ago, in TMEM) are all the next X batch reads
                     if (u < kLastX) {
                         fence_proxy_async_smem();
@@ -863,7 +726,7 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                         }
                         if (ny >= 3) mbar_wait(&bar_y0_empty[ny_slot], ny_par);
                         tc_fence_after_sync();
-                        store_a_tmem16_f<kInt>(t_opnd + kTmY0 + ny_slot * 32, v);
+                        store_a_tmem16_f<kFmt>(t_opnd + kTmY0 + ny_slot * 32, v);
                         tmem_st_wait();
                         tc_fence_before_sync();
                         __syncwarp();
@@ -894,8 +757,8 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                     if (h5) tmem_ld16_nowait(t_lane + 96, r5);
                     tmem_ld_wait();
                     float v[16];
-                    if (h3) { relu_bias(r3, 7, v); store_a_tmem16_f<kInt>(t_opnd + kTmP1 + (t3 % 3) * 32, v); }   // b5
-                    if (h4) { relu_bias(r4, 8, v); store_a_row16_f<kInt>(p2, row, c0, v); }              // b6
+                    if (h3) { relu_bias(r3, 7, v); store_a_tmem16_f<kFmt>(t_opnd + kTmP1 + (t3 % 3) * 32, v); }   // b5
+                    if (h4) { relu_bias(r4, 8, v); store_a_row16_f<kFmt>(p2, row, c0, v); }              // b6
                     fence_proxy_async_smem();
                     tmem_st_wait();
                     tc_fence_before_sync();
@@ -922,7 +785,7 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                                 acc2 = ffma2(make_float2(v[i], v[i + 1]), __ldg(reinterpret_cast<const float2*>(head_w + c0 + i)), acc2);
                             head_part[(((size_t)tile * kWindow + t5) * 2 + ch) * 128 + row] = acc2.x + acc2.y;
                         } else {
-                            store_a_row16_f<FMT>(reinterpret_cast<uint8_t*>(y_out) + ((size_t)tile * kWindow + t5) * kSliceBytes, row, c0, v);
+                            store_a_row16_f<kFmt>(reinterpret_cast<uint8_t*>(y_out) + ((size_t)tile * kWindow + t5) * kSliceBytes, row, c0, v);
                         }
                     }
                 }
@@ -934,393 +797,15 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
     if (warp == 16) tmem_dealloc<512>(tmem);
 }
 
-// ====================================================================== TK3: input projection
-// xp[blk][d*192 + n][w] = sum_k y[blk][w][k] Wx_d[k][n] + b[d*192 + n]
-// CTA = (direction, block slot): weights of one direction resident in smem (2 planes x K x 192),
-// A blocks streamed through a ring of bulk copies, two 192-column TMEM accumulators.
-// Warp 0 = producer, warp 1 = MMA issuer (+ TMEM owner), warps 2..5 = epilogue.
-template <int K> struct XprojCfg {
-    static constexpr int kStages = K >= 128 ? 2 : 4;
-    static constexpr uint32_t kABytes = 2u * 128 * K * 2;           // hi + lo block
-    static constexpr uint32_t kWBytes = 2u * K * kNX * 2;           // hi + lo weights of one direction
-    static constexpr uint32_t kSmem = kWBytes + kStages * kABytes + 256;
-};
-
-template <int K>
-__global__ void __launch_bounds__(192, 1)
-tc_xproj_kernel(const __nv_bfloat16* __restrict__ a_blocks, const __nv_bfloat16* __restrict__ wx,
-                const float* __restrict__ bias, float* __restrict__ xp, int n_blocks) {
-    using Cfg = XprojCfg<K>;
-    extern __shared__ __align__(128) uint8_t smem[];
-    uint8_t* w_s = smem;
-    uint8_t* a_s = smem + Cfg::kWBytes;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::kWBytes + Cfg::kStages * Cfg::kABytes);
-    uint64_t* full = bars;                       // [kStages]
-    uint64_t* empty = bars + Cfg::kStages;       // [kStages]
-    uint64_t* acc_full = empty + Cfg::kStages;   // [2]
-    uint64_t* acc_empty = acc_full + 2;          // [2]
-    uint64_t* w_bar = acc_empty + 2;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(w_bar + 1);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int dir = blockIdx.x & 1;
-    const int slot = blockIdx.x >> 1, n_slots = gridDim.x >> 1;
-
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < Cfg::kStages; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 128); }
-        mbar_init(w_bar, 1);
-        fence_mbar_init();
-    }
-    if (warp == 1) tmem_alloc<512>(tmem_slot);
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    const uint32_t tmem = *tmem_slot;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            mbar_expect_tx(w_bar, Cfg::kWBytes);
-            bulk_g2s(w_s, wx + (size_t)dir * (Cfg::kWBytes / 2), Cfg::kWBytes, w_bar);
-            int it = 0;
-            for (int b = slot; b < n_blocks; b += n_slots, ++it) {
-                const int s = it % Cfg::kStages;
-                mbar_wait(&empty[s], ((it / Cfg::kStages) & 1) ^ 1);
-                mbar_expect_tx(&full[s], Cfg::kABytes);
-                bulk_g2s(a_s + (size_t)s * Cfg::kABytes, a_blocks + (size_t)b * (Cfg::kABytes / 2), Cfg::kABytes, &full[s]);
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            constexpr uint32_t idesc = make_idesc_bf16(128, kNX);
-            constexpr uint32_t a_plane = 128u * K * 2, w_plane = (uint32_t)K * kNX * 2;
-            mbar_wait(w_bar, 0);
-            int it = 0;
-            for (int b = slot; b < n_blocks; b += n_slots, ++it) {
-                const int s = it % Cfg::kStages, ab = it & 1;
-                mbar_wait(&full[s], (it / Cfg::kStages) & 1);
-                mbar_wait(&acc_empty[ab], ((it >> 1) & 1) ^ 1);
-                tc_fence_after_sync();
-                const uint32_t a0 = smem_u32(a_s + (size_t)s * Cfg::kABytes), w0 = smem_u32(w_s);
-                const uint32_t d = tmem + ab * 256;
-#pragma unroll
-                for (int pass = 0; pass < 3; ++pass) {
-                    const uint32_t ap = a0 + (pass == 1 ? a_plane : 0);        // hi, lo, hi
-                    const uint32_t wp = w0 + (pass == 2 ? w_plane : 0);        // hi, hi, lo
-#pragma unroll
-                    for (int kk = 0; kk < K / 16; ++kk) {
-                        const uint64_t ad = make_smem_desc(ap + kk * 2 * (128 * 16), 128 * 16, 128);
-                        const uint64_t bd = make_smem_desc(wp + kk * 2 * (kNX * 16), kNX * 16, 128);
-                        umma_bf16(d, ad, bd, idesc, (pass | kk) != 0);
-                    }
-                }
-                umma_commit(&empty[s]);
-                umma_commit(&acc_full[ab]);
-            }
-        }
-    } else {
-        const int q = warp & 3;                    // TMEM lane quadrant this warp may access
-        const int row = q * 32 + lane;
-        const float* bias_d = bias + dir * kNX;
-        int it = 0;
-        for (int b = slot; b < n_blocks; b += n_slots, ++it) {
-            const int ab = it & 1;
-            mbar_wait(&acc_full[ab], (it >> 1) & 1);
-            tc_fence_after_sync();
-            float* dst = xp + ((size_t)b * (2 * kNX) + dir * kNX) * 128 + row;
-            const uint32_t t0 = tmem + ((uint32_t)(q * 32) << 16) + ab * 256;
-#pragma unroll 1
-            for (int c0 = 0; c0 < kNX; c0 += 16) {
-                float v[16];
-                tmem_ld16(t0 + c0, v);
-#pragma unroll
-                for (int i = 0; i < 16; ++i) dst[(size_t)(c0 + i) * 128] = v[i] + __ldg(bias_d + c0 + i);
-            }
-            tc_fence_before_sync();
-            mbar_arrive(&acc_empty[ab]);
-        }
-    }
-    tc_fence_before_sync();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc<512>(tmem);
-}
-
-// in == 1 (RNN-only layer 0): xp = x * w + b on CUDA cores.  x fp32 [block][128].
-__global__ void tc_xproj_k1_kernel(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias,
-                                   float* __restrict__ xp, int64_t n_blocks) {
-    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= n_blocks * 2 * kNX * 128) return;
-    const int row = (int)(idx % 128);
-    const int col = (int)((idx / 128) % (2 * kNX));
-    const int64_t blk = idx / (128 * 2 * kNX);
-    xp[idx] = fmaf(x[blk * 128 + row], w[col], bias[col]);
-}
-
-// ====================================================================== TK4: GRU recurrence
-// CTA = one tile of 128 windows at a time, both directions as two independent chains.
-//   warps 0-3: epilogue of chain 0 (forward), warps 4-7: epilogue of chain 1 (backward);
-//              thread = one window (TMEM lane), owns its h[64] in registers
-//   warp 8 / 9: MMA issuer of chain 0 / 1 (warp 8 also owns TMEM, warp 9 loads the weights)
-// Per step and chain (TF GRUCell, reset before the candidate matmul):
-//   G-MMA  Dg[128x128] = h Wgh                      -> bar_g
-//   G-EPI  r = s(Dg_r + xp_r); A <- r*h (bf16 hi/lo) -> bar_rh ; u = s(Dg_u + xp_u) stashed in TMEM
-//   C-MMA  Dc[128x64]  = (r*h) Wch                  -> bar_c
-//   C-EPI  c = tanh(Dc + xp_c); h = u h + (1-u) c; A <- h; y/head out -> bar_h
-constexpr uint32_t kGruWBytesDir = 2u * (kH * 2 * kH * 2) + 2u * (kH * kH * 2);   // 49152
-constexpr uint32_t kGruABytes = 2u * 128 * kH * 2;                                // 32768 (hi + lo)
-constexpr uint32_t kGruSmem = 2 * kGruWBytesDir + 2 * kGruABytes + 256;
-
-__global__ void __launch_bounds__(320, 1)
-tc_gru_kernel(const __nv_bfloat16* __restrict__ wh, const float* __restrict__ xp,
-              __nv_bfloat16* __restrict__ y_out, const float* __restrict__ head_w,
-              float* __restrict__ head_part, int n_tiles) {
-    extern __shared__ __align__(128) uint8_t smem[];
-    uint8_t* w_s = smem;                                   // [dir]{Wg hi, Wg lo, Wc hi, Wc lo}
-    uint8_t* a_s = smem + 2 * kGruWBytesDir;               // [chain]{hi, lo} each [8][128][8]
-    uint64_t* bars = reinterpret_cast<uint64_t*>(a_s + 2 * kGruABytes);
-    // per chain: bar_g, bar_c (MMA -> epilogue), bar_rh, bar_h (epilogue -> MMA)
-    uint64_t* w_bar = bars + 8;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 9);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-        for (int c = 0; c < 2; ++c) {
-            mbar_init(&bars[4 * c + 0], 1);
-            mbar_init(&bars[4 * c + 1], 1);
-            mbar_init(&bars[4 * c + 2], 128);
-            mbar_init(&bars[4 * c + 3], 128);
-        }
-        mbar_init(w_bar, 1);
-        fence_mbar_init();
-    }
-    if (warp == 8) tmem_alloc<512>(tmem_slot);
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    const uint32_t tmem = *tmem_slot;
-
-    if (warp >= 8) {
-        // ------------------------------------------------------------ MMA issuers
-        const int chain = warp - 8;
-        if (warp == 9 && lane == 0) {
-            mbar_expect_tx(w_bar, 2 * kGruWBytesDir);
-            bulk_g2s(w_s, wh, kGruWBytesDir, w_bar);
-            bulk_g2s(w_s + kGruWBytesDir, wh + kGruWBytesDir / 2, kGruWBytesDir, w_bar);
-        }
-        if (lane == 0) {
-            uint64_t* bar_g = &bars[4 * chain + 0];
-            uint64_t* bar_c = &bars[4 * chain + 1];
-            uint64_t* bar_rh = &bars[4 * chain + 2];
-            uint64_t* bar_h = &bars[4 * chain + 3];
-            constexpr uint32_t idesc_g = make_idesc_bf16(128, 2 * kH);
-            constexpr uint32_t idesc_c = make_idesc_bf16(128, kH);
-            const uint32_t a0 = smem_u32(a_s + (size_t)chain * kGruABytes);
-            const uint32_t wg0 = smem_u32(w_s + (size_t)chain * kGruWBytesDir);
-            const uint32_t wc0 = wg0 + 2 * (kH * 2 * kH * 2);
-            const uint32_t dg = tmem + chain * 256, dc = dg + 2 * kH;
-            mbar_wait(w_bar, 0);
-            uint32_t g = 0;
-            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-                for (int s = 0; s < kWindow; ++s, ++g) {
-                    mbar_wait(bar_h, g & 1);
-                    tc_fence_after_sync();
-#pragma unroll
-                    for (int pass = 0; pass < 3; ++pass) {
-                        const uint32_t ap = a0 + (pass == 1 ? 128 * kH * 2 : 0);
-                        const uint32_t wp = wg0 + (pass == 2 ? kH * 2 * kH * 2 : 0);
-#pragma unroll
-                        for (int kk = 0; kk < kH / 16; ++kk)
-                            umma_bf16(dg, make_smem_desc(ap + kk * 2 * (128 * 16), 128 * 16, 128),
-                                      make_smem_desc(wp + kk * 2 * (2 * kH * 16), 2 * kH * 16, 128), idesc_g,
-                                      (pass | kk) != 0);
-                    }
-                    umma_commit(bar_g);
-                    mbar_wait(bar_rh, g & 1);
-                    tc_fence_after_sync();
-#pragma unroll
-                    for (int pass = 0; pass < 3; ++pass) {
-                        const uint32_t ap = a0 + (pass == 1 ? 128 * kH * 2 : 0);
-                        const uint32_t wp = wc0 + (pass == 2 ? kH * kH * 2 : 0);
-#pragma unroll
-                        for (int kk = 0; kk < kH / 16; ++kk)
-                            umma_bf16(dc, make_smem_desc(ap + kk * 2 * (128 * 16), 128 * 16, 128),
-                                      make_smem_desc(wp + kk * 2 * (kH * 16), kH * 16, 128), idesc_c,
-                                      (pass | kk) != 0);
-                    }
-                    umma_commit(bar_c);
-                }
-            }
-        }
-    } else {
-        // ------------------------------------------------------------ epilogue: one window per thread
-        // State h lives in TMEM (fp32, columns 192..255 of the chain's half) next to the
-        // accumulators; registers hold a rolling prefetch P[64] of the xp addends so that every
-        // global load is issued one phase (>= 1000 cycles) before its use:
-        //   while r is computed from P = xp_r, P is refilled with xp_u; during u with xp_c;
-        //   during c with the next step's xp_r.
-        const int chain = warp >> 2;                     // 0 forward, 1 backward
-        const int q = warp & 3;
-        const int row = q * 32 + lane;
-        uint64_t* bar_g = &bars[4 * chain + 0];
-        uint64_t* bar_c = &bars[4 * chain + 1];
-        uint64_t* bar_rh = &bars[4 * chain + 2];
-        uint64_t* bar_h = &bars[4 * chain + 3];
-        uint8_t* a_hi = a_s + (size_t)chain * kGruABytes + row * 16;      // + (k/8) * 2048
-        uint8_t* a_lo = a_hi + 128 * kH * 2;
-        const uint32_t t_lane = tmem + ((uint32_t)(q * 32) << 16) + chain * 256;
-        const uint32_t t_r = t_lane, t_u = t_lane + kH, t_c = t_lane + 2 * kH, t_h = t_lane + 3 * kH;
-        const float* xp_row = xp + (size_t)chain * kNX * 128 + row;       // + blk * 384 * 128 + col * 128
-        auto blk_of = [&](int tile, int s) -> size_t { return (size_t)tile * kWindow + (chain ? kWindow - 1 - s : s); };
-        float P[kH];
-        uint32_t g = 0;
-        for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            {
-                float z[16];
-#pragma unroll
-                for (int i = 0; i < 16; ++i) z[i] = 0.f;
-#pragma unroll
-                for (int c0 = 0; c0 < kH; c0 += 16) tmem_st16(t_h + c0, z);
-#pragma unroll
-                for (int kg = 0; kg < kH / 8; ++kg) {
-                    *reinterpret_cast<uint4*>(a_hi + kg * 2048) = make_uint4(0, 0, 0, 0);
-                    *reinterpret_cast<uint4*>(a_lo + kg * 2048) = make_uint4(0, 0, 0, 0);
-                }
-                if (tile == (int)blockIdx.x) {           // later tiles were prefetched by the previous tile's last step
-                    const float* x0 = xp_row + blk_of(tile, 0) * (2 * kNX) * 128;
-#pragma unroll
-                    for (int j = 0; j < kH; ++j) P[j] = __ldg(x0 + (size_t)j * 128);
-                }
-                tmem_st_wait();
-                fence_proxy_async_smem();
-                tc_fence_before_sync();
-                mbar_arrive(bar_h);
-            }
-            for (int s = 0; s < kWindow; ++s, ++g) {
-                const size_t blk = blk_of(tile, s);
-                const float* xb = xp_row + blk * (2 * kNX) * 128;
-                // where the next reset-gate addends come from (next step, or the next tile's first step)
-                const float* xnext = nullptr;
-                if (s + 1 < kWindow) xnext = xp_row + blk_of(tile, s + 1) * (2 * kNX) * 128;
-                else if (tile + (int)gridDim.x < n_tiles) xnext = xp_row + blk_of(tile + gridDim.x, 0) * (2 * kNX) * 128;
-                // ---- G-EPI, reset gate first: the candidate MMA waits for r*h
-                mbar_wait(bar_g, g & 1);
-                tc_fence_after_sync();
-#pragma unroll
-                for (int c0 = 0; c0 < kH; c0 += 16) {
-                    uint32_t ar[16], hr[16];
-                    tmem_ld16_nowait(t_r + c0, ar);
-                    tmem_ld16_nowait(t_h + c0, hr);
-                    tmem_ld_wait();
-                    uint32_t hi[8], lo[8];
-#pragma unroll
-                    for (int i = 0; i < 16; i += 4) {
-                        float pre[4], r[4];
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) {
-                            pre[k] = __uint_as_float(ar[i + k]) + P[c0 + i + k];
-                            P[c0 + i + k] = __ldg(xb + (size_t)(kH + c0 + i + k) * 128);     // refill with xp_u
-                        }
-                        sigmoid4(pre, r);
-                        split_bf16x2(r[0] * __uint_as_float(hr[i]), r[1] * __uint_as_float(hr[i + 1]), hi[i >> 1], lo[i >> 1]);
-                        split_bf16x2(r[2] * __uint_as_float(hr[i + 2]), r[3] * __uint_as_float(hr[i + 3]), hi[(i >> 1) + 1], lo[(i >> 1) + 1]);
-                    }
-                    *reinterpret_cast<uint4*>(a_hi + (c0 / 8) * 2048) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                    *reinterpret_cast<uint4*>(a_hi + (c0 / 8 + 1) * 2048) = make_uint4(hi[4], hi[5], hi[6], hi[7]);
-                    *reinterpret_cast<uint4*>(a_lo + (c0 / 8) * 2048) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-                    *reinterpret_cast<uint4*>(a_lo + (c0 / 8 + 1) * 2048) = make_uint4(lo[4], lo[5], lo[6], lo[7]);
-                }
-                fence_proxy_async_smem();
-                tc_fence_before_sync();
-                mbar_arrive(bar_rh);
-                // ---- update gate while the candidate MMA runs; u replaces its own accumulator columns
-#pragma unroll
-                for (int c0 = 0; c0 < kH; c0 += 16) {
-                    float a[16];
-                    tmem_ld16(t_u + c0, a);
-#pragma unroll
-                    for (int i = 0; i < 16; i += 4) {
-                        float pre[4];
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) {
-                            pre[k] = a[i + k] + P[c0 + i + k];
-                            P[c0 + i + k] = __ldg(xb + (size_t)(2 * kH + c0 + i + k) * 128);  // refill with xp_c
-                        }
-                        sigmoid4(pre, a + i);
-                    }
-                    tmem_st16(t_u + c0, a);
-                }
-                tmem_st_wait();
-                // ---- C-EPI
-                mbar_wait(bar_c, g & 1);
-                tc_fence_after_sync();
-                float head_acc = 0.f;
-#pragma unroll
-                for (int c0 = 0; c0 < kH; c0 += 16) {
-                    uint32_t cr[16], ur[16], hr[16];
-                    tmem_ld16_nowait(t_c + c0, cr);
-                    tmem_ld16_nowait(t_u + c0, ur);
-                    tmem_ld16_nowait(t_h + c0, hr);
-                    tmem_ld_wait();
-                    uint32_t hi[8], lo[8];
-                    float hn[16];
-#pragma unroll
-                    for (int i = 0; i < 16; i += 4) {
-                        float pre[4], cv[4];
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) {
-                            pre[k] = __uint_as_float(cr[i + k]) + P[c0 + i + k];
-                            if (xnext) P[c0 + i + k] = __ldg(xnext + (size_t)(c0 + i + k) * 128);  // refill with next xp_r
-                        }
-                        tanh4(pre, cv);
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) {
-                            const float u = __uint_as_float(ur[i + k]);
-                            hn[i + k] = u * __uint_as_float(hr[i + k]) + (1.f - u) * cv[k];
-                        }
-                    }
-                    tmem_st16(t_h + c0, hn);
-#pragma unroll
-                    for (int i = 0; i < 16; i += 2) split_bf16x2(hn[i], hn[i + 1], hi[i >> 1], lo[i >> 1]);
-                    *reinterpret_cast<uint4*>(a_hi + (c0 / 8) * 2048) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                    *reinterpret_cast<uint4*>(a_hi + (c0 / 8 + 1) * 2048) = make_uint4(hi[4], hi[5], hi[6], hi[7]);
-                    *reinterpret_cast<uint4*>(a_lo + (c0 / 8) * 2048) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-                    *reinterpret_cast<uint4*>(a_lo + (c0 / 8 + 1) * 2048) = make_uint4(lo[4], lo[5], lo[6], lo[7]);
-                    if (y_out) {
-                        // next layer's A operand: block [plane][128/8][128][8], features chain*64 + j
-                        __nv_bfloat16* yb = y_out + blk * (2 * 128 * 2 * kH) + ((size_t)(chain * kH + c0) / 8 * 128 + row) * 8;
-                        *reinterpret_cast<uint4*>(yb) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                        *reinterpret_cast<uint4*>(yb + 128 * 8) = make_uint4(hi[4], hi[5], hi[6], hi[7]);
-                        *reinterpret_cast<uint4*>(yb + 128 * 2 * kH) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-                        *reinterpret_cast<uint4*>(yb + 128 * 2 * kH + 128 * 8) = make_uint4(lo[4], lo[5], lo[6], lo[7]);
-                    }
-                    if (head_part) {
-                        // dense 128 -> 1: this direction's half of the dot product (rnn_class.py:179)
-#pragma unroll
-                        for (int i = 0; i < 16; ++i) head_acc = fmaf(hn[i], __ldg(head_w + chain * kH + c0 + i), head_acc);
-                    }
-                }
-                if (head_part) head_part[(blk * 2 + chain) * 128 + row] = head_acc;
-                tmem_st_wait();
-                if (s + 1 < kWindow) {
-                    fence_proxy_async_smem();
-                    tc_fence_before_sync();
-                    mbar_arrive(bar_h);
-                }
-            }
-            tc_fence_before_sync();      // this tile's TMEM accesses precede the next tile's first MMA
-        }
-    }
-    tc_fence_before_sync();
-    __syncthreads();
-    if (warp == 8) tmem_dealloc<512>(tmem);
-}
-
 // ====================================================================== TK4G: fused GRU layer, two tiles per CTA
-// Same mathematics as TK4F, restructured so that the tensor pipe never idles behind one chain's
-// serial MMA -> epilogue -> MMA dependency: a CTA runs TWO independent chains (two tiles of the
-// same direction, sharing the resident weights).  To make room for the second chain the state
-// operand h / r*h no longer lives in shared memory: the epilogue writes it (packed, in the operand
-// format FMT) into tensor memory with tcgen05.st and the state-part MMAs read A from TMEM (".ts" form).
+// One GRU layer, input projection and recurrence in one kernel (TF GRUCell, reset gate applied before the
+// candidate matmul; rnn_class.py:142-175).  Per step and chain: the x part x W_x (N = 192: r | u | c) and the
+// state part h W_gh accumulate the gates, (r*h) W_ch adds to the candidate columns; the epilogue applies the
+// activations and h = u h + (1 - u) c.  So that the tensor pipe never idles behind one chain's serial
+// MMA -> epilogue -> MMA dependency, a CTA runs TWO independent chains (two tiles of the same direction,
+// sharing the resident weights).  To make room for the second chain the state operand h / r*h lives in
+// tensor memory: the epilogue writes it (packed, in the operand format FMT) with tcgen05.st and the
+// state-part MMAs read A from TMEM (".ts" form).
 // TMEM per chain (256 columns): gates accumulator 0..127, candidate 128..191, A plane 0 192..223,
 // A plane 1 224..255.  Shared memory: weights (147 KB) + ONE x ring (8 stages of 8 KB for a 128-wide input = one
 // entry per turn, 10 stages for a 32-wide one) that both chains
@@ -1363,9 +848,6 @@ __host__ __device__ constexpr uint32_t gru_out_block_bytes(int fmt) { return fmt
 constexpr int kGruF2Threads = 768;
 constexpr int kGruF2Converters = 2;               // warps 19.. rebuilding hi-byte slabs; must divide the ring's stages
 constexpr int kGruF2EpiRegs = 96, kGruF2ServiceRegs = 48;
-#ifndef CF_L2_PREFETCH
-#define CF_L2_PREFETCH 1
-#endif
 
 template <int KX, int FMT, int FMT_OUT>
 __global__ void __launch_bounds__(kGruF2Threads, 1)
@@ -1470,7 +952,7 @@ tc_gru_fused2_kernel(const uint8_t* __restrict__ wpk, const float* __restrict__ 
                 for (int c = 0; c < 2; ++c) {
                     if (c == 1 && gs >= total1) break;
                     const uint8_t* xb = xbase + blk_of(c, gs) * blk_bytes;
-                    if (kCompact && !(kExp & 1) && CF_L2_PREFETCH) {
+                    if (kCompact) {
                         // The ring holds about one entry, so an entry's chunks are requested only while the entry
                         // before it is being consumed, and when two x parts run back to back the second one waited
                         // an HBM latency (~1 500 cycles) per chunk.  Ask L2 for the NEXT entry one entry ahead.
@@ -1486,7 +968,6 @@ tc_gru_fused2_kernel(const uint8_t* __restrict__ wpk, const float* __restrict__ 
                         CF_TRC(5, gs, 80 + kk);
                         uint8_t* dst = smem + Cfg::kRing + st * 8192;
                         uint64_t* landed = &bars[(kCompact ? Cfg::kBarTma : Cfg::kBarFull) + st];
-                        if (kExp & 1) { mbar_arrive(landed); if (++st == Cfg::kStages) { st = 0; par ^= 1; } continue; }
                         if (kCompact) {
                             mbar_expect_tx(landed, 6144);
                             bulk_g2s(dst, xb + kk * 4096, 4096, landed);
@@ -1585,7 +1066,6 @@ tc_gru_fused2_kernel(const uint8_t* __restrict__ wpk, const float* __restrict__ 
                         const uint32_t a_lo = ring_lo + st * (8192 >> 4), w_lo = wx_lo + kk * (2 * kNX * 16 >> 4);
                         if (kE5) {
                             umma_bf16_pred(dg, ahi | a_lo, bhi | w_lo, idesc_x, kk != 0, elected);
-                            if (!(kExp & 2))
                             umma_f8_pred(dg, ahi | (a_lo + (4096 >> 4)), bhi | (w_lo + (KX * kNX * 2 >> 4)), idesc_x8, 1, elected);
                         } else {
 #pragma unroll
@@ -1627,7 +1107,6 @@ tc_gru_fused2_kernel(const uint8_t* __restrict__ wpk, const float* __restrict__ 
                     for (int kk = 0; kk < kH / 16; ++kk) {
                         const uint32_t w_lo = wgh_lo + kk * (2 * 128 * 16 >> 4);
                         umma_bf16_ts_pred(dg, ta + kk * 8, ghi | w_lo, idesc_g, !kNoX || kk != 0, elected);
-                        if (!(kExp & 2))
                         umma_f8_ts_pred(dg, ta + 32 + kk * 8, ghi | (w_lo + (kH * 128 * 2 >> 4)), idesc_g8, 1, elected);
                     }
                 } else {
@@ -1651,7 +1130,6 @@ tc_gru_fused2_kernel(const uint8_t* __restrict__ wpk, const float* __restrict__ 
                     for (int kk = 0; kk < kH / 16; ++kk) {
                         const uint32_t w_lo = wch_lo + kk * (2 * 64 * 16 >> 4);
                         umma_bf16_ts_pred(dc, ta + kk * 8, chi | w_lo, idesc_c, !kNoX || kk != 0, elected);
-                        if (!(kExp & 2))
                         umma_f8_ts_pred(dc, ta + 32 + kk * 8, chi | (w_lo + (kH * 64 * 2 >> 4)), idesc_c8, 1, elected);
                     }
                 } else {
@@ -1827,7 +1305,7 @@ tc_gru_fused2_kernel(const uint8_t* __restrict__ wpk, const float* __restrict__ 
                 if (lane == 0) mbar_arrive(&b[Cfg::kBarH]);
             }
             if (warp == 0 && lane == 0) CF_TR(2 + c, gs, 55);
-            if (y_out && !(kExp & 4)) {
+            if (y_out) {
                 // next layer's A operand, in the NEXT layer's operand format (a second split when it differs)
                 if (FMT_OUT != FMT) {
 #pragma unroll
@@ -1986,19 +1464,10 @@ int simt_conv_stack(SimtEngine* e, const HostModel& hm, const int16_t* raw, cons
                     WindowTable tab, int64_t tile0, int64_t tiles, int64_t chunk_tiles, const float** feat,
                     cudaStream_t stream, Profiler* prof);
 
-// The projection buffer (192 KB per block) is only needed by the unfused projection + recurrence pair.
-static bool tc_needs_xp(const TcEngine* e) {
-    if (!e->use_fused) return true;
-    for (const TcLayer& L : e->layers)
-        if (!L.wfused) return true;
-    return false;
-}
-
-static size_t tc_workspace_bytes(const TcEngine* e, int64_t tiles) {
+static size_t tc_workspace_bytes(int64_t tiles) {
     const size_t blocks = (size_t)tiles * kWindow;
     size_t b = 0;
     b += blocks * 128 * kC * 2 * 2;          // conv output as A operand (K = 32)
-    if (tc_needs_xp(e)) b += blocks * 2 * kNX * 128 * 4;   // xp
     b += 2 * blocks * 128 * 2 * kH * 2 * 2;  // y ping-pong (K = 128 operands)
     b += blocks * 8 * 128 * 4;               // head partials
     return b + 4096;
@@ -2010,28 +1479,22 @@ int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const doubl
     if (n_tiles <= 0) return CF_OK;
     if (bits && (e->layers.empty() || want_logits)) { set_error("label-bit output needs a GRU head"); return CF_ERR_BAD_ARG; }
     if (!e->attr_done) {
-        CF_CUDA(cudaFuncSetAttribute(tc_xproj_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, XprojCfg<32>::kSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_xproj_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, XprojCfg<128>::kSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_gru_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kGruSmem));
         CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<1, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<1>::kSmem));
         CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<1, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<1>::kSmem));
         CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<32, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<32>::kSmem));
         CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<32, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<32>::kSmem));
         CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<128, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<128>::kSmem));
         CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<128, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<128>::kSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_conv2_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_conv2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_conv4_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConv4Smem));
+        CF_CUDA(cudaFuncSetAttribute(tc_conv2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmem));
+        CF_CUDA(cudaFuncSetAttribute(tc_conv4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kConv4Smem));
         e->attr_done = true;
     }
     const int64_t chunk = n_tiles < kTcChunkTiles ? n_tiles : kTcChunkTiles;
-    CF_TRY(e->ws.ensure(tc_workspace_bytes(e, chunk)));
+    CF_TRY(e->ws.ensure(tc_workspace_bytes(chunk)));
     const size_t blocks_max = (size_t)chunk * kWindow;
     uint8_t* p = static_cast<uint8_t*>(e->ws.ptr);
     __nv_bfloat16* a0 = reinterpret_cast<__nv_bfloat16*>(p);
     p += blocks_max * 128 * kC * 2 * 2;
-    float* xp = reinterpret_cast<float*>(p);
-    if (tc_needs_xp(e)) p += blocks_max * 2 * kNX * 128 * 4;
     __nv_bfloat16* ybuf[2];
     ybuf[0] = reinterpret_cast<__nv_bfloat16*>(p);
     p += blocks_max * 128 * 2 * kH * 2 * 2;
@@ -2050,115 +1513,83 @@ int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const doubl
             ProfScope ps(prof, KC_K2_CONV, stream);
             const int grid = (int)std::min<int64_t>(tiles, e->n_sms);
             if (e->conv_nres == 2)
-                tc_conv4_kernel<0><<<grid, 576, kConv4Smem, stream>>>(e->conv_params, raw, stats, xwin, tab.src, tab.valid,
-                                                                     tab.read, tile0, (int)tiles, a0,
-                                                                     n_layers == 0 ? e->head_w : nullptr, n_layers == 0 ? head_part : nullptr);
+                tc_conv4_kernel<<<grid, 576, kConv4Smem, stream>>>(e->conv_params, raw, stats, xwin, tab.src, tab.valid,
+                                                                  tab.read, tile0, (int)tiles, a0,
+                                                                  n_layers == 0 ? e->head_w : nullptr, n_layers == 0 ? head_part : nullptr);
             else
-                tc_conv2_kernel<1><<<grid, 288, kConvSmem, stream>>>(e->conv_params, raw, stats, xwin, tab.src, tab.valid,
-                                                                     tab.read, tile0, (int)tiles, a0);
+                tc_conv2_kernel<<<grid, 288, kConvSmem, stream>>>(e->conv_params, raw, stats, xwin, tab.src, tab.valid,
+                                                                  tab.read, tile0, (int)tiles, a0);
             CF_LAUNCHED();
             a_in = a0;
         } else {
             CF_TRY(simt_conv_stack(e->simt, hm, raw, stats, xwin, tab, tile0, tiles, chunk, &feat, stream, prof));
         }
-        int head_parts = 2;
         for (int l = 0; l < n_layers; ++l) {
             const TcLayer& L = e->layers[l];
             const bool last = l + 1 == n_layers;
             __nv_bfloat16* yo = last ? nullptr : ybuf[l & 1];
-            if (L.wfused && e->use_fused) {
-                // input projection + recurrence in one kernel; a_in is the A-operand form of the layer input
-                if (l == 0 && !a_in && L.in == kC) {
-                    ProfScope ps(prof, KC_K3_XPROJ, stream);
-                    const int64_t total = rows * (kC / 8);
-                    tc_pack_a_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, stream>>>(feat, kC, rows, a0);
-                    CF_LAUNCHED();
-                    a_in = a0;
-                }
-                ProfScope ps(prof, KC_K4_GRU, stream);
-                long long* trace_dev = nullptr;
-                if (e->trace_path && !e->trace_done && L.in != kC) {
-                    CF_CUDA(cudaMalloc(&trace_dev, 6 * 200 * 2 * sizeof(long long)));
-                    CF_CUDA(cudaMemsetAsync(trace_dev, 0, 6 * 200 * 2 * sizeof(long long), stream));
-                }
-                const int grid2 = 2 * (int)std::min<int64_t>((tiles + 1) / 2, e->n_sms / 2);
-                const float* hw_l = last ? e->head_w : nullptr;
-                float* hp_l = last ? head_part : nullptr;
-                // operand format of this layer and of the layer that reads its output
-                const int fmt_out = last ? L.fmt : e->layers[l + 1].fmt;
-                if (L.in == 1) {
-                    // scalar input (RNN-only layer 0): x part in the epilogue from the fp32 signal rows
-                    if (L.fmt == kFmtF16E5)
-                        tc_gru_fused2_kernel<1, 1, 1><<<grid2, kGruF2Threads, GruF2Cfg<1>::kSmem, stream>>>(
-                            L.wfused, L.bz, nullptr, yo, hw_l, hp_l, (int)tiles, nullptr, feat, L.wxz);
-                    else
-                        tc_gru_fused2_kernel<1, 0, 0><<<grid2, kGruF2Threads, GruF2Cfg<1>::kSmem, stream>>>(
-                            L.wfused, L.bz, nullptr, yo, hw_l, hp_l, (int)tiles, nullptr, feat, L.wxz);
-                } else if (L.in == kC) {
-                    if (fmt_out == kFmtF16E5)
-                        tc_gru_fused2_kernel<32, 0, 1><<<grid2, kGruF2Threads, GruF2Cfg<32>::kSmem, stream>>>(
-                            L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, nullptr, nullptr, nullptr);
-                    else
-                        tc_gru_fused2_kernel<32, 0, 0><<<grid2, kGruF2Threads, GruF2Cfg<32>::kSmem, stream>>>(
-                            L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, nullptr, nullptr, nullptr);
-                } else if (L.fmt == kFmtF16E5) {
-                    tc_gru_fused2_kernel<128, 1, 1><<<grid2, kGruF2Threads, GruF2Cfg<128>::kSmem, stream>>>(
-                        L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, trace_dev, nullptr, nullptr);
-                } else {
-                    tc_gru_fused2_kernel<128, 0, 0><<<grid2, kGruF2Threads, GruF2Cfg<128>::kSmem, stream>>>(
-                        L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, trace_dev, nullptr, nullptr);
-                }
-                CF_LAUNCHED();
-                if (trace_dev) {
-                    // debug (CF_TC_TRACE=<file>): dump the timeline of block 0 once; results are unaffected
-                    CF_CUDA(cudaStreamSynchronize(stream));
-                    std::vector<long long> host(6 * 200 * 2);
-                    CF_CUDA(cudaMemcpy(host.data(), trace_dev, host.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-                    if (FILE* f = fopen(e->trace_path, "w")) {
-                        for (int rg = 0; rg < 6; ++rg)
-                            for (int k = 0; k < 200; ++k)
-                                if (host[(rg * 200 + k) * 2 + 1])
-                                    fprintf(f, "%d %lld %lld\n", rg, host[(rg * 200 + k) * 2], host[(rg * 200 + k) * 2 + 1]);
-                        fclose(f);
-                    }
-                    cudaFree(trace_dev);
-                    e->trace_done = true;
-                }
-                a_in = yo;
-                head_parts = 8;
-                continue;
-            }
-            head_parts = 2;
-            {
+            // input projection + recurrence in one kernel; a_in is the A-operand form of the layer input
+            if (l == 0 && !a_in && L.in == kC) {
                 ProfScope ps(prof, KC_K3_XPROJ, stream);
-                if (L.in == 1) {
-                    const int64_t total = blocks * 2 * kNX * 128;
-                    tc_xproj_k1_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, stream>>>(feat, L.wx_f32, L.bx, xp, blocks);
-                    CF_LAUNCHED();
-                } else {
-                    if (l == 0 && !a_in) {
-                        const int64_t total = rows * (kC / 8);
-                        tc_pack_a_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, stream>>>(feat, kC, rows, a0);
-                        CF_LAUNCHED();
-                        a_in = a0;
-                    }
-                    int grid = 2 * (int)std::min<int64_t>(blocks, e->n_sms / 2);
-                    if (L.in == kC) {
-                        tc_xproj_kernel<32><<<grid, 192, XprojCfg<32>::kSmem, stream>>>(a_in, L.wx, L.bx, xp, (int)blocks);
-                    } else {
-                        tc_xproj_kernel<128><<<grid, 192, XprojCfg<128>::kSmem, stream>>>(a_in, L.wx, L.bx, xp, (int)blocks);
-                    }
-                    CF_LAUNCHED();
-                }
-            }
-            {
-                ProfScope ps(prof, KC_K4_GRU, stream);
-                const int grid = (int)std::min<int64_t>(tiles, e->n_sms);
-                tc_gru_kernel<<<grid, 320, kGruSmem, stream>>>(L.wh, xp, yo, last ? e->head_w : nullptr,
-                                                               last ? head_part : nullptr, (int)tiles);
+                const int64_t total = rows * (kC / 8);
+                tc_pack_a_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, stream>>>(feat, kC, rows, a0);
                 CF_LAUNCHED();
-                a_in = yo;
+                a_in = a0;
             }
+            ProfScope ps(prof, KC_K4_GRU, stream);
+            long long* trace_dev = nullptr;
+#ifdef CF_TRACE_PROBES
+            if (e->trace_path && !e->trace_done && L.in != kC) {
+                CF_CUDA(cudaMalloc(&trace_dev, 6 * 200 * 2 * sizeof(long long)));
+                CF_CUDA(cudaMemsetAsync(trace_dev, 0, 6 * 200 * 2 * sizeof(long long), stream));
+            }
+#endif
+            const int grid2 = 2 * (int)std::min<int64_t>((tiles + 1) / 2, e->n_sms / 2);
+            const float* hw_l = last ? e->head_w : nullptr;
+            float* hp_l = last ? head_part : nullptr;
+            // operand format of this layer and of the layer that reads its output
+            const int fmt_out = last ? L.fmt : e->layers[l + 1].fmt;
+            if (L.in == 1) {
+                // scalar input (RNN-only layer 0): x part in the epilogue from the fp32 signal rows
+                if (L.fmt == kFmtF16E5)
+                    tc_gru_fused2_kernel<1, 1, 1><<<grid2, kGruF2Threads, GruF2Cfg<1>::kSmem, stream>>>(
+                        L.wfused, L.bz, nullptr, yo, hw_l, hp_l, (int)tiles, nullptr, feat, L.wxz);
+                else
+                    tc_gru_fused2_kernel<1, 0, 0><<<grid2, kGruF2Threads, GruF2Cfg<1>::kSmem, stream>>>(
+                        L.wfused, L.bz, nullptr, yo, hw_l, hp_l, (int)tiles, nullptr, feat, L.wxz);
+            } else if (L.in == kC) {
+                if (fmt_out == kFmtF16E5)
+                    tc_gru_fused2_kernel<32, 0, 1><<<grid2, kGruF2Threads, GruF2Cfg<32>::kSmem, stream>>>(
+                        L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, nullptr, nullptr, nullptr);
+                else
+                    tc_gru_fused2_kernel<32, 0, 0><<<grid2, kGruF2Threads, GruF2Cfg<32>::kSmem, stream>>>(
+                        L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, nullptr, nullptr, nullptr);
+            } else if (L.fmt == kFmtF16E5) {
+                tc_gru_fused2_kernel<128, 1, 1><<<grid2, kGruF2Threads, GruF2Cfg<128>::kSmem, stream>>>(
+                    L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, trace_dev, nullptr, nullptr);
+            } else {
+                tc_gru_fused2_kernel<128, 0, 0><<<grid2, kGruF2Threads, GruF2Cfg<128>::kSmem, stream>>>(
+                    L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, trace_dev, nullptr, nullptr);
+            }
+            CF_LAUNCHED();
+#ifdef CF_TRACE_PROBES
+            if (trace_dev) {
+                // debug (CF_TC_TRACE=<file>): dump the timeline of block 0 once; results are unaffected
+                CF_CUDA(cudaStreamSynchronize(stream));
+                std::vector<long long> host(6 * 200 * 2);
+                CF_CUDA(cudaMemcpy(host.data(), trace_dev, host.size() * sizeof(long long), cudaMemcpyDeviceToHost));
+                if (FILE* f = fopen(e->trace_path, "w")) {
+                    for (int rg = 0; rg < 6; ++rg)
+                        for (int k = 0; k < 200; ++k)
+                            if (host[(rg * 200 + k) * 2 + 1])
+                                fprintf(f, "%d %lld %lld\n", rg, host[(rg * 200 + k) * 2], host[(rg * 200 + k) * 2 + 1]);
+                    fclose(f);
+                }
+                cudaFree(trace_dev);
+                e->trace_done = true;
+            }
+#endif
+            a_in = yo;
         }
         if (n_layers == 0 && e->conv_nres == 2) {
             // ResNet-only, two residual blocks: the conv kernel's epilogue already took the dense layer (two partial dots)
@@ -2174,49 +1605,14 @@ int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const doubl
                 a_in, e->head_w, e->head_b, tab.src, tab.valid, tab.read, raw ? stats : nullptr, tile0, rows, probs, want_logits ? 1 : 0);
             CF_LAUNCHED();
         } else {
+            // GRU head: the last layer's epilogue wrote eight partial dots per position (2 directions x 4 unit groups)
             ProfScope ps(prof, KC_K5_HEAD, stream);
             tc_head_kernel<<<(unsigned)tiles, 256, 0, stream>>>(
-                head_part, head_parts, e->head_b, tab.src, tab.valid, tab.read, raw ? stats : nullptr, tile0, rows, probs, want_logits ? 1 : 0,
+                head_part, 8, e->head_b, tab.src, tab.valid, tab.read, raw ? stats : nullptr, tile0, rows, probs, want_logits ? 1 : 0,
                 bits ? bits->lwords : nullptr, bits ? bits->threshold : 0.0);
             CF_LAUNCHED();
         }
     }
-    return CF_OK;
-}
-
-// ====================================================================== self-test of TK3
-// out[blk][n][w] = sum_k a[blk*128 + w][k] wx[k][n] + bias[n] for n in [0, 384), through the same
-// pack / bulk-copy / tcgen05 path the engine uses.  All pointers are device pointers except wx/bias.
-int tc_selftest_xproj(const float* a_dev, int64_t n_blocks, int K, const float* wx_host, const float* bias_host,
-                      float* out_dev, cudaStream_t stream) {
-    if (K != 32 && K != 128) { set_error("selftest: K must be 32 or 128"); return CF_ERR_BAD_ARG; }
-    std::vector<__nv_bfloat16> wpk;
-    pack_b_operand(wx_host, K, kNX, 2 * kNX, 0, &wpk);
-    pack_b_operand(wx_host, K, kNX, 2 * kNX, kNX, &wpk);
-    DevBuf w, b, a;
-    CF_TRY(w.ensure(wpk.size() * 2));
-    CF_TRY(b.ensure(2 * kNX * 4));
-    CF_TRY(a.ensure((size_t)n_blocks * 128 * K * 4));
-    CF_CUDA(cudaMemcpyAsync(w.ptr, wpk.data(), wpk.size() * 2, cudaMemcpyHostToDevice, stream));
-    CF_CUDA(cudaMemcpyAsync(b.ptr, bias_host, 2 * kNX * 4, cudaMemcpyHostToDevice, stream));
-    const int64_t rows = n_blocks * 128;
-    tc_pack_a_kernel<<<(unsigned)ceil_div(rows * (K / 8), 256), 256, 0, stream>>>(a_dev, K, rows, a.as<__nv_bfloat16>());
-    CF_LAUNCHED();
-    int sms = 148;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int grid = 2 * (int)std::min<int64_t>(n_blocks, sms / 2);
-    if (K == 32) {
-        CF_CUDA(cudaFuncSetAttribute(tc_xproj_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, XprojCfg<32>::kSmem));
-        tc_xproj_kernel<32><<<grid, 192, XprojCfg<32>::kSmem, stream>>>(a.as<__nv_bfloat16>(), w.as<__nv_bfloat16>(), b.as<float>(), out_dev, (int)n_blocks);
-    } else {
-        CF_CUDA(cudaFuncSetAttribute(tc_xproj_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, XprojCfg<128>::kSmem));
-        tc_xproj_kernel<128><<<grid, 192, XprojCfg<128>::kSmem, stream>>>(a.as<__nv_bfloat16>(), w.as<__nv_bfloat16>(), b.as<float>(), out_dev, (int)n_blocks);
-    }
-    CF_LAUNCHED();
-    CF_CUDA(cudaStreamSynchronize(stream));
-    w.release(); b.release(); a.release();
     return CF_OK;
 }
 

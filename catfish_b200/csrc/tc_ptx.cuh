@@ -426,16 +426,10 @@ __device__ __forceinline__ float tanh_zb(float acc, float bk) { return tanh_appr
 // two values at a time: packed argument / result arithmetic around the two MUFU.TANH
 __device__ __forceinline__ float2 sigmoid_zb2(float2 acc, float2 bk) {
     const float2 z = ffma2(acc, splat2(kSigArgScale), bk);
-#if defined(CF_EXP) && (CF_EXP & 8)
-    return ffma2(z, splat2(0.01f), splat2(0.5f));       // build-time experiment only: no MUFU
-#endif
     return ffma2(make_float2(tanh_approx(z.x), tanh_approx(z.y)), splat2(0.5f), splat2(0.5f));
 }
 __device__ __forceinline__ float2 tanh_zb2(float2 acc, float2 bk) {
     const float2 z = ffma2(acc, splat2(kTanhArgScale), bk);
-#if defined(CF_EXP) && (CF_EXP & 8)
-    return fmul2(z, splat2(0.01f));                      // build-time experiment only: no MUFU
-#endif
     return make_float2(tanh_approx(z.x), tanh_approx(z.y));
 }
 #endif

@@ -200,7 +200,7 @@ def infer_reads_arrays(raws, model, threshold=0.5, min_run=15, extension_left=11
 
 _PIPELINE_MIN_SAMPLES = 24_000_000      # batches of at least ~2 engine passes take the pipelined path
 _GROUP_SAMPLES = 10_400_000             # one engine pass (2368 tiles of 128 windows) per group
-_FIRST_GROUP_SAMPLES = int(os.environ.get("CF_FIRST_GROUP_SAMPLES", 2_600_000))
+_FIRST_GROUP_SAMPLES = 2_600_000       # a quarter pass, see _infer_reads_pipelined
 _DEVBUF = {}                            # device index -> dict of cached device / pinned result buffers
 
 

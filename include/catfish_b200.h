@@ -89,8 +89,8 @@ int cf_model_num_tensors(const cf_model_desc* desc);
 /* Which engine the handle resolved to (cf_engine value). */
 int cf_model_engine(const cf_model* model);
 /* Tensor-core operand format of the handle: 0 = split bf16, three MMA passes ("bf16x3"); 1 = fp16 main
- * product + e5m2 correction product, two pass-equivalents ("f16e5", the default where every kernel of
- * the pass supports it; CF_TC_FMT=0 in the environment forces 0); -1 = fp32 CUDA-core engine. */
+ * product + e5m2 correction product, two pass-equivalents ("f16e5"; chosen when every tensor-core kernel
+ * of the pass supports it and the GRU weights fit fp16's range); -1 = fp32 CUDA-core engine. */
 int cf_model_operand_format(const cf_model* model);
 
 /* Pre-size the handle's workspace so later calls do not allocate
@@ -254,16 +254,6 @@ int cf_validate_windows(cf_model* model, const float* x_dev, const uint8_t* labe
 int cf_vote_events(int32_t device, const double* scores_dev, int64_t n_scores, const int64_t* event_lengths_host,
                    int64_t n_events, int64_t start, int64_t length, int32_t* classes_dev, int64_t* n_voted_out,
                    int64_t* start_event_out, int64_t* final_event_out, int32_t* empty_event_out, void* stream);
-
-/*
- * cf_selftest_xproj - unit self-test of the tcgen05 GEMM path (no reference counterpart): the GRU
- * input projection out[blk][n][w] = sum_k a[blk*128 + w][k] * wx[k][n] + bias[n], n in [0, 384),
- * through the engine's operand packing, bulk (TMA) copies, tcgen05.mma and TMEM epilogue.
- * a_dev float32 [n_blocks*128][k] (device), wx_host [k][384], bias_host [384] (host),
- * out_dev float32 [n_blocks][384][128] (device); k is 32 or 128.  Synchronises.
- */
-int cf_selftest_xproj(int32_t device, const float* a_dev, int64_t n_blocks, int32_t k, const float* wx_host,
-                      const float* bias_host, float* out_dev, void* stream);
 
 /*
  * cf_selftest_f16e5 - unit self-test of the fp16 + e5m2-correction MMA pair (no reference counterpart):

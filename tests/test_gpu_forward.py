@@ -128,19 +128,24 @@ def test_engine_cross_check_large():
         _check_intervals(a, sa, sb.astype(np.float64))
 
 
-@pytest.mark.parametrize("env", [{"CF_TC_UNFUSED": "1"}, {"CF_TC_FMT": "0"}], ids=["unfused-pair", "bf16x3-operands"])
-def test_tcgen05_kernel_variants(env, monkeypatch):
-    """The two remaining switches of the tcgen05 engine - projection + recurrence as two kernels, and split-bf16
-    operands in every layer - stay parity-green: they are the cross-checks of the default kernels."""
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
+@pytest.mark.parametrize("kind,n_res", [("ResNetRNN", 1), ("ResNetRNN", 3), ("ResNet", 1)],
+                         ids=["resnetrnn-1-block", "resnetrnn-3-blocks", "resnet-1-block"])
+def test_tcgen05_kernel_variants(kind, n_res):
+    """Networks off the default path, which run split-bf16 operands in every layer, against the fp32 SIMT engine:
+    one residual block (tc_conv2_kernel, then the 32- and 128-wide GRU layers or tc_head_conv_kernel) and three
+    (the CUDA-core conv stack, tc_pack_a_kernel, then the GRU layers).  The longest input spans more tiles than
+    the GPU has SMs, so a CTA of every kernel runs several tiles."""
+    w = weights.random_init(kind, seed=30 + n_res, n_layers_res=n_res)
+    m = _model(kind, "auto", w, n_layers_res=n_res)
+    assert m.resolved_engine == "tcgen05" and m.operand_format == "bf16x3"
+    ref = _model(kind, "simt", w, n_layers_res=n_res)
+    if kind == "ResNet":
+        x = np.random.default_rng(31).normal(0, 1.5, size=(20000, 35, 1)).astype(np.float32)
+        assert np.abs(m.infer(x) - ref.infer(x)).max() < PROB_TOL
+        return
     g = golden("forward_resnetrnn_shipped.npz")
-    m = _model("ResNetRNN", "auto")
-    if m.resolved_engine != "tcgen05":
-        pytest.skip("tcgen05 engine not available")
-    reads = [g["read%d" % i] for i in range(int(g["n_reads"]))] + synth.synth_reads([30000, 4481], base_seed=77)
+    reads = [g["read%d" % i] for i in range(int(g["n_reads"]))] + synth.synth_reads([30000, 4481, 700000], base_seed=77)
     hps, lengths, scores = infer.infer_reads(reads, m, return_scores=True)
-    ref = _model("ResNetRNN", "simt")
     hps2, lengths2, scores2 = infer.infer_reads(reads, ref, return_scores=True)
     assert lengths == lengths2
     for a, b_, sa, sb in zip(hps, hps2, scores, scores2):

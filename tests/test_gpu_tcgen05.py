@@ -1,31 +1,9 @@
-"""GPU: unit test of the tcgen05 GEMM path (operand packing, bulk copies, UMMA descriptors, TMEM
-epilogue) against a float64 matmul.  Split-bf16 operands: relative error ~2^-16 per product."""
+"""GPU: unit test of the fp16 + e5m2-correction MMA pair (operand packing, UMMA descriptors, mixed MMA kinds
+on one TMEM accumulator) against a float64 matmul and a bit-level model of the scheme."""
 import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.mark.parametrize("k,n_blocks", [(32, 1), (32, 5), (128, 1), (128, 3), (32, 200), (128, 333)])
-def test_xproj_gemm_matches_float64(k, n_blocks):
-    import torch
-    from catfish_b200 import _cabi
-    lib = _cabi.load_library()
-    rng = np.random.default_rng(k + n_blocks)
-    a = rng.normal(0, 1, size=(n_blocks * 128, k)).astype(np.float32)
-    a[::7] *= 30.0                                            # mixed magnitudes
-    w = rng.normal(0, 0.3, size=(k, 384)).astype(np.float32)
-    bias = rng.normal(0, 1, size=384).astype(np.float32)
-    ad = torch.from_numpy(a).cuda()
-    out = torch.full((n_blocks, 384, 128), float("nan"), dtype=torch.float32, device="cuda")
-    _cabi.check(lib.cf_selftest_xproj(0, ad.data_ptr(), n_blocks, k, w.ctypes.data, bias.ctypes.data,
-                                      out.data_ptr(), torch.cuda.current_stream().cuda_stream))
-    got = out.cpu().numpy().transpose(0, 2, 1).reshape(n_blocks * 128, 384)
-    want = a.astype(np.float64) @ w.astype(np.float64) + bias
-    scale = np.abs(a).astype(np.float64) @ np.abs(w).astype(np.float64) + 1.0
-    err = np.abs(got - want) / scale
-    assert np.isfinite(got).all()
-    assert err.max() < 5e-5, err.max()
 
 
 def _f16e5_emulated(a, w, s=64.0):
