@@ -632,7 +632,7 @@ int cf_model_create(const cf_model_desc* desc, const float* const* tensors, cons
     int engine = desc->engine;
     if (engine == CF_ENGINE_AUTO) engine = cf::tc_supported(m->hm) ? CF_ENGINE_TCGEN05 : CF_ENGINE_SIMT;
     if (engine == CF_ENGINE_TCGEN05 && !cf::tc_supported(m->hm)) {
-        cf::set_error("the tcgen05 engine supports layer_size_res 32 / layer_size 64 only");
+        cf::set_error("the tcgen05 engine supports layer_size_res <= 32 and layer_size <= 64 only");
         delete m;
         return CF_ERR_BAD_ARG;
     }

@@ -1,7 +1,9 @@
 // tcgen05 engine: the GEMM-shaped part of the forward graph on 5th-gen tensor cores.
 //
-// Specialised for the shipped hyper-parameters (conv channels C = 32, GRU units H = 64; any
-// number of layers; network types ResNetRNN, RNN and ResNet).  Single bf16/fp16 operands do not
+// Specialised for the shipped widths (conv channels C = 32, GRU units H = 64; any number of residual
+// blocks and GRU layers; network types ResNetRNN, RNN and ResNet).  Narrower networks (C < 32, H < 64)
+// run on the same kernels: tc_create pads them once with zero channels and units, which stay exactly
+// zero through every layer (pad_model).  Single bf16/fp16 operands do not
 // meet the 1e-3 probability contract (DESIGN.md, precision table), so every product is evaluated
 // with split operands and fp32 accumulation in TMEM, in one of two formats:
 //   bf16x3  a_hi w_hi + a_lo w_hi + a_hi w_lo, three kind::f16 MMAs per K = 16 chunk
@@ -13,9 +15,9 @@
 //   TK4G  tc_gru_fused2_kernel   one GRU layer (input projection + recurrence), two tiles per CTA
 //   TK5   tc_head_kernel         dense 128 -> 1 + sigmoid from the partial dots of the last layer
 // (the conv stack and the GRU layer it feeds use bf16x3, the 128-wide GRU layers f16e5).
-// Other shapes: tc_conv2_kernel (networks with ONE residual block), tc_head_conv_kernel (ResNet-only
-// networks with one residual block), tc_pack_a_kernel (conv stacks of more than two blocks run on the
-// CUDA-core engine; their output is packed into the first GRU layer's operand form).  Layer 0 of
+// Other shapes: tc_conv2_kernel (networks with ONE residual block), tc_conv_block_kernel (every block
+// after the second of deeper stacks, once per block, from and to the K = 32 operand form),
+// tc_head_conv_kernel (ResNet-only networks other than two blocks).  Layer 0 of
 // RNN-only networks, whose input is 1 wide, is the KX = 1 form of TK4G: no x MMAs, the rank-1 update
 // x_t * w_row is added in the epilogue.
 //
@@ -108,8 +110,9 @@ struct TcLayer {
 };
 
 struct TcEngine {
-    SimtEngine* simt = nullptr;       // fp32 conv stack for shapes TK2 is not specialised for
-    uint8_t* conv_params = nullptr;   // TK2 parameter block (see ConvParams), nullptr = use simt
+    SimtEngine* simt = nullptr;       // RNN-only networks: normalised scalar input (simt_conv_stack without blocks)
+    uint8_t* conv_params = nullptr;   // TK2 parameter block (see ConvParams), nullptr = no residual blocks
+    uint8_t* block_params = nullptr;  // [conv_nres - 2] parameter blocks of tc_conv_block_kernel (block-1 slots)
     int conv_nres = 0;
     std::vector<TcLayer> layers;
     float* head_w = nullptr;          // [128]
@@ -128,11 +131,65 @@ struct TcEngine {
 };
 
 bool tc_supported(const HostModel& hm) {
-    if (hm.desc.network_type == CF_NET_RESNET)                        // conv stack (TK2) + dense 32 -> 1
-        return hm.desc.layer_size_res == kC && hm.desc.n_layers_res >= 1 && hm.desc.n_layers_res <= 2;
-    if (hm.desc.layer_size != kH) return false;
-    if (hm.desc.network_type == CF_NET_RESNET_RNN && hm.desc.layer_size_res != kC) return false;
+    if (hm.n_res() > 0 && hm.conv_channels() > kC) return false;     // any number of residual blocks
+    if (hm.n_rnn() > 0 && hm.desc.layer_size > kH) return false;      // any number of GRU layers
     return true;
+}
+
+// The network padded to C = 32 channels and H = 64 units with zero weights and biases.  A zero channel stays
+// relu(0) = 0; a zero unit keeps h = 0 through every GRU step (candidate tanh(0) = 0, h' = u 0 + (1 - u) 0);
+// zero rows add nothing to the real outputs.  So the padded network computes exactly what the narrow one does.
+// Layout: channel c stays at c; unit j of each gate group (r, u, candidate) stays at j of its 64-wide group;
+// a 2H-wide input [fw | bw] (GRU layers after the first, the dense head) puts fw unit j at j and bw unit j at 64 + j.
+static HostModel pad_model(const HostModel& hm) {
+    HostModel p = hm;
+    if (hm.n_res() > 0) {
+        const int C = hm.conv_channels();
+        p.desc.layer_size_res = kC;
+        for (size_t i = 0; i < hm.convs.size(); ++i) {
+            const ConvLayer& s = hm.convs[i];
+            ConvLayer& d = p.convs[i];
+            const bool scalar_in = i < 2;                 // the two Cin = 1 convolutions of block 0
+            d.cin = scalar_in ? 1 : kC;
+            d.cout = kC;
+            d.w.assign((size_t)d.k * d.cin * kC, 0.f);
+            d.b.assign(kC, 0.f);
+            for (int co = 0; co < C; ++co) d.b[co] = s.b[co];
+            for (int k = 0; k < s.k; ++k)
+                for (int ci = 0; ci < s.cin; ++ci)
+                    for (int co = 0; co < C; ++co) d.w[((size_t)k * d.cin + ci) * kC + co] = s.w[((size_t)k * s.cin + ci) * C + co];
+        }
+    }
+    auto unit2 = [](int r, int H) { return r < H ? r : kH + (r - H); };       // row of a [fw | bw] input
+    if (hm.n_rnn() > 0) {
+        const int H = hm.desc.layer_size;
+        p.desc.layer_size = kH;
+        auto col = [&](int j) { return (j / H) * kH + j % H; };                // column of an r | u | c group
+        for (size_t i = 0; i < hm.gru.size(); ++i) {
+            const GruDir& s = hm.gru[i];
+            GruDir& d = p.gru[i];
+            const bool first = i < 2;
+            d.in = first ? (hm.n_res() > 0 ? kC : 1) : 2 * kH;
+            d.h = kH;
+            d.wx.assign((size_t)d.in * kNX, 0.f);
+            d.bx.assign(kNX, 0.f);
+            d.wgh.assign((size_t)kH * 2 * kH, 0.f);
+            d.wch.assign((size_t)kH * kH, 0.f);
+            for (int r = 0; r < s.in; ++r)
+                for (int j = 0; j < 3 * H; ++j) d.wx[(size_t)(first ? r : unit2(r, H)) * kNX + col(j)] = s.wx[(size_t)r * 3 * H + j];
+            for (int j = 0; j < 3 * H; ++j) d.bx[col(j)] = s.bx[j];
+            for (int r = 0; r < H; ++r) {
+                for (int j = 0; j < 2 * H; ++j) d.wgh[(size_t)r * 2 * kH + col(j)] = s.wgh[(size_t)r * 2 * H + j];
+                for (int j = 0; j < H; ++j) d.wch[(size_t)r * kH + j] = s.wch[(size_t)r * H + j];
+            }
+        }
+        p.head_w.assign(2 * kH, 0.f);
+        for (int r = 0; r < 2 * H; ++r) p.head_w[unit2(r, H)] = hm.head_w[r];
+    } else {
+        p.head_w.assign(kC, 0.f);
+        std::copy(hm.head_w.begin(), hm.head_w.end(), p.head_w.begin());
+    }
+    return p;
 }
 
 template <typename T>
@@ -144,12 +201,13 @@ static T* tc_upload(TcEngine* e, const std::vector<T>& v) {
     return d;
 }
 
-TcEngine* tc_create(const HostModel& hm) {
+TcEngine* tc_create(const HostModel& narrow) {
     TcEngine* e = new TcEngine();
     int dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&e->n_sms, cudaDevAttrMultiProcessorCount, dev);
-    e->simt = simt_create(hm);
+    if (narrow.n_res() == 0) e->simt = simt_create(narrow);
+    const HostModel hm = pad_model(narrow);          // everything below, the operand format included, sees C = 32 / H = 64
 #ifdef CF_TRACE_PROBES
     e->trace_path = getenv("CF_TC_TRACE");
 #endif
@@ -167,17 +225,17 @@ TcEngine* tc_create(const HostModel& hm) {
         const bool in_range = wmax * kCandScale * kCorrScale < 60000.f;
         e->fmt = covered && in_range ? kFmtF16E5 : kFmtBf16x3;
     }
-    if (hm.n_res() >= 1 && hm.n_res() <= 2 && hm.conv_channels() == kC) {
-        // TK2 parameter block: fp32 vectors, then the B operands, split bf16 (see ConvParams)
-        std::vector<uint8_t> blk(ConvParams::kBytes, 0);
-        float* fp = reinterpret_cast<float*>(blk.data());
+    if (hm.n_res() >= 1) {
+        // TK2 parameter block: fp32 vectors, then the B operands, split bf16 (see ConvParams).  Blocks 0 and 1 go
+        // to TK2; every further block b gets a block of its own with only the block-1 slots filled, from convs[4 b..].
+        const int n_extra = std::max(hm.n_res() - 2, 0);
+        std::vector<uint8_t> all((size_t)(1 + n_extra) * ConvParams::kBytes, 0);
+        uint8_t* blk = all.data();
+        float* fp = reinterpret_cast<float*>(blk);
         auto put = [&](int slot, const std::vector<float>& v) { memcpy(fp + 32 * slot, v.data(), 32 * sizeof(float)); };
-        put(0, hm.convs[0].w); put(1, hm.convs[0].b);          // shortcut of block 0: [1][1][32]
-        put(2, hm.convs[1].w); put(3, hm.convs[1].b);
-        put(4, hm.convs[2].b); put(5, hm.convs[3].b);
         auto put_w = [&](int off, const float* w, int n, int ldw, int col0, int dst_col0, int n_total) {
             // pack a [32][n] matrix into columns [dst_col0, dst_col0 + n) of a {hi, lo} x [4][n_total][8] operand
-            __nv_bfloat16* hi = reinterpret_cast<__nv_bfloat16*>(blk.data() + off);
+            __nv_bfloat16* hi = reinterpret_cast<__nv_bfloat16*>(blk + off);
             __nv_bfloat16* lo = hi + 32 * n_total;
             for (int k = 0; k < 32; ++k)
                 for (int j = 0; j < n; ++j) {
@@ -188,16 +246,27 @@ TcEngine* tc_create(const HostModel& hm) {
                     lo[idx] = __float2bfloat16_rn(v - __bfloat162float(h));
                 }
         };
+        auto put_block1 = [&](int i) {                    // a residual block with a 32-wide input, convs[i .. i + 3]
+            put(6, hm.convs[i].b); put(7, hm.convs[i + 1].b); put(8, hm.convs[i + 2].b); put(9, hm.convs[i + 3].b);
+            put_w(ConvParams::kW45, hm.convs[i].w.data(), 32, 32, 0, 0, 64);           // shortcut columns 0..31
+            put_w(ConvParams::kW45, hm.convs[i + 1].w.data(), 32, 32, 0, 32, 64);      // p1 columns 32..63
+            for (int tap = 0; tap < 3; ++tap) put_w(ConvParams::kW6 + tap * 4096, hm.convs[i + 2].w.data() + tap * 32 * 32, 32, 32, 0, 0, 32);
+            put_w(ConvParams::kW7, hm.convs[i + 3].w.data(), 32, 32, 0, 0, 32);
+        };
+        put(0, hm.convs[0].w); put(1, hm.convs[0].b);          // shortcut of block 0: [1][1][32]
+        put(2, hm.convs[1].w); put(3, hm.convs[1].b);
+        put(4, hm.convs[2].b); put(5, hm.convs[3].b);
         for (int tap = 0; tap < 3; ++tap) put_w(ConvParams::kW2 + tap * 4096, hm.convs[2].w.data() + tap * 32 * 32, 32, 32, 0, 0, 32);
         put_w(ConvParams::kW3, hm.convs[3].w.data(), 32, 32, 0, 0, 32);
-        if (hm.n_res() == 2) {
-            put(6, hm.convs[4].b); put(7, hm.convs[5].b); put(8, hm.convs[6].b); put(9, hm.convs[7].b);
-            put_w(ConvParams::kW45, hm.convs[4].w.data(), 32, 32, 0, 0, 64);       // sc1 columns 0..31
-            put_w(ConvParams::kW45, hm.convs[5].w.data(), 32, 32, 0, 32, 64);      // p1 columns 32..63
-            for (int tap = 0; tap < 3; ++tap) put_w(ConvParams::kW6 + tap * 4096, hm.convs[6].w.data() + tap * 32 * 32, 32, 32, 0, 0, 32);
-            put_w(ConvParams::kW7, hm.convs[7].w.data(), 32, 32, 0, 0, 32);
+        if (hm.n_res() >= 2) put_block1(4);
+        for (int b = 2; b < hm.n_res(); ++b) {
+            blk = all.data() + (size_t)(b - 1) * ConvParams::kBytes;
+            fp = reinterpret_cast<float*>(blk);
+            put_block1(4 * b);
         }
-        e->conv_params = tc_upload(e, blk);
+        uint8_t* dev_blocks = tc_upload(e, all);
+        e->conv_params = dev_blocks;
+        if (n_extra > 0) e->block_params = dev_blocks + ConvParams::kBytes;
         e->conv_nres = hm.n_res();
     }
     for (int l = 0; l < hm.n_rnn(); ++l) {
@@ -248,26 +317,6 @@ void tc_destroy(TcEngine* e) {
     for (void* p : e->owned) cudaFree(p);
     e->ws.release();
     delete e;
-}
-
-// ====================================================================== A-operand packing
-// fp32 rows [(tile*35+t)*128 + w][K] -> per block: hi plane, lo plane, each [K/8][128][8] bf16.
-// One thread per (row, 8-column group): one 16-byte store per plane, coalesced over rows.
-__global__ void tc_pack_a_kernel(const float* __restrict__ in, int K, int64_t n_rows, __nv_bfloat16* __restrict__ out) {
-    const int kg = K / 8;
-    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= n_rows * kg) return;
-    const int64_t blk = idx / (kg * 128);
-    const int rem = (int)(idx % (kg * 128));
-    const int g = rem / 128, w = rem % 128;
-    const float* src = in + (blk * 128 + w) * K + g * 8;
-    uint32_t hi[4], lo[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) split_bf16x2(src[2 * i], src[2 * i + 1], hi[i], lo[i]);
-    const size_t plane = (size_t)128 * K;
-    __nv_bfloat16* dst = out + (size_t)blk * 2 * plane + ((size_t)g * 128 + w) * 8;
-    *reinterpret_cast<uint4*>(dst) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-    *reinterpret_cast<uint4*>(dst + plane) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
 }
 
 // ====================================================================== TK2: residual conv stack
@@ -795,6 +844,164 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
     tc_fence_before_sync();
     __syncthreads();
     if (warp == 16) tmem_dealloc<512>(tmem);
+}
+
+// ====================================================================== TK2, one further residual block
+// Blocks after the second of a deeper conv stack, one launch per block.  Input and output are the K = 32 operand form
+// TK2 writes (one 16 KB slice per (tile, t)), so the first GRU layer and tc_head_conv_kernel read the last block's
+// output unchanged.  Per position t it is chain Y of tc_conv4_kernel with its input streamed from HBM:
+//   [sc | p1] = y[t] [W_sc | W_1]                        N = 64, TMEM ring of 4 at 64 k (sc waits three positions)
+//   p2[t] = relu(conv3(relu(p1 + b5)) + b6)              taps over p1 operands t-1, t, t+1; SAME padding = skipped MMA
+//   y_out[t] = relu(relu(p2 W_3 + b7) + sc + b4)
+// The stages are skewed so that one batch per iteration u = 0..37 issues [sc|p1][u], p2[u-2] and p3[u-3]; one
+// epilogue pass then writes the p1 operand of u, the p2 operand of u-2 and the output of u-3.
+//   warps 0-7 : epilogue; thread = (window, 16 of the 32 channels)
+//   warp 8    : MMA issuer (warp-converged issue, elected lane)
+//   warp 9    : producer, input slices by cp.async.bulk into a ring of 4
+constexpr int kBlockRing = 4;
+constexpr uint32_t kBlockSmem = ConvParams::kBytes + (kBlockRing + 3 + 1) * kSliceBytes + 256;
+
+__global__ void __launch_bounds__(320, 1)
+tc_conv_block_kernel(const uint8_t* __restrict__ params, const __nv_bfloat16* __restrict__ y_in, int n_tiles,
+                     __nv_bfloat16* __restrict__ y_out) {
+    constexpr int kFmt = kFmtBf16x3;
+    extern __shared__ __align__(128) uint8_t smem[];
+    uint8_t* prm = smem;
+    uint8_t* yin = smem + ConvParams::kBytes;         // ring of kBlockRing input slices
+    uint8_t* p1 = yin + kBlockRing * kSliceBytes;     // ring of 3 p1 operand slices (slot t % 3)
+    uint8_t* p2 = p1 + 3 * kSliceBytes;
+    uint64_t* bars = reinterpret_cast<uint64_t*>(p2 + kSliceBytes);
+    uint64_t* bar_ready = &bars[0];
+    uint64_t* bar_mma = &bars[1];
+    uint64_t* bar_prm = &bars[2];
+    uint64_t* bar_full = &bars[3];                    // [kBlockRing] input slice landed
+    uint64_t* bar_empty = &bars[3 + kBlockRing];      // [kBlockRing] its MMA completed
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 + 2 * kBlockRing);
+    const float* fp = reinterpret_cast<const float*>(prm);
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) {
+        mbar_init(bar_ready, 8);
+        mbar_init(bar_mma, 1);
+        mbar_init(bar_prm, 1);
+        for (int i = 0; i < kBlockRing; ++i) { mbar_init(&bar_full[i], 1); mbar_init(&bar_empty[i], 1); }
+        fence_mbar_init();
+        mbar_expect_tx(bar_prm, ConvParams::kBytes);
+        bulk_g2s(prm, params, ConvParams::kBytes, bar_prm);
+    }
+    if (warp == 8) tmem_alloc<512>(tmem_slot);
+    tc_fence_before_sync();
+    __syncthreads();
+    tc_fence_after_sync();
+    const uint32_t tmem = *tmem_slot;
+    constexpr int kLastU = kWindow + 2;               // p3[34] at u = 37
+    constexpr uint32_t kTmP2 = 256, kTmP3 = 288;      // [sc|p1] ring at 0, 64, 128, 192
+    mbar_wait(bar_prm, 0);
+
+    if (warp == 8) {
+        // ------------------------------------------------------------ issuer (all lanes converged)
+        const uint32_t elected = elect_one();
+        const uint32_t prm_u = smem_u32(prm), yin_u = smem_u32(yin), p1_u = smem_u32(p1), p2_u = smem_u32(p2);
+        uint32_t it = 0, n = 0;                       // n = input slices consumed so far
+        for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+            for (int u = 0; u <= kLastU; ++u, ++it) {
+                mbar_wait(bar_ready, it & 1);
+                tc_fence_after_sync();
+                const int t2 = u - 2, t3 = u - 3;
+                if (u < kWindow) {
+                    const uint32_t slot = n % kBlockRing;
+                    mbar_wait(&bar_full[slot], (n / kBlockRing) & 1);
+                    conv_mma_pred<64>(tmem + (u & 3) * 64, yin_u + slot * kSliceBytes, prm_u + ConvParams::kW45, true, elected);
+                    umma_commit_pred(&bar_empty[slot], elected);
+                    ++n;
+                }
+                if (t2 >= 0 && t2 < kWindow) {
+                    bool first = true;
+#pragma unroll
+                    for (int tap = 0; tap < 3; ++tap) {
+                        const int tt = t2 + tap - 1;
+                        if (tt < 0 || tt >= kWindow) continue;
+                        conv_mma_pred<32>(tmem + kTmP2, p1_u + (tt % 3) * kSliceBytes, prm_u + ConvParams::kW6 + tap * 4096, first, elected);
+                        first = false;
+                    }
+                }
+                if (t3 >= 0 && t3 < kWindow) conv_mma_pred<32>(tmem + kTmP3, p2_u, prm_u + ConvParams::kW7, true, elected);
+                umma_commit_pred(bar_mma, elected);
+            }
+        }
+    } else if (warp == 9) {
+        // ------------------------------------------------------------ producer
+        if (lane == 0) {
+            const uint8_t* src = reinterpret_cast<const uint8_t*>(y_in);
+            uint32_t n = 0;
+            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x)
+                for (int t = 0; t < kWindow; ++t, ++n) {
+                    const uint32_t slot = n % kBlockRing;
+                    if (n >= kBlockRing) mbar_wait(&bar_empty[slot], (n / kBlockRing - 1) & 1);
+                    mbar_expect_tx(&bar_full[slot], kSliceBytes);
+                    bulk_g2s(yin + slot * kSliceBytes, src + ((size_t)tile * kWindow + t) * kSliceBytes, kSliceBytes, &bar_full[slot]);
+                }
+        }
+    } else {
+        // ------------------------------------------------------------ epilogue
+        const int q = warp & 3, ch = warp >> 2;
+        const int row = q * 32 + lane;
+        const int c0 = ch * 16;
+        const uint32_t t_lane = tmem + ((uint32_t)(q * 32) << 16) + c0;
+        auto relu_bias = [&](uint32_t* r, int slot, float* v) {
+#pragma unroll
+            for (int i = 0; i < 16; i += 4) {
+                const float4 b4 = *reinterpret_cast<const float4*>(fp + 32 * slot + c0 + i);
+                const float2 s0 = fadd2(make_float2(__uint_as_float(r[i]), __uint_as_float(r[i + 1])), make_float2(b4.x, b4.y));
+                const float2 s1 = fadd2(make_float2(__uint_as_float(r[i + 2]), __uint_as_float(r[i + 3])), make_float2(b4.z, b4.w));
+                v[i] = fmaxf(s0.x, 0.f);
+                v[i + 1] = fmaxf(s0.y, 0.f);
+                v[i + 2] = fmaxf(s1.x, 0.f);
+                v[i + 3] = fmaxf(s1.y, 0.f);
+            }
+        };
+        uint32_t it = 0;
+        if (lane == 0) mbar_arrive(bar_ready);        // nothing to prepare for the first batch
+        for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+            for (int u = 0; u <= kLastU; ++u, ++it) {
+                const int t2 = u - 2, t3 = u - 3;
+                const bool h1 = u < kWindow, h2 = t2 >= 0 && t2 < kWindow, h3 = t3 >= 0 && t3 < kWindow;
+                mbar_wait(bar_mma, it & 1);
+                tc_fence_after_sync();
+                uint32_t r1[16], r2[16], r3[16], rs[16];
+                if (h1) tmem_ld16_nowait(t_lane + (u & 3) * 64 + 32, r1);
+                if (h2) tmem_ld16_nowait(t_lane + kTmP2, r2);
+                if (h3) {
+                    tmem_ld16_nowait(t_lane + kTmP3, r3);
+                    tmem_ld16_nowait(t_lane + (t3 & 3) * 64, rs);
+                }
+                tmem_ld_wait();
+                float v[16];
+                if (h1) { relu_bias(r1, 7, v); store_a_row16_f<kFmt>(p1 + (u % 3) * kSliceBytes, row, c0, v); }   // b5
+                if (h2) { relu_bias(r2, 8, v); store_a_row16_f<kFmt>(p2, row, c0, v); }                        // b6
+                // the next batch's operands are written and every accumulator it overwrites has been read
+                fence_proxy_async_smem();
+                tc_fence_before_sync();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(bar_ready);
+                if (h3) {
+                    relu_bias(r3, 9, v);                                                         // b7
+#pragma unroll
+                    for (int i = 0; i < 16; i += 2) {                                             // + (sc + b4)
+                        const float2 sc = fadd2(make_float2(__uint_as_float(rs[i]), __uint_as_float(rs[i + 1])),
+                                                *reinterpret_cast<const float2*>(fp + 192 + c0 + i));
+                        const float2 o = fadd2(make_float2(v[i], v[i + 1]), sc);
+                        v[i] = fmaxf(o.x, 0.f);
+                        v[i + 1] = fmaxf(o.y, 0.f);
+                    }
+                    store_a_row16_f<kFmt>(reinterpret_cast<uint8_t*>(y_out) + ((size_t)tile * kWindow + t3) * kSliceBytes, row, c0, v);
+                }
+            }
+        }
+    }
+    tc_fence_before_sync();
+    __syncthreads();
+    if (warp == 8) tmem_dealloc<512>(tmem);
 }
 
 // ====================================================================== TK4G: fused GRU layer, two tiles per CTA
@@ -1487,6 +1694,7 @@ int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const doubl
         CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<128, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<128>::kSmem));
         CF_CUDA(cudaFuncSetAttribute(tc_conv2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmem));
         CF_CUDA(cudaFuncSetAttribute(tc_conv4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kConv4Smem));
+        CF_CUDA(cudaFuncSetAttribute(tc_conv_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBlockSmem));
         e->attr_done = true;
     }
     const int64_t chunk = n_tiles < kTcChunkTiles ? n_tiles : kTcChunkTiles;
@@ -1507,20 +1715,30 @@ int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const doubl
         const int64_t tiles = std::min<int64_t>(kTcChunkTiles, n_tiles - tile0);
         const int64_t blocks = tiles * kWindow;
         const int64_t rows = blocks * 128;
-        const float* feat = nullptr;             // fp32 rows: conv output [rows][32] or x [rows]
+        const float* feat = nullptr;             // RNN-only networks: the normalised scalar input x [rows]
         const __nv_bfloat16* a_in = nullptr;
         if (e->conv_params) {
             ProfScope ps(prof, KC_K2_CONV, stream);
             const int grid = (int)std::min<int64_t>(tiles, e->n_sms);
-            if (e->conv_nres == 2)
+            const bool fused_head = n_layers == 0 && e->conv_nres == 2;
+            if (e->conv_nres >= 2)
                 tc_conv4_kernel<<<grid, 576, kConv4Smem, stream>>>(e->conv_params, raw, stats, xwin, tab.src, tab.valid,
                                                                   tab.read, tile0, (int)tiles, a0,
-                                                                  n_layers == 0 ? e->head_w : nullptr, n_layers == 0 ? head_part : nullptr);
+                                                                  fused_head ? e->head_w : nullptr, fused_head ? head_part : nullptr);
             else
                 tc_conv2_kernel<<<grid, 288, kConvSmem, stream>>>(e->conv_params, raw, stats, xwin, tab.src, tab.valid,
                                                                   tab.read, tile0, (int)tiles, a0);
             CF_LAUNCHED();
             a_in = a0;
+            // further blocks alternate between a0 and ybuf[1], which the GRU layers do not touch before layer 1
+            // writes it; the last block's output is never in ybuf[0], which GRU layer 0 writes while reading it
+            for (int b = 2; b < e->conv_nres; ++b) {
+                __nv_bfloat16* out = a_in == a0 ? ybuf[1] : a0;
+                tc_conv_block_kernel<<<grid, 320, kBlockSmem, stream>>>(e->block_params + (size_t)(b - 2) * ConvParams::kBytes,
+                                                                        a_in, (int)tiles, out);
+                CF_LAUNCHED();
+                a_in = out;
+            }
         } else {
             CF_TRY(simt_conv_stack(e->simt, hm, raw, stats, xwin, tab, tile0, tiles, chunk, &feat, stream, prof));
         }
@@ -1529,13 +1747,6 @@ int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const doubl
             const bool last = l + 1 == n_layers;
             __nv_bfloat16* yo = last ? nullptr : ybuf[l & 1];
             // input projection + recurrence in one kernel; a_in is the A-operand form of the layer input
-            if (l == 0 && !a_in && L.in == kC) {
-                ProfScope ps(prof, KC_K3_XPROJ, stream);
-                const int64_t total = rows * (kC / 8);
-                tc_pack_a_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, stream>>>(feat, kC, rows, a0);
-                CF_LAUNCHED();
-                a_in = a0;
-            }
             ProfScope ps(prof, KC_K4_GRU, stream);
             long long* trace_dev = nullptr;
 #ifdef CF_TRACE_PROBES

@@ -41,7 +41,7 @@ typedef enum cf_network_type {
 
 typedef enum cf_engine {
     CF_ENGINE_AUTO = 0,       /* tcgen05 kernels when the shape is supported, else SIMT */
-    CF_ENGINE_TCGEN05 = 1,    /* bf16x3 split operands on tcgen05/TMEM (C = 32, H = 64) */
+    CF_ENGINE_TCGEN05 = 1,    /* split operands on tcgen05/TMEM (C <= 32, H <= 64, any depth) */
     CF_ENGINE_SIMT = 2        /* fp32 CUDA-core kernels, any shape (on-device cross-check) */
 } cf_engine;
 
