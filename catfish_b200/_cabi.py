@@ -53,6 +53,12 @@ SIGNATURES = {
     "cf_infer_reads_host": (ctypes.c_int, [c_void, c_void, c_i64_p, ctypes.c_int32, c_void, c_void, c_void,
                                            ctypes.c_int64, ctypes.c_double, ctypes.c_int32, ctypes.c_int32,
                                            ctypes.c_int32, c_i64_p, c_void]),
+    "cf_exec_create": (ctypes.c_int, [c_void, ctypes.POINTER(c_void)]),
+    "cf_exec_destroy": (None, [c_void]),
+    "cf_exec_reserve": (ctypes.c_int, [c_void, ctypes.c_int64, ctypes.c_int32]),
+    "cf_exec_infer_reads": (ctypes.c_int, [c_void, c_void, c_i64_p, ctypes.c_int32, c_void, c_void, c_void,
+                                           ctypes.c_int64, ctypes.c_double, ctypes.c_int32, ctypes.c_int32,
+                                           ctypes.c_int32, c_void]),
     "cf_max_intervals": (ctypes.c_int64, [ctypes.c_int64, ctypes.c_int32, ctypes.c_int32]),
     "cf_normalize_reads": (ctypes.c_int, [ctypes.c_int32, c_void, c_i64_p, ctypes.c_int32, c_void, c_void, c_void]),
     "cf_call_intervals": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int32, c_i64_p, ctypes.c_int32,

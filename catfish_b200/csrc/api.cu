@@ -234,30 +234,67 @@ __global__ void dense_window_table_kernel(int64_t n_windows, int64_t n_slots, in
 
 }  // namespace cf
 
-// ---------------------------------------------------------------- handle
+// ---------------------------------------------------------------- execution context
+namespace cf {
+
+// Everything an inference call writes.  The model (weights, engine, operand format) is read-only after
+// cf_model_create; calls on different contexts of one model share nothing else and may overlap on the device.
+struct Exec {
+    HostBuf pin_plan;                // offsets + win_off staging
+    cudaEvent_t plan_copied = nullptr;
+    HostBuf pin_chunks;              // K1 chunk-table staging
+    cudaEvent_t chunks_copied = nullptr;
+    DevBuf plan_dev;                 // offsets[R+1] | win_off[R+1]
+    DevBuf stats, wide_flags, wide_scratch, k1_chunked, k1_chunk_tab;
+    DevBuf tab_src, tab_valid, tab_read;
+    DevBuf probs_internal;
+    DevBuf val_logits, val_partial;  // validation row (N4)
+    IntervalScratch k6;
+    // host-buffer entry point
+    DevBuf h_raw, h_intervals, h_ioff, h_probs;
+    HostBuf pin_io;
+    // engine workspaces: the tensor-core pass, and the CUDA-core pass (the tensor-core engine uses it for the
+    // scalar input of RNN-only networks)
+    DevBuf tc_ws, simt_ws;
+    cudaEvent_t last_done = nullptr; // end of the previous asynchronous call on this context (ExecCall)
+    std::mutex mu;
+
+    void release() {
+        pin_plan.release(); plan_dev.release(); stats.release(); wide_flags.release();
+        wide_scratch.release(); k1_chunked.release(); k1_chunk_tab.release(); tab_src.release(); tab_valid.release(); tab_read.release();
+        probs_internal.release();
+        val_logits.release(); val_partial.release();
+        k6.bits.release(); k6.block_cnt.release(); k6.read_cnt.release(); k6.misc.release();
+        h_raw.release(); h_intervals.release(); h_ioff.release(); h_probs.release();
+        pin_io.release();
+        tc_ws.release(); simt_ws.release();
+        if (plan_copied) cudaEventDestroy(plan_copied);
+        plan_copied = nullptr;
+        pin_chunks.release();
+        if (chunks_copied) cudaEventDestroy(chunks_copied);
+        chunks_copied = nullptr;
+        if (last_done) cudaEventDestroy(last_done);
+        last_done = nullptr;
+    }
+};
+
+}  // namespace cf
+
+// ---------------------------------------------------------------- handles
 struct cf_model {
     cf::HostModel hm;
     int device = 0;
     int engine = CF_ENGINE_SIMT;
     cf::SimtEngine* simt = nullptr;
     cf::TcEngine* tc = nullptr;
-    // per-batch scratch
-    cf::HostBuf pin_plan;            // offsets + win_off staging
-    cudaEvent_t plan_copied = nullptr;
-    cf::HostBuf pin_chunks;          // K1 chunk-table staging
-    cudaEvent_t chunks_copied = nullptr;
-    cf::DevBuf plan_dev;             // offsets[R+1] | win_off[R+1]
-    cf::DevBuf stats, wide_flags, wide_scratch, k1_chunked, k1_chunk_tab;
-    cf::DevBuf tab_src, tab_valid, tab_read;
-    cf::DevBuf probs_internal;
-    cf::DevBuf val_logits, val_partial;   // validation row (N4)
-    cf::IntervalScratch k6;
-    cf::Profiler prof;
-    // host-buffer entry point
-    cf::DevBuf h_raw, h_intervals, h_ioff, h_probs;
-    cf::HostBuf pin_io;
-    cudaEvent_t last_done = nullptr; // end of the previous asynchronous call on this handle (handle_begin / handle_end)
-    std::mutex mu;
+    cf::Exec def;                    // the default context of every cf_model_* / cf_infer_* / cf_validate_* call
+    cf::Profiler prof;               // cf_profile_*: timing of the default context's calls
+    std::atomic<int> refs{1};        // the handle itself + one per live cf_exec
+};
+
+struct cf_exec {
+    cf_model* model = nullptr;
+    cf::Exec x;
 };
 
 namespace cf {
@@ -297,28 +334,33 @@ int DeviceGuard::set(int device) {
     return CF_OK;
 }
 
-// One handle = one set of scratch buffers: a call on stream B must not start while the previous call's
-// kernels (possibly on stream A) still use them.  Every asynchronous entry point waits on the event of the
-// previous call first (a no-op on the same stream) and records it again when its own work is enqueued.
-static int handle_begin(cf_model* m, cudaStream_t st);
-static int handle_end(cf_model* m, cudaStream_t st);
+// One context = one set of scratch buffers: a call on stream B must not start while the previous call's
+// kernels (possibly on stream A) still use them.  Every asynchronous call waits on the event of the previous
+// call on its context first (a no-op on the same stream) and records it again when it returns - on every
+// path, so that a call that fails after enqueueing work still orders the next call after that work.
+struct ExecCall {
+    Exec* x;
+    cudaStream_t st;
+    bool armed = false;
+    ExecCall(Exec* ex, cudaStream_t stream) : x(ex), st(stream) {}
+    int begin() {
+        if (!x->last_done) CF_CUDA(cudaEventCreateWithFlags(&x->last_done, cudaEventDisableTiming));
+        armed = true;
+        CF_CUDA(cudaStreamWaitEvent(st, x->last_done, 0));
+        return CF_OK;
+    }
+    ~ExecCall() {
+        if (armed && cudaEventRecord(x->last_done, st) != cudaSuccess) cudaGetLastError();
+    }
+};
 
-static int engine_forward(cf_model* m, const int16_t* raw, const double* stats, const float* xwin,
-                          WindowTable tab, int64_t n_tiles, float* probs, cudaStream_t stream,
+static int engine_forward(cf_model* m, Exec* x, Profiler* prof, const int16_t* raw, const double* stats,
+                          const float* xwin, WindowTable tab, int64_t n_tiles, float* probs, cudaStream_t stream,
                           bool want_logits = false, const LabelBits* bits = nullptr) {
     if (m->engine == CF_ENGINE_TCGEN05)
-        return tc_forward(m->tc, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream, &m->prof, want_logits, bits);
-    return simt_forward(m->simt, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream, &m->prof, want_logits);
-}
-
-static int handle_begin(cf_model* m, cudaStream_t st) {
-    if (m->last_done) CF_CUDA(cudaStreamWaitEvent(st, m->last_done, 0));
-    return CF_OK;
-}
-static int handle_end(cf_model* m, cudaStream_t st) {
-    if (!m->last_done) CF_CUDA(cudaEventCreateWithFlags(&m->last_done, cudaEventDisableTiming));
-    CF_CUDA(cudaEventRecord(m->last_done, st));
-    return CF_OK;
+        return tc_forward(m->tc, &x->tc_ws, &x->simt_ws, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream, prof,
+                          want_logits, bits);
+    return simt_forward(m->simt, &x->simt_ws, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream, prof, want_logits);
 }
 
 // Validate offsets and lay out the windows of every read (infer.py:32-43).
@@ -351,20 +393,20 @@ static int make_plan(const int64_t* offsets, int32_t n_reads, BatchPlan* p) {
 }
 
 // Copy offsets (rebased to 0) and win_off to the device through the pinned staging buffer.
-static int upload_plan(cf_model* m, const int64_t* offsets, const BatchPlan& p, cudaStream_t stream,
+static int upload_plan(Exec* x, const int64_t* offsets, const BatchPlan& p, cudaStream_t stream,
                        const int64_t** offsets_dev, const int64_t** win_off_dev) {
     const size_t n = (size_t)p.n_reads + 1;
-    if (m->plan_copied) CF_CUDA(cudaEventSynchronize(m->plan_copied));   // staging still in flight?
-    CF_TRY(m->pin_plan.ensure(2 * n * sizeof(int64_t)));
-    CF_TRY(m->plan_dev.ensure(2 * n * sizeof(int64_t)));
-    int64_t* st = m->pin_plan.as<int64_t>();
+    if (x->plan_copied) CF_CUDA(cudaEventSynchronize(x->plan_copied));   // staging still in flight?
+    CF_TRY(x->pin_plan.ensure(2 * n * sizeof(int64_t)));
+    CF_TRY(x->plan_dev.ensure(2 * n * sizeof(int64_t)));
+    int64_t* st = x->pin_plan.as<int64_t>();
     for (size_t i = 0; i < n; ++i) st[i] = offsets[i] - offsets[0];
     memcpy(st + n, p.win_off.data(), n * sizeof(int64_t));
-    CF_CUDA(cudaMemcpyAsync(m->plan_dev.ptr, st, 2 * n * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
-    if (!m->plan_copied) CF_CUDA(cudaEventCreateWithFlags(&m->plan_copied, cudaEventDisableTiming));
-    CF_CUDA(cudaEventRecord(m->plan_copied, stream));
-    *offsets_dev = m->plan_dev.as<int64_t>();
-    *win_off_dev = m->plan_dev.as<int64_t>() + n;
+    CF_CUDA(cudaMemcpyAsync(x->plan_dev.ptr, st, 2 * n * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
+    if (!x->plan_copied) CF_CUDA(cudaEventCreateWithFlags(&x->plan_copied, cudaEventDisableTiming));
+    CF_CUDA(cudaEventRecord(x->plan_copied, stream));
+    *offsets_dev = x->plan_dev.as<int64_t>();
+    *win_off_dev = x->plan_dev.as<int64_t>() + n;
     return CF_OK;
 }
 
@@ -426,19 +468,19 @@ static int compute_read_stats(const int16_t* raw0, const int64_t* offsets_host, 
                                  sc.chunked->ptr, stats, sc.flags->as<int32_t>(), sc.wide->as<uint32_t>(), kWideSlots, stream);
 }
 
-static int ensure_table(cf_model* m, int64_t n_tiles, WindowTable* tab) {
+static int ensure_table(Exec* x, int64_t n_tiles, WindowTable* tab) {
     const size_t slots = (size_t)n_tiles * kTileWindows;
-    CF_TRY(m->tab_src.ensure(slots * sizeof(int64_t)));
-    CF_TRY(m->tab_valid.ensure(slots * sizeof(int32_t)));
-    CF_TRY(m->tab_read.ensure(slots * sizeof(int32_t)));
-    tab->src = m->tab_src.as<int64_t>();
-    tab->valid = m->tab_valid.as<int32_t>();
-    tab->read = m->tab_read.as<int32_t>();
+    CF_TRY(x->tab_src.ensure(slots * sizeof(int64_t)));
+    CF_TRY(x->tab_valid.ensure(slots * sizeof(int32_t)));
+    CF_TRY(x->tab_read.ensure(slots * sizeof(int32_t)));
+    tab->src = x->tab_src.as<int64_t>();
+    tab->valid = x->tab_valid.as<int32_t>();
+    tab->read = x->tab_read.as<int32_t>();
     return CF_OK;
 }
 
-static int infer_reads_device(cf_model* m, const int16_t* raw_dev, const int64_t* offsets_host,
-                              int32_t n_reads, float* probs_dev, int64_t* intervals_dev,
+static int infer_reads_device(cf_model* m, Exec* x, Profiler* prof, const int16_t* raw_dev,
+                              const int64_t* offsets_host, int32_t n_reads, float* probs_dev, int64_t* intervals_dev,
                               int64_t* interval_offsets_dev, int64_t capacity, double threshold,
                               int32_t min_run, int32_t ext_left, int32_t ext_right,
                               cudaStream_t stream) {
@@ -450,10 +492,10 @@ static int infer_reads_device(cf_model* m, const int16_t* raw_dev, const int64_t
     }
     const int16_t* raw0 = raw_dev + offsets_host[0];
     const int64_t *offsets_dev, *win_off_dev;
-    CF_TRY(upload_plan(m, offsets_host, plan, stream, &offsets_dev, &win_off_dev));
-    CF_TRY(m->stats.ensure(sizeof(double) * 2 * (size_t)n_reads));
+    CF_TRY(upload_plan(x, offsets_host, plan, stream, &offsets_dev, &win_off_dev));
+    CF_TRY(x->stats.ensure(sizeof(double) * 2 * (size_t)n_reads));
     WindowTable tab;
-    CF_TRY(ensure_table(m, plan.n_tiles, &tab));
+    CF_TRY(ensure_table(x, plan.n_tiles, &tab));
     // When the caller does not want the probabilities, the head kernel thresholds them itself and emits label bits
     // (no 4 B/sample write + 4 B/sample read between the network and the interval caller).
     const bool fused_bits = !probs_dev && m->engine == CF_ENGINE_TCGEN05 && tc_can_emit_bits(m->tc);
@@ -461,34 +503,34 @@ static int infer_reads_device(cf_model* m, const int16_t* raw_dev, const int64_t
     bits.threshold = threshold;
     float* probs = probs_dev;
     if (fused_bits) {
-        CF_TRY(k6_bits_prepare(m->k6, plan.total_samples, &bits, stream));
+        CF_TRY(k6_bits_prepare(x->k6, plan.total_samples, &bits, stream));
     } else if (!probs) {
-        CF_TRY(m->probs_internal.ensure(sizeof(float) * (size_t)plan.total_samples));
-        probs = m->probs_internal.as<float>();
+        CF_TRY(x->probs_internal.ensure(sizeof(float) * (size_t)plan.total_samples));
+        probs = x->probs_internal.as<float>();
     }
     {
-        StatsScratch sc{&m->wide_flags, &m->wide_scratch, &m->k1_chunked, &m->k1_chunk_tab, &m->pin_chunks, &m->chunks_copied};
+        StatsScratch sc{&x->wide_flags, &x->wide_scratch, &x->k1_chunked, &x->k1_chunk_tab, &x->pin_chunks, &x->chunks_copied};
         const bool chunks = stats_use_chunks(offsets_host, n_reads);
         if (chunks) {   // allocate before the timed bracket
-            CF_TRY(m->k1_chunked.ensure(k1_chunked_scratch_bytes(n_reads)));
+            CF_TRY(x->k1_chunked.ensure(k1_chunked_scratch_bytes(n_reads)));
         }
-        ProfScope ps(&m->prof, KC_K1_STATS, stream, chunks ? 4 : 2);
-        CF_TRY(compute_read_stats(raw0, offsets_host, offsets_dev, n_reads, m->stats.as<double>(), sc, stream));
+        ProfScope ps(prof, KC_K1_STATS, stream, chunks ? 4 : 2);
+        CF_TRY(compute_read_stats(raw0, offsets_host, offsets_dev, n_reads, x->stats.as<double>(), sc, stream));
     }
     {
-        ProfScope ps(&m->prof, KC_K1_TABLE, stream);
+        ProfScope ps(prof, KC_K1_TABLE, stream);
         CF_TRY(k1_window_table(offsets_dev, win_off_dev, n_reads, plan.total_windows, plan.n_tiles, tab, stream,
                                fused_bits ? bits.bwords : nullptr, plan.total_samples));
     }
-    CF_TRY(engine_forward(m, raw0, m->stats.as<double>(), nullptr, tab, plan.n_tiles, probs, stream, false,
+    CF_TRY(engine_forward(m, x, prof, raw0, x->stats.as<double>(), nullptr, tab, plan.n_tiles, probs, stream, false,
                           fused_bits ? &bits : nullptr));
     if (fused_bits) {
-        ProfScope ps(&m->prof, KC_K6_INTERVALS, stream, 3);
-        CF_TRY(k6_intervals_from_bits(m->k6, bits, offsets_dev, n_reads, plan.total_samples, intervals_dev,
+        ProfScope ps(prof, KC_K6_INTERVALS, stream, 3);
+        CF_TRY(k6_intervals_from_bits(x->k6, bits, offsets_dev, n_reads, plan.total_samples, intervals_dev,
                                       interval_offsets_dev, capacity, min_run, ext_left, ext_right, stream));
     } else {
-        ProfScope ps(&m->prof, KC_K6_INTERVALS, stream, 7);
-        CF_TRY(k6_call_intervals(m->k6, probs, BITS_FROM_F32, threshold, 1, offsets_dev, n_reads,
+        ProfScope ps(prof, KC_K6_INTERVALS, stream, 7);
+        CF_TRY(k6_call_intervals(x->k6, probs, BITS_FROM_F32, threshold, 1, offsets_dev, n_reads,
                                  plan.total_samples, intervals_dev, interval_offsets_dev, nullptr, capacity,
                                  min_run, ext_left, ext_right, stream));
     }
@@ -641,7 +683,8 @@ int cf_model_create(const cf_model_desc* desc, const float* const* tensors, cons
     else m->simt = cf::simt_create(m->hm);
     cudaError_t e = cudaDeviceSynchronize();
     if (e != cudaSuccess || (!m->tc && !m->simt)) {
-        cf::set_error("cf_model_create: uploading weights failed: %s", cudaGetErrorString(e));
+        // a failed engine creation has already said why; otherwise the device did
+        if (e != cudaSuccess) cf::set_error("cf_model_create: uploading weights failed: %s", cudaGetErrorString(e));
         cf_model_destroy(m);
         return CF_ERR_CUDA;
     }
@@ -649,26 +692,49 @@ int cf_model_create(const cf_model_desc* desc, const float* const* tensors, cons
     return CF_OK;
 }
 
+// Drop one reference (the handle's or a context's); the last one frees the weights.  The caller has selected
+// the model's device.
+static void model_unref(cf_model* m) {
+    if (m->refs.fetch_sub(1) != 1) return;
+    cudaDeviceSynchronize();
+    cf::simt_destroy(m->simt);
+    cf::tc_destroy(m->tc);
+    delete m;
+}
+
 void cf_model_destroy(cf_model* m) {
     if (!m) return;
     cf::DeviceGuard guard;
     if (guard.set(m->device) != CF_OK) cudaSetDevice(m->device);
     cudaDeviceSynchronize();
-    cf::simt_destroy(m->simt);
-    cf::tc_destroy(m->tc);
-    m->pin_plan.release(); m->plan_dev.release(); m->stats.release(); m->wide_flags.release();
-    m->wide_scratch.release(); m->k1_chunked.release(); m->k1_chunk_tab.release(); m->tab_src.release(); m->tab_valid.release(); m->tab_read.release();
-    m->probs_internal.release();
-    m->val_logits.release(); m->val_partial.release();
-    m->k6.bits.release(); m->k6.block_cnt.release(); m->k6.read_cnt.release(); m->k6.misc.release();
-    m->h_raw.release(); m->h_intervals.release(); m->h_ioff.release(); m->h_probs.release();
-    m->pin_io.release();
+    m->def.release();
     m->prof.release();
-    if (m->plan_copied) cudaEventDestroy(m->plan_copied);
-    m->pin_chunks.release();
-    if (m->chunks_copied) cudaEventDestroy(m->chunks_copied);
-    if (m->last_done) cudaEventDestroy(m->last_done);
-    delete m;
+    model_unref(m);
+}
+
+int cf_exec_create(cf_model* m, cf_exec** out) {
+    if (!m || !out) { cf::set_error("cf_exec_create: NULL argument"); return CF_ERR_BAD_ARG; }
+    *out = nullptr;
+    cf::DeviceGuard guard;
+    CF_TRY(guard.set(m->device));
+    cf_exec* ex = new cf_exec();
+    ex->model = m;
+    m->refs.fetch_add(1);
+    *out = ex;
+    return CF_OK;
+}
+
+void cf_exec_destroy(cf_exec* ex) {
+    if (!ex) return;
+    cf::DeviceGuard guard;
+    if (guard.set(ex->model->device) != CF_OK) cudaSetDevice(ex->model->device);
+    {
+        std::lock_guard<std::mutex> lock(ex->x.mu);
+        if (ex->x.last_done) cudaEventSynchronize(ex->x.last_done);
+        ex->x.release();
+    }
+    model_unref(ex->model);
+    delete ex;
 }
 
 int cf_model_engine(const cf_model* m) { return m ? m->engine : CF_ERR_BAD_ARG; }
@@ -679,7 +745,7 @@ int cf_model_operand_format(const cf_model* m) {
 
 int cf_profile_enable(cf_model* m, int32_t on) {
     if (!m) { cf::set_error("cf_profile_enable: NULL model"); return CF_ERR_BAD_ARG; }
-    std::lock_guard<std::mutex> lock(m->mu);
+    std::lock_guard<std::mutex> lock(m->def.mu);
     cf::DeviceGuard guard;
     CF_TRY(guard.set(m->device));
     m->prof.reset();
@@ -692,7 +758,7 @@ const char* cf_profile_class_name(int32_t cls) { return cf::kernel_class_name(cl
 
 int cf_profile_read(cf_model* m, double* ms_out, int64_t* launches_out, int32_t n) {
     if (!m || !ms_out || !launches_out || n < cf::KC_COUNT) { cf::set_error("cf_profile_read: bad argument"); return CF_ERR_BAD_ARG; }
-    std::lock_guard<std::mutex> lock(m->mu);
+    std::lock_guard<std::mutex> lock(m->def.mu);
     cf::DeviceGuard guard;
     CF_TRY(guard.set(m->device));
     m->prof.collect();
@@ -700,21 +766,38 @@ int cf_profile_read(cf_model* m, double* ms_out, int64_t* launches_out, int32_t 
     return CF_OK;
 }
 
-int cf_model_reserve(cf_model* m, int64_t max_samples, int32_t max_reads) {
-    if (!m || max_samples < 0 || max_reads < 0) { cf::set_error("cf_model_reserve: bad argument"); return CF_ERR_BAD_ARG; }
-    std::lock_guard<std::mutex> lock(m->mu);
+static int reserve(cf_model* m, cf::Exec* x, int64_t max_samples, int32_t max_reads) {
+    std::lock_guard<std::mutex> lock(x->mu);
     cf::DeviceGuard guard;
     CF_TRY(guard.set(m->device));
     const int64_t windows = max_samples / cf::kWindow + max_reads;
     const int64_t tiles = cf::ceil_div(windows, cf::kTileWindows);
     cf::WindowTable tab;
-    CF_TRY(cf::ensure_table(m, tiles, &tab));
-    CF_TRY(m->stats.ensure(sizeof(double) * 2 * (size_t)max_reads));
-    CF_TRY(m->wide_flags.ensure(sizeof(int32_t) * (size_t)max_reads));
-    CF_TRY(m->wide_scratch.ensure(cf::k1_wide_scratch_bytes(cf::kWideSlots)));
-    if (max_reads > 0 && max_reads <= 8192) CF_TRY(m->k1_chunked.ensure(cf::k1_chunked_scratch_bytes(max_reads)));
-    CF_TRY(m->probs_internal.ensure(sizeof(float) * (size_t)max_samples));
+    CF_TRY(cf::ensure_table(x, tiles, &tab));
+    CF_TRY(x->stats.ensure(sizeof(double) * 2 * (size_t)max_reads));
+    CF_TRY(x->wide_flags.ensure(sizeof(int32_t) * (size_t)max_reads));
+    CF_TRY(x->wide_scratch.ensure(cf::k1_wide_scratch_bytes(cf::kWideSlots)));
+    if (max_reads > 0 && max_reads <= 8192) CF_TRY(x->k1_chunked.ensure(cf::k1_chunked_scratch_bytes(max_reads)));
+    CF_TRY(x->probs_internal.ensure(sizeof(float) * (size_t)max_samples));
     return CF_OK;
+}
+
+int cf_model_reserve(cf_model* m, int64_t max_samples, int32_t max_reads) {
+    if (!m || max_samples < 0 || max_reads < 0) { cf::set_error("cf_model_reserve: bad argument"); return CF_ERR_BAD_ARG; }
+    return reserve(m, &m->def, max_samples, max_reads);
+}
+
+int cf_exec_reserve(cf_exec* ex, int64_t max_samples, int32_t max_reads) {
+    if (!ex || max_samples < 0 || max_reads < 0) { cf::set_error("cf_exec_reserve: bad argument"); return CF_ERR_BAD_ARG; }
+    CF_TRY(reserve(ex->model, &ex->x, max_samples, max_reads));
+    // and the engine workspaces, the largest allocations of a call
+    cf_model* m = ex->model;
+    std::lock_guard<std::mutex> lock(ex->x.mu);
+    cf::DeviceGuard guard;
+    CF_TRY(guard.set(m->device));
+    const int64_t tiles = cf::ceil_div(max_samples / cf::kWindow + max_reads, cf::kTileWindows);
+    if (m->engine == CF_ENGINE_TCGEN05) return cf::tc_reserve(m->tc, &ex->x.tc_ws, &ex->x.simt_ws, m->hm, tiles);
+    return cf::simt_reserve(&ex->x.simt_ws, m->hm, tiles);
 }
 
 int cf_infer_windows(cf_model* m, const float* x_dev, int64_t n_windows, float* probs_dev, void* stream) {
@@ -723,20 +806,19 @@ int cf_infer_windows(cf_model* m, const float* x_dev, int64_t n_windows, float* 
         return CF_ERR_BAD_ARG;
     }
     if (n_windows == 0) return CF_OK;
-    std::lock_guard<std::mutex> lock(m->mu);
+    std::lock_guard<std::mutex> lock(m->def.mu);
     cf::DeviceGuard guard;
     CF_TRY(guard.set(m->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int64_t tiles = cf::ceil_div(n_windows, cf::kTileWindows);
     cf::WindowTable tab;
-    CF_TRY(cf::ensure_table(m, tiles, &tab));
+    CF_TRY(cf::ensure_table(&m->def, tiles, &tab));
     const int64_t slots = tiles * cf::kTileWindows;
-    CF_TRY(cf::handle_begin(m, st));
+    cf::ExecCall call(&m->def, st);
+    CF_TRY(call.begin());
     cf::dense_window_table_kernel<<<(unsigned)cf::ceil_div(slots, 256), 256, 0, st>>>(n_windows, slots, tab.src, tab.valid, tab.read);
     CF_LAUNCHED();
-    const int rc = cf::engine_forward(m, nullptr, nullptr, x_dev, tab, tiles, probs_dev, st);
-    CF_TRY(cf::handle_end(m, st));
-    return rc;
+    return cf::engine_forward(m, &m->def, &m->prof, nullptr, nullptr, x_dev, tab, tiles, probs_dev, st);
 }
 
 int cf_validate_windows(cf_model* m, const float* x_dev, const uint8_t* labels_dev, int64_t n_windows,
@@ -746,29 +828,33 @@ int cf_validate_windows(cf_model* m, const float* x_dev, const uint8_t* labels_d
         cf::set_error("cf_validate_windows: bad argument");
         return CF_ERR_BAD_ARG;
     }
-    std::lock_guard<std::mutex> lock(m->mu);
+    std::lock_guard<std::mutex> lock(m->def.mu);
     cf::DeviceGuard guard;
     CF_TRY(guard.set(m->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
+    cf::Exec* x = &m->def;
     const int64_t n = n_windows * cf::kWindow;
     const int64_t tiles = cf::ceil_div(n_windows, cf::kTileWindows);
     const int blocks = cf::k9_validation_blocks(n);
-    CF_TRY(m->val_logits.ensure(sizeof(float) * (size_t)n));
-    CF_TRY(m->val_partial.ensure(sizeof(long long) * 6 * ((size_t)blocks + 1)));
+    CF_TRY(x->val_logits.ensure(sizeof(float) * (size_t)n));
+    CF_TRY(x->val_partial.ensure(sizeof(long long) * 6 * ((size_t)blocks + 1)));
     cf::WindowTable tab;
-    CF_TRY(cf::ensure_table(m, tiles, &tab));
+    CF_TRY(cf::ensure_table(x, tiles, &tab));
     const int64_t slots = tiles * cf::kTileWindows;
-    CF_TRY(cf::handle_begin(m, st));
-    cf::dense_window_table_kernel<<<(unsigned)cf::ceil_div(slots, 256), 256, 0, st>>>(n_windows, slots, tab.src, tab.valid, tab.read);
-    CF_LAUNCHED();
-    CF_TRY(cf::engine_forward(m, nullptr, nullptr, x_dev, tab, tiles, m->val_logits.as<float>(), st, /*want_logits=*/true));
-    long long* partial = m->val_partial.as<long long>();
-    long long* result = partial + (size_t)blocks * 6;
-    CF_TRY(cf::k9_validate(m->val_logits.as<float>(), labels_dev, n, threshold, partial, result, st));
     long long host[6];
-    CF_CUDA(cudaMemcpyAsync(host, result, sizeof(host), cudaMemcpyDeviceToHost, st));
-    CF_CUDA(cudaStreamSynchronize(st));
-    CF_TRY(cf::handle_end(m, st));
+    {
+        cf::ExecCall call(x, st);
+        CF_TRY(call.begin());
+        cf::dense_window_table_kernel<<<(unsigned)cf::ceil_div(slots, 256), 256, 0, st>>>(n_windows, slots, tab.src, tab.valid, tab.read);
+        CF_LAUNCHED();
+        CF_TRY(cf::engine_forward(m, x, &m->prof, nullptr, nullptr, x_dev, tab, tiles, x->val_logits.as<float>(), st,
+                                  /*want_logits=*/true));
+        long long* partial = x->val_partial.as<long long>();
+        long long* result = partial + (size_t)blocks * 6;
+        CF_TRY(cf::k9_validate(x->val_logits.as<float>(), labels_dev, n, threshold, partial, result, st));
+        CF_CUDA(cudaMemcpyAsync(host, result, sizeof(host), cudaMemcpyDeviceToHost, st));
+        CF_CUDA(cudaStreamSynchronize(st));
+    }
     counts_out[0] = host[0];
     counts_out[1] = host[1];
     counts_out[2] = host[2] - padding_size;      // rnn_class.py:247
@@ -826,24 +912,41 @@ int cf_vote_events(int32_t device, const double* scores_dev, int64_t n_scores, c
     return CF_OK;
 }
 
+static int infer_reads_call(const char* name, cf_model* m, cf::Exec* x, cf::Profiler* prof, const int16_t* raw_dev,
+                            const int64_t* offsets_host, int32_t n_reads, float* probs_dev, int64_t* intervals_dev,
+                            int64_t* interval_offsets_dev, int64_t capacity, double threshold, int32_t min_run,
+                            int32_t ext_left, int32_t ext_right, void* stream) {
+    if (!m || n_reads < 0 || !offsets_host || !interval_offsets_dev || capacity < 0 ||
+        (n_reads > 0 && !raw_dev) || (capacity > 0 && !intervals_dev)) {
+        cf::set_error("%s: bad argument", name);
+        return CF_ERR_BAD_ARG;
+    }
+    std::lock_guard<std::mutex> lock(x->mu);
+    cf::DeviceGuard guard;
+    CF_TRY(guard.set(m->device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    cf::ExecCall call(x, st);
+    CF_TRY(call.begin());
+    return cf::infer_reads_device(m, x, prof, raw_dev, offsets_host, n_reads, probs_dev, intervals_dev,
+                                  interval_offsets_dev, capacity, threshold, min_run, ext_left, ext_right, st);
+}
+
 int cf_infer_reads(cf_model* m, const int16_t* raw_dev, const int64_t* offsets_host, int32_t n_reads,
                    float* probs_dev, int64_t* intervals_dev, int64_t* interval_offsets_dev,
                    int64_t capacity, double threshold, int32_t min_run, int32_t ext_left,
                    int32_t ext_right, void* stream) {
-    if (!m || n_reads < 0 || !offsets_host || !interval_offsets_dev || capacity < 0 ||
-        (n_reads > 0 && !raw_dev) || (capacity > 0 && !intervals_dev)) {
-        cf::set_error("cf_infer_reads: bad argument");
-        return CF_ERR_BAD_ARG;
-    }
-    std::lock_guard<std::mutex> lock(m->mu);
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(m->device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    CF_TRY(cf::handle_begin(m, st));
-    const int rc = cf::infer_reads_device(m, raw_dev, offsets_host, n_reads, probs_dev, intervals_dev,
-                                          interval_offsets_dev, capacity, threshold, min_run, ext_left, ext_right, st);
-    CF_TRY(cf::handle_end(m, st));
-    return rc;
+    return infer_reads_call("cf_infer_reads", m, m ? &m->def : nullptr, m ? &m->prof : nullptr, raw_dev, offsets_host,
+                            n_reads, probs_dev, intervals_dev, interval_offsets_dev, capacity, threshold, min_run,
+                            ext_left, ext_right, stream);
+}
+
+int cf_exec_infer_reads(cf_exec* ex, const int16_t* raw_dev, const int64_t* offsets_host, int32_t n_reads,
+                        float* probs_dev, int64_t* intervals_dev, int64_t* interval_offsets_dev,
+                        int64_t capacity, double threshold, int32_t min_run, int32_t ext_left,
+                        int32_t ext_right, void* stream) {
+    return infer_reads_call("cf_exec_infer_reads", ex ? ex->model : nullptr, ex ? &ex->x : nullptr, nullptr, raw_dev,
+                            offsets_host, n_reads, probs_dev, intervals_dev, interval_offsets_dev, capacity, threshold,
+                            min_run, ext_left, ext_right, stream);
 }
 
 int64_t cf_max_intervals(int64_t total_samples, int32_t n_reads, int32_t min_run) {
@@ -862,20 +965,21 @@ int cf_infer_reads_host(cf_model* m, const int16_t* raw_host, const int64_t* off
         cf::set_error("cf_infer_reads_host: bad argument");
         return CF_ERR_BAD_ARG;
     }
-    std::lock_guard<std::mutex> lock(m->mu);
+    std::lock_guard<std::mutex> lock(m->def.mu);
     cf::DeviceGuard guard;
     CF_TRY(guard.set(m->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
+    cf::Exec* x = &m->def;
     const int64_t base = n_reads > 0 ? offsets_host[0] : 0;
     const int64_t total = n_reads > 0 ? offsets_host[n_reads] - base : 0;
     if (total < 0) { cf::set_error("cf_infer_reads_host: offsets decrease"); return CF_ERR_BAD_ARG; }
-    CF_TRY(m->h_raw.ensure(sizeof(int16_t) * (size_t)(total > 0 ? total : 1)));
-    CF_TRY(m->h_intervals.ensure(sizeof(int64_t) * 2 * (size_t)(capacity > 0 ? capacity : 1)));
-    CF_TRY(m->h_ioff.ensure(sizeof(int64_t) * ((size_t)n_reads + 1)));
+    CF_TRY(x->h_raw.ensure(sizeof(int16_t) * (size_t)(total > 0 ? total : 1)));
+    CF_TRY(x->h_intervals.ensure(sizeof(int64_t) * 2 * (size_t)(capacity > 0 ? capacity : 1)));
+    CF_TRY(x->h_ioff.ensure(sizeof(int64_t) * ((size_t)n_reads + 1)));
     float* probs_dev = nullptr;
     if (probs_host) {
-        CF_TRY(m->h_probs.ensure(sizeof(float) * (size_t)(total > 0 ? total : 1)));
-        probs_dev = m->h_probs.as<float>();
+        CF_TRY(x->h_probs.ensure(sizeof(float) * (size_t)(total > 0 ? total : 1)));
+        probs_dev = x->h_probs.as<float>();
     }
     // offsets rebased so that raw_dev + offsets[0] is the staged copy
     std::vector<int64_t> off((size_t)n_reads + 1);
@@ -884,27 +988,30 @@ int cf_infer_reads_host(cf_model* m, const int16_t* raw_host, const int64_t* off
         cf::BatchPlan whole;                       // reject bad / empty reads before any asynchronous copy reads the caller's buffer
         CF_TRY(cf::make_plan(off.data(), n_reads, &whole));
     }
-    CF_TRY(cf::handle_begin(m, st));
-    // (Cutting the batch into groups of whole passes whose copies overlap the previous group's kernels was
-    // measured: no gain - the copy is 1.2-1.5 ms of a 75 ms step and the extra K1 / K6 sequences cost as much.)
-    if (total > 0)
-        CF_CUDA(cudaMemcpyAsync(m->h_raw.ptr, raw_host + base, sizeof(int16_t) * (size_t)total, cudaMemcpyHostToDevice, st));
-    CF_TRY(cf::infer_reads_device(m, m->h_raw.as<int16_t>(), off.data(), n_reads, probs_dev,
-                                  m->h_intervals.as<int64_t>(), m->h_ioff.as<int64_t>(), capacity, threshold,
-                                  min_run, ext_left, ext_right, st));
-    CF_CUDA(cudaMemcpyAsync(interval_offsets_host, m->h_ioff.ptr, sizeof(int64_t) * ((size_t)n_reads + 1),
-                            cudaMemcpyDeviceToHost, st));
-    CF_CUDA(cudaStreamSynchronize(st));
-    const int64_t found = interval_offsets_host[n_reads];
-    if (n_intervals_out) *n_intervals_out = found;
-    const int64_t ncopy = found < capacity ? found : capacity;
-    if (ncopy > 0)
-        CF_CUDA(cudaMemcpyAsync(intervals_host, m->h_intervals.ptr, sizeof(int64_t) * 2 * (size_t)ncopy,
+    int64_t found = 0;
+    {
+        cf::ExecCall call(x, st);
+        CF_TRY(call.begin());
+        // (Cutting the batch into groups of whole passes whose copies overlap the previous group's kernels was
+        // measured: no gain - the copy is 1.2-1.5 ms of a 75 ms step and the extra K1 / K6 sequences cost as much.)
+        if (total > 0)
+            CF_CUDA(cudaMemcpyAsync(x->h_raw.ptr, raw_host + base, sizeof(int16_t) * (size_t)total, cudaMemcpyHostToDevice, st));
+        CF_TRY(cf::infer_reads_device(m, x, &m->prof, x->h_raw.as<int16_t>(), off.data(), n_reads, probs_dev,
+                                      x->h_intervals.as<int64_t>(), x->h_ioff.as<int64_t>(), capacity, threshold,
+                                      min_run, ext_left, ext_right, st));
+        CF_CUDA(cudaMemcpyAsync(interval_offsets_host, x->h_ioff.ptr, sizeof(int64_t) * ((size_t)n_reads + 1),
                                 cudaMemcpyDeviceToHost, st));
-    if (probs_host && total > 0)
-        CF_CUDA(cudaMemcpyAsync(probs_host, probs_dev, sizeof(float) * (size_t)total, cudaMemcpyDeviceToHost, st));
-    CF_CUDA(cudaStreamSynchronize(st));
-    CF_TRY(cf::handle_end(m, st));
+        CF_CUDA(cudaStreamSynchronize(st));
+        found = interval_offsets_host[n_reads];
+        if (n_intervals_out) *n_intervals_out = found;
+        const int64_t ncopy = found < capacity ? found : capacity;
+        if (ncopy > 0)
+            CF_CUDA(cudaMemcpyAsync(intervals_host, x->h_intervals.ptr, sizeof(int64_t) * 2 * (size_t)ncopy,
+                                    cudaMemcpyDeviceToHost, st));
+        if (probs_host && total > 0)
+            CF_CUDA(cudaMemcpyAsync(probs_host, probs_dev, sizeof(float) * (size_t)total, cudaMemcpyDeviceToHost, st));
+        CF_CUDA(cudaStreamSynchronize(st));
+    }
     if (found > capacity) {
         cf::set_error("cf_infer_reads_host: %lld intervals found, capacity %lld", (long long)found, (long long)capacity);
         return CF_ERR_CAPACITY;

@@ -1,4 +1,5 @@
-// Model handle: folded / re-packed weights and per-handle workspace.
+// Model handle: folded / re-packed weights.  The engines own only what is read-only after creation; the
+// workspace a forward pass writes belongs to the caller's execution context and is passed in.
 #pragma once
 
 #include <vector>
@@ -53,9 +54,15 @@ void simt_destroy(SimtEngine* e);
 // per-read (shift, scale) or already-normalised float windows; output probabilities are
 // scattered to probs[tab.src[g] + t] for t < tab.valid[g].  With want_logits the dense layer's output
 // (rnn_class.py:178-183) is written instead of its sigmoid - the validation row needs it for the loss.
-int simt_forward(SimtEngine* e, const HostModel& hm, const int16_t* raw, const double* stats,
+// ws: the calling context's workspace, grown to the pass's needs.
+int simt_forward(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* raw, const double* stats,
                  const float* xwin, WindowTable tab, int64_t n_tiles, float* probs,
                  cudaStream_t stream, Profiler* prof, bool want_logits = false);
+
+// Grow ws to what simt_forward needs for a pass over n_tiles tiles.
+int simt_reserve(DevBuf* ws, const HostModel& hm, int64_t n_tiles);
+// Grow ws to what simt_conv_stack needs for passes of chunk_tiles tiles (the tensor-core engine's RNN-only input).
+int simt_conv_stack_reserve(DevBuf* ws, const HostModel& hm, int64_t chunk_tiles);
 
 // ---------------------------------------------------------------- tcgen05 engine
 struct TcEngine;
@@ -66,9 +73,14 @@ int tc_operand_format(const TcEngine* e);    // 0 = split bf16 (3 MMA passes), 1
 // bits != nullptr (networks with a GRU head): the head thresholds its own scores and ORs label bits into
 // bits->lwords (k6_bits_prepare) instead of writing probabilities - probs may then be nullptr.
 bool tc_can_emit_bits(const TcEngine* e);
-int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const double* stats,
+// ws: the calling context's tensor-core workspace; simt_ws: its CUDA-core workspace (RNN-only networks normalise
+// their scalar input with simt_conv_stack).  Both grow to the pass's needs.
+int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, const int16_t* raw, const double* stats,
                const float* xwin, WindowTable tab, int64_t n_tiles, float* probs,
                cudaStream_t stream, Profiler* prof, bool want_logits = false, const LabelBits* bits = nullptr);
+
+// Grow ws / simt_ws to what tc_forward needs for a pass over n_tiles tiles.
+int tc_reserve(const TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, int64_t n_tiles);
 
 int tc_selftest_f16e5(const float* a_dev, int K, int N, const float* w_host, int mode, float* out_dev, cudaStream_t stream);
 

@@ -25,7 +25,6 @@ struct SimtEngine {
     float* head_w = nullptr;
     float head_b = 0.f;
     std::vector<void*> owned;
-    DevBuf ws;
 };
 
 static float* upload(SimtEngine* e, const std::vector<float>& v) {
@@ -69,7 +68,6 @@ SimtEngine* simt_create(const HostModel& hm) {
 void simt_destroy(SimtEngine* e) {
     if (!e) return;
     for (void* p : e->owned) cudaFree(p);
-    e->ws.release();
     delete e;
 }
 
@@ -271,15 +269,15 @@ __global__ void simt_head_kernel(const float* __restrict__ y, const float* __res
 // Carve the workspace for passes of at most `chunk_tiles` tiles.
 struct SimtBufs { float *x, *ca, *cb, *csc, *cout, *xproj, *y0, *y1; };
 
-static int simt_prepare(SimtEngine* e, const HostModel& hm, int64_t chunk_tiles, bool with_rnn, SimtBufs* b) {
+static int simt_prepare(DevBuf* ws, const HostModel& hm, int64_t chunk_tiles, bool with_rnn, SimtBufs* b) {
     const int64_t rows = chunk_tiles * kWindow * kTileWindows;
     const int C = hm.conv_channels(), H = hm.desc.layer_size;
     const bool res = hm.n_res() > 0, rnn = with_rnn && hm.n_rnn() > 0;
     size_t fl = (size_t)rows;
     if (res) fl += (size_t)rows * C * 4;
     if (rnn) fl += (size_t)rows * (6 * H + 2 * 2 * H);
-    CF_TRY(e->ws.ensure(fl * sizeof(float) + 1024));
-    b->x = e->ws.as<float>();
+    CF_TRY(ws->ensure(fl * sizeof(float) + 1024));
+    b->x = ws->as<float>();
     b->ca = b->x + rows;
     b->cb = b->ca + (res ? rows * C : 0);
     b->csc = b->cb + (res ? rows * C : 0);
@@ -323,21 +321,33 @@ static int conv_stack(SimtEngine* e, const HostModel& hm, const SimtBufs& b, con
     return CF_OK;
 }
 
-int simt_conv_stack(SimtEngine* e, const HostModel& hm, const int16_t* raw, const double* stats, const float* xwin,
-                    WindowTable tab, int64_t tile0, int64_t tiles, int64_t chunk_tiles, const float** feat,
-                    cudaStream_t stream, Profiler* prof) {
+int simt_conv_stack(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* raw, const double* stats,
+                    const float* xwin, WindowTable tab, int64_t tile0, int64_t tiles, int64_t chunk_tiles,
+                    const float** feat, cudaStream_t stream, Profiler* prof) {
     SimtBufs b;
-    CF_TRY(simt_prepare(e, hm, chunk_tiles, false, &b));
+    CF_TRY(simt_prepare(ws, hm, chunk_tiles, false, &b));
     return conv_stack(e, hm, b, raw, stats, xwin, tab, tile0, tiles, feat, stream, prof);
 }
 
-int simt_forward(SimtEngine* e, const HostModel& hm, const int16_t* raw, const double* stats,
+int simt_reserve(DevBuf* ws, const HostModel& hm, int64_t n_tiles) {
+    if (n_tiles <= 0) return CF_OK;
+    SimtBufs b;
+    return simt_prepare(ws, hm, n_tiles < kSimtChunkTiles ? n_tiles : kSimtChunkTiles, true, &b);
+}
+
+int simt_conv_stack_reserve(DevBuf* ws, const HostModel& hm, int64_t chunk_tiles) {
+    if (chunk_tiles <= 0) return CF_OK;
+    SimtBufs b;
+    return simt_prepare(ws, hm, chunk_tiles, false, &b);
+}
+
+int simt_forward(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* raw, const double* stats,
                  const float* xwin, WindowTable tab, int64_t n_tiles, float* probs,
                  cudaStream_t stream, Profiler* prof, bool want_logits) {
     if (n_tiles <= 0) return CF_OK;
     const int64_t chunk = n_tiles < kSimtChunkTiles ? n_tiles : kSimtChunkTiles;
     SimtBufs b;
-    CF_TRY(simt_prepare(e, hm, chunk, true, &b));
+    CF_TRY(simt_prepare(ws, hm, chunk, true, &b));
     const int H = hm.desc.layer_size;
     for (int64_t tile0 = 0; tile0 < n_tiles; tile0 += kSimtChunkTiles) {
         const int64_t tiles = (n_tiles - tile0) < kSimtChunkTiles ? (n_tiles - tile0) : kSimtChunkTiles;

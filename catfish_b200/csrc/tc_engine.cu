@@ -118,9 +118,7 @@ struct TcEngine {
     float* head_w = nullptr;          // [128]
     float head_b = 0.f;
     std::vector<void*> owned;
-    DevBuf ws;
     int n_sms = 148;
-    bool attr_done = false;
 #ifdef CF_TRACE_PROBES
     bool trace_done = false;
     const char* trace_path = nullptr; // CF_TC_TRACE=<file>: in-kernel timeline of one TK4G launch (debug; results unaffected)
@@ -201,7 +199,10 @@ static T* tc_upload(TcEngine* e, const std::vector<T>& v) {
     return d;
 }
 
+static int tc_set_attributes();
+
 TcEngine* tc_create(const HostModel& narrow) {
+    if (tc_set_attributes() != CF_OK) return nullptr;
     TcEngine* e = new TcEngine();
     int dev = 0;
     cudaGetDevice(&dev);
@@ -315,7 +316,6 @@ void tc_destroy(TcEngine* e) {
     if (!e) return;
     simt_destroy(e->simt);
     for (void* p : e->owned) cudaFree(p);
-    e->ws.release();
     delete e;
 }
 
@@ -1667,9 +1667,9 @@ tc_head_conv_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict
 }
 
 // ====================================================================== forward
-int simt_conv_stack(SimtEngine* e, const HostModel& hm, const int16_t* raw, const double* stats, const float* xwin,
-                    WindowTable tab, int64_t tile0, int64_t tiles, int64_t chunk_tiles, const float** feat,
-                    cudaStream_t stream, Profiler* prof);
+int simt_conv_stack(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* raw, const double* stats,
+                    const float* xwin, WindowTable tab, int64_t tile0, int64_t tiles, int64_t chunk_tiles,
+                    const float** feat, cudaStream_t stream, Profiler* prof);
 
 static size_t tc_workspace_bytes(int64_t tiles) {
     const size_t blocks = (size_t)tiles * kWindow;
@@ -1680,27 +1680,49 @@ static size_t tc_workspace_bytes(int64_t tiles) {
     return b + 4096;
 }
 
-int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const double* stats, const float* xwin,
-               WindowTable tab, int64_t n_tiles, float* probs, cudaStream_t stream, Profiler* prof, bool want_logits,
-               const LabelBits* bits) {
+int tc_reserve(const TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, int64_t n_tiles) {
+    if (n_tiles <= 0) return CF_OK;
+    const int64_t chunk = n_tiles < kTcChunkTiles ? n_tiles : kTcChunkTiles;
+    CF_TRY(ws->ensure(tc_workspace_bytes(chunk)));
+    if (!e->conv_params) CF_TRY(simt_conv_stack_reserve(simt_ws, hm, chunk));
+    return CF_OK;
+}
+
+// Every tensor-core kernel allocates all 512 TMEM columns of its SM.  Calls on different execution contexts may
+// run kernels at the same time, so a second TMEM CTA must never be placed on an SM that already holds one (its
+// allocation would wait for the first CTA to finish): each such kernel's dynamic shared memory is more than half
+// of an SM's 228 KiB.
+constexpr uint32_t kSmemPerSm = 228 * 1024;
+static_assert(GruF2Cfg<128>::kSmem > kSmemPerSm / 2, "two tc_gru_fused2_kernel<128> CTAs could share an SM's TMEM");
+static_assert(GruF2Cfg<32>::kSmem > kSmemPerSm / 2, "two tc_gru_fused2_kernel<32> CTAs could share an SM's TMEM");
+static_assert(GruF2Cfg<1>::kSmem > kSmemPerSm / 2, "two tc_gru_fused2_kernel<1> CTAs could share an SM's TMEM");
+static_assert(kConv4Smem > kSmemPerSm / 2, "two tc_conv4_kernel CTAs could share an SM's TMEM");
+static_assert(kBlockSmem > kSmemPerSm / 2, "two tc_conv_block_kernel CTAs could share an SM's TMEM");
+static_assert(kConvSmem > kSmemPerSm / 2, "two tc_conv2_kernel CTAs could share an SM's TMEM");
+
+// The opt-in to more than 48 KB of dynamic shared memory, once per engine (called from tc_create).
+static int tc_set_attributes() {
+    CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<1, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<1>::kSmem));
+    CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<1, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<1>::kSmem));
+    CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<32, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<32>::kSmem));
+    CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<32, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<32>::kSmem));
+    CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<128, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<128>::kSmem));
+    CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<128, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<128>::kSmem));
+    CF_CUDA(cudaFuncSetAttribute(tc_conv2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmem));
+    CF_CUDA(cudaFuncSetAttribute(tc_conv4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kConv4Smem));
+    CF_CUDA(cudaFuncSetAttribute(tc_conv_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBlockSmem));
+    return CF_OK;
+}
+
+int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, const int16_t* raw, const double* stats,
+               const float* xwin, WindowTable tab, int64_t n_tiles, float* probs, cudaStream_t stream, Profiler* prof,
+               bool want_logits, const LabelBits* bits) {
     if (n_tiles <= 0) return CF_OK;
     if (bits && (e->layers.empty() || want_logits)) { set_error("label-bit output needs a GRU head"); return CF_ERR_BAD_ARG; }
-    if (!e->attr_done) {
-        CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<1, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<1>::kSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<1, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<1>::kSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<32, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<32>::kSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<32, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<32>::kSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<128, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<128>::kSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_gru_fused2_kernel<128, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GruF2Cfg<128>::kSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_conv2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmem));
-        CF_CUDA(cudaFuncSetAttribute(tc_conv4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kConv4Smem));
-        CF_CUDA(cudaFuncSetAttribute(tc_conv_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBlockSmem));
-        e->attr_done = true;
-    }
     const int64_t chunk = n_tiles < kTcChunkTiles ? n_tiles : kTcChunkTiles;
-    CF_TRY(e->ws.ensure(tc_workspace_bytes(chunk)));
+    CF_TRY(ws->ensure(tc_workspace_bytes(chunk)));
     const size_t blocks_max = (size_t)chunk * kWindow;
-    uint8_t* p = static_cast<uint8_t*>(e->ws.ptr);
+    uint8_t* p = static_cast<uint8_t*>(ws->ptr);
     __nv_bfloat16* a0 = reinterpret_cast<__nv_bfloat16*>(p);
     p += blocks_max * 128 * kC * 2 * 2;
     __nv_bfloat16* ybuf[2];
@@ -1740,7 +1762,7 @@ int tc_forward(TcEngine* e, const HostModel& hm, const int16_t* raw, const doubl
                 a_in = out;
             }
         } else {
-            CF_TRY(simt_conv_stack(e->simt, hm, raw, stats, xwin, tab, tile0, tiles, chunk, &feat, stream, prof));
+            CF_TRY(simt_conv_stack(e->simt, simt_ws, hm, raw, stats, xwin, tab, tile0, tiles, chunk, &feat, stream, prof));
         }
         for (int l = 0; l < n_layers; ++l) {
             const TcLayer& L = e->layers[l];

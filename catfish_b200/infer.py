@@ -9,6 +9,7 @@ reference (catfish/infer.py)  here                        C-ABI entry
 infer_class_from_signal :12   infer_class_from_signal     cf_infer_reads_host
 (array-level twins)           infer_class_from_raw,       cf_infer_reads_host
                               infer_reads
+(the CLI's per-file loop)     infer_stream                cf_exec_infer_reads
 process_signal :77            process_signal (h5py)       cf_normalize_reads
 normalize_raw_signal :96      normalize_raw_signal        cf_normalize_reads
 reshape_input :108            reshape_input               (pure reshape, host)
@@ -20,9 +21,12 @@ correct_short :174            correct_short               cf_correct_short
 PyTorch tensors are used only to hold device buffers and to name the stream.
 """
 
+import collections
 import collections.abc
 import ctypes
 import os
+import threading
+import time
 
 import numpy as np
 
@@ -77,6 +81,7 @@ class IntervalList(collections.abc.Sequence):
 
 
 _POOL = None
+_POOL_LOCK = threading.Lock()
 
 
 def _concat_into(stage, arrays, offsets):
@@ -89,9 +94,10 @@ def _concat_into(stage, arrays, offsets):
     if total < (1 << 23) or len(arrays) < 2 * workers or workers < 2:
         np.concatenate(arrays, out=stage)
         return
-    if _POOL is None:
-        import concurrent.futures
-        _POOL = concurrent.futures.ThreadPoolExecutor(max_workers=workers, thread_name_prefix="catfish-stage")
+    with _POOL_LOCK:
+        if _POOL is None:
+            import concurrent.futures
+            _POOL = concurrent.futures.ThreadPoolExecutor(max_workers=workers, thread_name_prefix="catfish-stage")
     cuts = np.searchsorted(offsets, np.linspace(0, total, workers + 1)[1:-1]).tolist()
     bounds = [0] + cuts + [len(arrays)]
     jobs = []
@@ -273,6 +279,183 @@ def _infer_reads_pipelined(arrays, offsets, model, threshold, min_run, ext_left,
         parts = [iv_pin[int(cap_off[g]):int(cap_off[g]) + n_g] for g, n_g in enumerate(found) if n_g]
         intervals = np.concatenate(parts) if parts else np.zeros((0, 2), np.int64)
     return intervals, ioff
+
+
+_STREAM_DEPTH = 2                       # groups in flight in infer_stream
+_STREAM_GROUP_SAMPLES = 2_600_000       # samples per group of infer_stream: a quarter pass (profiles/r3_stream.txt)
+
+
+def infer_stream(reads, model, threshold=0.5, min_run=15, extension_left=11, extension_right=16, window_size=35,
+                 return_scores=False, group_samples=None, max_wait_s=None, depth=_STREAM_DEPTH):
+    """Streaming ``infer_reads``: yields ``(intervals, len_read)`` - plus the float32 scores with ``return_scores`` -
+    for every read of the iterable ``reads``, in input order, with the results ``infer_reads`` gives for the whole list.
+
+    Reads are pulled lazily and grouped: consecutive reads until the group holds ``group_samples`` samples (default:
+    a quarter of an engine pass), or fewer when the input ends or when ``max_wait_s`` seconds have passed since the group's first
+    read was taken (checked as each read arrives).  Up to ``depth`` groups run at once, each on its own execution
+    context of the model (``cf_exec``), CUDA stream, pinned staging and device buffers, so that small groups overlap
+    on the device instead of running one after another.  At most ``depth + 1`` groups of reads are pulled and not
+    yet yielded.
+
+    A read that ``infer_reads`` would reject (empty: ``IndexError``; not integer DAC values: ``ValueError``), or an
+    exception raised by ``reads`` itself, ends the stream the way the reference's one-file-at-a-time loop meets it:
+    every earlier read's result is yielded first, then the exception is raised.  The stream owns all of its buffers
+    and contexts and releases them when it is exhausted, closed or collected; streams on one model are independent
+    of each other and of ``infer_reads``."""
+    if window_size != model.window:
+        raise ValueError("window_size must equal the model's window (%d)" % model.window)
+    depth = int(depth)
+    if depth < 1:
+        raise ValueError("depth must be at least 1")
+    group_samples = _STREAM_GROUP_SAMPLES if group_samples is None else int(group_samples)
+    if group_samples < 1:
+        raise ValueError("group_samples must be at least 1")
+    params = (float(threshold), int(min_run), int(extension_left), int(extension_right))
+    return _stream(iter(reads), model, params, bool(return_scores), group_samples, max_wait_s, depth)
+
+
+class _StreamSlot(object):
+    """One group in flight of ``infer_stream``: an execution context of the model, a CUDA stream, and pinned / device
+    buffers that grow to the largest group the slot has run."""
+
+    def __init__(self, torch, lib, model):
+        self.torch, self.lib, self.dev = torch, lib, int(model.device)
+        self.ex = None
+        ex = ctypes.c_void_p()
+        _cabi.check(lib.cf_exec_create(model.handle, ctypes.byref(ex)))
+        self.ex = ex
+        with torch.cuda.device(self.dev):
+            self.stream = torch.cuda.Stream()
+            self.event = torch.cuda.Event()
+        self.buf = {}
+        self.group = None
+
+    def _ensure(self, name, n, dtype, pinned=False):
+        t = self.buf.get(name)
+        if t is None or t.numel() < n:
+            n = max(n + n // 4, 1024)
+            self.buf[name] = None
+            t = self.torch.empty(n, dtype=dtype, pin_memory=pinned) if pinned else \
+                self.torch.empty(n, dtype=dtype, device="cuda:%d" % self.dev)
+            self.buf[name] = t
+        return t
+
+    def submit(self, arrays, params, return_scores):
+        """Stage, copy and enqueue one group on this slot's stream (returns without waiting for the device)."""
+        torch = self.torch
+        threshold, min_run, ext_left, ext_right = params
+        n = len(arrays)
+        offsets = np.zeros(n + 1, np.int64)
+        np.cumsum([a.size for a in arrays], out=offsets[1:])
+        total = int(offsets[-1])
+        cap = int(self.lib.cf_max_intervals(total, n, min_run))
+        with torch.cuda.device(self.dev), torch.cuda.stream(self.stream):
+            stage = self._ensure("stage", total, torch.int16, pinned=True)
+            raw = self._ensure("raw", total, torch.int16)
+            iv = self._ensure("iv", 2 * cap, torch.int64)
+            ioff = self._ensure("ioff", n + 1, torch.int64)
+            ioff_pin = self._ensure("ioff_pin", n + 1, torch.int64, pinned=True)
+            probs = self._ensure("probs", total, torch.float32) if return_scores else None
+            probs_pin = self._ensure("probs_pin", total, torch.float32, pinned=True) if return_scores else None
+            _concat_into(stage.numpy()[:total], arrays, offsets)
+            raw[:total].copy_(stage[:total], non_blocking=True)
+            _cabi.check(self.lib.cf_exec_infer_reads(
+                self.ex, raw.data_ptr(), _offsets_ptr(offsets), n, probs.data_ptr() if return_scores else None,
+                iv.data_ptr(), ioff.data_ptr(), cap, threshold, min_run, ext_left, ext_right, self.stream.cuda_stream))
+            ioff_pin[:n + 1].copy_(ioff[:n + 1], non_blocking=True)
+            if return_scores:
+                probs_pin[:total].copy_(probs[:total], non_blocking=True)
+            self.event.record(self.stream)
+        self.group = (offsets, cap, return_scores)
+
+    def done(self):
+        return self.event.query()
+
+    def results(self):
+        """Wait for the group and return its per-read results, in order; the slot is then free."""
+        torch = self.torch
+        offsets, cap, return_scores = self.group
+        self.group = None
+        n, total = len(offsets) - 1, int(offsets[-1])
+        self.event.synchronize()
+        ioff = self.buf["ioff_pin"].numpy()[:n + 1].copy()
+        found = int(ioff[-1])
+        if found > cap:
+            raise _cabi.CatfishError("interval capacity exceeded (%d > %d)" % (found, cap))
+        intervals = np.zeros((0, 2), np.int64)
+        if found:
+            iv_pin = self._ensure("iv_pin", 2 * found, torch.int64, pinned=True)
+            with torch.cuda.device(self.dev), torch.cuda.stream(self.stream):
+                iv_pin[:2 * found].copy_(self.buf["iv"][:2 * found], non_blocking=True)
+            self.stream.synchronize()
+            intervals = iv_pin.numpy()[:2 * found].reshape(found, 2).copy()
+        bounds, lengths = ioff.tolist(), np.diff(offsets).tolist()
+        hps = [IntervalList(intervals[bounds[r]:bounds[r + 1]]) for r in range(n)]
+        if not return_scores:
+            return list(zip(hps, lengths))
+        scores = self.buf["probs_pin"].numpy()[:total].copy()
+        return [(hps[r], lengths[r], scores[int(offsets[r]):int(offsets[r + 1])]) for r in range(n)]
+
+    def close(self):
+        if self.ex is not None:
+            self.stream.synchronize()           # copies enqueued after the context's own work
+            self.lib.cf_exec_destroy(self.ex)
+            self.ex = None
+        self.buf.clear()
+
+
+def _stream(it, model, params, return_scores, group_samples, max_wait_s, depth):
+    torch = _torch()
+    lib = _cabi.load_library()
+    slots, idle, inflight = [], [], collections.deque()      # inflight: slots in input order
+
+    def retire():
+        s = inflight.popleft()
+        out = s.results()
+        idle.append(s)
+        return out
+
+    def launch(group):
+        if len(inflight) == depth:                           # bounded read-ahead: the oldest group goes out first
+            yield from retire()
+        if not idle:
+            slots.append(_StreamSlot(torch, lib, model))
+            idle.append(slots[-1])
+        s = idle.pop()
+        s.submit(group, params, return_scores)
+        inflight.append(s)
+
+    error = None
+    try:
+        group, n_samples, t_first = [], 0, 0.0
+        while True:
+            while inflight and inflight[0].done():             # finished groups go out as soon as they are found
+                yield from retire()
+            try:
+                a = _as_int16(next(it))
+                if a.size == 0:
+                    raise IndexError("list index out of range")  # infer.py:184 on an empty read
+            except StopIteration:
+                break
+            except Exception as e:                             # earlier reads' results first, then this
+                error = e
+                break
+            if not group:
+                t_first = time.monotonic()
+            group.append(a)
+            n_samples += a.size
+            if n_samples >= group_samples or (max_wait_s is not None and time.monotonic() - t_first >= max_wait_s):
+                yield from launch(group)
+                group, n_samples = [], 0
+        if group:
+            yield from launch(group)
+        while inflight:
+            yield from retire()
+    finally:
+        for s in slots:
+            s.close()
+    if error is not None:
+        raise error
 
 
 def infer_concatenated(raw, offsets, model, threshold=0.5, min_run=15, extension_left=11,

@@ -140,6 +140,40 @@ int cf_infer_reads_host(cf_model* model, const int16_t* raw_host, const int64_t*
                         int32_t min_run, int32_t ext_left, int32_t ext_right,
                         int64_t* n_intervals_out, void* stream);
 
+/*
+ * Execution contexts (no reference counterpart): concurrent inference on one model.
+ *
+ * A model handle holds the weights, which no call changes, and one default context: the scratch
+ * buffers, workspaces and completion event that every cf_model_* / cf_infer_* / cf_validate_* call
+ * above uses.  Calls on the default context are serialised on the device, whatever their streams.
+ * A cf_exec is one more such context of the same model, with buffers of its own:
+ *   - calls on one context are serialised on the device as calls on the handle are (each waits for
+ *     the previous call's work on that context, on any stream); they may come from any thread, one
+ *     at a time (a context holds a mutex for the duration of a call);
+ *   - calls on different contexts of one model, and calls on the default context, may overlap on
+ *     the device when they are enqueued on different streams;
+ *   - a context's buffers and engine workspaces grow to the largest batch it has run
+ *     (cf_exec_reserve pre-sizes all of them) and are freed by cf_exec_destroy;
+ *   - a context holds a reference on its model: cf_model_destroy while contexts are alive releases
+ *     the handle's own buffers, and the weights are freed when the last context is destroyed;
+ *   - context calls are not timed by cf_profile_* (which covers the default context only).
+ * The caller's current device is restored by every call.
+ */
+typedef struct cf_exec cf_exec;
+/* A new context on the model's device (allocates nothing until its first call). */
+int cf_exec_create(cf_model* model, cf_exec** out);
+/* Waits for the context's last work, then frees its buffers (and the model, if it was the last reference). */
+void cf_exec_destroy(cf_exec* ex);
+/* Pre-size one context's buffers for calls of at most max_samples samples / max_reads reads: what
+ * cf_model_reserve sizes, and also the engine workspaces (tensor-core engine: up to ~12.6 GB at a
+ * full pass of 2368 tiles), so that such calls allocate nothing. */
+int cf_exec_reserve(cf_exec* ex, int64_t max_samples, int32_t max_reads);
+/* cf_infer_reads on a context: same arguments after the model, same semantics and outputs; asynchronous. */
+int cf_exec_infer_reads(cf_exec* ex, const int16_t* raw_dev, const int64_t* offsets_host,
+                        int32_t n_reads, float* probs_dev, int64_t* intervals_dev,
+                        int64_t* interval_offsets_dev, int64_t capacity, double threshold,
+                        int32_t min_run, int32_t ext_left, int32_t ext_right, void* stream);
+
 /* Upper bound on the number of intervals cf_infer_reads can emit. */
 int64_t cf_max_intervals(int64_t total_samples, int32_t n_reads, int32_t min_run);
 
