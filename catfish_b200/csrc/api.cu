@@ -4,6 +4,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 
@@ -28,7 +29,7 @@ void set_error(const char* fmt, ...) {
 
 int DevBuf::ensure(size_t want) {
     if (want <= bytes) return CF_OK;
-    if (ptr) { cudaFree(ptr); ptr = nullptr; bytes = 0; }
+    { DevBuf old(std::move(*this)); }      // free the smaller allocation before making the larger one
     const size_t grow = want + want / 8 + 256;
     cudaError_t e = cudaMalloc(&ptr, grow);
     if (e != cudaSuccess) {
@@ -66,17 +67,14 @@ void Profiler::reset() {
     collect();
     for (int i = 0; i < KC_COUNT; ++i) { ms[i] = 0; launches[i] = 0; }
 }
-void Profiler::release() {
+Profiler::~Profiler() {
     collect();
     for (cudaEvent_t e : pool) cudaEventDestroy(e);
-    pool.clear();
 }
-
-void DevBuf::release() { if (ptr) cudaFree(ptr); ptr = nullptr; bytes = 0; }
 
 int HostBuf::ensure(size_t want) {
     if (want <= bytes) return CF_OK;
-    if (ptr) { cudaFreeHost(ptr); ptr = nullptr; bytes = 0; }
+    { HostBuf old(std::move(*this)); }     // free the smaller allocation before making the larger one
     const size_t grow = want + want / 8 + 256;
     cudaError_t e = cudaMallocHost(&ptr, grow);
     if (e != cudaSuccess) {
@@ -88,7 +86,6 @@ int HostBuf::ensure(size_t want) {
     bytes = grow;
     return CF_OK;
 }
-void HostBuf::release() { if (ptr) cudaFreeHost(ptr); ptr = nullptr; bytes = 0; }
 
 // ---------------------------------------------------------------- weights
 static int check_desc(const cf_model_desc& d) {
@@ -239,11 +236,12 @@ namespace cf {
 
 // Everything an inference call writes.  The model (weights, engine, operand format) is read-only after
 // cf_model_create; calls on different contexts of one model share nothing else and may overlap on the device.
+// Its members free themselves; destroy it with the model's device current.
 struct Exec {
     HostBuf pin_plan;                // offsets + win_off staging
-    cudaEvent_t plan_copied = nullptr;
+    Event plan_copied;
     HostBuf pin_chunks;              // K1 chunk-table staging
-    cudaEvent_t chunks_copied = nullptr;
+    Event chunks_copied;
     DevBuf plan_dev;                 // offsets[R+1] | win_off[R+1]
     DevBuf stats, wide_flags, wide_scratch, k1_chunked, k1_chunk_tab;
     DevBuf tab_src, tab_valid, tab_read;
@@ -252,30 +250,12 @@ struct Exec {
     IntervalScratch k6;
     // host-buffer entry point
     DevBuf h_raw, h_intervals, h_ioff, h_probs;
-    HostBuf pin_io;
     // engine workspaces: the tensor-core pass, and the CUDA-core pass (the tensor-core engine uses it for the
     // scalar input of RNN-only networks)
     DevBuf tc_ws, simt_ws;
-    cudaEvent_t last_done = nullptr; // end of the previous asynchronous call on this context (ExecCall)
+    Profiler prof;                   // cf_profile_*: switched on for the model's default context only
+    Event last_done;                 // end of the previous asynchronous call on this context (CallScope)
     std::mutex mu;
-
-    void release() {
-        pin_plan.release(); plan_dev.release(); stats.release(); wide_flags.release();
-        wide_scratch.release(); k1_chunked.release(); k1_chunk_tab.release(); tab_src.release(); tab_valid.release(); tab_read.release();
-        probs_internal.release();
-        val_logits.release(); val_partial.release();
-        k6.bits.release(); k6.block_cnt.release(); k6.read_cnt.release(); k6.misc.release();
-        h_raw.release(); h_intervals.release(); h_ioff.release(); h_probs.release();
-        pin_io.release();
-        tc_ws.release(); simt_ws.release();
-        if (plan_copied) cudaEventDestroy(plan_copied);
-        plan_copied = nullptr;
-        pin_chunks.release();
-        if (chunks_copied) cudaEventDestroy(chunks_copied);
-        chunks_copied = nullptr;
-        if (last_done) cudaEventDestroy(last_done);
-        last_done = nullptr;
-    }
 };
 
 }  // namespace cf
@@ -285,10 +265,10 @@ struct cf_model {
     cf::HostModel hm;
     int device = 0;
     int engine = CF_ENGINE_SIMT;
-    cf::SimtEngine* simt = nullptr;
-    cf::TcEngine* tc = nullptr;
-    cf::Exec def;                    // the default context of every cf_model_* / cf_infer_* / cf_validate_* call
-    cf::Profiler prof;               // cf_profile_*: timing of the default context's calls
+    cf::SimtEnginePtr simt;
+    cf::TcEnginePtr tc;
+    // the default context of every cf_model_* / cf_infer_* / cf_validate_* call; cf_model_destroy frees it
+    std::unique_ptr<cf::Exec> def = std::make_unique<cf::Exec>();
     std::atomic<int> refs{1};        // the handle itself + one per live cf_exec
 };
 
@@ -334,33 +314,44 @@ int DeviceGuard::set(int device) {
     return CF_OK;
 }
 
-// One context = one set of scratch buffers: a call on stream B must not start while the previous call's
-// kernels (possibly on stream A) still use them.  Every asynchronous call waits on the event of the previous
-// call on its context first (a no-op on the same stream) and records it again when it returns - on every
-// path, so that a call that fails after enqueueing work still orders the next call after that work.
-struct ExecCall {
+// The scope of one call on a context.  It holds the context's mutex and makes the model's device current.  A call
+// that enqueues work also orders it on the device: one context = one set of scratch buffers, so a call on stream B
+// must not start while the previous call's kernels (possibly on stream A) still use them.  Such a call waits on
+// the event of the previous call on its context (a no-op on the same stream) and records it again when the scope
+// ends - on every path, so that a call that fails after enqueueing work still orders the next call after that work.
+// The destructor records the event while the model's device is current; the members then restore the caller's
+// device and only after that release the mutex.
+struct CallScope {
+    std::lock_guard<std::mutex> lock;
+    DeviceGuard device;
     Exec* x;
-    cudaStream_t st;
-    bool armed = false;
-    ExecCall(Exec* ex, cudaStream_t stream) : x(ex), st(stream) {}
-    int begin() {
-        if (!x->last_done) CF_CUDA(cudaEventCreateWithFlags(&x->last_done, cudaEventDisableTiming));
-        armed = true;
-        CF_CUDA(cudaStreamWaitEvent(st, x->last_done, 0));
-        return CF_OK;
+    cudaStream_t st = nullptr;
+    bool ordered = false;
+    explicit CallScope(Exec* ex) : lock(ex->mu), x(ex) {}
+    ~CallScope() {
+        if (ordered && cudaEventRecord(x->last_done.ev, st) != cudaSuccess) cudaGetLastError();
     }
-    ~ExecCall() {
-        if (armed && cudaEventRecord(x->last_done, st) != cudaSuccess) cudaGetLastError();
+    // Selects the model's device (reserve, profiling).
+    int enter(int dev) { return device.set(dev); }
+    // Also orders the call's work on `stream` after the previous call on this context.
+    int enter(int dev, cudaStream_t stream) {
+        CF_TRY(device.set(dev));
+        CF_TRY(x->last_done.create());
+        st = stream;
+        ordered = true;
+        CF_CUDA(cudaStreamWaitEvent(st, x->last_done.ev, 0));
+        return CF_OK;
     }
 };
 
-static int engine_forward(cf_model* m, Exec* x, Profiler* prof, const int16_t* raw, const double* stats,
-                          const float* xwin, WindowTable tab, int64_t n_tiles, float* probs, cudaStream_t stream,
+static int engine_forward(cf_model* m, Exec* x, const int16_t* raw, const double* stats, const float* xwin,
+                          WindowTable tab, int64_t n_tiles, float* probs, cudaStream_t stream,
                           bool want_logits = false, const LabelBits* bits = nullptr) {
     if (m->engine == CF_ENGINE_TCGEN05)
-        return tc_forward(m->tc, &x->tc_ws, &x->simt_ws, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream, prof,
-                          want_logits, bits);
-    return simt_forward(m->simt, &x->simt_ws, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream, prof, want_logits);
+        return tc_forward(m->tc.get(), &x->tc_ws, &x->simt_ws, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream,
+                          &x->prof, want_logits, bits);
+    return simt_forward(m->simt.get(), &x->simt_ws, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream, &x->prof,
+                        want_logits);
 }
 
 // Validate offsets and lay out the windows of every read (infer.py:32-43).
@@ -396,15 +387,14 @@ static int make_plan(const int64_t* offsets, int32_t n_reads, BatchPlan* p) {
 static int upload_plan(Exec* x, const int64_t* offsets, const BatchPlan& p, cudaStream_t stream,
                        const int64_t** offsets_dev, const int64_t** win_off_dev) {
     const size_t n = (size_t)p.n_reads + 1;
-    if (x->plan_copied) CF_CUDA(cudaEventSynchronize(x->plan_copied));   // staging still in flight?
+    CF_TRY(x->plan_copied.sync());                  // staging still in flight?
     CF_TRY(x->pin_plan.ensure(2 * n * sizeof(int64_t)));
     CF_TRY(x->plan_dev.ensure(2 * n * sizeof(int64_t)));
     int64_t* st = x->pin_plan.as<int64_t>();
     for (size_t i = 0; i < n; ++i) st[i] = offsets[i] - offsets[0];
     memcpy(st + n, p.win_off.data(), n * sizeof(int64_t));
     CF_CUDA(cudaMemcpyAsync(x->plan_dev.ptr, st, 2 * n * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
-    if (!x->plan_copied) CF_CUDA(cudaEventCreateWithFlags(&x->plan_copied, cudaEventDisableTiming));
-    CF_CUDA(cudaEventRecord(x->plan_copied, stream));
+    CF_TRY(x->plan_copied.record(stream));
     *offsets_dev = x->plan_dev.as<int64_t>();
     *win_off_dev = x->plan_dev.as<int64_t>() + n;
     return CF_OK;
@@ -414,17 +404,25 @@ static int upload_plan(Exec* x, const int64_t* offsets, const BatchPlan& p, cuda
 struct StatsScratch {
     DevBuf* flags; DevBuf* wide; DevBuf* chunked; DevBuf* chunk_tab;
     HostBuf* pinned = nullptr;        // optional pinned staging for the chunk table (keeps the call asynchronous)
-    cudaEvent_t* staged = nullptr;    // recorded after the staging copy; waited on before the buffer is reused
+    Event* staged = nullptr;          // recorded after the staging copy; waited on before the buffer is reused
 };
+// Whether a call of n_reads reads may take the chunked path, which needs k1_chunked_scratch_bytes(n_reads);
+// stats_use_chunks decides from the read lengths.
+static bool stats_may_use_chunks(int32_t n_reads) { return n_reads > 0 && n_reads <= 8192; }
 static bool stats_use_chunks(const int64_t* offsets, int32_t n_reads) {
+    if (!stats_may_use_chunks(n_reads)) return false;
     const int64_t total = offsets[n_reads] - offsets[0];
-    return n_reads <= 8192 && (total / n_reads >= 2 * kK1ChunkSamples || n_reads < 2 * 148);
+    return total / n_reads >= 2 * kK1ChunkSamples || n_reads < 2 * 148;
 }
 static int compute_read_stats(const int16_t* raw0, const int64_t* offsets_host, const int64_t* offsets_dev,
-                              int32_t n_reads, double* stats, StatsScratch sc, cudaStream_t stream) {
+                              int32_t n_reads, double* stats, StatsScratch sc, cudaStream_t stream,
+                              Profiler* prof = nullptr) {
+    const bool chunks = stats_use_chunks(offsets_host, n_reads);
     CF_TRY(sc.flags->ensure(sizeof(int32_t) * (size_t)n_reads));
     CF_TRY(sc.wide->ensure(k1_wide_scratch_bytes(kWideSlots)));
-    if (!stats_use_chunks(offsets_host, n_reads))
+    if (chunks) CF_TRY(sc.chunked->ensure(k1_chunked_scratch_bytes(n_reads)));   // allocate before the timed bracket
+    ProfScope ps(prof, KC_K1_STATS, stream, chunks ? 4 : 2);
+    if (!chunks)
         return k1_read_stats(raw0, offsets_dev, n_reads, stats, sc.flags->as<int32_t>(), sc.wide->as<uint32_t>(), kWideSlots, stream);
     // chunk table: [beg int64 | read int32 | len int32] per chunk, built on the host
     size_t nc = 0;
@@ -432,7 +430,7 @@ static int compute_read_stats(const int16_t* raw0, const int64_t* offsets_host, 
     std::vector<uint8_t> pageable;
     uint8_t* host = nullptr;
     if (sc.pinned) {
-        if (*sc.staged) CF_CUDA(cudaEventSynchronize(*sc.staged));
+        CF_TRY(sc.staged->sync());
         CF_TRY(sc.pinned->ensure(nc * 16 + 64));
         host = sc.pinned->as<uint8_t>();
     } else {
@@ -452,13 +450,11 @@ static int compute_read_stats(const int16_t* raw0, const int64_t* offsets_host, 
         }
     }
     CF_TRY(sc.chunk_tab->ensure(nc * 16 + 64));
-    CF_TRY(sc.chunked->ensure(k1_chunked_scratch_bytes(n_reads)));
     uint8_t* tab = static_cast<uint8_t*>(sc.chunk_tab->ptr);
     if (nc) {
         CF_CUDA(cudaMemcpyAsync(tab, host, nc * 16, cudaMemcpyHostToDevice, stream));
         if (sc.pinned) {
-            if (!*sc.staged) CF_CUDA(cudaEventCreateWithFlags(sc.staged, cudaEventDisableTiming));
-            CF_CUDA(cudaEventRecord(*sc.staged, stream));
+            CF_TRY(sc.staged->record(stream));
         } else {
             CF_CUDA(cudaStreamSynchronize(stream));        // pageable, local staging
         }
@@ -479,7 +475,7 @@ static int ensure_table(Exec* x, int64_t n_tiles, WindowTable* tab) {
     return CF_OK;
 }
 
-static int infer_reads_device(cf_model* m, Exec* x, Profiler* prof, const int16_t* raw_dev,
+static int infer_reads_device(cf_model* m, Exec* x, const int16_t* raw_dev,
                               const int64_t* offsets_host, int32_t n_reads, float* probs_dev, int64_t* intervals_dev,
                               int64_t* interval_offsets_dev, int64_t capacity, double threshold,
                               int32_t min_run, int32_t ext_left, int32_t ext_right,
@@ -498,7 +494,7 @@ static int infer_reads_device(cf_model* m, Exec* x, Profiler* prof, const int16_
     CF_TRY(ensure_table(x, plan.n_tiles, &tab));
     // When the caller does not want the probabilities, the head kernel thresholds them itself and emits label bits
     // (no 4 B/sample write + 4 B/sample read between the network and the interval caller).
-    const bool fused_bits = !probs_dev && m->engine == CF_ENGINE_TCGEN05 && tc_can_emit_bits(m->tc);
+    const bool fused_bits = !probs_dev && m->engine == CF_ENGINE_TCGEN05 && tc_can_emit_bits(m->tc.get());
     LabelBits bits;
     bits.threshold = threshold;
     float* probs = probs_dev;
@@ -508,28 +504,21 @@ static int infer_reads_device(cf_model* m, Exec* x, Profiler* prof, const int16_
         CF_TRY(x->probs_internal.ensure(sizeof(float) * (size_t)plan.total_samples));
         probs = x->probs_internal.as<float>();
     }
+    StatsScratch sc{&x->wide_flags, &x->wide_scratch, &x->k1_chunked, &x->k1_chunk_tab, &x->pin_chunks, &x->chunks_copied};
+    CF_TRY(compute_read_stats(raw0, offsets_host, offsets_dev, n_reads, x->stats.as<double>(), sc, stream, &x->prof));
     {
-        StatsScratch sc{&x->wide_flags, &x->wide_scratch, &x->k1_chunked, &x->k1_chunk_tab, &x->pin_chunks, &x->chunks_copied};
-        const bool chunks = stats_use_chunks(offsets_host, n_reads);
-        if (chunks) {   // allocate before the timed bracket
-            CF_TRY(x->k1_chunked.ensure(k1_chunked_scratch_bytes(n_reads)));
-        }
-        ProfScope ps(prof, KC_K1_STATS, stream, chunks ? 4 : 2);
-        CF_TRY(compute_read_stats(raw0, offsets_host, offsets_dev, n_reads, x->stats.as<double>(), sc, stream));
-    }
-    {
-        ProfScope ps(prof, KC_K1_TABLE, stream);
+        ProfScope ps(&x->prof, KC_K1_TABLE, stream);
         CF_TRY(k1_window_table(offsets_dev, win_off_dev, n_reads, plan.total_windows, plan.n_tiles, tab, stream,
                                fused_bits ? bits.bwords : nullptr, plan.total_samples));
     }
-    CF_TRY(engine_forward(m, x, prof, raw0, x->stats.as<double>(), nullptr, tab, plan.n_tiles, probs, stream, false,
+    CF_TRY(engine_forward(m, x, raw0, x->stats.as<double>(), nullptr, tab, plan.n_tiles, probs, stream, false,
                           fused_bits ? &bits : nullptr));
     if (fused_bits) {
-        ProfScope ps(prof, KC_K6_INTERVALS, stream, 3);
+        ProfScope ps(&x->prof, KC_K6_INTERVALS, stream, 3);
         CF_TRY(k6_intervals_from_bits(x->k6, bits, offsets_dev, n_reads, plan.total_samples, intervals_dev,
                                       interval_offsets_dev, capacity, min_run, ext_left, ext_right, stream));
     } else {
-        ProfScope ps(prof, KC_K6_INTERVALS, stream, 7);
+        ProfScope ps(&x->prof, KC_K6_INTERVALS, stream, 7);
         CF_TRY(k6_call_intervals(x->k6, probs, BITS_FROM_F32, threshold, 1, offsets_dev, n_reads,
                                  plan.total_samples, intervals_dev, interval_offsets_dev, nullptr, capacity,
                                  min_run, ext_left, ext_right, stream));
@@ -542,12 +531,6 @@ static int infer_reads_device(cf_model* m, Exec* x, Profiler* prof, const int16_
 // ================================================================== extern "C"
 // ---------------------------------------------------------------- model-free helpers
 namespace {
-struct TempBufs {
-    std::vector<cf::DevBuf*> bufs;
-    ~TempBufs() { for (auto* b : bufs) { b->release(); delete b; } }
-    cf::DevBuf* make() { bufs.push_back(new cf::DevBuf()); return bufs.back(); }
-};
-
 int upload_offsets(const int64_t* offsets_host, int32_t n_reads, cf::DevBuf* buf, cudaStream_t st) {
     CF_TRY(buf->ensure(sizeof(int64_t) * ((size_t)n_reads + 1)));
     std::vector<int64_t> off((size_t)n_reads + 1);
@@ -583,22 +566,19 @@ int cf_merge_chunks(int32_t device, const int64_t* intervals_dev, const int64_t*
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int64_t n_int = interval_offsets_host[n_reads] - interval_offsets_host[0];
     if (n_int < 0 || (n_int > 0 && !intervals_dev)) { cf::set_error("cf_merge_chunks: bad offsets"); return CF_ERR_BAD_ARG; }
-    TempBufs tmp;
-    cf::DevBuf* work = tmp.make();
-    cf::DevBuf* idx = tmp.make();
-    cf::DevBuf* meta = tmp.make();
-    CF_TRY(work->ensure(sizeof(int64_t) * 2 * (size_t)(n_int + 1)));
-    CF_TRY(idx->ensure(sizeof(int32_t) * (size_t)(n_int + n_reads + 1)));
-    CF_TRY(meta->ensure(sizeof(int64_t) * (2 * (size_t)n_reads + 1)));
+    cf::DevBuf work, idx, meta;
+    CF_TRY(work.ensure(sizeof(int64_t) * 2 * (size_t)(n_int + 1)));
+    CF_TRY(idx.ensure(sizeof(int32_t) * (size_t)(n_int + n_reads + 1)));
+    CF_TRY(meta.ensure(sizeof(int64_t) * (2 * (size_t)n_reads + 1)));
     std::vector<int64_t> host((size_t)2 * n_reads + 1);
     for (int32_t r = 0; r <= n_reads; ++r) host[r] = interval_offsets_host[r] - interval_offsets_host[0];
     for (int32_t r = 0; r < n_reads; ++r) host[n_reads + 1 + r] = read_lengths_host[r];
-    CF_CUDA(cudaMemcpyAsync(meta->ptr, host.data(), sizeof(int64_t) * host.size(), cudaMemcpyHostToDevice, st));
+    CF_CUDA(cudaMemcpyAsync(meta.ptr, host.data(), sizeof(int64_t) * host.size(), cudaMemcpyHostToDevice, st));
     if (n_int > 0)
-        CF_CUDA(cudaMemcpyAsync(work->ptr, intervals_dev + 2 * interval_offsets_host[0], sizeof(int64_t) * 2 * (size_t)n_int,
+        CF_CUDA(cudaMemcpyAsync(work.ptr, intervals_dev + 2 * interval_offsets_host[0], sizeof(int64_t) * 2 * (size_t)n_int,
                                 cudaMemcpyDeviceToDevice, st));
-    int s = cf::k7_merge_chunks(work->as<int64_t>(), meta->as<int64_t>(), meta->as<int64_t>() + n_reads + 1, n_reads,
-                                chunk_size, idx->as<int32_t>(), merged_dev, merged_count_dev, nonhp_dev, nonhp_count_dev, st);
+    int s = cf::k7_merge_chunks(work.as<int64_t>(), meta.as<int64_t>(), meta.as<int64_t>() + n_reads + 1, n_reads,
+                                chunk_size, idx.as<int32_t>(), merged_dev, merged_count_dev, nonhp_dev, nonhp_count_dev, st);
     cudaStreamSynchronize(st);
     return s;
 }
@@ -614,13 +594,11 @@ int cf_split_raw(int32_t device, const int16_t* raw_dev, const int64_t* offsets_
     cf::DeviceGuard guard;
     CF_TRY(guard.set(device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    TempBufs tmp;
-    cf::DevBuf* off = tmp.make();
-    cf::DevBuf* len = tmp.make();
-    if (n_reads > 0) CF_TRY(upload_offsets(offsets_host, n_reads, off, st));
-    CF_TRY(len->ensure(sizeof(int64_t) * (size_t)(n_ranges + 1)));
+    cf::DevBuf off, len;
+    if (n_reads > 0) CF_TRY(upload_offsets(offsets_host, n_reads, &off, st));
+    CF_TRY(len.ensure(sizeof(int64_t) * (size_t)(n_ranges + 1)));
     const int16_t* raw0 = n_reads > 0 ? raw_dev + offsets_host[0] : raw_dev;
-    int s = cf::k8_split_raw(raw0, off->as<int64_t>(), ranges_dev, range_read_dev, n_ranges, len->as<int64_t>(),
+    int s = cf::k8_split_raw(raw0, off.as<int64_t>(), ranges_dev, range_read_dev, n_ranges, len.as<int64_t>(),
                              piece_offsets_dev, capacity, out_dev, st);
     cudaStreamSynchronize(st);
     return s;
@@ -668,26 +646,29 @@ int cf_model_create(const cf_model_desc* desc, const float* const* tensors, cons
     }
     cf::DeviceGuard guard;
     CF_TRY(guard.set(device));
-    cf_model* m = new cf_model();
-    m->device = device;
-    cf::build_host_model(*desc, tensors, &m->hm);
+    cf::HostModel hm;
+    cf::build_host_model(*desc, tensors, &hm);
     int engine = desc->engine;
-    if (engine == CF_ENGINE_AUTO) engine = cf::tc_supported(m->hm) ? CF_ENGINE_TCGEN05 : CF_ENGINE_SIMT;
-    if (engine == CF_ENGINE_TCGEN05 && !cf::tc_supported(m->hm)) {
+    if (engine == CF_ENGINE_AUTO) engine = cf::tc_supported(hm) ? CF_ENGINE_TCGEN05 : CF_ENGINE_SIMT;
+    if (engine == CF_ENGINE_TCGEN05 && !cf::tc_supported(hm)) {
         cf::set_error("the tcgen05 engine supports layer_size_res <= 32 and layer_size <= 64 only");
-        delete m;
         return CF_ERR_BAD_ARG;
     }
-    m->engine = engine;
-    if (engine == CF_ENGINE_TCGEN05) m->tc = cf::tc_create(m->hm);
-    else m->simt = cf::simt_create(m->hm);
-    cudaError_t e = cudaDeviceSynchronize();
-    if (e != cudaSuccess || (!m->tc && !m->simt)) {
-        // a failed engine creation has already said why; otherwise the device did
-        if (e != cudaSuccess) cf::set_error("cf_model_create: uploading weights failed: %s", cudaGetErrorString(e));
-        cf_model_destroy(m);
+    // a failed creation frees what it made (the engine pointers' destructors) and returns its status
+    cf::TcEnginePtr tc;
+    cf::SimtEnginePtr simt;
+    CF_TRY(engine == CF_ENGINE_TCGEN05 ? cf::tc_create(hm, &tc) : cf::simt_create(hm, &simt));
+    const cudaError_t e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) {
+        cf::set_error("cf_model_create: uploading weights failed: %s", cudaGetErrorString(e));
         return CF_ERR_CUDA;
     }
+    cf_model* m = new cf_model();
+    m->hm = std::move(hm);
+    m->device = device;
+    m->engine = engine;
+    m->tc = std::move(tc);
+    m->simt = std::move(simt);
     *out_model = m;
     return CF_OK;
 }
@@ -697,8 +678,6 @@ int cf_model_create(const cf_model_desc* desc, const float* const* tensors, cons
 static void model_unref(cf_model* m) {
     if (m->refs.fetch_sub(1) != 1) return;
     cudaDeviceSynchronize();
-    cf::simt_destroy(m->simt);
-    cf::tc_destroy(m->tc);
     delete m;
 }
 
@@ -707,8 +686,7 @@ void cf_model_destroy(cf_model* m) {
     cf::DeviceGuard guard;
     if (guard.set(m->device) != CF_OK) cudaSetDevice(m->device);
     cudaDeviceSynchronize();
-    m->def.release();
-    m->prof.release();
+    m->def.reset();
     model_unref(m);
 }
 
@@ -729,27 +707,26 @@ void cf_exec_destroy(cf_exec* ex) {
     cf::DeviceGuard guard;
     if (guard.set(ex->model->device) != CF_OK) cudaSetDevice(ex->model->device);
     {
-        std::lock_guard<std::mutex> lock(ex->x.mu);
-        if (ex->x.last_done) cudaEventSynchronize(ex->x.last_done);
-        ex->x.release();
+        std::lock_guard<std::mutex> lock(ex->x.mu);      // a call on another thread finishes enqueueing first
+        ex->x.last_done.sync();
     }
-    model_unref(ex->model);
-    delete ex;
+    cf_model* m = ex->model;
+    delete ex;                                          // unlocked: a locked mutex must not be destroyed
+    model_unref(m);
 }
 
 int cf_model_engine(const cf_model* m) { return m ? m->engine : CF_ERR_BAD_ARG; }
 int cf_model_operand_format(const cf_model* m) {
     if (!m) return CF_ERR_BAD_ARG;
-    return m->engine == CF_ENGINE_TCGEN05 ? cf::tc_operand_format(m->tc) : -1;
+    return m->engine == CF_ENGINE_TCGEN05 ? cf::tc_operand_format(m->tc.get()) : -1;
 }
 
 int cf_profile_enable(cf_model* m, int32_t on) {
     if (!m) { cf::set_error("cf_profile_enable: NULL model"); return CF_ERR_BAD_ARG; }
-    std::lock_guard<std::mutex> lock(m->def.mu);
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(m->device));
-    m->prof.reset();
-    m->prof.on = on != 0;
+    cf::CallScope call(m->def.get());
+    CF_TRY(call.enter(m->device));
+    m->def->prof.reset();
+    m->def->prof.on = on != 0;
     return CF_OK;
 }
 
@@ -758,46 +735,39 @@ const char* cf_profile_class_name(int32_t cls) { return cf::kernel_class_name(cl
 
 int cf_profile_read(cf_model* m, double* ms_out, int64_t* launches_out, int32_t n) {
     if (!m || !ms_out || !launches_out || n < cf::KC_COUNT) { cf::set_error("cf_profile_read: bad argument"); return CF_ERR_BAD_ARG; }
-    std::lock_guard<std::mutex> lock(m->def.mu);
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(m->device));
-    m->prof.collect();
-    for (int i = 0; i < cf::KC_COUNT; ++i) { ms_out[i] = m->prof.ms[i]; launches_out[i] = m->prof.launches[i]; }
+    cf::CallScope call(m->def.get());
+    CF_TRY(call.enter(m->device));
+    cf::Profiler& prof = m->def->prof;
+    prof.collect();
+    for (int i = 0; i < cf::KC_COUNT; ++i) { ms_out[i] = prof.ms[i]; launches_out[i] = prof.launches[i]; }
     return CF_OK;
 }
 
+// Grow every buffer of context x, the engine workspaces included, to what a call of at most max_samples samples
+// and max_reads reads needs.
 static int reserve(cf_model* m, cf::Exec* x, int64_t max_samples, int32_t max_reads) {
-    std::lock_guard<std::mutex> lock(x->mu);
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(m->device));
-    const int64_t windows = max_samples / cf::kWindow + max_reads;
-    const int64_t tiles = cf::ceil_div(windows, cf::kTileWindows);
+    cf::CallScope call(x);
+    CF_TRY(call.enter(m->device));
+    const int64_t tiles = cf::ceil_div(max_samples / cf::kWindow + max_reads, cf::kTileWindows);
     cf::WindowTable tab;
     CF_TRY(cf::ensure_table(x, tiles, &tab));
     CF_TRY(x->stats.ensure(sizeof(double) * 2 * (size_t)max_reads));
     CF_TRY(x->wide_flags.ensure(sizeof(int32_t) * (size_t)max_reads));
     CF_TRY(x->wide_scratch.ensure(cf::k1_wide_scratch_bytes(cf::kWideSlots)));
-    if (max_reads > 0 && max_reads <= 8192) CF_TRY(x->k1_chunked.ensure(cf::k1_chunked_scratch_bytes(max_reads)));
+    if (cf::stats_may_use_chunks(max_reads)) CF_TRY(x->k1_chunked.ensure(cf::k1_chunked_scratch_bytes(max_reads)));
     CF_TRY(x->probs_internal.ensure(sizeof(float) * (size_t)max_samples));
-    return CF_OK;
+    if (m->engine == CF_ENGINE_TCGEN05) return cf::tc_reserve(m->tc.get(), &x->tc_ws, &x->simt_ws, m->hm, tiles);
+    return cf::simt_reserve(&x->simt_ws, m->hm, tiles);
 }
 
 int cf_model_reserve(cf_model* m, int64_t max_samples, int32_t max_reads) {
     if (!m || max_samples < 0 || max_reads < 0) { cf::set_error("cf_model_reserve: bad argument"); return CF_ERR_BAD_ARG; }
-    return reserve(m, &m->def, max_samples, max_reads);
+    return reserve(m, m->def.get(), max_samples, max_reads);
 }
 
 int cf_exec_reserve(cf_exec* ex, int64_t max_samples, int32_t max_reads) {
     if (!ex || max_samples < 0 || max_reads < 0) { cf::set_error("cf_exec_reserve: bad argument"); return CF_ERR_BAD_ARG; }
-    CF_TRY(reserve(ex->model, &ex->x, max_samples, max_reads));
-    // and the engine workspaces, the largest allocations of a call
-    cf_model* m = ex->model;
-    std::lock_guard<std::mutex> lock(ex->x.mu);
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(m->device));
-    const int64_t tiles = cf::ceil_div(max_samples / cf::kWindow + max_reads, cf::kTileWindows);
-    if (m->engine == CF_ENGINE_TCGEN05) return cf::tc_reserve(m->tc, &ex->x.tc_ws, &ex->x.simt_ws, m->hm, tiles);
-    return cf::simt_reserve(&ex->x.simt_ws, m->hm, tiles);
+    return reserve(ex->model, &ex->x, max_samples, max_reads);
 }
 
 int cf_infer_windows(cf_model* m, const float* x_dev, int64_t n_windows, float* probs_dev, void* stream) {
@@ -806,19 +776,17 @@ int cf_infer_windows(cf_model* m, const float* x_dev, int64_t n_windows, float* 
         return CF_ERR_BAD_ARG;
     }
     if (n_windows == 0) return CF_OK;
-    std::lock_guard<std::mutex> lock(m->def.mu);
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(m->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
+    cf::Exec* x = m->def.get();
+    cf::CallScope call(x);
+    CF_TRY(call.enter(m->device, st));
     const int64_t tiles = cf::ceil_div(n_windows, cf::kTileWindows);
     cf::WindowTable tab;
-    CF_TRY(cf::ensure_table(&m->def, tiles, &tab));
+    CF_TRY(cf::ensure_table(x, tiles, &tab));
     const int64_t slots = tiles * cf::kTileWindows;
-    cf::ExecCall call(&m->def, st);
-    CF_TRY(call.begin());
     cf::dense_window_table_kernel<<<(unsigned)cf::ceil_div(slots, 256), 256, 0, st>>>(n_windows, slots, tab.src, tab.valid, tab.read);
     CF_LAUNCHED();
-    return cf::engine_forward(m, &m->def, &m->prof, nullptr, nullptr, x_dev, tab, tiles, probs_dev, st);
+    return cf::engine_forward(m, x, nullptr, nullptr, x_dev, tab, tiles, probs_dev, st);
 }
 
 int cf_validate_windows(cf_model* m, const float* x_dev, const uint8_t* labels_dev, int64_t n_windows,
@@ -828,11 +796,10 @@ int cf_validate_windows(cf_model* m, const float* x_dev, const uint8_t* labels_d
         cf::set_error("cf_validate_windows: bad argument");
         return CF_ERR_BAD_ARG;
     }
-    std::lock_guard<std::mutex> lock(m->def.mu);
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(m->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cf::Exec* x = &m->def;
+    cf::Exec* x = m->def.get();
+    cf::CallScope call(x);
+    CF_TRY(call.enter(m->device, st));
     const int64_t n = n_windows * cf::kWindow;
     const int64_t tiles = cf::ceil_div(n_windows, cf::kTileWindows);
     const int blocks = cf::k9_validation_blocks(n);
@@ -841,20 +808,16 @@ int cf_validate_windows(cf_model* m, const float* x_dev, const uint8_t* labels_d
     cf::WindowTable tab;
     CF_TRY(cf::ensure_table(x, tiles, &tab));
     const int64_t slots = tiles * cf::kTileWindows;
+    cf::dense_window_table_kernel<<<(unsigned)cf::ceil_div(slots, 256), 256, 0, st>>>(n_windows, slots, tab.src, tab.valid, tab.read);
+    CF_LAUNCHED();
+    CF_TRY(cf::engine_forward(m, x, nullptr, nullptr, x_dev, tab, tiles, x->val_logits.as<float>(), st,
+                              /*want_logits=*/true));
+    long long* partial = x->val_partial.as<long long>();
+    long long* result = partial + (size_t)blocks * 6;
+    CF_TRY(cf::k9_validate(x->val_logits.as<float>(), labels_dev, n, threshold, partial, result, st));
     long long host[6];
-    {
-        cf::ExecCall call(x, st);
-        CF_TRY(call.begin());
-        cf::dense_window_table_kernel<<<(unsigned)cf::ceil_div(slots, 256), 256, 0, st>>>(n_windows, slots, tab.src, tab.valid, tab.read);
-        CF_LAUNCHED();
-        CF_TRY(cf::engine_forward(m, x, &m->prof, nullptr, nullptr, x_dev, tab, tiles, x->val_logits.as<float>(), st,
-                                  /*want_logits=*/true));
-        long long* partial = x->val_partial.as<long long>();
-        long long* result = partial + (size_t)blocks * 6;
-        CF_TRY(cf::k9_validate(x->val_logits.as<float>(), labels_dev, n, threshold, partial, result, st));
-        CF_CUDA(cudaMemcpyAsync(host, result, sizeof(host), cudaMemcpyDeviceToHost, st));
-        CF_CUDA(cudaStreamSynchronize(st));
-    }
+    CF_CUDA(cudaMemcpyAsync(host, result, sizeof(host), cudaMemcpyDeviceToHost, st));
+    CF_CUDA(cudaStreamSynchronize(st));
     counts_out[0] = host[0];
     counts_out[1] = host[1];
     counts_out[2] = host[2] - padding_size;      // rnn_class.py:247
@@ -897,22 +860,20 @@ int cf_vote_events(int32_t device, const double* scores_dev, int64_t n_scores, c
     cf::DeviceGuard guard;
     CF_TRY(guard.set(device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    TempBufs tmp;
-    cf::DevBuf* ev = tmp.make();
-    cf::DevBuf* flag = tmp.make();
-    CF_TRY(ev->ensure(sizeof(int64_t) * (size_t)(n_voted + 1)));
-    CF_TRY(flag->ensure(sizeof(int32_t)));
-    CF_CUDA(cudaMemcpyAsync(ev->ptr, begin.data() + start_event, sizeof(int64_t) * (size_t)(n_voted + 1),
+    cf::DevBuf ev, flag;
+    CF_TRY(ev.ensure(sizeof(int64_t) * (size_t)(n_voted + 1)));
+    CF_TRY(flag.ensure(sizeof(int32_t)));
+    CF_CUDA(cudaMemcpyAsync(ev.ptr, begin.data() + start_event, sizeof(int64_t) * (size_t)(n_voted + 1),
                             cudaMemcpyHostToDevice, st));
-    CF_TRY(cf::k10_vote_events(scores_dev, n_scores, ev->as<int64_t>(), 0, n_voted, classes_dev, flag->as<int32_t>(), st));
+    CF_TRY(cf::k10_vote_events(scores_dev, n_scores, ev.as<int64_t>(), 0, n_voted, classes_dev, flag.as<int32_t>(), st));
     int32_t empty = 0;
-    CF_CUDA(cudaMemcpyAsync(&empty, flag->ptr, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CF_CUDA(cudaMemcpyAsync(&empty, flag.ptr, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CF_CUDA(cudaStreamSynchronize(st));
     if (empty_event_out) *empty_event_out = empty;
     return CF_OK;
 }
 
-static int infer_reads_call(const char* name, cf_model* m, cf::Exec* x, cf::Profiler* prof, const int16_t* raw_dev,
+static int infer_reads_call(const char* name, cf_model* m, cf::Exec* x, const int16_t* raw_dev,
                             const int64_t* offsets_host, int32_t n_reads, float* probs_dev, int64_t* intervals_dev,
                             int64_t* interval_offsets_dev, int64_t capacity, double threshold, int32_t min_run,
                             int32_t ext_left, int32_t ext_right, void* stream) {
@@ -921,13 +882,10 @@ static int infer_reads_call(const char* name, cf_model* m, cf::Exec* x, cf::Prof
         cf::set_error("%s: bad argument", name);
         return CF_ERR_BAD_ARG;
     }
-    std::lock_guard<std::mutex> lock(x->mu);
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(m->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cf::ExecCall call(x, st);
-    CF_TRY(call.begin());
-    return cf::infer_reads_device(m, x, prof, raw_dev, offsets_host, n_reads, probs_dev, intervals_dev,
+    cf::CallScope call(x);
+    CF_TRY(call.enter(m->device, st));
+    return cf::infer_reads_device(m, x, raw_dev, offsets_host, n_reads, probs_dev, intervals_dev,
                                   interval_offsets_dev, capacity, threshold, min_run, ext_left, ext_right, st);
 }
 
@@ -935,16 +893,16 @@ int cf_infer_reads(cf_model* m, const int16_t* raw_dev, const int64_t* offsets_h
                    float* probs_dev, int64_t* intervals_dev, int64_t* interval_offsets_dev,
                    int64_t capacity, double threshold, int32_t min_run, int32_t ext_left,
                    int32_t ext_right, void* stream) {
-    return infer_reads_call("cf_infer_reads", m, m ? &m->def : nullptr, m ? &m->prof : nullptr, raw_dev, offsets_host,
-                            n_reads, probs_dev, intervals_dev, interval_offsets_dev, capacity, threshold, min_run,
-                            ext_left, ext_right, stream);
+    return infer_reads_call("cf_infer_reads", m, m ? m->def.get() : nullptr, raw_dev, offsets_host, n_reads, probs_dev,
+                            intervals_dev, interval_offsets_dev, capacity, threshold, min_run, ext_left, ext_right,
+                            stream);
 }
 
 int cf_exec_infer_reads(cf_exec* ex, const int16_t* raw_dev, const int64_t* offsets_host, int32_t n_reads,
                         float* probs_dev, int64_t* intervals_dev, int64_t* interval_offsets_dev,
                         int64_t capacity, double threshold, int32_t min_run, int32_t ext_left,
                         int32_t ext_right, void* stream) {
-    return infer_reads_call("cf_exec_infer_reads", ex ? ex->model : nullptr, ex ? &ex->x : nullptr, nullptr, raw_dev,
+    return infer_reads_call("cf_exec_infer_reads", ex ? ex->model : nullptr, ex ? &ex->x : nullptr, raw_dev,
                             offsets_host, n_reads, probs_dev, intervals_dev, interval_offsets_dev, capacity, threshold,
                             min_run, ext_left, ext_right, stream);
 }
@@ -965,11 +923,10 @@ int cf_infer_reads_host(cf_model* m, const int16_t* raw_host, const int64_t* off
         cf::set_error("cf_infer_reads_host: bad argument");
         return CF_ERR_BAD_ARG;
     }
-    std::lock_guard<std::mutex> lock(m->def.mu);
-    cf::DeviceGuard guard;
-    CF_TRY(guard.set(m->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cf::Exec* x = &m->def;
+    cf::Exec* x = m->def.get();
+    cf::CallScope call(x);
+    CF_TRY(call.enter(m->device, st));
     const int64_t base = n_reads > 0 ? offsets_host[0] : 0;
     const int64_t total = n_reads > 0 ? offsets_host[n_reads] - base : 0;
     if (total < 0) { cf::set_error("cf_infer_reads_host: offsets decrease"); return CF_ERR_BAD_ARG; }
@@ -988,30 +945,25 @@ int cf_infer_reads_host(cf_model* m, const int16_t* raw_host, const int64_t* off
         cf::BatchPlan whole;                       // reject bad / empty reads before any asynchronous copy reads the caller's buffer
         CF_TRY(cf::make_plan(off.data(), n_reads, &whole));
     }
-    int64_t found = 0;
-    {
-        cf::ExecCall call(x, st);
-        CF_TRY(call.begin());
-        // (Cutting the batch into groups of whole passes whose copies overlap the previous group's kernels was
-        // measured: no gain - the copy is 1.2-1.5 ms of a 75 ms step and the extra K1 / K6 sequences cost as much.)
-        if (total > 0)
-            CF_CUDA(cudaMemcpyAsync(x->h_raw.ptr, raw_host + base, sizeof(int16_t) * (size_t)total, cudaMemcpyHostToDevice, st));
-        CF_TRY(cf::infer_reads_device(m, x, &m->prof, x->h_raw.as<int16_t>(), off.data(), n_reads, probs_dev,
-                                      x->h_intervals.as<int64_t>(), x->h_ioff.as<int64_t>(), capacity, threshold,
-                                      min_run, ext_left, ext_right, st));
-        CF_CUDA(cudaMemcpyAsync(interval_offsets_host, x->h_ioff.ptr, sizeof(int64_t) * ((size_t)n_reads + 1),
+    // (Cutting the batch into groups of whole passes whose copies overlap the previous group's kernels was
+    // measured: no gain - the copy is 1.2-1.5 ms of a 75 ms step and the extra K1 / K6 sequences cost as much.)
+    if (total > 0)
+        CF_CUDA(cudaMemcpyAsync(x->h_raw.ptr, raw_host + base, sizeof(int16_t) * (size_t)total, cudaMemcpyHostToDevice, st));
+    CF_TRY(cf::infer_reads_device(m, x, x->h_raw.as<int16_t>(), off.data(), n_reads, probs_dev,
+                                  x->h_intervals.as<int64_t>(), x->h_ioff.as<int64_t>(), capacity, threshold,
+                                  min_run, ext_left, ext_right, st));
+    CF_CUDA(cudaMemcpyAsync(interval_offsets_host, x->h_ioff.ptr, sizeof(int64_t) * ((size_t)n_reads + 1),
+                            cudaMemcpyDeviceToHost, st));
+    CF_CUDA(cudaStreamSynchronize(st));
+    const int64_t found = interval_offsets_host[n_reads];
+    if (n_intervals_out) *n_intervals_out = found;
+    const int64_t ncopy = found < capacity ? found : capacity;
+    if (ncopy > 0)
+        CF_CUDA(cudaMemcpyAsync(intervals_host, x->h_intervals.ptr, sizeof(int64_t) * 2 * (size_t)ncopy,
                                 cudaMemcpyDeviceToHost, st));
-        CF_CUDA(cudaStreamSynchronize(st));
-        found = interval_offsets_host[n_reads];
-        if (n_intervals_out) *n_intervals_out = found;
-        const int64_t ncopy = found < capacity ? found : capacity;
-        if (ncopy > 0)
-            CF_CUDA(cudaMemcpyAsync(intervals_host, x->h_intervals.ptr, sizeof(int64_t) * 2 * (size_t)ncopy,
-                                    cudaMemcpyDeviceToHost, st));
-        if (probs_host && total > 0)
-            CF_CUDA(cudaMemcpyAsync(probs_host, probs_dev, sizeof(float) * (size_t)total, cudaMemcpyDeviceToHost, st));
-        CF_CUDA(cudaStreamSynchronize(st));
-    }
+    if (probs_host && total > 0)
+        CF_CUDA(cudaMemcpyAsync(probs_host, probs_dev, sizeof(float) * (size_t)total, cudaMemcpyDeviceToHost, st));
+    CF_CUDA(cudaStreamSynchronize(st));
     if (found > capacity) {
         cf::set_error("cf_infer_reads_host: %lld intervals found, capacity %lld", (long long)found, (long long)capacity);
         return CF_ERR_CAPACITY;
@@ -1032,24 +984,18 @@ int cf_normalize_reads(int32_t device, const int16_t* raw_dev, const int64_t* of
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     for (int32_t r = 0; r < n_reads; ++r)
         if (offsets_host[r + 1] < offsets_host[r]) { cf::set_error("cf_normalize_reads: offsets decrease"); return CF_ERR_BAD_ARG; }
-    TempBufs tmp;
-    cf::DevBuf* off = tmp.make();
-    CF_TRY(upload_offsets(offsets_host, n_reads, off, st));
-    cf::DevBuf* flags = tmp.make();
-    cf::DevBuf* wide = tmp.make();
-    cf::DevBuf* chunked = tmp.make();
-    cf::DevBuf* chunk_tab = tmp.make();
-    cf::DevBuf* stats_tmp = tmp.make();
+    cf::DevBuf off, flags, wide, chunked, chunk_tab, stats_tmp;
+    CF_TRY(upload_offsets(offsets_host, n_reads, &off, st));
     double* stats = stats_dev;
     if (!stats) {
-        CF_TRY(stats_tmp->ensure(sizeof(double) * 2 * (size_t)n_reads));
-        stats = stats_tmp->as<double>();
+        CF_TRY(stats_tmp.ensure(sizeof(double) * 2 * (size_t)n_reads));
+        stats = stats_tmp.as<double>();
     }
     const int16_t* raw0 = raw_dev + offsets_host[0];
-    cf::StatsScratch sc{flags, wide, chunked, chunk_tab};
-    CF_TRY(cf::compute_read_stats(raw0, offsets_host, off->as<int64_t>(), n_reads, stats, sc, st));
+    cf::StatsScratch sc{&flags, &wide, &chunked, &chunk_tab};
+    CF_TRY(cf::compute_read_stats(raw0, offsets_host, off.as<int64_t>(), n_reads, stats, sc, st));
     if (norm_dev)
-        CF_TRY(cf::k1_normalize_f64(raw0, off->as<int64_t>(), n_reads, offsets_host[n_reads] - offsets_host[0],
+        CF_TRY(cf::k1_normalize_f64(raw0, off.as<int64_t>(), n_reads, offsets_host[n_reads] - offsets_host[0],
                                     stats, norm_dev, st));
     CF_CUDA(cudaStreamSynchronize(st));      // scratch is freed on return
     return CF_OK;
@@ -1073,16 +1019,14 @@ int cf_call_intervals(int32_t device, const void* probs_dev, int32_t probs_is_f6
         if (offsets_host[r + 1] < offsets_host[r]) { cf::set_error("cf_call_intervals: offsets decrease"); return CF_ERR_BAD_ARG; }
     const int64_t total = offsets_host[n_reads] - offsets_host[0];
     if (total > 0 && !probs_dev) { cf::set_error("cf_call_intervals: probs is NULL"); return CF_ERR_BAD_ARG; }
-    TempBufs tmp;
-    cf::DevBuf* off = tmp.make();
-    CF_TRY(upload_offsets(offsets_host, n_reads, off, st));
+    cf::DevBuf off;
+    CF_TRY(upload_offsets(offsets_host, n_reads, &off, st));
     cf::IntervalScratch scratch;
     const char* base = static_cast<const char*>(probs_dev) + (size_t)offsets_host[0] * (probs_is_f64 ? 8 : 4);
     int s = cf::k6_call_intervals(scratch, base, probs_is_f64 ? cf::BITS_FROM_F64 : cf::BITS_FROM_F32, threshold, 1,
-                                  off->as<int64_t>(), n_reads, total, intervals_dev, interval_offsets_dev, nullptr,
+                                  off.as<int64_t>(), n_reads, total, intervals_dev, interval_offsets_dev, nullptr,
                                   capacity, min_run, ext_left, ext_right, st);
     cudaStreamSynchronize(st);
-    scratch.bits.release(); scratch.block_cnt.release(); scratch.read_cnt.release(); scratch.misc.release();
     return s;
 }
 
@@ -1115,17 +1059,14 @@ int cf_hp_in_pred(int32_t device, const int64_t* labels_dev, int64_t n, int32_t 
     cf::DeviceGuard guard;
     CF_TRY(guard.set(device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    TempBufs tmp;
-    cf::DevBuf* off = tmp.make();
-    cf::DevBuf* ioff = tmp.make();
+    cf::DevBuf off, ioff;
     const int64_t offsets[2] = {0, n};
-    CF_TRY(upload_offsets(offsets, 1, off, st));
-    CF_TRY(ioff->ensure(sizeof(int64_t) * 2));
+    CF_TRY(upload_offsets(offsets, 1, &off, st));
+    CF_TRY(ioff.ensure(sizeof(int64_t) * 2));
     cf::IntervalScratch scratch;
-    int s = cf::k6_call_intervals(scratch, labels_dev, cf::BITS_FROM_I64_EQ, 0.0, label, off->as<int64_t>(), 1, n,
-                                  intervals_dev, ioff->as<int64_t>(), n_out_dev, capacity, 1, ext_left, ext_right, st);
+    int s = cf::k6_call_intervals(scratch, labels_dev, cf::BITS_FROM_I64_EQ, 0.0, label, off.as<int64_t>(), 1, n,
+                                  intervals_dev, ioff.as<int64_t>(), n_out_dev, capacity, 1, ext_left, ext_right, st);
     cudaStreamSynchronize(st);
-    scratch.bits.release(); scratch.block_cnt.release(); scratch.read_cnt.release(); scratch.misc.release();
     return s;
 }
 

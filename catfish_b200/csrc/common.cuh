@@ -73,10 +73,13 @@ struct Profiler {
     std::vector<cudaEvent_t> pool;
     double ms[KC_COUNT] = {};
     long long launches[KC_COUNT] = {};
+    Profiler() = default;
+    Profiler(const Profiler&) = delete;
+    Profiler& operator=(const Profiler&) = delete;
+    ~Profiler();             // waits for the recorded events, then destroys every event
     cudaEvent_t get();
     void collect();          // synchronises on the recorded events and folds them into ms[]
     void reset();
-    void release();
 };
 
 // RAII bracket: records an event pair around the launches issued in its scope.
@@ -94,22 +97,60 @@ struct ProfScope {
 };
 
 // ---------------------------------------------------------------- device buffers
-// A growable device allocation owned by a handle; grows only when asked for more.
+// A growable device allocation, freed by its destructor; grows only when asked for more.  Move-only: a moved-from
+// buffer is empty.
 struct DevBuf {
     void* ptr = nullptr;
     size_t bytes = 0;
+    DevBuf() = default;
+    DevBuf(DevBuf&& o) noexcept : ptr(o.ptr), bytes(o.bytes) { o.ptr = nullptr; o.bytes = 0; }
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() { if (ptr) cudaFree(ptr); }
     int ensure(size_t want);
-    void release();
+    // ensure + a synchronous copy of v from the host: the engines' weights
+    template <typename T> int upload(const std::vector<T>& v) {
+        CF_TRY(ensure(sizeof(T) * v.size()));
+        CF_CUDA(cudaMemcpy(ptr, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice));
+        return CF_OK;
+    }
     template <typename T> T* as() const { return reinterpret_cast<T*>(ptr); }
 };
 
-// Pinned host staging buffer.
+// Pinned host staging buffer, freed by its destructor.
 struct HostBuf {
     void* ptr = nullptr;
     size_t bytes = 0;
+    HostBuf() = default;
+    HostBuf(HostBuf&& o) noexcept : ptr(o.ptr), bytes(o.bytes) { o.ptr = nullptr; o.bytes = 0; }
+    HostBuf(const HostBuf&) = delete;
+    HostBuf& operator=(const HostBuf&) = delete;
+    ~HostBuf() { if (ptr) cudaFreeHost(ptr); }
     int ensure(size_t want);
-    void release();
     template <typename T> T* as() const { return reinterpret_cast<T*>(ptr); }
+};
+
+// A CUDA event without timing, created on first use and destroyed by its destructor.
+struct Event {
+    cudaEvent_t ev = nullptr;
+    Event() = default;
+    Event(const Event&) = delete;
+    Event& operator=(const Event&) = delete;
+    ~Event() { if (ev) cudaEventDestroy(ev); }
+    int create() {
+        if (!ev) CF_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+        return CF_OK;
+    }
+    int record(cudaStream_t stream) {
+        CF_TRY(create());
+        CF_CUDA(cudaEventRecord(ev, stream));
+        return CF_OK;
+    }
+    // Waits for the last record; an event never recorded has nothing to wait for.
+    int sync() {
+        if (ev) CF_CUDA(cudaEventSynchronize(ev));
+        return CF_OK;
+    }
 };
 
 // ---------------------------------------------------------------- ragged batch plan

@@ -2,6 +2,7 @@
 // workspace a forward pass writes belongs to the caller's execution context and is passed in.
 #pragma once
 
+#include <memory>
 #include <vector>
 
 #include "common.cuh"
@@ -46,10 +47,19 @@ struct HostModel {
 int expected_tensor_shapes(const cf_model_desc& d, std::vector<std::vector<int64_t>>* shapes);
 int build_host_model(const cf_model_desc& d, const float* const* tensors, HostModel* out);
 
-// ---------------------------------------------------------------- SIMT (fp32) engine
+// An engine owns its weights; each engine's source defines how one is deleted.
 struct SimtEngine;
-SimtEngine* simt_create(const HostModel& hm);
-void simt_destroy(SimtEngine* e);
+struct TcEngine;
+struct EngineDelete {
+    void operator()(SimtEngine* e) const;
+    void operator()(TcEngine* e) const;
+};
+using SimtEnginePtr = std::unique_ptr<SimtEngine, EngineDelete>;
+using TcEnginePtr = std::unique_ptr<TcEngine, EngineDelete>;
+
+// ---------------------------------------------------------------- SIMT (fp32) engine
+// Uploads the weights; CF_ERR_ALLOC / CF_ERR_CUDA when an allocation / a copy fails.
+int simt_create(const HostModel& hm, SimtEnginePtr* out);
 // Forward pass over n_tiles tiles of 128 windows.  Input is either the raw int16 signal with
 // per-read (shift, scale) or already-normalised float windows; output probabilities are
 // scattered to probs[tab.src[g] + t] for t < tab.valid[g].  With want_logits the dense layer's output
@@ -65,10 +75,10 @@ int simt_reserve(DevBuf* ws, const HostModel& hm, int64_t n_tiles);
 int simt_conv_stack_reserve(DevBuf* ws, const HostModel& hm, int64_t chunk_tiles);
 
 // ---------------------------------------------------------------- tcgen05 engine
-struct TcEngine;
 bool tc_supported(const HostModel& hm);
-TcEngine* tc_create(const HostModel& hm);
-void tc_destroy(TcEngine* e);
+// Sets the kernels' attributes and uploads the weights; CF_ERR_ALLOC / CF_ERR_CUDA when an allocation / a CUDA call
+// fails.
+int tc_create(const HostModel& hm, TcEnginePtr* out);
 int tc_operand_format(const TcEngine* e);    // 0 = split bf16 (3 MMA passes), 1 = fp16 + e5m2 corrections (2 pass-equivalents)
 // bits != nullptr (networks with a GRU head): the head thresholds its own scores and ORs label bits into
 // bits->lwords (k6_bits_prepare) instead of writing probabilities - probs may then be nullptr.

@@ -19,27 +19,26 @@ constexpr int kSimtChunkTiles = 256;
 
 struct SimtEngine {
     // weights
-    std::vector<float*> conv_w, conv_b;
-    std::vector<float*> gru_wx, gru_bx;      // per layer: [in][6H], [6H] (fw r|u|c, bw r|u|c)
-    std::vector<float*> gru_wgh, gru_wch;    // per layer*2+dir
-    float* head_w = nullptr;
+    std::vector<DevBuf> conv_w, conv_b;
+    std::vector<DevBuf> gru_wx, gru_bx;      // per layer: [in][6H], [6H] (fw r|u|c, bw r|u|c)
+    std::vector<DevBuf> gru_wgh, gru_wch;    // per layer*2+dir
+    DevBuf head_w;
     float head_b = 0.f;
-    std::vector<void*> owned;
 };
 
-static float* upload(SimtEngine* e, const std::vector<float>& v) {
-    float* d = nullptr;
-    if (cudaMalloc(&d, sizeof(float) * (v.size() ? v.size() : 1)) != cudaSuccess) return nullptr;
-    cudaMemcpy(d, v.data(), sizeof(float) * v.size(), cudaMemcpyHostToDevice);
-    e->owned.push_back(d);
-    return d;
+void EngineDelete::operator()(SimtEngine* e) const { delete e; }
+
+// Appends a device copy of v to list.
+static int upload(std::vector<DevBuf>* list, const std::vector<float>& v) {
+    list->emplace_back();
+    return list->back().upload(v);
 }
 
-SimtEngine* simt_create(const HostModel& hm) {
-    SimtEngine* e = new SimtEngine();
+int simt_create(const HostModel& hm, SimtEnginePtr* out) {
+    SimtEnginePtr e(new SimtEngine());
     for (const ConvLayer& c : hm.convs) {
-        e->conv_w.push_back(upload(e, c.w));
-        e->conv_b.push_back(upload(e, c.b));
+        CF_TRY(upload(&e->conv_w, c.w));
+        CF_TRY(upload(&e->conv_b, c.b));
     }
     const int n_rnn = hm.n_rnn();
     for (int l = 0; l < n_rnn; ++l) {
@@ -53,22 +52,17 @@ SimtEngine* simt_create(const HostModel& hm) {
                 wx[(size_t)k * 2 * h3 + h3 + j] = b.wx[(size_t)k * h3 + j];
             }
         for (int j = 0; j < h3; ++j) { bx[j] = f.bx[j]; bx[h3 + j] = b.bx[j]; }
-        e->gru_wx.push_back(upload(e, wx));
-        e->gru_bx.push_back(upload(e, bx));
+        CF_TRY(upload(&e->gru_wx, wx));
+        CF_TRY(upload(&e->gru_bx, bx));
         for (int d = 0; d < 2; ++d) {
-            e->gru_wgh.push_back(upload(e, hm.gru[2 * l + d].wgh));
-            e->gru_wch.push_back(upload(e, hm.gru[2 * l + d].wch));
+            CF_TRY(upload(&e->gru_wgh, hm.gru[2 * l + d].wgh));
+            CF_TRY(upload(&e->gru_wch, hm.gru[2 * l + d].wch));
         }
     }
-    e->head_w = upload(e, hm.head_w);
+    CF_TRY(e->head_w.upload(hm.head_w));
     e->head_b = hm.head_b;
-    return e;
-}
-
-void simt_destroy(SimtEngine* e) {
-    if (!e) return;
-    for (void* p : e->owned) cudaFree(p);
-    delete e;
+    *out = std::move(e);
+    return CF_OK;
 }
 
 // ---------------------------------------------------------------- input
@@ -307,7 +301,7 @@ static int conv_stack(SimtEngine* e, const HostModel& hm, const SimtBufs& b, con
             const int64_t total = rows * c.cout;
             ProfScope ps(prof, KC_K2_CONV, stream);
             simt_conv_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, stream>>>(
-                in, e->conv_w[i], e->conv_b[i], res, out, rows, c.k, c.cin, c.cout, relu);
+                in, e->conv_w[i].as<float>(), e->conv_b[i].as<float>(), res, out, rows, c.k, c.cin, c.cout, relu);
             CF_LAUNCHED();
             return CF_OK;
         };
@@ -362,7 +356,8 @@ int simt_forward(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* 
             dim3 grid((unsigned)ceil_div(rows, 64), (unsigned)ceil_div(6 * H, 64));
             {
                 ProfScope ps(prof, KC_K3_XPROJ, stream);
-                simt_gemm_bias_kernel<<<grid, 256, 0, stream>>>(a, e->gru_wx[l], e->gru_bx[l], b.xproj, rows, 6 * H, in_dim);
+                simt_gemm_bias_kernel<<<grid, 256, 0, stream>>>(a, e->gru_wx[l].as<float>(), e->gru_bx[l].as<float>(), b.xproj,
+                                                                rows, 6 * H, in_dim);
                 CF_LAUNCHED();
             }
             float* yout = (l & 1) ? b.y1 : b.y0;
@@ -372,7 +367,8 @@ int simt_forward(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* 
             {
                 ProfScope ps(prof, KC_K4_GRU, stream);
                 simt_gru_kernel<<<dim3((unsigned)tiles, 4, 2), 256, smem, stream>>>(
-                    b.xproj, e->gru_wgh[2 * l], e->gru_wch[2 * l], e->gru_wgh[2 * l + 1], e->gru_wch[2 * l + 1], yout, H);
+                    b.xproj, e->gru_wgh[2 * l].as<float>(), e->gru_wch[2 * l].as<float>(), e->gru_wgh[2 * l + 1].as<float>(),
+                    e->gru_wch[2 * l + 1].as<float>(), yout, H);
                 CF_LAUNCHED();
             }
             yin = yout;
@@ -380,7 +376,7 @@ int simt_forward(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* 
         const float* hin = hm.n_rnn() ? yin : feat;
         ProfScope ps(prof, KC_K5_HEAD, stream);
         simt_head_kernel<<<(unsigned)ceil_div(rows, 256), 256, 0, stream>>>(
-            hin, e->head_w, e->head_b, hm.head_features(), tab.src, tab.valid, tab.read, raw ? stats : nullptr,
+            hin, e->head_w.as<float>(), e->head_b, hm.head_features(), tab.src, tab.valid, tab.read, raw ? stats : nullptr,
             tile0, rows, probs, want_logits ? 1 : 0);
         CF_LAUNCHED();
     }

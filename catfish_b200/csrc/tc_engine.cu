@@ -103,21 +103,20 @@ static void pack_b_operand_f16e5(const float* w, int K, int N, int ldw, int col0
 
 struct TcLayer {
     int in = 0;                       // input features of this GRU layer (1, 32 or 128)
-    uint8_t* wfused = nullptr;        // [dir]{Wgx, Wcx, Wgh, Wch} as in GruF2Cfg (no Wgx, Wcx for in = 1), exponent domain
+    DevBuf wfused;                    // [dir]{Wgx, Wcx, Wgh, Wch} as in GruF2Cfg (no Wgx, Wcx for in = 1), exponent domain
     int fmt = 0;                      // operand format of wfused / of this layer's x and state operands
-    float* bz = nullptr;              // [384] biases in the exponent domain
-    float* wxz = nullptr;             // [384] the single x row of gates / candidate kernels, exponent domain (in == 1)
+    DevBuf bz;                        // float [384] biases in the exponent domain
+    DevBuf wxz;                       // float [384] the single x row of gates / candidate kernels, exponent domain (in == 1)
 };
 
 struct TcEngine {
-    SimtEngine* simt = nullptr;       // RNN-only networks: normalised scalar input (simt_conv_stack without blocks)
-    uint8_t* conv_params = nullptr;   // TK2 parameter block (see ConvParams), nullptr = no residual blocks
-    uint8_t* block_params = nullptr;  // [conv_nres - 2] parameter blocks of tc_conv_block_kernel (block-1 slots)
+    SimtEnginePtr simt;               // RNN-only networks: normalised scalar input (simt_conv_stack without blocks)
+    DevBuf conv_params;               // TK2 parameter block (see ConvParams), then [conv_nres - 2] parameter blocks of
+                                      // tc_conv_block_kernel (block-1 slots); empty = no residual blocks
     int conv_nres = 0;
     std::vector<TcLayer> layers;
-    float* head_w = nullptr;          // [128]
+    DevBuf head_w;                    // float [128]
     float head_b = 0.f;
-    std::vector<void*> owned;
     int n_sms = 148;
 #ifdef CF_TRACE_PROBES
     bool trace_done = false;
@@ -190,24 +189,17 @@ static HostModel pad_model(const HostModel& hm) {
     return p;
 }
 
-template <typename T>
-static T* tc_upload(TcEngine* e, const std::vector<T>& v) {
-    T* d = nullptr;
-    if (cudaMalloc(&d, sizeof(T) * (v.size() ? v.size() : 1)) != cudaSuccess) return nullptr;
-    cudaMemcpy(d, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice);
-    e->owned.push_back(d);
-    return d;
-}
+void EngineDelete::operator()(TcEngine* e) const { delete e; }
 
 static int tc_set_attributes();
 
-TcEngine* tc_create(const HostModel& narrow) {
-    if (tc_set_attributes() != CF_OK) return nullptr;
-    TcEngine* e = new TcEngine();
+int tc_create(const HostModel& narrow, TcEnginePtr* out) {
+    CF_TRY(tc_set_attributes());
+    TcEnginePtr e(new TcEngine());
     int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&e->n_sms, cudaDevAttrMultiProcessorCount, dev);
-    if (narrow.n_res() == 0) e->simt = simt_create(narrow);
+    CF_CUDA(cudaGetDevice(&dev));
+    CF_CUDA(cudaDeviceGetAttribute(&e->n_sms, cudaDevAttrMultiProcessorCount, dev));
+    if (narrow.n_res() == 0) CF_TRY(simt_create(narrow, &e->simt));
     const HostModel hm = pad_model(narrow);          // everything below, the operand format included, sees C = 32 / H = 64
 #ifdef CF_TRACE_PROBES
     e->trace_path = getenv("CF_TC_TRACE");
@@ -265,13 +257,12 @@ TcEngine* tc_create(const HostModel& narrow) {
             fp = reinterpret_cast<float*>(blk);
             put_block1(4 * b);
         }
-        uint8_t* dev_blocks = tc_upload(e, all);
-        e->conv_params = dev_blocks;
-        if (n_extra > 0) e->block_params = dev_blocks + ConvParams::kBytes;
+        CF_TRY(e->conv_params.upload(all));
         e->conv_nres = hm.n_res();
     }
+    e->layers.resize(hm.n_rnn());
     for (int l = 0; l < hm.n_rnn(); ++l) {
-        TcLayer L;
+        TcLayer& L = e->layers[l];
         L.in = hm.gru[2 * l].in;
         // The layer fed by the conv stack stays bf16x3: it contributes nearly all of f16e5's extra error
         // (emulation: 5.8e-5 of 6.1e-5; conv activations span 2^-10 .. 60 and would need an fp16 range
@@ -287,12 +278,12 @@ TcEngine* tc_create(const HostModel& narrow) {
             pack(g.wgh.data(), kH, 2 * kH, 2 * kH, 0, &wf, kGateScale, 1 << 30, 1.f);
             pack(g.wch.data(), kH, kH, kH, 0, &wf, kCandScale, 1 << 30, 1.f);
         }
-        L.wfused = reinterpret_cast<uint8_t*>(tc_upload(e, wf));
+        CF_TRY(L.wfused.upload(wf));
         std::vector<float> bz(2 * kNX);
         for (int d = 0; d < 2; ++d)
             for (int j = 0; j < kNX; ++j)
                 bz[d * kNX + j] = hm.gru[2 * l + d].bx[j] * (j < 2 * kH ? kGateScale : kCandScale);
-        L.bz = tc_upload(e, bz);
+        CF_TRY(L.bz.upload(bz));
         if (L.in == 1) {
             // RNN-only layer 0 (neural_network.py:17-18): the x part of concat([x, h]) W is a rank-1 update
             // x_t * w_row, added to the bias in the epilogue of the fused kernel - no MMA
@@ -300,24 +291,17 @@ TcEngine* tc_create(const HostModel& narrow) {
             for (int d = 0; d < 2; ++d)
                 for (int j = 0; j < kNX; ++j)
                     wxz[d * kNX + j] = hm.gru[2 * l + d].wx[j] * (j < 2 * kH ? kGateScale : kCandScale);
-            L.wxz = tc_upload(e, wxz);
+            CF_TRY(L.wxz.upload(wxz));
         }
-        e->layers.push_back(L);
     }
-    e->head_w = tc_upload(e, hm.head_w);
+    CF_TRY(e->head_w.upload(hm.head_w));
     e->head_b = hm.head_b;
-    return e;
+    *out = std::move(e);
+    return CF_OK;
 }
 
 int tc_operand_format(const TcEngine* e) { return e ? e->fmt : 0; }
 bool tc_can_emit_bits(const TcEngine* e) { return e && !e->layers.empty(); }
-
-void tc_destroy(TcEngine* e) {
-    if (!e) return;
-    simt_destroy(e->simt);
-    for (void* p : e->owned) cudaFree(p);
-    delete e;
-}
 
 // ====================================================================== TK2: residual conv stack
 // Fuses, per tile of 128 windows: median/MAD normalisation of the raw signal, the 35-sample
@@ -1684,7 +1668,7 @@ int tc_reserve(const TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& 
     if (n_tiles <= 0) return CF_OK;
     const int64_t chunk = n_tiles < kTcChunkTiles ? n_tiles : kTcChunkTiles;
     CF_TRY(ws->ensure(tc_workspace_bytes(chunk)));
-    if (!e->conv_params) CF_TRY(simt_conv_stack_reserve(simt_ws, hm, chunk));
+    if (!e->conv_params.ptr) CF_TRY(simt_conv_stack_reserve(simt_ws, hm, chunk));
     return CF_OK;
 }
 
@@ -1739,16 +1723,17 @@ int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, co
         const int64_t rows = blocks * 128;
         const float* feat = nullptr;             // RNN-only networks: the normalised scalar input x [rows]
         const __nv_bfloat16* a_in = nullptr;
-        if (e->conv_params) {
+        if (e->conv_params.ptr) {
             ProfScope ps(prof, KC_K2_CONV, stream);
             const int grid = (int)std::min<int64_t>(tiles, e->n_sms);
             const bool fused_head = n_layers == 0 && e->conv_nres == 2;
             if (e->conv_nres >= 2)
-                tc_conv4_kernel<<<grid, 576, kConv4Smem, stream>>>(e->conv_params, raw, stats, xwin, tab.src, tab.valid,
-                                                                  tab.read, tile0, (int)tiles, a0,
-                                                                  fused_head ? e->head_w : nullptr, fused_head ? head_part : nullptr);
+                tc_conv4_kernel<<<grid, 576, kConv4Smem, stream>>>(e->conv_params.as<uint8_t>(), raw, stats, xwin, tab.src,
+                                                                  tab.valid, tab.read, tile0, (int)tiles, a0,
+                                                                  fused_head ? e->head_w.as<float>() : nullptr,
+                                                                  fused_head ? head_part : nullptr);
             else
-                tc_conv2_kernel<<<grid, 288, kConvSmem, stream>>>(e->conv_params, raw, stats, xwin, tab.src, tab.valid,
+                tc_conv2_kernel<<<grid, 288, kConvSmem, stream>>>(e->conv_params.as<uint8_t>(), raw, stats, xwin, tab.src, tab.valid,
                                                                   tab.read, tile0, (int)tiles, a0);
             CF_LAUNCHED();
             a_in = a0;
@@ -1756,13 +1741,13 @@ int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, co
             // writes it; the last block's output is never in ybuf[0], which GRU layer 0 writes while reading it
             for (int b = 2; b < e->conv_nres; ++b) {
                 __nv_bfloat16* out = a_in == a0 ? ybuf[1] : a0;
-                tc_conv_block_kernel<<<grid, 320, kBlockSmem, stream>>>(e->block_params + (size_t)(b - 2) * ConvParams::kBytes,
-                                                                        a_in, (int)tiles, out);
+                tc_conv_block_kernel<<<grid, 320, kBlockSmem, stream>>>(
+                    e->conv_params.as<uint8_t>() + (size_t)(b - 1) * ConvParams::kBytes, a_in, (int)tiles, out);
                 CF_LAUNCHED();
                 a_in = out;
             }
         } else {
-            CF_TRY(simt_conv_stack(e->simt, simt_ws, hm, raw, stats, xwin, tab, tile0, tiles, chunk, &feat, stream, prof));
+            CF_TRY(simt_conv_stack(e->simt.get(), simt_ws, hm, raw, stats, xwin, tab, tile0, tiles, chunk, &feat, stream, prof));
         }
         for (int l = 0; l < n_layers; ++l) {
             const TcLayer& L = e->layers[l];
@@ -1778,7 +1763,7 @@ int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, co
             }
 #endif
             const int grid2 = 2 * (int)std::min<int64_t>((tiles + 1) / 2, e->n_sms / 2);
-            const float* hw_l = last ? e->head_w : nullptr;
+            const float* hw_l = last ? e->head_w.as<float>() : nullptr;
             float* hp_l = last ? head_part : nullptr;
             // operand format of this layer and of the layer that reads its output
             const int fmt_out = last ? L.fmt : e->layers[l + 1].fmt;
@@ -1786,23 +1771,23 @@ int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, co
                 // scalar input (RNN-only layer 0): x part in the epilogue from the fp32 signal rows
                 if (L.fmt == kFmtF16E5)
                     tc_gru_fused2_kernel<1, 1, 1><<<grid2, kGruF2Threads, GruF2Cfg<1>::kSmem, stream>>>(
-                        L.wfused, L.bz, nullptr, yo, hw_l, hp_l, (int)tiles, nullptr, feat, L.wxz);
+                        L.wfused.as<uint8_t>(), L.bz.as<float>(), nullptr, yo, hw_l, hp_l, (int)tiles, nullptr, feat, L.wxz.as<float>());
                 else
                     tc_gru_fused2_kernel<1, 0, 0><<<grid2, kGruF2Threads, GruF2Cfg<1>::kSmem, stream>>>(
-                        L.wfused, L.bz, nullptr, yo, hw_l, hp_l, (int)tiles, nullptr, feat, L.wxz);
+                        L.wfused.as<uint8_t>(), L.bz.as<float>(), nullptr, yo, hw_l, hp_l, (int)tiles, nullptr, feat, L.wxz.as<float>());
             } else if (L.in == kC) {
                 if (fmt_out == kFmtF16E5)
                     tc_gru_fused2_kernel<32, 0, 1><<<grid2, kGruF2Threads, GruF2Cfg<32>::kSmem, stream>>>(
-                        L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, nullptr, nullptr, nullptr);
+                        L.wfused.as<uint8_t>(), L.bz.as<float>(), a_in, yo, hw_l, hp_l, (int)tiles, nullptr, nullptr, nullptr);
                 else
                     tc_gru_fused2_kernel<32, 0, 0><<<grid2, kGruF2Threads, GruF2Cfg<32>::kSmem, stream>>>(
-                        L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, nullptr, nullptr, nullptr);
+                        L.wfused.as<uint8_t>(), L.bz.as<float>(), a_in, yo, hw_l, hp_l, (int)tiles, nullptr, nullptr, nullptr);
             } else if (L.fmt == kFmtF16E5) {
                 tc_gru_fused2_kernel<128, 1, 1><<<grid2, kGruF2Threads, GruF2Cfg<128>::kSmem, stream>>>(
-                    L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, trace_dev, nullptr, nullptr);
+                    L.wfused.as<uint8_t>(), L.bz.as<float>(), a_in, yo, hw_l, hp_l, (int)tiles, trace_dev, nullptr, nullptr);
             } else {
                 tc_gru_fused2_kernel<128, 0, 0><<<grid2, kGruF2Threads, GruF2Cfg<128>::kSmem, stream>>>(
-                    L.wfused, L.bz, a_in, yo, hw_l, hp_l, (int)tiles, trace_dev, nullptr, nullptr);
+                    L.wfused.as<uint8_t>(), L.bz.as<float>(), a_in, yo, hw_l, hp_l, (int)tiles, trace_dev, nullptr, nullptr);
             }
             CF_LAUNCHED();
 #ifdef CF_TRACE_PROBES
@@ -1835,7 +1820,7 @@ int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, co
             // ResNet-only: dense on the conv output
             ProfScope ps(prof, KC_K5_HEAD, stream);
             tc_head_conv_kernel<<<(unsigned)tiles, 256, 0, stream>>>(
-                a_in, e->head_w, e->head_b, tab.src, tab.valid, tab.read, raw ? stats : nullptr, tile0, rows, probs, want_logits ? 1 : 0);
+                a_in, e->head_w.as<float>(), e->head_b, tab.src, tab.valid, tab.read, raw ? stats : nullptr, tile0, rows, probs, want_logits ? 1 : 0);
             CF_LAUNCHED();
         } else {
             // GRU head: the last layer's epilogue wrote eight partial dots per position (2 directions x 4 unit groups)
@@ -1939,7 +1924,6 @@ int tc_selftest_f16e5(const float* a_dev, int K, int N, const float* w_host, int
     tc_selftest_f16e5_kernel<<<1, 128, smem, stream>>>(a_dev, w.as<uint8_t>(), K, N, mode, out_dev);
     CF_LAUNCHED();
     CF_CUDA(cudaStreamSynchronize(stream));
-    w.release();
     return CF_OK;
 }
 

@@ -93,8 +93,9 @@ int cf_model_engine(const cf_model* model);
  * of the pass supports it and the GRU weights fit fp16's range); -1 = fp32 CUDA-core engine. */
 int cf_model_operand_format(const cf_model* model);
 
-/* Pre-size the handle's workspace so later calls do not allocate
- * (max total samples / reads per call).  Optional. */
+/* Pre-size the handle's buffers and engine workspaces (tensor-core engine: up to ~12.6 GB at a full pass
+ * of 2368 tiles) for calls of at most max_samples samples / max_reads reads, so that such calls do not
+ * allocate.  Optional: otherwise the first call that needs more allocates it. */
 int cf_model_reserve(cf_model* model, int64_t max_samples, int32_t max_reads);
 
 /*
@@ -164,9 +165,7 @@ typedef struct cf_exec cf_exec;
 int cf_exec_create(cf_model* model, cf_exec** out);
 /* Waits for the context's last work, then frees its buffers (and the model, if it was the last reference). */
 void cf_exec_destroy(cf_exec* ex);
-/* Pre-size one context's buffers for calls of at most max_samples samples / max_reads reads: what
- * cf_model_reserve sizes, and also the engine workspaces (tensor-core engine: up to ~12.6 GB at a
- * full pass of 2368 tiles), so that such calls allocate nothing. */
+/* cf_model_reserve on a context: pre-sizes its buffers and engine workspaces. */
 int cf_exec_reserve(cf_exec* ex, int64_t max_samples, int32_t max_reads);
 /* cf_infer_reads on a context: same arguments after the model, same semantics and outputs; asynchronous. */
 int cf_exec_infer_reads(cf_exec* ex, const int16_t* raw_dev, const int64_t* offsets_host,

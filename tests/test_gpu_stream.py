@@ -242,15 +242,24 @@ def test_context_outlives_model_handle():
     _cabi.check(lib.cf_infer_reads(model.handle, *c.args(s)))
     s.synchronize()
     want = c.result()
-    ex = ctypes.c_void_p()
+    ex, idle = ctypes.c_void_p(), ctypes.c_void_p()
     _cabi.check(lib.cf_exec_create(model.handle, ctypes.byref(ex)))
-    model.close()                                  # cf_model_destroy: the context keeps the weights alive
+    _cabi.check(lib.cf_exec_create(model.handle, ctypes.byref(idle)))
+    model.close()                                  # cf_model_destroy: the contexts keep the weights alive
+    lib.cf_exec_destroy(idle)                      # a context that never ran
     for _ in range(2):
         c = _Call(torch, lib, raw, off)
         _cabi.check(lib.cf_exec_infer_reads(ex, *c.args(s)))
         s.synchronize()
         _same(c.result(), want)
+    # the last reference goes while the context's last call is still in flight on another stream: destroying the
+    # context waits for that call before it frees the context and the weights
+    s2 = torch.cuda.Stream()
+    c = _Call(torch, lib, raw, off)
+    _cabi.check(lib.cf_exec_infer_reads(ex, *c.args(s2)))
     lib.cf_exec_destroy(ex)
+    s2.synchronize()
+    _same(c.result(), want)
 
 
 def test_two_threads_stream_through_one_model(shipped):
@@ -277,11 +286,16 @@ def test_two_threads_stream_through_one_model(shipped):
 
 @pytest.mark.parametrize("kind", ["RNN", "simt"])
 def test_reserved_context_matches_default_context(kind):
-    """cf_exec_reserve sizes the engine workspaces too (the CUDA-core one for the CUDA-core engine and for the
-    tensor-core engine's RNN-only input); a call within the reservation gives the default context's results."""
+    """cf_exec_reserve and cf_model_reserve size the engine workspaces too (the CUDA-core one for the CUDA-core engine
+    and for the tensor-core engine's RNN-only input); a call within the reservation gives the results of a default
+    context that was not reserved."""
     import torch
     lib = _cabi.load_library()
-    model = _model("RNN") if kind == "RNN" else neural_network.load_network("ResNetRNN", None, 30000, engine="simt")
+
+    def make():
+        return _model("RNN") if kind == "RNN" else neural_network.load_network("ResNetRNN", None, 30000, engine="simt")
+
+    model = make()
     raw, off = _batch(41, 20)
     s = torch.cuda.Stream()
     c = _Call(torch, lib, raw, off)
@@ -298,3 +312,10 @@ def test_reserved_context_matches_default_context(kind):
         _same(c.result(), want)
     finally:
         lib.cf_exec_destroy(ex)
+    # the default context of a second model with the same weights, reserved before its first call
+    reserved = make()
+    _cabi.check(lib.cf_model_reserve(reserved.handle, int(off[-1]), len(off) - 1))
+    c = _Call(torch, lib, raw, off)
+    _cabi.check(lib.cf_infer_reads(reserved.handle, *c.args(s)))
+    s.synchronize()
+    _same(c.result(), want)
