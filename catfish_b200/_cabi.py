@@ -78,6 +78,11 @@ SIGNATURES = {
                                     ctypes.c_int64, c_void, c_void]),
     "cf_validate_windows": (ctypes.c_int, [c_void, c_void, c_void, ctypes.c_int64, ctypes.c_int64, ctypes.c_double, c_i64_p,
                                            ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double), c_void]),
+    "cf_validate_windows_sweep": (ctypes.c_int, [c_void, c_void, c_void, ctypes.c_int64, ctypes.c_int64, c_void, ctypes.c_int32,
+                                                 c_i64_p, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double),
+                                                 c_void]),
+    "cf_sweep_thresholds": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int32, c_void, ctypes.c_int64, c_void, ctypes.c_int32,
+                                           c_i64_p, c_void]),
     "cf_vote_events": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int64, c_i64_p, ctypes.c_int64, ctypes.c_int64,
                                       ctypes.c_int64, c_void, c_i64_p, c_i64_p, c_i64_p, ctypes.POINTER(ctypes.c_int32),
                                       c_void]),

@@ -247,6 +247,7 @@ struct Exec {
     DevBuf tab_src, tab_valid, tab_read;
     DevBuf probs_internal;
     DevBuf val_logits, val_partial;  // validation row (N4)
+    DevBuf val_sweep;                // its threshold sweep (K11 scratch)
     IntervalScratch k6;
     // host-buffer entry point
     DevBuf h_raw, h_intervals, h_ioff, h_probs;
@@ -756,6 +757,7 @@ static int reserve(cf_model* m, cf::Exec* x, int64_t max_samples, int32_t max_re
     CF_TRY(x->wide_scratch.ensure(cf::k1_wide_scratch_bytes(cf::kWideSlots)));
     if (cf::stats_may_use_chunks(max_reads)) CF_TRY(x->k1_chunked.ensure(cf::k1_chunked_scratch_bytes(max_reads)));
     CF_TRY(x->probs_internal.ensure(sizeof(float) * (size_t)max_samples));
+    CF_TRY(x->val_sweep.ensure(cf::k11_scratch_bytes(cf::kSweepMaxThresholds)));
     if (m->engine == CF_ENGINE_TCGEN05) return cf::tc_reserve(m->tc.get(), &x->tc_ws, &x->simt_ws, m->hm, tiles);
     return cf::simt_reserve(&x->simt_ws, m->hm, tiles);
 }
@@ -789,17 +791,10 @@ int cf_infer_windows(cf_model* m, const float* x_dev, int64_t n_windows, float* 
     return cf::engine_forward(m, x, nullptr, nullptr, x_dev, tab, tiles, probs_dev, st);
 }
 
-int cf_validate_windows(cf_model* m, const float* x_dev, const uint8_t* labels_dev, int64_t n_windows,
-                        int64_t padding_size, double threshold, int64_t* counts_out, double* accuracy_out,
-                        double* loss_out, void* stream) {
-    if (!m || n_windows <= 0 || !x_dev || !labels_dev || padding_size < 0 || !counts_out) {
-        cf::set_error("cf_validate_windows: bad argument");
-        return CF_ERR_BAD_ARG;
-    }
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cf::Exec* x = m->def.get();
-    cf::CallScope call(x);
-    CF_TRY(call.enter(m->device, st));
+// The forward pass of the validation row: the logits of n_windows dense windows into x->val_logits, then K9 over
+// all n_windows * 35 positions at `threshold`.  *result (device): tp, fp, tn, fn, correct (int64) | loss sum (double).
+static int validate_forward(cf_model* m, cf::Exec* x, const float* x_dev, const uint8_t* labels_dev, int64_t n_windows,
+                            double threshold, cudaStream_t st, const long long** result) {
     const int64_t n = n_windows * cf::kWindow;
     const int64_t tiles = cf::ceil_div(n_windows, cf::kTileWindows);
     const int blocks = cf::k9_validation_blocks(n);
@@ -813,8 +808,45 @@ int cf_validate_windows(cf_model* m, const float* x_dev, const uint8_t* labels_d
     CF_TRY(cf::engine_forward(m, x, nullptr, nullptr, x_dev, tab, tiles, x->val_logits.as<float>(), st,
                               /*want_logits=*/true));
     long long* partial = x->val_partial.as<long long>();
-    long long* result = partial + (size_t)blocks * 6;
-    CF_TRY(cf::k9_validate(x->val_logits.as<float>(), labels_dev, n, threshold, partial, result, st));
+    long long* res = partial + (size_t)blocks * 6;
+    CF_TRY(cf::k9_validate(x->val_logits.as<float>(), labels_dev, n, threshold, partial, res, st));
+    *result = res;
+    return CF_OK;
+}
+
+// K9's accuracy and mean loss from its result (host copy) over n positions.
+static void validate_means(const long long* host, int64_t n, double* accuracy_out, double* loss_out) {
+    double loss_sum;
+    std::memcpy(&loss_sum, &host[5], sizeof(double));
+    if (accuracy_out) *accuracy_out = (double)host[4] / (double)n;
+    if (loss_out) *loss_out = loss_sum / (double)n;
+}
+
+// K11's counts (sorted-threshold order) to the caller's threshold order, tn minus tn_shift.
+static void sweep_scatter(const std::vector<long long>& sorted_counts, const std::vector<int>& index, int64_t tn_shift,
+                          int64_t* out) {
+    for (size_t i = 0; i < index.size(); ++i) {
+        const long long* c = sorted_counts.data() + 4 * (size_t)index[i];
+        out[4 * i + 0] = c[0];
+        out[4 * i + 1] = c[1];
+        out[4 * i + 2] = c[2] - tn_shift;
+        out[4 * i + 3] = c[3];
+    }
+}
+
+int cf_validate_windows(cf_model* m, const float* x_dev, const uint8_t* labels_dev, int64_t n_windows,
+                        int64_t padding_size, double threshold, int64_t* counts_out, double* accuracy_out,
+                        double* loss_out, void* stream) {
+    if (!m || n_windows <= 0 || !x_dev || !labels_dev || padding_size < 0 || !counts_out) {
+        cf::set_error("cf_validate_windows: bad argument");
+        return CF_ERR_BAD_ARG;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    cf::Exec* x = m->def.get();
+    cf::CallScope call(x);
+    CF_TRY(call.enter(m->device, st));
+    const long long* result;
+    CF_TRY(validate_forward(m, x, x_dev, labels_dev, n_windows, threshold, st, &result));
     long long host[6];
     CF_CUDA(cudaMemcpyAsync(host, result, sizeof(host), cudaMemcpyDeviceToHost, st));
     CF_CUDA(cudaStreamSynchronize(st));
@@ -822,10 +854,67 @@ int cf_validate_windows(cf_model* m, const float* x_dev, const uint8_t* labels_d
     counts_out[1] = host[1];
     counts_out[2] = host[2] - padding_size;      // rnn_class.py:247
     counts_out[3] = host[3];
-    double loss_sum;
-    std::memcpy(&loss_sum, &host[5], sizeof(double));
-    if (accuracy_out) *accuracy_out = (double)host[4] / (double)n;
-    if (loss_out) *loss_out = loss_sum / (double)n;
+    validate_means(host, n_windows * cf::kWindow, accuracy_out, loss_out);
+    return CF_OK;
+}
+
+int cf_validate_windows_sweep(cf_model* m, const float* x_dev, const uint8_t* labels_dev, int64_t n_windows,
+                              int64_t padding_size, const double* thresholds_host, int32_t n_thresholds,
+                              int64_t* counts_out_host, double* accuracy_out, double* loss_out, void* stream) {
+    if (!m || n_windows <= 0 || !x_dev || !labels_dev || padding_size < 0 || !counts_out_host) {
+        cf::set_error("cf_validate_windows_sweep: bad argument");
+        return CF_ERR_BAD_ARG;
+    }
+    std::vector<float> sorted;
+    std::vector<int> index;
+    CF_TRY(cf::k11_prepare_thresholds(thresholds_host, n_thresholds, &sorted, &index));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    cf::Exec* x = m->def.get();
+    cf::CallScope call(x);
+    CF_TRY(call.enter(m->device, st));
+    CF_TRY(x->val_sweep.ensure(cf::k11_scratch_bytes((int)sorted.size())));
+    const long long* result;
+    // K9's counts at 0.5 are not used: it runs for the accuracy and the loss, which no threshold changes
+    CF_TRY(validate_forward(m, x, x_dev, labels_dev, n_windows, 0.5, st, &result));
+    const int64_t n = n_windows * cf::kWindow;
+    std::vector<long long> counts(4 * sorted.size());
+    CF_TRY(cf::k11_sweep(x->val_logits.as<float>(), true, labels_dev, n, sorted, x->val_sweep.ptr, counts.data(), st));
+    long long host[6];
+    CF_CUDA(cudaMemcpyAsync(host, result, sizeof(host), cudaMemcpyDeviceToHost, st));
+    CF_CUDA(cudaStreamSynchronize(st));
+    sweep_scatter(counts, index, padding_size, counts_out_host);      // rnn_class.py:247 at every threshold
+    validate_means(host, n, accuracy_out, loss_out);
+    return CF_OK;
+}
+
+int cf_sweep_thresholds(int32_t device, const float* values_dev, int32_t values_are_logits, const uint8_t* labels_dev,
+                        int64_t n, const double* thresholds_host, int32_t n_thresholds, int64_t* counts_out_host,
+                        void* stream) {
+    if (n < 0 || !counts_out_host || (n > 0 && (!values_dev || !labels_dev))) {
+        cf::set_error("cf_sweep_thresholds: bad argument");
+        return CF_ERR_BAD_ARG;
+    }
+    std::vector<float> sorted;
+    std::vector<int> index;
+    CF_TRY(cf::k11_prepare_thresholds(thresholds_host, n_thresholds, &sorted, &index));
+    if (n == 0) {
+        std::fill(counts_out_host, counts_out_host + 4 * (size_t)n_thresholds, 0);
+        return CF_OK;
+    }
+    cf::DeviceGuard guard;
+    CF_TRY(guard.set(device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    cf::DevBuf scratch;
+    CF_TRY(scratch.ensure(cf::k11_scratch_bytes((int)sorted.size())));
+    std::vector<long long> counts(4 * sorted.size());
+    const int s = cf::k11_sweep(values_dev, values_are_logits != 0, labels_dev, n, sorted, scratch.ptr, counts.data(), st);
+    const cudaError_t e = cudaStreamSynchronize(st);    // scratch is freed on return, also after a failed launch
+    CF_TRY(s);
+    if (e != cudaSuccess) {
+        cf::set_error("cf_sweep_thresholds: %s", cudaGetErrorString(e));
+        return CF_ERR_CUDA;
+    }
+    sweep_scatter(counts, index, 0, counts_out_host);
     return CF_OK;
 }
 

@@ -237,6 +237,19 @@ int k9_validation_blocks(int64_t n);
 int k9_validate(const float* logits, const uint8_t* labels, int64_t n, double threshold, long long* partial,
                 long long* result, cudaStream_t stream);
 
+// ---------------------------------------------------------------- k11: threshold sweep
+constexpr int kSweepMaxThresholds = 4096;   // 3 x 4097 uint32 counters = 48 KiB of shared memory per block
+// Checks the caller's thresholds (1..kSweepMaxThresholds, none NaN) and turns them into the sorted, deduplicated
+// float thresholds K11 compares with; index[i] is the position of caller threshold i in `sorted`.
+int k11_prepare_thresholds(const double* thresholds, int n_thresholds, std::vector<float>* sorted,
+                           std::vector<int>* index);
+// Device scratch of k11_sweep for n_thresholds thresholds.
+size_t k11_scratch_bytes(int n_thresholds);
+// Enqueues the sweep over n values (probabilities, or logits with values_are_logits) and the copy of the counts,
+// int64 [sorted.size()][4] = tp, fp, tn, fn in sorted order, to counts_host; the caller synchronises the stream.
+int k11_sweep(const float* values, bool values_are_logits, const uint8_t* labels, int64_t n,
+              const std::vector<float>& sorted, void* scratch, long long* counts_host, cudaStream_t stream);
+
 // ---------------------------------------------------------------- k10: event voting (next row N3)
 int k10_vote_events(const double* scores, int64_t n_scores, const int64_t* ev_begin, int64_t first_event,
                     int64_t n_voted, int32_t* classes, int32_t* empty_flag, cudaStream_t stream);

@@ -10,6 +10,7 @@ infer_class_from_signal :12   infer_class_from_signal     cf_infer_reads_host
 (array-level twins)           infer_class_from_raw,       cf_infer_reads_host
                               infer_reads
 (the CLI's per-file loop)     infer_stream                cf_exec_infer_reads
+(precision_recall_ROC.py)     evaluate_reads              cf_infer_reads + cf_sweep_thresholds
 process_signal :77            process_signal (h5py)       cf_normalize_reads
 normalize_raw_signal :96      normalize_raw_signal        cf_normalize_reads
 reshape_input :108            reshape_input               (pure reshape, host)
@@ -279,6 +280,82 @@ def _infer_reads_pipelined(arrays, offsets, model, threshold, min_run, ext_left,
         parts = [iv_pin[int(cap_off[g]):int(cap_off[g]) + n_g] for g, n_g in enumerate(found) if n_g]
         intervals = np.concatenate(parts) if parts else np.zeros((0, 2), np.int64)
     return intervals, ioff
+
+
+def evaluate_reads(raws, labels, model, thresholds, window_size=35):
+    """Confusion counts of labelled raw reads at every threshold: int64 ``[T, 4]`` rows of (tp, fp, tn, fn), in the
+    order of ``thresholds`` (1..4096 of them, unsorted / repeated allowed).
+
+    ``labels[i]`` holds one label per sample of ``raws[i]`` (0 / 1; other small integers count as
+    ``metrics.confusion_matrix`` counts them).  The reads take the production path - median / MAD normalisation,
+    windowing, network - with the probabilities left on the device, and every real sample is counted at every
+    threshold on the device (``cf_sweep_thresholds``; padding never enters: the probabilities are already unpadded).
+    Row i equals ``metrics.confusion_matrix`` of the labels against ``scores >= thresholds[i]`` for the scores
+    ``infer_reads(..., return_scores=True)`` gives; reads with MAD = 0 have NaN scores, predicted 0 everywhere.
+    Batches are processed in groups of about one engine pass; no probability travels to the host."""
+    if window_size != model.window:
+        raise ValueError("window_size must equal the model's window (%d)" % model.window)
+    arrays = [_as_int16(r) for r in raws]
+    labels = list(labels)
+    if len(labels) != len(arrays):
+        raise ValueError("one label array per read is needed (%d reads, %d label arrays)" % (len(arrays), len(labels)))
+    labs = []
+    for r, (a, y) in enumerate(zip(arrays, labels)):
+        if a.size == 0:
+            raise IndexError("list index out of range")        # infer.py:184 on an empty read
+        y = np.asarray(y).reshape(-1)
+        if y.size != a.size:
+            raise ValueError("read %d has %d samples and %d labels" % (r, a.size, y.size))
+        y8 = y.astype(np.uint8)
+        if not np.array_equal(y8, y):
+            raise ValueError("labels must be small non-negative integers")
+        labs.append(y8)
+    th = np.ascontiguousarray(np.asarray(thresholds, dtype=np.float64).reshape(-1))
+    n_th = min(th.size, 2 ** 31 - 1)
+    counts = np.zeros((th.size, 4), np.int64)
+    lib = _cabi.load_library()
+    # no positions: checks the thresholds on the host, before any device work, and leaves the counts at zero
+    _cabi.check(lib.cf_sweep_thresholds(0, None, 0, None, 0, th.ctypes.data, n_th, counts.ctypes.data_as(_cabi.c_i64_p),
+                                        None))
+    if not arrays:
+        return counts
+    torch = _torch()
+    dev = int(model.device)
+    n_reads = len(arrays)
+    offsets = np.zeros(n_reads + 1, np.int64)
+    np.cumsum([a.size for a in arrays], out=offsets[1:])
+    cuts = [0]                                                 # groups of whole reads, about one engine pass each
+    while cuts[-1] < n_reads:
+        lo = cuts[-1]
+        hi = int(np.searchsorted(offsets, offsets[lo] + _GROUP_SAMPLES, side="right")) - 1
+        cuts.append(min(n_reads, max(hi, lo + 1)))
+    groups = list(zip(cuts[:-1], cuts[1:]))
+    most = max(int(offsets[hi] - offsets[lo]) for lo, hi in groups)
+    part = np.zeros_like(counts)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream()
+        stage = _staging(torch, dev, most)
+        lab_pin = torch.empty(most, dtype=torch.uint8).pin_memory()
+        raw_d = torch.empty(most, dtype=torch.int16, device="cuda")
+        lab_d = torch.empty(most, dtype=torch.uint8, device="cuda")
+        probs = torch.empty(most, dtype=torch.float32, device="cuda")
+        ioff = torch.empty(max(hi - lo for lo, hi in groups) + 1, dtype=torch.int64, device="cuda")
+        for lo, hi in groups:
+            off_g = np.ascontiguousarray(offsets[lo:hi + 1] - offsets[lo])
+            n = int(off_g[-1])
+            _concat_into(stage.numpy()[:n], arrays[lo:hi], off_g)
+            np.concatenate(labs[lo:hi], out=lab_pin.numpy()[:n])
+            raw_d[:n].copy_(stage[:n], non_blocking=True)
+            lab_d[:n].copy_(lab_pin[:n], non_blocking=True)
+            # intervals are not wanted: capacity 0 (the per-read interval counts still land in ioff)
+            _cabi.check(lib.cf_infer_reads(model.handle, raw_d.data_ptr(), _offsets_ptr(off_g), hi - lo,
+                                           probs.data_ptr(), None, ioff.data_ptr(), 0, 0.5, 15, 11, 16,
+                                           stream.cuda_stream))
+            # synchronises: the pinned staging is free again for the next group
+            _cabi.check(lib.cf_sweep_thresholds(dev, probs.data_ptr(), 0, lab_d.data_ptr(), n, th.ctypes.data, n_th,
+                                                part.ctypes.data_as(_cabi.c_i64_p), stream.cuda_stream))
+            counts += part
+    return counts
 
 
 _STREAM_DEPTH = 2                       # groups in flight in infer_stream

@@ -47,6 +47,7 @@ class RNN(object):
         self._handle = None
         self._weights = None
         self.tp = self.fp = self.tn = self.fn = 0
+        self.sweep_counts = None        # test_network_sweep's [T, 4] accumulator (reset_sweep)
 
     # ------------------------------------------------------------------ hyper-parameters
     def _hpm(self):
@@ -150,16 +151,7 @@ class RNN(object):
         ``padding_size``, :247) and returns ``(test_acc, test_loss)`` over all positions,
         padding included, like the reference's ``sess.run([self.accuracy, self.loss])``."""
         import torch
-        x = np.ascontiguousarray(np.asarray(test_x, dtype=np.float32))
-        if x.ndim != 3 or x.shape[1] != self.window or x.shape[2] != self.n_inputs:
-            raise ValueError("Cannot feed value of shape %s for Tensor 'data/Placeholder:0', "
-                             "which has shape '(?, %d, %d)'" % (x.shape, self.window, self.n_inputs))
-        y = np.asarray(test_y).reshape(-1)
-        if y.size != x.shape[0] * self.window:
-            raise ValueError("Length of labels to compare is not equal.")
-        y8 = y.astype(np.uint8)
-        if not np.array_equal(y8, y):
-            raise ValueError("labels must be small non-negative integers")
+        x, y8 = self._validation_arrays(test_x, test_y)
         n_windows = x.shape[0]
         dev = torch.device("cuda", self.device)
         counts = np.zeros(4, np.int64)
@@ -176,6 +168,51 @@ class RNN(object):
         self.tn += int(counts[2])
         self.fn += int(counts[3])
         return np.float32(acc.value), np.float32(loss.value)
+
+    def test_network_sweep(self, test_x, test_y, thresholds, padding_size=0):
+        """``test_network`` at every threshold of ``thresholds`` (unsorted / repeated allowed, 1..4096 of them) from
+        ONE forward pass.  Adds the int64 ``[T, 4]`` rows (tp, fp, tn - padding_size, fn), in the order given, to
+        ``self.sweep_counts`` (cleared by ``reset_sweep``; a sweep over another number of thresholds needs a reset
+        first) and returns ``(test_acc, test_loss)`` exactly as ``test_network`` does: neither depends on the
+        threshold.  Row i equals what ``test_network(..., threshold=thresholds[i])`` adds to tp / fp / tn / fn."""
+        import torch
+        x, y8 = self._validation_arrays(test_x, test_y)
+        th = np.ascontiguousarray(np.asarray(thresholds, dtype=np.float64).reshape(-1))
+        if self.sweep_counts is not None and self.sweep_counts.shape[0] != th.size:
+            raise ValueError("sweep_counts holds %d thresholds, this sweep has %d: call reset_sweep() first"
+                             % (self.sweep_counts.shape[0], th.size))
+        n_windows = x.shape[0]
+        dev = torch.device("cuda", self.device)
+        counts = np.zeros((th.size, 4), np.int64)
+        acc, loss = ctypes.c_double(), ctypes.c_double()
+        with torch.cuda.device(dev):
+            xd = torch.from_numpy(x.reshape(n_windows, self.window)).to(dev)
+            yd = torch.from_numpy(np.ascontiguousarray(y8)).to(dev)
+            stream = torch.cuda.current_stream(dev)
+            _cabi.check(_cabi.load_library().cf_validate_windows_sweep(
+                self.handle, xd.data_ptr(), yd.data_ptr(), n_windows, int(padding_size), th.ctypes.data,
+                min(th.size, 2 ** 31 - 1), counts.ctypes.data_as(_cabi.c_i64_p), ctypes.byref(acc), ctypes.byref(loss),
+                stream.cuda_stream))
+        self.sweep_counts = counts if self.sweep_counts is None else self.sweep_counts + counts
+        return np.float32(acc.value), np.float32(loss.value)
+
+    def reset_sweep(self):
+        """Clear ``self.sweep_counts``."""
+        self.sweep_counts = None
+
+    def _validation_arrays(self, test_x, test_y):
+        """The padded ``[n_windows, 35, 1]`` input as float32 and its labels as uint8, checked."""
+        x = np.ascontiguousarray(np.asarray(test_x, dtype=np.float32))
+        if x.ndim != 3 or x.shape[1] != self.window or x.shape[2] != self.n_inputs:
+            raise ValueError("Cannot feed value of shape %s for Tensor 'data/Placeholder:0', "
+                             "which has shape '(?, %d, %d)'" % (x.shape, self.window, self.n_inputs))
+        y = np.asarray(test_y).reshape(-1)
+        if y.size != x.shape[0] * self.window:
+            raise ValueError("Length of labels to compare is not equal.")
+        y8 = y.astype(np.uint8)
+        if not np.array_equal(y8, y):
+            raise ValueError("labels must be small non-negative integers")
+        return x, y8
 
     def _release(self):
         if getattr(self, "_handle", None) is not None:

@@ -272,6 +272,29 @@ int cf_validate_windows(cf_model* model, const float* x_dev, const uint8_t* labe
                         double* loss_out, void* stream);
 
 /*
+ * Threshold sweeps (K11; the reference's networks/precision_recall_ROC.py thresholds the scores once per point):
+ * confusion counts at up to 4096 thresholds from one pass over the scores.  A position is predicted 1 at
+ * threshold t when (double)p >= t (class_from_threshold, infer.py:128); NaN scores are predicted 0 at every
+ * threshold; labels other than 0 / 1 count as metrics.confusion_matrix counts them (a positive is a TP only for
+ * label 1, a negative a TN only for label 0).  thresholds_host may be unsorted and may repeat; 1 <= n_thresholds
+ * <= 4096 and no threshold NaN, else CF_ERR_BAD_ARG.  counts_out_host int64 [n_thresholds][4] = tp, fp, tn, fn,
+ * in the caller's threshold order.  Integer counts: the result is exact and deterministic.
+ */
+/* Confusion counts at T thresholds over n positions.  values_dev holds probabilities (values_are_logits = 0) or
+ * logits (1; p = 1 / (1 + exp(-z)) in fp32, as K9 and the head kernels).  labels_dev uint8 [n].  Needs no model:
+ * scratch is allocated and freed inside.  Synchronises. */
+int cf_sweep_thresholds(int32_t device, const float* values_dev, int32_t values_are_logits, const uint8_t* labels_dev,
+                        int64_t n, const double* thresholds_host, int32_t n_thresholds, int64_t* counts_out_host,
+                        void* stream);
+
+/* cf_validate_windows at T thresholds, one forward pass: per threshold tn has padding_size subtracted
+ * (rnn_class.py:247); accuracy / loss do not depend on the threshold and are returned once (either may be NULL).
+ * Runs on the model's default context.  Synchronises. */
+int cf_validate_windows_sweep(cf_model* model, const float* x_dev, const uint8_t* labels_dev, int64_t n_windows,
+                              int64_t padding_size, const double* thresholds_host, int32_t n_thresholds,
+                              int64_t* counts_out_host, double* accuracy_out, double* loss_out, void* stream);
+
+/*
  * cf_vote_events - "next" row N3: the arithmetic of correct_events (networks/correct_output.py:38-61,
  * unfinished in the reference): walk the events as the reference's loop does (start found at the
  * first event whose first measurement is >= start; stop before the event that would pass `length`,
