@@ -6,8 +6,8 @@ the arithmetic runs on the GPU through the C ABI (include/catfish_b200.h):
 ===========================  ==========================  =========================
 reference (catfish/infer.py)  here                        C-ABI entry
 ===========================  ==========================  =========================
-infer_class_from_signal :12   infer_class_from_signal     cf_infer_reads_host
-(array-level twins)           infer_class_from_raw,       cf_infer_reads_host
+infer_class_from_signal :12   infer_class_from_signal     cf_infer_reads
+(array-level twins)           infer_class_from_raw,       cf_infer_reads
                               infer_reads
 (the CLI's per-file loop)     infer_stream                cf_exec_infer_reads
 (precision_recall_ROC.py)     evaluate_reads              cf_infer_reads + cf_sweep_thresholds
@@ -32,8 +32,6 @@ import time
 import numpy as np
 
 from . import _cabi
-
-_STAGING = {}        # device index -> pinned int16 torch tensor the ragged batch is concatenated into
 
 
 class IntervalList(collections.abc.Sequence):
@@ -109,15 +107,6 @@ def _concat_into(stage, arrays, offsets):
         j.result()
 
 
-def _staging(torch, device, n):
-    """Pinned host buffer of at least n int16 samples for `device` (grows geometrically, reused across calls)."""
-    buf = _STAGING.get(device)
-    if buf is None or buf.numel() < n:
-        buf = torch.empty(max(n + n // 4, 1 << 20), dtype=torch.int16).pin_memory()
-        _STAGING[device] = buf
-    return buf
-
-
 def _torch():
     import torch
     if not torch.cuda.is_available():
@@ -158,10 +147,10 @@ def infer_reads(raws, model, threshold=0.5, min_run=15, extension_left=11, exten
 
     Returns ``(hps, lengths)`` - per read the [start, end] intervals (an ``IntervalList``: list-like, Python
     ints on access, as the reference) and ``len(labels)`` - plus the per-position float32 scores when
-    ``return_scores`` is set.  One C-ABI call: host->device copy of the signal, median/MAD
-    normalisation, windowing, network, threshold / short-run removal / interval emission,
-    device->host copy of the results.  The ragged batch is concatenated straight into a pinned staging
-    buffer (one host pass, then DMA at PCIe rate instead of a pageable copy)."""
+    ``return_scores`` is set.  The batch runs as groups of whole reads, about one engine pass each (the first a
+    quarter pass, so that the device starts early), with two groups in flight: while the device works on one group
+    (``cf_infer_reads``: median/MAD normalisation, windowing, network, threshold / short-run removal / interval
+    emission), the host concatenates the next one straight into pinned staging and starts its copy."""
     res = infer_reads_arrays(raws, model, threshold, min_run, extension_left, extension_right, window_size,
                              return_scores)
     intervals, ioff, lengths = res[0], res[1], res[2]
@@ -182,104 +171,36 @@ def infer_reads_arrays(raws, model, threshold=0.5, min_run=15, extension_left=11
     for a in arrays:
         if a.size == 0:
             raise IndexError("list index out of range")        # infer.py:184 on an empty read
-    n_reads = len(arrays)
     lengths = np.array([a.size for a in arrays], np.int64)
-    offsets = np.zeros(n_reads + 1, np.int64)
+    offsets = np.zeros(len(arrays) + 1, np.int64)
     np.cumsum(lengths, out=offsets[1:])
-    total = int(offsets[-1])
-    if total >= _PIPELINE_MIN_SAMPLES and not return_scores:
-        intervals, ioff = _infer_reads_pipelined(arrays, offsets, model, threshold, min_run, extension_left,
-                                                 extension_right)
-        return intervals, ioff, lengths
-    if n_reads:
-        stage = _staging(_torch(), int(model.device), total).numpy()[:total]
-        _concat_into(stage, arrays, offsets)
-        raw = stage
-    else:
-        raw = np.zeros(0, np.int16)
-    res = infer_concatenated(raw, offsets, model, threshold, min_run, extension_left, extension_right,
-                             return_scores)
+    params = (float(threshold), int(min_run), int(extension_left), int(extension_right))
+    results = _run_on_model(model, [(arrays[lo:hi], params, return_scores)
+                                    for lo, hi in _cut_groups(offsets, _FIRST_GROUP_SAMPLES, _GROUP_SAMPLES)])
+    intervals, ioff = np.zeros((0, 2), np.int64), np.zeros(len(arrays) + 1, np.int64)
+    if results:
+        intervals = np.concatenate([iv for _, iv, _, _ in results])
+        np.cumsum(np.concatenate([np.diff(ioff_g) for _, _, ioff_g, _ in results]), out=ioff[1:])
     if return_scores:
-        scores = [res[2][int(offsets[r]):int(offsets[r + 1])] for r in range(n_reads)]
-        return res[0], res[1], lengths, scores
-    return res[0], res[1], lengths
+        scores = [s[int(off[r]):int(off[r + 1])] for off, _, _, s in results for r in range(len(off) - 1)]
+        return intervals, ioff, lengths, scores
+    return intervals, ioff, lengths
 
 
-_PIPELINE_MIN_SAMPLES = 24_000_000      # batches of at least ~2 engine passes take the pipelined path
 _GROUP_SAMPLES = 10_400_000             # one engine pass (2368 tiles of 128 windows) per group
-_FIRST_GROUP_SAMPLES = 2_600_000       # a quarter pass, see _infer_reads_pipelined
-_DEVBUF = {}                            # device index -> dict of cached device / pinned result buffers
+_FIRST_GROUP_SAMPLES = 2_600_000        # a quarter pass: the device starts after ~0.5 ms of staging instead of ~2 ms
+_DEPTH = 2                              # groups in flight of infer_reads_arrays and evaluate_reads
 
 
-def _infer_reads_pipelined(arrays, offsets, model, threshold, min_run, ext_left, ext_right):
-    """A large ragged batch as a pipeline of groups of whole reads (about one engine pass each): while the GPU
-    works on group g (asynchronous ``cf_infer_reads`` on the device-resident copy), the host concatenates
-    group g+1 into pinned staging and starts its copy - the host pass over the signal disappears behind the
-    kernels instead of preceding them.  Same results as one ``cf_infer_reads_host`` call (reads are independent;
-    batch invariance is part of the parity suite).  Returns (intervals [n, 2], interval_offsets [R + 1])."""
-    torch = _torch()
-    lib = _cabi.load_library()
-    dev = int(model.device)
-    n_reads = len(arrays)
-    total = int(offsets[-1])
-    # groups of consecutive reads
-    cuts = [0]
-    while cuts[-1] < n_reads:
-        lo = cuts[-1]
-        # the first group is a quarter pass: the GPU starts after ~0.5 ms of staging instead of ~2 ms
-        want = _GROUP_SAMPLES if lo else _FIRST_GROUP_SAMPLES
-        hi = int(np.searchsorted(offsets, offsets[lo] + want, side="right")) - 1
-        cuts.append(min(n_reads, max(hi, lo + 1)))
-    groups = list(zip(cuts[:-1], cuts[1:]))
-    caps = [int(lib.cf_max_intervals(int(offsets[hi] - offsets[lo]), hi - lo, min_run)) for lo, hi in groups]
-    cap_off = np.concatenate([[0], np.cumsum(caps)]).astype(np.int64)
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream()
-        buf = _DEVBUF.setdefault(dev, {})
-        if buf.get("n_raw", 0) < total:
-            buf["raw"] = torch.empty(total + total // 4, dtype=torch.int16, device="cuda")
-            buf["n_raw"] = buf["raw"].numel()
-        if buf.get("n_iv", 0) < cap_off[-1]:
-            buf["iv"] = torch.empty((int(cap_off[-1]) * 5 // 4, 2), dtype=torch.int64, device="cuda")
-            buf["iv_pin"] = torch.empty((int(cap_off[-1]) * 5 // 4, 2), dtype=torch.int64).pin_memory()
-            buf["n_iv"] = buf["iv"].shape[0]
-        n_off = n_reads + len(groups)
-        if buf.get("n_off", 0) < n_off:
-            buf["ioff"] = torch.empty(n_off * 2, dtype=torch.int64, device="cuda")
-            buf["ioff_pin"] = torch.empty(n_off * 2, dtype=torch.int64).pin_memory()
-            buf["n_off"] = n_off * 2
-        stage_t = _staging(torch, dev, total)
-        stage = stage_t.numpy()
-        raw_dev, iv_dev, ioff_dev = buf["raw"], buf["iv"], buf["ioff"]
-        for g, (lo, hi) in enumerate(groups):
-            a, b = int(offsets[lo]), int(offsets[hi])
-            _concat_into(stage[a:b], arrays[lo:hi], offsets[lo:hi + 1] - offsets[lo])
-            raw_dev[a:b].copy_(stage_t[a:b], non_blocking=True)
-            off_g = np.ascontiguousarray(offsets[lo:hi + 1])
-            _cabi.check(lib.cf_infer_reads(
-                model.handle, raw_dev.data_ptr(), _offsets_ptr(off_g), hi - lo, None,
-                iv_dev.data_ptr() + 16 * int(cap_off[g]), ioff_dev.data_ptr() + 8 * (lo + g), caps[g],
-                float(threshold), int(min_run), int(ext_left), int(ext_right), stream.cuda_stream))
-        buf["ioff_pin"][:n_off].copy_(ioff_dev[:n_off], non_blocking=True)
-        stream.synchronize()
-        ioff_all = buf["ioff_pin"].numpy()
-        ioff = np.zeros(n_reads + 1, np.int64)
-        found = []
-        for g, (lo, hi) in enumerate(groups):
-            local = ioff_all[lo + g:hi + g + 1]
-            n_g = int(local[-1])
-            if n_g > caps[g]:
-                raise _cabi.CatfishError("interval capacity exceeded (%d > %d)" % (n_g, caps[g]))
-            ioff[lo + 1:hi + 1] = ioff[lo] + local[1:]
-            found.append(n_g)
-            if n_g:
-                c0 = int(cap_off[g])
-                buf["iv_pin"][c0:c0 + n_g].copy_(iv_dev[c0:c0 + n_g], non_blocking=True)
-        stream.synchronize()
-        iv_pin = buf["iv_pin"].numpy()
-        parts = [iv_pin[int(cap_off[g]):int(cap_off[g]) + n_g] for g, n_g in enumerate(found) if n_g]
-        intervals = np.concatenate(parts) if parts else np.zeros((0, 2), np.int64)
-    return intervals, ioff
+def _cut_groups(offsets, first, later):
+    """``(lo, hi)`` ranges of consecutive whole reads, in order, of the batch with CSR ``offsets``: the first group
+    holds at most ``first`` samples, every later one at most ``later``, unless a single read is longer."""
+    groups, lo, want = [], 0, first
+    while lo < len(offsets) - 1:
+        hi = max(int(np.searchsorted(offsets, offsets[lo] + want, side="right")) - 1, lo + 1)
+        groups.append((lo, hi))
+        lo, want = hi, later
+    return groups
 
 
 def evaluate_reads(raws, labels, model, thresholds, window_size=35):
@@ -311,50 +232,18 @@ def evaluate_reads(raws, labels, model, thresholds, window_size=35):
             raise ValueError("labels must be small non-negative integers")
         labs.append(y8)
     th = np.ascontiguousarray(np.asarray(thresholds, dtype=np.float64).reshape(-1))
-    n_th = min(th.size, 2 ** 31 - 1)
     counts = np.zeros((th.size, 4), np.int64)
-    lib = _cabi.load_library()
     # no positions: checks the thresholds on the host, before any device work, and leaves the counts at zero
-    _cabi.check(lib.cf_sweep_thresholds(0, None, 0, None, 0, th.ctypes.data, n_th, counts.ctypes.data_as(_cabi.c_i64_p),
-                                        None))
+    _cabi.check(_cabi.load_library().cf_sweep_thresholds(0, None, 0, None, 0, th.ctypes.data, min(th.size, 2 ** 31 - 1),
+                                                         counts.ctypes.data_as(_cabi.c_i64_p), None))
     if not arrays:
         return counts
-    torch = _torch()
-    dev = int(model.device)
-    n_reads = len(arrays)
-    offsets = np.zeros(n_reads + 1, np.int64)
+    offsets = np.zeros(len(arrays) + 1, np.int64)
     np.cumsum([a.size for a in arrays], out=offsets[1:])
-    cuts = [0]                                                 # groups of whole reads, about one engine pass each
-    while cuts[-1] < n_reads:
-        lo = cuts[-1]
-        hi = int(np.searchsorted(offsets, offsets[lo] + _GROUP_SAMPLES, side="right")) - 1
-        cuts.append(min(n_reads, max(hi, lo + 1)))
-    groups = list(zip(cuts[:-1], cuts[1:]))
-    most = max(int(offsets[hi] - offsets[lo]) for lo, hi in groups)
-    part = np.zeros_like(counts)
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream()
-        stage = _staging(torch, dev, most)
-        lab_pin = torch.empty(most, dtype=torch.uint8).pin_memory()
-        raw_d = torch.empty(most, dtype=torch.int16, device="cuda")
-        lab_d = torch.empty(most, dtype=torch.uint8, device="cuda")
-        probs = torch.empty(most, dtype=torch.float32, device="cuda")
-        ioff = torch.empty(max(hi - lo for lo, hi in groups) + 1, dtype=torch.int64, device="cuda")
-        for lo, hi in groups:
-            off_g = np.ascontiguousarray(offsets[lo:hi + 1] - offsets[lo])
-            n = int(off_g[-1])
-            _concat_into(stage.numpy()[:n], arrays[lo:hi], off_g)
-            np.concatenate(labs[lo:hi], out=lab_pin.numpy()[:n])
-            raw_d[:n].copy_(stage[:n], non_blocking=True)
-            lab_d[:n].copy_(lab_pin[:n], non_blocking=True)
-            # intervals are not wanted: capacity 0 (the per-read interval counts still land in ioff)
-            _cabi.check(lib.cf_infer_reads(model.handle, raw_d.data_ptr(), _offsets_ptr(off_g), hi - lo,
-                                           probs.data_ptr(), None, ioff.data_ptr(), 0, 0.5, 15, 11, 16,
-                                           stream.cuda_stream))
-            # synchronises: the pinned staging is free again for the next group
-            _cabi.check(lib.cf_sweep_thresholds(dev, probs.data_ptr(), 0, lab_d.data_ptr(), n, th.ctypes.data, n_th,
-                                                part.ctypes.data_as(_cabi.c_i64_p), stream.cuda_stream))
-            counts += part
+    params = (0.5, 15, 11, 16)                                 # only the probabilities are used
+    for part in _run_on_model(model, [(arrays[lo:hi], params, False, labs[lo:hi], th)
+                                      for lo, hi in _cut_groups(offsets, _GROUP_SAMPLES, _GROUP_SAMPLES)]):
+        counts += part
     return counts
 
 
@@ -391,16 +280,23 @@ def infer_stream(reads, model, threshold=0.5, min_run=15, extension_left=11, ext
     return _stream(iter(reads), model, params, bool(return_scores), group_samples, max_wait_s, depth)
 
 
-class _StreamSlot(object):
-    """One group in flight of ``infer_stream``: an execution context of the model, a CUDA stream, and pinned / device
-    buffers that grow to the largest group the slot has run."""
+class _Slot(object):
+    """Runs one group of reads at a time: a CUDA stream, an event, pinned / device buffers that grow to the largest
+    group the slot has run, and the execution context the group runs on - a context of its own (``cf_exec_create``)
+    or the model's default context.  Slots on the default context still have a stream each, so that a retired
+    group's copies back do not queue behind the next group's kernels; the library orders calls on one context
+    across streams."""
 
-    def __init__(self, torch, lib, model):
+    def __init__(self, torch, lib, model, own_context):
         self.torch, self.lib, self.dev = torch, lib, int(model.device)
         self.ex = None
-        ex = ctypes.c_void_p()
-        _cabi.check(lib.cf_exec_create(model.handle, ctypes.byref(ex)))
-        self.ex = ex
+        if own_context:
+            ex = ctypes.c_void_p()
+            _cabi.check(lib.cf_exec_create(model.handle, ctypes.byref(ex)))
+            self.ex = ex
+        # cf_exec_infer_reads is cf_infer_reads on a context: the two calls differ only in their first argument
+        self.target = self.ex if own_context else model.handle
+        self.infer = lib.cf_exec_infer_reads if own_context else lib.cf_infer_reads
         with torch.cuda.device(self.dev):
             self.stream = torch.cuda.Stream()
             self.event = torch.cuda.Event()
@@ -417,74 +313,81 @@ class _StreamSlot(object):
             self.buf[name] = t
         return t
 
-    def submit(self, arrays, params, return_scores):
-        """Stage, copy and enqueue one group on this slot's stream (returns without waiting for the device)."""
+    def submit(self, arrays, params, return_scores, labels=None, thresholds=None):
+        """Stage, copy and enqueue one group on this slot's stream (returns without waiting for the device).  With
+        ``labels`` (one uint8 array per read) the group is counted at ``thresholds`` instead of returning intervals."""
         torch = self.torch
         threshold, min_run, ext_left, ext_right = params
         n = len(arrays)
         offsets = np.zeros(n + 1, np.int64)
         np.cumsum([a.size for a in arrays], out=offsets[1:])
         total = int(offsets[-1])
-        cap = int(self.lib.cf_max_intervals(total, n, min_run))
+        cap = 0 if labels is not None else int(self.lib.cf_max_intervals(total, n, min_run))
         with torch.cuda.device(self.dev), torch.cuda.stream(self.stream):
             stage = self._ensure("stage", total, torch.int16, pinned=True)
             raw = self._ensure("raw", total, torch.int16)
-            iv = self._ensure("iv", 2 * cap, torch.int64)
-            ioff = self._ensure("ioff", n + 1, torch.int64)
-            ioff_pin = self._ensure("ioff_pin", n + 1, torch.int64, pinned=True)
-            probs = self._ensure("probs", total, torch.float32) if return_scores else None
-            probs_pin = self._ensure("probs_pin", total, torch.float32, pinned=True) if return_scores else None
+            # the intervals [cap, 2], then the n + 1 interval offsets: one copy brings both back
+            m = 2 * cap + n + 1
+            out = self._ensure("out", m, torch.int64)
+            probs = self._ensure("probs", total, torch.float32) if return_scores or labels is not None else None
             _concat_into(stage.numpy()[:total], arrays, offsets)
             raw[:total].copy_(stage[:total], non_blocking=True)
-            _cabi.check(self.lib.cf_exec_infer_reads(
-                self.ex, raw.data_ptr(), _offsets_ptr(offsets), n, probs.data_ptr() if return_scores else None,
-                iv.data_ptr(), ioff.data_ptr(), cap, threshold, min_run, ext_left, ext_right, self.stream.cuda_stream))
-            ioff_pin[:n + 1].copy_(ioff[:n + 1], non_blocking=True)
+            if labels is not None:
+                lab_pin = self._ensure("lab_pin", total, torch.uint8, pinned=True)
+                np.concatenate(labels, out=lab_pin.numpy()[:total])
+                self._ensure("lab", total, torch.uint8)[:total].copy_(lab_pin[:total], non_blocking=True)
+            _cabi.check(self.infer(
+                self.target, raw.data_ptr(), _offsets_ptr(offsets), n, probs.data_ptr() if probs is not None else None,
+                out.data_ptr(), out.data_ptr() + 16 * cap, cap, threshold, min_run, ext_left, ext_right,
+                self.stream.cuda_stream))
+            self._ensure("out_pin", m, torch.int64, pinned=True)[:m].copy_(out[:m], non_blocking=True)
             if return_scores:
+                probs_pin = self._ensure("probs_pin", total, torch.float32, pinned=True)
                 probs_pin[:total].copy_(probs[:total], non_blocking=True)
             self.event.record(self.stream)
-        self.group = (offsets, cap, return_scores)
+        self.group = (offsets, cap, return_scores, thresholds if labels is not None else None)
 
     def done(self):
         return self.event.query()
 
     def results(self):
-        """Wait for the group and return its per-read results, in order; the slot is then free."""
-        torch = self.torch
-        offsets, cap, return_scores = self.group
+        """Wait for the group and return ``(offsets, intervals, interval_offsets, scores or None)`` of its reads - or,
+        for a group submitted with labels, its int64 ``[T, 4]`` confusion counts.  The slot is then free."""
+        offsets, cap, return_scores, thresholds = self.group
         self.group = None
         n, total = len(offsets) - 1, int(offsets[-1])
+        if thresholds is not None:
+            counts = np.zeros((thresholds.size, 4), np.int64)
+            # queued behind the group on the slot's stream; synchronises
+            _cabi.check(self.lib.cf_sweep_thresholds(
+                self.dev, self.buf["probs"].data_ptr(), 0, self.buf["lab"].data_ptr(), total, thresholds.ctypes.data,
+                thresholds.size, counts.ctypes.data_as(_cabi.c_i64_p), self.stream.cuda_stream))
+            return counts
         self.event.synchronize()
-        ioff = self.buf["ioff_pin"].numpy()[:n + 1].copy()
+        out = self.buf["out_pin"].numpy()
+        ioff = out[2 * cap:2 * cap + n + 1].copy()
         found = int(ioff[-1])
         if found > cap:
             raise _cabi.CatfishError("interval capacity exceeded (%d > %d)" % (found, cap))
-        intervals = np.zeros((0, 2), np.int64)
-        if found:
-            iv_pin = self._ensure("iv_pin", 2 * found, torch.int64, pinned=True)
-            with torch.cuda.device(self.dev), torch.cuda.stream(self.stream):
-                iv_pin[:2 * found].copy_(self.buf["iv"][:2 * found], non_blocking=True)
-            self.stream.synchronize()
-            intervals = iv_pin.numpy()[:2 * found].reshape(found, 2).copy()
-        bounds, lengths = ioff.tolist(), np.diff(offsets).tolist()
-        hps = [IntervalList(intervals[bounds[r]:bounds[r + 1]]) for r in range(n)]
-        if not return_scores:
-            return list(zip(hps, lengths))
-        scores = self.buf["probs_pin"].numpy()[:total].copy()
-        return [(hps[r], lengths[r], scores[int(offsets[r]):int(offsets[r + 1])]) for r in range(n)]
+        intervals = out[:2 * found].reshape(found, 2).copy()
+        scores = self.buf["probs_pin"].numpy()[:total].copy() if return_scores else None
+        return offsets, intervals, ioff, scores
 
     def close(self):
+        self.stream.synchronize()               # copies enqueued after the context's own work
         if self.ex is not None:
-            self.stream.synchronize()           # copies enqueued after the context's own work
             self.lib.cf_exec_destroy(self.ex)
             self.ex = None
         self.buf.clear()
 
 
-def _stream(it, model, params, return_scores, group_samples, max_wait_s, depth):
-    torch = _torch()
-    lib = _cabi.load_library()
-    slots, idle, inflight = [], [], collections.deque()      # inflight: slots in input order
+def _in_order(groups, depth, take_slot):
+    """Runs every group of the iterable ``groups`` (each the arguments of ``_Slot.submit``) and yields the groups'
+    ``results`` in input order.  Up to ``depth`` groups are in flight, on slots from ``take_slot()`` that are reused
+    once retired: while the device works on one group, the host stages the next.  A finished group goes out as soon
+    as it is found; a ``None`` in ``groups`` submits nothing and only gives that chance.  Groups still in flight when
+    the caller stops early are waited for, so that their slots can be reused or freed."""
+    idle, inflight = [], collections.deque()
 
     def retire():
         s = inflight.popleft()
@@ -492,22 +395,56 @@ def _stream(it, model, params, return_scores, group_samples, max_wait_s, depth):
         idle.append(s)
         return out
 
-    def launch(group):
-        if len(inflight) == depth:                           # bounded read-ahead: the oldest group goes out first
-            yield from retire()
-        if not idle:
-            slots.append(_StreamSlot(torch, lib, model))
-            idle.append(slots[-1])
-        s = idle.pop()
-        s.submit(group, params, return_scores)
-        inflight.append(s)
-
-    error = None
     try:
+        for group in groups:
+            while inflight and inflight[0].done():
+                yield retire()
+            if group is None:
+                continue
+            if len(inflight) == depth:                       # bounded read-ahead: the oldest group goes out first
+                yield retire()
+            s = idle.pop() if idle else take_slot()
+            inflight.append(s)                               # first: a failed submit may have enqueued copies
+            s.submit(*group)
+        while inflight:
+            yield retire()
+    finally:
+        for s in inflight:
+            s.stream.synchronize()
+
+
+def _run_on_model(model, groups):
+    """The list of ``_in_order`` results of ``groups`` on default-context slots of the model's pool, ``_DEPTH`` in
+    flight.  The call takes the slots it needs from the pool (new ones when it is short) and puts them back when it
+    ends, so that concurrent calls never share a buffer and the next call finds its buffers warm."""
+    torch, lib = _torch(), _cabi.load_library()
+    taken = []
+
+    def take_slot():
+        with model._slot_lock:
+            s = model._slots.pop() if model._slots else None
+        taken.append(s if s is not None else _Slot(torch, lib, model, own_context=False))
+        return taken[-1]
+
+    try:
+        return list(_in_order(groups, _DEPTH, take_slot))
+    finally:
+        with model._slot_lock:
+            model._slots.extend(taken)
+
+
+def _stream(it, model, params, return_scores, group_samples, max_wait_s, depth):
+    torch, lib = _torch(), _cabi.load_library()
+    slots, error = [], []
+
+    def take_slot():
+        slots.append(_Slot(torch, lib, model, own_context=True))
+        return slots[-1]
+
+    def groups():
         group, n_samples, t_first = [], 0, 0.0
         while True:
-            while inflight and inflight[0].done():             # finished groups go out as soon as they are found
-                yield from retire()
+            yield None                                         # finished groups go out as soon as they are found
             try:
                 a = _as_int16(next(it))
                 if a.size == 0:
@@ -515,24 +452,29 @@ def _stream(it, model, params, return_scores, group_samples, max_wait_s, depth):
             except StopIteration:
                 break
             except Exception as e:                             # earlier reads' results first, then this
-                error = e
+                error.append(e)
                 break
             if not group:
                 t_first = time.monotonic()
             group.append(a)
             n_samples += a.size
             if n_samples >= group_samples or (max_wait_s is not None and time.monotonic() - t_first >= max_wait_s):
-                yield from launch(group)
+                yield group, params, return_scores
                 group, n_samples = [], 0
         if group:
-            yield from launch(group)
-        while inflight:
-            yield from retire()
+            yield group, params, return_scores
+
+    try:
+        for offsets, intervals, ioff, scores in _in_order(groups(), depth, take_slot):
+            bounds, lengths = ioff.tolist(), np.diff(offsets).tolist()
+            for r in range(len(lengths)):
+                hps = IntervalList(intervals[bounds[r]:bounds[r + 1]])
+                yield (hps, lengths[r]) if scores is None else (hps, lengths[r], scores[offsets[r]:offsets[r + 1]])
     finally:
         for s in slots:
             s.close()
-    if error is not None:
-        raise error
+    if error:
+        raise error[0]
 
 
 def infer_concatenated(raw, offsets, model, threshold=0.5, min_run=15, extension_left=11,

@@ -10,6 +10,7 @@ follows the validation twin networks/rnn_class.py:222-261.  Training
 
 import ctypes
 import os
+import threading
 
 import numpy as np
 
@@ -48,6 +49,10 @@ class RNN(object):
         self._weights = None
         self.tp = self.fp = self.tn = self.fn = 0
         self.sweep_counts = None        # test_network_sweep's [T, 4] accumulator (reset_sweep)
+        # idle slots (infer._Slot: stream, buffers) of infer_reads / evaluate_reads on the default context; a call
+        # takes what it needs and puts it back, so concurrent calls never share a buffer
+        self._slots = []
+        self._slot_lock = threading.Lock()
 
     # ------------------------------------------------------------------ hyper-parameters
     def _hpm(self):
@@ -215,6 +220,14 @@ class RNN(object):
         return x, y8
 
     def _release(self):
+        if getattr(self, "_slots", None):
+            with self._slot_lock:
+                slots, self._slots = self._slots, []
+            for s in slots:
+                try:
+                    s.close()
+                except Exception:
+                    pass
         if getattr(self, "_handle", None) is not None:
             try:
                 _cabi.load_library().cf_model_destroy(self._handle)

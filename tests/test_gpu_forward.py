@@ -269,9 +269,10 @@ def test_outlier_windows_stay_in_contract():
     assert np.isfinite(a[keep]).all() and np.abs(a[keep] - b[keep]).max() < PROB_TOL
 
 
-def test_large_host_call_equals_smaller_calls():
+def test_large_batch_in_groups_equals_host_calls():
     """A batch of several engine passes through cf_infer_reads_host: CSR offsets, intervals and probabilities
-    equal those of smaller calls over sub-ranges of the same reads (batch invariance at the host boundary)."""
+    equal those of smaller calls over sub-ranges of the same reads (batch invariance at the host boundary), and
+    infer_reads, which runs the batch as several groups of reads, gives the same intervals and scores."""
     m = _model("ResNetRNN", "auto")
     lengths = synth.ragged_lengths(300, 60_000, 120_000, seed=3)           # ~27M samples = 5 passes
     reads = synth.synth_reads(lengths, base_seed=9000)
@@ -285,15 +286,16 @@ def test_large_host_call_equals_smaller_calls():
         assert np.array_equal(ioff2, ioff[lo:hi + 1] - ioff[lo])
         assert np.array_equal(iv2, iv[ioff[lo]:ioff[hi]])
         assert np.array_equal(scores2, scores[off[lo]:off[hi]])
-    # the Python entry point takes the pipelined path for a batch of this size (groups of reads, device-side
-    # calls overlapped with the host's staging): identical per-read results, list-like and as arrays
-    assert int(off[-1]) >= infer._PIPELINE_MIN_SAMPLES
-    hps, lens = infer.infer_reads(reads, m)
+    # the Python entry point runs a batch of this size as several groups of reads (device-side calls overlapped
+    # with the host's staging): identical per-read results and scores, list-like and as arrays
+    assert len(infer._cut_groups(off, infer._FIRST_GROUP_SAMPLES, infer._GROUP_SAMPLES)) > 1
+    hps, lens, scores_py = infer.infer_reads(reads, m, return_scores=True)
     assert lens == [len(r) for r in reads]
     for r in range(len(reads)):
         assert np.array_equal(hps[r].array, iv[ioff[r]:ioff[r + 1]])
+        assert np.array_equal(scores_py[r], scores[off[r]:off[r + 1]])
     assert hps[7] == iv[ioff[7]:ioff[8]].tolist() and isinstance(hps[7][0][0], int)
-    hps_again, _ = infer.infer_reads(reads, m)                     # cached staging / device buffers reused
+    hps_again, _ = infer.infer_reads(reads, m)                     # the model's pooled buffers reused
     assert all(a == b for a, b in zip(hps, hps_again))
 
 

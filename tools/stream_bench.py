@@ -65,7 +65,7 @@ def main():
         ("B: 512 x U{50k..200k} samples", synth.synth_reads(synth.ragged_lengths(512, 50_000, 200_000, seed=1), base_seed=1)),
     ]
     groups = (infer._GROUP_SAMPLES // 4, infer._GROUP_SAMPLES)
-    make_slot = infer._StreamSlot
+    make_slot = infer._Slot
     lib = _cabi.load_library()
     for name, reads in workloads:
         samples = sum(r.size for r in reads)
@@ -88,22 +88,22 @@ def main():
         def warm_streamed():
             pool = []
 
-            def slot(*a):
+            def slot(*a, **kw):
                 if pool:
                     return pool.pop()
-                s = make_slot(*a)
+                s = make_slot(*a, **kw)
                 s.destroy, s.close = s.close, (lambda: None)         # kept alive across runs
                 kept.append(s)
                 return s
 
             def run():
                 pool[:] = kept
-                infer._StreamSlot = slot
+                infer._Slot = slot
                 try:
                     outputs.append(list(infer.infer_stream(iter(reads), model)))
                     torch.cuda.synchronize()
                 finally:
-                    infer._StreamSlot = make_slot
+                    infer._Slot = make_slot
             return run
 
         configs = [("infer_reads (whole list)", batched), ("infer_stream default", streamed()),
