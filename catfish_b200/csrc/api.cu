@@ -498,10 +498,9 @@ static int infer_reads_device(cf_model* m, Exec* x, const int16_t* raw_dev,
     const bool fused_bits = !probs_dev && m->engine == CF_ENGINE_TCGEN05 && tc_can_emit_bits(m->tc.get());
     LabelBits bits;
     bits.threshold = threshold;
+    CF_TRY(k6_bits_prepare(x->k6, plan.total_samples, &bits, stream));
     float* probs = probs_dev;
-    if (fused_bits) {
-        CF_TRY(k6_bits_prepare(x->k6, plan.total_samples, &bits, stream));
-    } else if (!probs) {
+    if (!fused_bits && !probs) {
         CF_TRY(x->probs_internal.ensure(sizeof(float) * (size_t)plan.total_samples));
         probs = x->probs_internal.as<float>();
     }
@@ -510,20 +509,14 @@ static int infer_reads_device(cf_model* m, Exec* x, const int16_t* raw_dev,
     {
         ProfScope ps(&x->prof, KC_K1_TABLE, stream);
         CF_TRY(k1_window_table(offsets_dev, win_off_dev, n_reads, plan.total_windows, plan.n_tiles, tab, stream,
-                               fused_bits ? bits.bwords : nullptr, plan.total_samples));
+                               bits.bwords, plan.total_samples));
     }
     CF_TRY(engine_forward(m, x, raw0, x->stats.as<double>(), nullptr, tab, plan.n_tiles, probs, stream, false,
                           fused_bits ? &bits : nullptr));
-    if (fused_bits) {
-        ProfScope ps(&x->prof, KC_K6_INTERVALS, stream, 3);
-        CF_TRY(k6_intervals_from_bits(x->k6, bits, offsets_dev, n_reads, plan.total_samples, intervals_dev,
-                                      interval_offsets_dev, capacity, min_run, ext_left, ext_right, stream));
-    } else {
-        ProfScope ps(&x->prof, KC_K6_INTERVALS, stream, 7);
-        CF_TRY(k6_call_intervals(x->k6, probs, BITS_FROM_F32, threshold, 1, offsets_dev, n_reads,
-                                 plan.total_samples, intervals_dev, interval_offsets_dev, nullptr, capacity,
-                                 min_run, ext_left, ext_right, stream));
-    }
+    ProfScope ps(&x->prof, KC_K6_INTERVALS, stream, fused_bits ? 3 : 4);
+    if (!fused_bits) CF_TRY(k6_pack_bits(probs, BITS_FROM_F32, threshold, 1, plan.total_samples, bits, stream));
+    CF_TRY(k6_intervals_from_bits(x->k6, bits, offsets_dev, n_reads, plan.total_samples, intervals_dev,
+                                  interval_offsets_dev, nullptr, capacity, min_run, ext_left, ext_right, stream));
     return CF_OK;
 }
 
@@ -539,6 +532,25 @@ int upload_offsets(const int64_t* offsets_host, int32_t n_reads, cf::DevBuf* buf
     CF_CUDA(cudaMemcpyAsync(buf->ptr, off.data(), sizeof(int64_t) * off.size(), cudaMemcpyHostToDevice, st));
     CF_CUDA(cudaStreamSynchronize(st));     // `off` is pageable and about to go out of scope
     return CF_OK;
+}
+
+// cf_call_intervals and cf_hp_in_pred: read-start bits from the offsets, label bits from `values` (k6_pack_bits), then
+// the intervals.  Synchronises the stream on every path: the scratch is freed on return.
+int model_free_intervals(const void* values, int source, double threshold, int64_t label, const int64_t* offsets_host,
+                         int32_t n_reads, int64_t* intervals, int64_t* interval_offsets, int64_t* total_out,
+                         int64_t capacity, int32_t min_run, int32_t ext_left, int32_t ext_right, cudaStream_t st) {
+    const int64_t total = offsets_host[n_reads] - offsets_host[0];
+    cf::DevBuf off;
+    CF_TRY(upload_offsets(offsets_host, n_reads, &off, st));
+    cf::IntervalScratch scratch;
+    cf::LabelBits bits;
+    int s = cf::k6_bits_prepare(scratch, total, &bits, st);
+    if (s == CF_OK) s = cf::k6_read_starts(off.as<int64_t>(), n_reads, total, bits, st);
+    if (s == CF_OK) s = cf::k6_pack_bits(values, source, threshold, label, total, bits, st);
+    if (s == CF_OK) s = cf::k6_intervals_from_bits(scratch, bits, off.as<int64_t>(), n_reads, total, intervals,
+                                                   interval_offsets, total_out, capacity, min_run, ext_left, ext_right, st);
+    cudaStreamSynchronize(st);
+    return s;
 }
 }  // namespace
 
@@ -1100,23 +1112,14 @@ int cf_call_intervals(int32_t device, const void* probs_dev, int32_t probs_is_f6
     cf::DeviceGuard guard;
     CF_TRY(guard.set(device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (n_reads == 0) {
-        CF_CUDA(cudaMemsetAsync(interval_offsets_dev, 0, sizeof(int64_t), st));
-        return CF_OK;
-    }
     for (int32_t r = 0; r < n_reads; ++r)
         if (offsets_host[r + 1] < offsets_host[r]) { cf::set_error("cf_call_intervals: offsets decrease"); return CF_ERR_BAD_ARG; }
     const int64_t total = offsets_host[n_reads] - offsets_host[0];
     if (total > 0 && !probs_dev) { cf::set_error("cf_call_intervals: probs is NULL"); return CF_ERR_BAD_ARG; }
-    cf::DevBuf off;
-    CF_TRY(upload_offsets(offsets_host, n_reads, &off, st));
-    cf::IntervalScratch scratch;
     const char* base = static_cast<const char*>(probs_dev) + (size_t)offsets_host[0] * (probs_is_f64 ? 8 : 4);
-    int s = cf::k6_call_intervals(scratch, base, probs_is_f64 ? cf::BITS_FROM_F64 : cf::BITS_FROM_F32, threshold, 1,
-                                  off.as<int64_t>(), n_reads, total, intervals_dev, interval_offsets_dev, nullptr,
-                                  capacity, min_run, ext_left, ext_right, st);
-    cudaStreamSynchronize(st);
-    return s;
+    return model_free_intervals(base, probs_is_f64 ? cf::BITS_FROM_F64 : cf::BITS_FROM_F32, threshold, 1, offsets_host,
+                                n_reads, intervals_dev, interval_offsets_dev, nullptr, capacity, min_run, ext_left,
+                                ext_right, st);
 }
 
 int cf_class_from_threshold(int32_t device, const double* scores_dev, int64_t n, double threshold,
@@ -1148,15 +1151,11 @@ int cf_hp_in_pred(int32_t device, const int64_t* labels_dev, int64_t n, int32_t 
     cf::DeviceGuard guard;
     CF_TRY(guard.set(device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cf::DevBuf off, ioff;
+    cf::DevBuf ioff;
     const int64_t offsets[2] = {0, n};
-    CF_TRY(upload_offsets(offsets, 1, &off, st));
     CF_TRY(ioff.ensure(sizeof(int64_t) * 2));
-    cf::IntervalScratch scratch;
-    int s = cf::k6_call_intervals(scratch, labels_dev, cf::BITS_FROM_I64_EQ, 0.0, label, off.as<int64_t>(), 1, n,
-                                  intervals_dev, ioff.as<int64_t>(), n_out_dev, capacity, 1, ext_left, ext_right, st);
-    cudaStreamSynchronize(st);
-    return s;
+    return model_free_intervals(labels_dev, cf::BITS_FROM_I64_EQ, 0.0, label, offsets, 1, intervals_dev,
+                                ioff.as<int64_t>(), n_out_dev, capacity, 1, ext_left, ext_right, st);
 }
 
 }  // extern "C"

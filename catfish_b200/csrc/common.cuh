@@ -177,10 +177,11 @@ int k1_read_stats(const int16_t* raw, const int64_t* offsets_dev, int32_t n_read
 int k1_normalize_f64(const int16_t* raw, const int64_t* offsets_dev, int32_t n_reads,
                      int64_t total_samples, const double* stats, double* norm,
                      cudaStream_t stream);
-// bwords (optional): read-start bit words of the interval caller, set here so that k6 needs no pass of its own
+// Also sets the read-start bits of the interval caller (LabelBits::bwords, zeroed by k6_bits_prepare), so that k6
+// needs no pass of its own.
 int k1_window_table(const int64_t* offsets_dev, const int64_t* win_off_dev, int32_t n_reads,
                     int64_t total_windows, int64_t n_tiles, WindowTable tab, cudaStream_t stream,
-                    unsigned* bwords = nullptr, int64_t total_samples = 0);
+                    unsigned* bwords, int64_t total_samples);
 size_t k1_wide_scratch_bytes(int n_slots);
 constexpr int kK1ChunkSamples = 32768;
 size_t k1_chunked_scratch_bytes(int n_reads);
@@ -198,24 +199,29 @@ struct IntervalScratch {
     bool misc_zeroed = false;
 };
 enum BitSource { BITS_FROM_F32 = 0, BITS_FROM_F64 = 1, BITS_FROM_I64_EQ = 2 };
-// Label bits produced elsewhere (the head kernel of the network thresholds its own probabilities, so they never
-// make the HBM round trip): k6_bits_prepare sizes and zeroes the label / read-start words, the producers OR
-// their bits in, k6_intervals_from_bits turns them into intervals in three launches (count + scan by the last
+// Label bits and read-start bits over the concatenated sample index space.  k6_bits_prepare sizes and zeroes them; the
+// producers set them; k6_intervals_from_bits turns them into intervals in three launches (count + scan by the last
 // block, emit, per-read offsets).
+//   label bits: the head kernel of the tensor-core engine thresholds its own probabilities and ORs them in (they
+//               never make the HBM round trip); every other caller has the values in memory and calls k6_pack_bits.
+//   read-start bits: k1_window_table on the inference path, k6_read_starts for the model-free entry points.
 struct LabelBits {
     unsigned* lwords = nullptr;     // [n_words + 1] label bits over the concatenated sample index space
     unsigned* bwords = nullptr;     // [n_words + 1] read-start bits
     double threshold = 0.5;
 };
 int k6_bits_prepare(IntervalScratch& s, int64_t total_samples, LabelBits* out, cudaStream_t stream);
+// One launch: writes the label bits of n values, (double)value >= threshold for BITS_FROM_F32 / _F64 (NaN gives 0),
+// value == label for BITS_FROM_I64_EQ.
+int k6_pack_bits(const void* values, int source, double threshold, int64_t label, int64_t n, const LabelBits& bits,
+                 cudaStream_t stream);
+// One launch (none without reads): sets the read-start bit of every non-empty read.
+int k6_read_starts(const int64_t* offsets_dev, int32_t n_reads, int64_t total_samples, const LabelBits& bits,
+                   cudaStream_t stream);
+// With no reads or no samples it zeroes interval_offsets[0..n_reads] and *total_out (if given) and launches nothing.
 int k6_intervals_from_bits(IntervalScratch& s, const LabelBits& bits, const int64_t* offsets_dev, int32_t n_reads,
-                           int64_t total_samples, int64_t* intervals, int64_t* interval_offsets, int64_t capacity,
-                           int32_t min_run, int32_t ext_left, int32_t ext_right, cudaStream_t stream);
-int k6_call_intervals(IntervalScratch& s, const void* values, int source, double threshold,
-                      int64_t label, const int64_t* offsets_dev, int32_t n_reads,
-                      int64_t total_samples, int64_t* intervals, int64_t* interval_offsets,
-                      int64_t* total_out, int64_t capacity, int32_t min_run, int32_t ext_left,
-                      int32_t ext_right, cudaStream_t stream);
+                           int64_t total_samples, int64_t* intervals, int64_t* interval_offsets, int64_t* total_out,
+                           int64_t capacity, int32_t min_run, int32_t ext_left, int32_t ext_right, cudaStream_t stream);
 int k6_class_from_threshold(const double* scores, int64_t n, double threshold, int64_t* labels,
                             cudaStream_t stream);
 int k6_correct_short(const int64_t* labels, int64_t n, int32_t threshold, int64_t* out,

@@ -350,7 +350,7 @@ __global__ void k1_window_table_kernel(const int64_t* __restrict__ offsets, cons
                                        int64_t* __restrict__ src, int32_t* __restrict__ valid,
                                        int32_t* __restrict__ read, unsigned* __restrict__ bwords, int64_t total_samples) {
     const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (bwords && g < n_reads) {             // read-start bits for the interval caller (k6): one per non-empty read
+    if (g < n_reads) {                       // read-start bits for the interval caller (k6): one per non-empty read
         const int64_t o = offsets[g];
         if (o < total_samples && offsets[g + 1] > o) atomicOr(&bwords[o >> 5], 1u << (o & 31));
     }

@@ -9,9 +9,10 @@
 // coordinates, unclamped, unmerged, ordered by start.  Runs never span two reads.
 //
 // Bit-parallel formulation over the concatenated sample index space:
-//   L word  : label bits (warp ballot / nibble merge of 128-bit loads)
-//   B word  : read-start bits (scattered from the offsets)
-//   S word  : run-start bits  S = L & (~(L << 1 | carry) | B)
+//   L word  : label bits, ORed in by the network's head kernel (tc_engine.cu) or written by
+//             k6_pack_bits from values in memory (warp ballot / nibble merge of 128-bit loads)
+//   B word  : read-start bits (k1_window_table, or k6_read_starts from the offsets)
+//   S word  : run-start bits  S = L & (~(L << 1 | carry) | B), evaluated where needed, not stored
 //   run ends: E = L & (~(L >> 1 | next) | B >> 1); the start of the run ending at e is the
 //             nearest S bit at or below e (scan S words backwards).
 // Output order is the global rank of the run (count -> exclusive scan -> emit), so the
@@ -19,8 +20,6 @@
 #include "common.cuh"
 
 namespace cf {
-
-constexpr int kWordsPerBlock = 256;   // one thread per 32-sample word, 8192 samples per block
 
 __device__ __forceinline__ int find_read(const int64_t* __restrict__ off, int n, int64_t i) {
     int lo = 0, hi = n;
@@ -40,7 +39,15 @@ __global__ void k6_bounds_kernel(const int64_t* __restrict__ offsets, int n_read
     if (o < total && offsets[r + 1] > o) atomicOr(&bwords[o >> 5], 1u << (o & 31));
 }
 
-// ---------------------------------------------------------------- label + start bits
+int k6_read_starts(const int64_t* offsets_dev, int32_t n_reads, int64_t total_samples, const LabelBits& bits,
+                   cudaStream_t stream) {
+    if (n_reads <= 0) return CF_OK;
+    k6_bounds_kernel<<<(unsigned)ceil_div(n_reads, 256), 256, 0, stream>>>(offsets_dev, n_reads, total_samples, bits.bwords);
+    CF_LAUNCHED();
+    return CF_OK;
+}
+
+// ---------------------------------------------------------------- label bits from values in memory
 template <int SRC> struct Src;
 template <> struct Src<BITS_FROM_F32> {
     typedef float T;
@@ -58,8 +65,7 @@ template <> struct Src<BITS_FROM_I64_EQ> {
 // Generic path: one warp per 32-sample word per iteration, ballot.
 template <int SRC>
 __global__ void k6_pack_kernel(const typename Src<SRC>::T* __restrict__ vals, int64_t n, double thr,
-                               int64_t label, int64_t n_words, const unsigned* __restrict__ bwords,
-                               unsigned* __restrict__ lwords, unsigned* __restrict__ swords) {
+                               int64_t label, int64_t n_words, unsigned* __restrict__ lwords) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -67,12 +73,7 @@ __global__ void k6_pack_kernel(const typename Src<SRC>::T* __restrict__ vals, in
         const int64_t i = (w << 5) + lane;
         const bool h = i < n && Src<SRC>::hit(vals[i], thr, label);
         const unsigned L = __ballot_sync(0xffffffffu, h);
-        if (lane == 0) {
-            unsigned carry = 0;
-            if (w > 0) carry = Src<SRC>::hit(vals[(w << 5) - 1], thr, label) ? 1u : 0u;
-            lwords[w] = L;
-            swords[w] = L & (~((L << 1) | carry) | bwords[w]);
-        }
+        if (lane == 0) lwords[w] = L;
     }
 }
 
@@ -80,8 +81,7 @@ __global__ void k6_pack_kernel(const typename Src<SRC>::T* __restrict__ vals, in
 // independent 128-sample groups per warp iteration keep 4 loads per thread in flight (HBM-bound).
 __global__ void __launch_bounds__(256)
 k6_pack_f32x4_kernel(const float* __restrict__ vals, int64_t n, double thr,
-                     int64_t n_words, const unsigned* __restrict__ bwords,
-                     unsigned* __restrict__ lwords, unsigned* __restrict__ swords) {
+                     int64_t n_words, unsigned* __restrict__ lwords) {
     constexpr int kUnroll = 4;
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -127,221 +127,38 @@ k6_pack_f32x4_kernel(const float* __restrict__ vals, int64_t n, double thr,
             L |= __shfl_xor_sync(0xffffffffu, L, 1);
             L |= __shfl_xor_sync(0xffffffffu, L, 2);
             L |= __shfl_xor_sync(0xffffffffu, L, 4);
-            // carry = label of the sample before this word = top bit of the previous lane-group's word
-            unsigned prev = __shfl_up_sync(0xffffffffu, L, 8);
             const int64_t w = (g << 2) + (lane >> 3);
-            if ((lane & 7) == 0 && w < n_words) {
-                unsigned carry;
-                if (lane >= 8) carry = prev >> 31;
-                else carry = w > 0 ? (((double)vals[(w << 5) - 1] >= thr) ? 1u : 0u) : 0u;
-                lwords[w] = L;
-                swords[w] = L & (~((L << 1) | carry) | bwords[w]);
-            }
+            if ((lane & 7) == 0 && w < n_words) lwords[w] = L;
         }
     }
 }
 
-// ---------------------------------------------------------------- runs: count / emit
-// For the run ending at global position e (bit eb of word w), return its start.
-__device__ __forceinline__ int64_t run_start(const unsigned* __restrict__ swords, int64_t w, int eb) {
-    unsigned s = swords[w] & (eb == 31 ? 0xffffffffu : ((2u << eb) - 1u));
-    while (s == 0) {                 // the run began in an earlier word (all ones in between)
-        --w;
-        s = swords[w];
-    }
-    return (w << 5) + (31 - __clz(s));
-}
-
-template <bool EMIT>
-__global__ void __launch_bounds__(kWordsPerBlock)
-k6_runs_kernel(const unsigned* __restrict__ lwords, const unsigned* __restrict__ swords,
-               const unsigned* __restrict__ bwords, int64_t n_words, const int64_t* __restrict__ offsets,
-               int n_reads, int min_run, int ext_left, int ext_right,
-               unsigned* __restrict__ block_cnt, const int64_t* __restrict__ block_base,
-               int64_t* __restrict__ run_start_global, int64_t* __restrict__ intervals,
-               int64_t capacity) {
-    __shared__ unsigned warp_sums[kWordsPerBlock / 32];
-    const int64_t w = (int64_t)blockIdx.x * kWordsPerBlock + threadIdx.x;
-    unsigned L = 0, E = 0;
-    if (w < n_words) {
-        L = lwords[w];
-        unsigned next = 0, bnext = 0;
-        if (w + 1 < n_words) { next = lwords[w + 1] & 1u; bnext = bwords[w + 1] & 1u; }
-        E = L & (~((L >> 1) | (next << 31)) | (bwords[w] >> 1) | (bnext << 31));
-    }
-    // qualifying runs that end in this word
-    unsigned qual = 0;
-    int64_t starts[4];               // a word holds few qualifying ends; recomputed if more
-    int nq = 0;
-    for (unsigned e = E; e; e &= e - 1) {
-        const int eb = __ffs(e) - 1;
-        const int64_t s = run_start(swords, w, eb);
-        const int64_t len = (w << 5) + eb - s + 1;
-        if (len >= min_run) {
-            qual |= 1u << eb;
-            if (nq < 4) starts[nq] = s;
-            ++nq;
-        }
-    }
-    // block-level exclusive scan of nq
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned inc = (unsigned)nq;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        unsigned o = __shfl_up_sync(0xffffffffu, inc, d);
-        if (lane >= d) inc += o;
-    }
-    if (lane == 31) warp_sums[warp] = inc;
-    __syncthreads();
-    unsigned base = 0, total = 0;
-    for (int i = 0; i < kWordsPerBlock / 32; ++i) {
-        unsigned v = warp_sums[i];
-        if (i < warp) base += v;
-        total += v;
-    }
-    if (!EMIT) {
-        if (threadIdx.x == 0) block_cnt[blockIdx.x] = total;
-    } else {
-        int64_t rank = block_base[blockIdx.x] + base + inc - (unsigned)nq;
-        int k = 0;
-        for (unsigned q = qual; q; q &= q - 1, ++k, ++rank) {
-            const int eb = __ffs(q) - 1;
-            const int64_t s = k < 4 ? starts[k] : run_start(swords, w, eb);
-            const int64_t len = (w << 5) + eb - s + 1;
-            run_start_global[rank] = s;
-            if (rank < capacity) {
-                const int64_t local = s - offsets[find_read(offsets, n_reads, s)];
-                intervals[2 * rank] = local - ext_left;
-                intervals[2 * rank + 1] = local + len + ext_right;
-            }
-        }
-    }
-}
-
-// interval_offsets[r] = number of emitted runs that start before read r = lower bound of
-// offsets[r] in the (ascending) global run starts.  No atomics, any number of reads.
-__global__ void k6_read_offsets_kernel(const int64_t* __restrict__ run_start_global, const int64_t* __restrict__ total_runs,
-                                       const int64_t* __restrict__ offsets, int n_reads,
-                                       int64_t* __restrict__ interval_offsets, int64_t* __restrict__ total_out) {
-    const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r > n_reads) return;
-    const int64_t n = *total_runs;
-    const int64_t key = offsets[r];
-    int64_t lo = 0, hi = n;
-    while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (run_start_global[mid] < key) lo = mid + 1; else hi = mid;
-    }
-    interval_offsets[r] = lo;
-    if (r == n_reads && total_out) *total_out = n;
-}
-
-// ---------------------------------------------------------------- single-block exclusive scans
-template <typename TIn>
-__global__ void __launch_bounds__(1024)
-k6_scan_kernel(const TIn* __restrict__ in, int64_t n, int64_t* __restrict__ out, int64_t* __restrict__ total_out) {
-    __shared__ long long warp_sums[32];
-    __shared__ long long carry;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (int64_t base = 0; base < n; base += 1024) {
-        const int64_t i = base + threadIdx.x;
-        const long long v = i < n ? (long long)in[i] : 0;
-        long long inc = v;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            long long o = __shfl_up_sync(0xffffffffu, inc, d);
-            if (lane >= d) inc += o;
-        }
-        if (lane == 31) warp_sums[warp] = inc;
-        __syncthreads();
-        long long wbase = 0, tot = 0;
-        for (int k = 0; k < 32; ++k) {
-            long long s = warp_sums[k];
-            if (k < warp) wbase += s;
-            tot += s;
-        }
-        const long long c = carry;
-        if (i < n) out[i] = c + wbase + inc - v;
-        __syncthreads();
-        if (threadIdx.x == 0) carry = c + tot;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) {
-        out[n] = carry;
-        if (total_out) *total_out = carry;
-    }
-}
-
-// ---------------------------------------------------------------- host orchestration
-int k6_call_intervals(IntervalScratch& s, const void* values, int source, double threshold,
-                      int64_t label, const int64_t* offsets_dev, int32_t n_reads,
-                      int64_t total_samples, int64_t* intervals, int64_t* interval_offsets,
-                      int64_t* total_out, int64_t capacity, int32_t min_run, int32_t ext_left,
-                      int32_t ext_right, cudaStream_t stream) {
-    const int64_t n = total_samples;
+int k6_pack_bits(const void* values, int source, double threshold, int64_t label, int64_t n, const LabelBits& bits,
+                 cudaStream_t stream) {
     const int64_t n_words = ceil_div(n, 32);
-    const int64_t n_blocks = ceil_div(n_words, kWordsPerBlock);
-    if (n_reads <= 0 || n <= 0) {
-        CF_CUDA(cudaMemsetAsync(interval_offsets, 0, sizeof(int64_t) * (size_t)((n_reads > 0 ? n_reads : 0) + 1), stream));
-        if (total_out) CF_CUDA(cudaMemsetAsync(total_out, 0, sizeof(int64_t), stream));
-        return CF_OK;
-    }
-    // words are padded by one so that neighbours can be read unconditionally
-    CF_TRY(s.bits.ensure(sizeof(unsigned) * (size_t)(3 * (n_words + 1))));
-    unsigned* lwords = s.bits.as<unsigned>();
-    unsigned* swords = lwords + (n_words + 1);
-    unsigned* bwords = swords + (n_words + 1);
-    CF_TRY(s.block_cnt.ensure(sizeof(unsigned) * (size_t)n_blocks + sizeof(int64_t) * (size_t)(n_blocks + 1) + 16));
-    int64_t* block_base = s.block_cnt.as<int64_t>();
-    unsigned* block_cnt = reinterpret_cast<unsigned*>(block_base + n_blocks + 1);
-    // global start of every emitted run (ascending): at most one run per min_run + 1 samples
-    const int64_t max_runs = n / ((min_run < 1 ? 1 : min_run) + 1) + n_reads + 1;
-    CF_TRY(s.read_cnt.ensure(sizeof(int64_t) * (size_t)max_runs));
-    int64_t* run_start_global = s.read_cnt.as<int64_t>();
-
-    CF_CUDA(cudaMemsetAsync(bwords, 0, sizeof(unsigned) * (size_t)(n_words + 1), stream));
-    k6_bounds_kernel<<<(unsigned)ceil_div(n_reads, 256), 256, 0, stream>>>(offsets_dev, n_reads, n, bwords);
-    CF_LAUNCHED();
-
     int64_t pack_blocks = ceil_div(n_words, 8 * 16);  // 8 warps per block, 16 words per warp iteration
     if (pack_blocks < 1) pack_blocks = 1;
     if (pack_blocks > 148 * 8) pack_blocks = 148 * 8;
     if (source == BITS_FROM_F32) {
         if ((reinterpret_cast<uintptr_t>(values) & 15) == 0) {
             k6_pack_f32x4_kernel<<<(unsigned)pack_blocks, 256, 0, stream>>>(
-                static_cast<const float*>(values), n, threshold, n_words, bwords, lwords, swords);
+                static_cast<const float*>(values), n, threshold, n_words, bits.lwords);
         } else {
             k6_pack_kernel<BITS_FROM_F32><<<(unsigned)pack_blocks, 256, 0, stream>>>(
-                static_cast<const float*>(values), n, threshold, label, n_words, bwords, lwords, swords);
+                static_cast<const float*>(values), n, threshold, label, n_words, bits.lwords);
         }
     } else if (source == BITS_FROM_F64) {
         k6_pack_kernel<BITS_FROM_F64><<<(unsigned)pack_blocks, 256, 0, stream>>>(
-            static_cast<const double*>(values), n, threshold, label, n_words, bwords, lwords, swords);
+            static_cast<const double*>(values), n, threshold, label, n_words, bits.lwords);
     } else {
         k6_pack_kernel<BITS_FROM_I64_EQ><<<(unsigned)pack_blocks, 256, 0, stream>>>(
-            static_cast<const int64_t*>(values), n, threshold, label, n_words, bwords, lwords, swords);
+            static_cast<const int64_t*>(values), n, threshold, label, n_words, bits.lwords);
     }
-    CF_LAUNCHED();
-
-    k6_runs_kernel<false><<<(unsigned)n_blocks, kWordsPerBlock, 0, stream>>>(
-        lwords, swords, bwords, n_words, offsets_dev, n_reads, min_run, ext_left, ext_right,
-        block_cnt, nullptr, nullptr, nullptr, 0);
-    CF_LAUNCHED();
-    k6_scan_kernel<unsigned><<<1, 1024, 0, stream>>>(block_cnt, n_blocks, block_base, nullptr);
-    CF_LAUNCHED();
-    k6_runs_kernel<true><<<(unsigned)n_blocks, kWordsPerBlock, 0, stream>>>(
-        lwords, swords, bwords, n_words, offsets_dev, n_reads, min_run, ext_left, ext_right,
-        nullptr, block_base, run_start_global, intervals, capacity);
-    CF_LAUNCHED();
-    k6_read_offsets_kernel<<<(unsigned)ceil_div(n_reads + 1, 256), 256, 0, stream>>>(
-        run_start_global, block_base + n_blocks, offsets_dev, n_reads, interval_offsets, total_out);
     CF_LAUNCHED();
     return CF_OK;
 }
 
-// ---------------------------------------------------------------- label bits produced by the network's head kernel
+// ---------------------------------------------------------------- runs: count / emit
 // S words are not stored: S[w] = L[w] & (~(L[w] << 1 | L[w-1] >> 31) | B[w]).
 __device__ __forceinline__ unsigned start_word(const unsigned* __restrict__ lwords, const unsigned* __restrict__ bwords, int64_t w) {
     const unsigned L = lwords[w];
@@ -477,10 +294,28 @@ k6_runs_bits_kernel(const unsigned* __restrict__ lwords, const unsigned* __restr
     }
 }
 
+// interval_offsets[r] = number of emitted runs that start before read r = lower bound of
+// offsets[r] in the (ascending) global run starts.  No atomics, any number of reads.
+__global__ void k6_read_offsets_kernel(const int64_t* __restrict__ run_start_global, const int64_t* __restrict__ total_runs,
+                                       const int64_t* __restrict__ offsets, int n_reads,
+                                       int64_t* __restrict__ interval_offsets, int64_t* __restrict__ total_out) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r > n_reads) return;
+    const int64_t n = *total_runs;
+    const int64_t key = offsets[r];
+    int64_t lo = 0, hi = n;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (run_start_global[mid] < key) lo = mid + 1; else hi = mid;
+    }
+    interval_offsets[r] = lo;
+    if (r == n_reads && total_out) *total_out = n;
+}
+
 int k6_bits_prepare(IntervalScratch& s, int64_t total_samples, LabelBits* out, cudaStream_t stream) {
     const int64_t n_words = ceil_div(total_samples > 0 ? total_samples : 1, 32);
     const int64_t stride = (n_words + 1 + 3) / 4 * 4;             // both word arrays 16-byte aligned (128-bit loads)
-    CF_TRY(s.bits.ensure(sizeof(unsigned) * (size_t)(3 * stride)));
+    CF_TRY(s.bits.ensure(sizeof(unsigned) * (size_t)(2 * stride)));
     CF_TRY(s.misc.ensure(256));
     static_assert(sizeof(unsigned) == 4, "");
     out->lwords = s.bits.as<unsigned>();
@@ -490,14 +325,20 @@ int k6_bits_prepare(IntervalScratch& s, int64_t total_samples, LabelBits* out, c
 }
 
 int k6_intervals_from_bits(IntervalScratch& s, const LabelBits& bits, const int64_t* offsets_dev, int32_t n_reads,
-                           int64_t total_samples, int64_t* intervals, int64_t* interval_offsets, int64_t capacity,
-                           int32_t min_run, int32_t ext_left, int32_t ext_right, cudaStream_t stream) {
+                           int64_t total_samples, int64_t* intervals, int64_t* interval_offsets, int64_t* total_out,
+                           int64_t capacity, int32_t min_run, int32_t ext_left, int32_t ext_right, cudaStream_t stream) {
     const int64_t n = total_samples;
     const int64_t n_words = ceil_div(n, 32);
     const int64_t n_blocks = ceil_div(n_words, kBitsWordsPerBlock);
+    if (n_reads <= 0 || n <= 0) {
+        CF_CUDA(cudaMemsetAsync(interval_offsets, 0, sizeof(int64_t) * (size_t)((n_reads > 0 ? n_reads : 0) + 1), stream));
+        if (total_out) CF_CUDA(cudaMemsetAsync(total_out, 0, sizeof(int64_t), stream));
+        return CF_OK;
+    }
     CF_TRY(s.block_cnt.ensure(sizeof(unsigned) * (size_t)n_blocks + sizeof(int64_t) * (size_t)(n_blocks + 1) + 16));
     int64_t* block_base = s.block_cnt.as<int64_t>();
     unsigned* block_cnt = reinterpret_cast<unsigned*>(block_base + n_blocks + 1);
+    // global start of every emitted run (ascending): at most one run per min_run + 1 samples
     const int64_t max_runs = n / ((min_run < 1 ? 1 : min_run) + 1) + n_reads + 1;
     CF_TRY(s.read_cnt.ensure(sizeof(int64_t) * (size_t)max_runs));
     int64_t* run_start_global = s.read_cnt.as<int64_t>();
@@ -515,7 +356,7 @@ int k6_intervals_from_bits(IntervalScratch& s, const LabelBits& bits, const int6
         run_start_global, intervals, capacity);
     CF_LAUNCHED();
     k6_read_offsets_kernel<<<(unsigned)ceil_div(n_reads + 1, 256), 256, 0, stream>>>(
-        run_start_global, block_base + n_blocks, offsets_dev, n_reads, interval_offsets, nullptr);
+        run_start_global, block_base + n_blocks, offsets_dev, n_reads, interval_offsets, total_out);
     CF_LAUNCHED();
     return CF_OK;
 }

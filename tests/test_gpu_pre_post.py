@@ -53,15 +53,16 @@ def test_read_stats_long_read():
     assert st[0] == shift and st[1] == np.median(np.abs(raw - shift))
 
 
-def _call_intervals(probs_list, dtype, **kw):
-    """cf_call_intervals on a ragged batch of probability arrays."""
+def _call_intervals(probs_list, dtype, lead=0, **kw):
+    """cf_call_intervals on a ragged batch of probability arrays, placed after `lead` values that belong to no read
+    (lead 1-3 moves the first read's device pointer off 16-byte alignment)."""
     import ctypes
     import torch
     from catfish_b200 import _cabi
     lib = _cabi.load_library()
-    offsets = np.zeros(len(probs_list) + 1, np.int64)
-    offsets[1:] = np.cumsum([len(p) for p in probs_list])
-    flat = np.concatenate(probs_list).astype(dtype)
+    offsets = np.full(len(probs_list) + 1, lead, np.int64)
+    offsets[1:] += np.cumsum([len(p) for p in probs_list], dtype=np.int64)
+    flat = np.concatenate([np.ones(lead)] + list(probs_list)).astype(dtype)
     min_run = kw.get("min_run", 15)
     cap = int(lib.cf_max_intervals(len(flat), len(probs_list), min_run))
     pd = torch.from_numpy(flat).cuda()
@@ -93,9 +94,10 @@ def test_call_intervals_ragged_random(dtype):
         p = np.where(lab == 1, 0.5 + 0.5 * rng.random(n), 0.5 * rng.random(n) - 1e-9).astype(dtype)
         p[rng.integers(0, n, size=max(1, n // 50))] = 0.5                  # exactly on the threshold: counts as 1
         probs.append(p)
-    got = _call_intervals(probs, dtype)
-    for p, g in zip(probs, got):
-        assert g == _oracle_intervals(p.astype(np.float64))
+    for lead in (0, 1, 2, 3):          # f32 at leads 1-3: the unaligned (ballot) pack kernel
+        got = _call_intervals(probs, dtype, lead=lead)
+        for p, g in zip(probs, got):
+            assert g == _oracle_intervals(p.astype(np.float64))
     # other parameters
     got = _call_intervals(probs, dtype, threshold=0.9, min_run=4, ext_left=0, ext_right=3)
     for p, g in zip(probs, got):
@@ -116,6 +118,10 @@ def test_call_intervals_edge_patterns():
     # runs must not leak across read boundaries: all-ones neighbours stay separate intervals
     got = _call_intervals([ones(10), ones(10), ones(40), ones(7)], np.float32)
     assert got == [[], [], [[-11, 56]], []]
+    # empty reads have no intervals and keep their non-empty neighbours apart
+    got = _call_intervals([ones(0), ones(20), ones(0), ones(20), zeros(3), ones(0)], np.float32)
+    assert got == [[], [[-11, 36]], [], [[-11, 36]], [], []]
+    assert _call_intervals([], np.float32) == [] and _call_intervals([ones(0), ones(0)], np.float32) == [[], []]
 
 
 def test_python_helpers_match_golden():
