@@ -13,6 +13,8 @@ elementwise math stay exact, as in the CUDA engine.  Schemes:
   fp16+e5m2  a_hi w_hi in fp16 + [a_lo 2^s | a_hi 2^-s] [w_hi 2^-s ; w_lo 2^s] in e5m2, the a_hi 2^-s byte
              truncated (it is the top byte of the fp16 value, never stored in HBM)
              (1 fp16 pass + 1 fp8 pass with doubled K = 2 pass-equivalents; DESIGN.md section 4)
+  fp16+e5m2 faults, each a correction term lost:  "-lo" drops a_lo w_hi, "-hi" drops a_hi w_lo, "-both" drops both
+engine_mm(kind) picks the format per matmul the way the tensor-core engine does.
 Test infrastructure only (imports oracle/).
 """
 import os
@@ -59,16 +61,59 @@ def make_mm(scheme, s_corr=6):
         if scheme == "fp16x2":
             ah, al = split(a, hf)
             return (ah + al) @ rnd(w, hf)
-        if scheme == "fp16+e5m2":
+        if scheme.startswith("fp16+e5m2"):
+            fault = scheme[len("fp16+e5m2"):]
+            if fault not in ("", "-lo", "-hi", "-both"):
+                raise ValueError(scheme)
             wh = rnd(w, hf)
             ah = 2.0 ** s_corr * rnd(rnd(a, hf) / 2.0 ** s_corr, hf)      # main plane = fp16(fp16(a) 2^-s)
             al, wl = a - ah, w - wh
             k = 2.0 ** s_corr
-            # the a_hi 2^-s byte is the top byte of the fp16 main value (truncated e5m2), as the kernels build it
-            corr = rnd(al * k, e5) @ rnd(wh / k, e5) + trunc_e5(ah / k) @ rnd(wl * k, e5)
-            return ah @ wh + corr
+            out = ah @ wh
+            if fault not in ("-lo", "-both"):
+                out = out + rnd(al * k, e5) @ rnd(wh / k, e5)
+            if fault not in ("-hi", "-both"):
+                # the a_hi 2^-s byte is the top byte of the fp16 main value (truncated e5m2), as the kernels build it
+                out = out + trunc_e5(ah / k) @ rnd(wl * k, e5)
+            return out
         raise ValueError(scheme)
     return mm
+
+
+def engine_mm(kind, f16e5="fp16+e5m2"):
+    """Matmul in the operand format the tensor-core engine uses for each product of the H = 64 networks, with
+    `f16e5` (a fp16+e5m2 scheme, possibly a fault) where the engine runs f16e5.  ResNetRNN: the convolutions
+    (K = 32) and GRU layer 0 (K = 32 + 64) are bf16x3, the 128-wide layers (K = 128 + 64) f16e5.  RNN: every layer is
+    f16e5, except that layer 0's scalar input row (K = 1 + 64) is an exact rank-1 update."""
+    if kind not in ("ResNetRNN", "RNN"):
+        raise ValueError(kind)
+    bf3, f16 = make_mm("bf16x3"), make_mm(f16e5)
+
+    def mm(a, w):
+        k = np.shape(a)[1]
+        if kind == "RNN" and k == 1 + 64:
+            a, w = np.asarray(a, np.float64), np.asarray(w, np.float64)
+            return a[:, :1] @ w[:1] + f16(a[:, 1:], w[1:])
+        return f16(a, w) if kind == "RNN" or k == 128 + 64 else bf3(a, w)
+    return mm
+
+
+def synthetic_windows(n_windows, read_len=7000, seed=300):
+    """The first n_windows windows [n, 35, 1] of normalised synthetic reads (seeds seed, seed + 1, ...)."""
+    xs, n = [], 0
+    while n < n_windows:
+        raw = synth.synth_read(read_len, seed + len(xs))
+        xs.append(postprocess.pad_and_window(postprocess.normalize_raw_signal(raw))[0])
+        n += xs[-1].shape[0]
+    return np.concatenate(xs, 0)[:n_windows]
+
+
+def tile_rms(p, ref, tile=128):
+    """RMS of p - ref over each tile of `tile` windows (35 positions each); the last tile counts only the windows
+    it has.  A fault confined to some tiles (one chain of the fused GRU kernel) shows in those tiles undiluted."""
+    d = np.asarray(p, np.float64) - np.asarray(ref, np.float64)
+    per = tile * tf_graph.WINDOW
+    return np.array([np.sqrt(np.mean(d[i:i + per] ** 2)) for i in range(0, d.size, per)])
 
 
 def forward(w, x, mm):
