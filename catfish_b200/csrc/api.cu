@@ -218,17 +218,6 @@ int build_host_model(const cf_model_desc& d, const float* const* t, HostModel* o
     return CF_OK;
 }
 
-// dense window table for cf_infer_windows: window g covers x[35 g .. 35 g + 35)
-__global__ void dense_window_table_kernel(int64_t n_windows, int64_t n_slots, int64_t* __restrict__ src,
-                                          int32_t* __restrict__ valid, int32_t* __restrict__ read) {
-    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= n_slots) return;
-    const bool real = g < n_windows;
-    src[g] = real ? g * kWindow : -1;
-    valid[g] = real ? kWindow : 0;
-    read[g] = -1;
-}
-
 }  // namespace cf
 
 // ---------------------------------------------------------------- execution context
@@ -245,15 +234,12 @@ struct Exec {
     DevBuf plan_dev;                 // offsets[R+1] | win_off[R+1]
     DevBuf stats, wide_flags, wide_scratch, k1_chunked, k1_chunk_tab;
     DevBuf tab_src, tab_valid, tab_read;
-    DevBuf probs_internal;
     DevBuf val_logits, val_partial;  // validation row (N4)
     DevBuf val_sweep;                // its threshold sweep (K11 scratch)
     IntervalScratch k6;
     // host-buffer entry point
     DevBuf h_raw, h_intervals, h_ioff, h_probs;
-    // engine workspaces: the tensor-core pass, and the CUDA-core pass (the tensor-core engine uses it for the
-    // scalar input of RNN-only networks)
-    DevBuf tc_ws, simt_ws;
+    DevBuf ws;                       // the engine's workspace
     Profiler prof;                   // cf_profile_*: switched on for the model's default context only
     Event last_done;                 // end of the previous asynchronous call on this context (CallScope)
     std::mutex mu;
@@ -349,10 +335,9 @@ static int engine_forward(cf_model* m, Exec* x, const int16_t* raw, const double
                           WindowTable tab, int64_t n_tiles, float* probs, cudaStream_t stream,
                           bool want_logits = false, const LabelBits* bits = nullptr) {
     if (m->engine == CF_ENGINE_TCGEN05)
-        return tc_forward(m->tc.get(), &x->tc_ws, &x->simt_ws, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream,
-                          &x->prof, want_logits, bits);
-    return simt_forward(m->simt.get(), &x->simt_ws, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream, &x->prof,
-                        want_logits);
+        return tc_forward(m->tc.get(), &x->ws, raw, stats, xwin, tab, n_tiles, probs, stream, &x->prof, want_logits, bits);
+    return simt_forward(m->simt.get(), &x->ws, m->hm, raw, stats, xwin, tab, n_tiles, probs, stream, &x->prof,
+                        want_logits, bits);
 }
 
 // Validate offsets and lay out the windows of every read (infer.py:32-43).
@@ -493,17 +478,11 @@ static int infer_reads_device(cf_model* m, Exec* x, const int16_t* raw_dev,
     CF_TRY(x->stats.ensure(sizeof(double) * 2 * (size_t)n_reads));
     WindowTable tab;
     CF_TRY(ensure_table(x, plan.n_tiles, &tab));
-    // When the caller does not want the probabilities, the head kernel thresholds them itself and emits label bits
-    // (no 4 B/sample write + 4 B/sample read between the network and the interval caller).
-    const bool fused_bits = !probs_dev && m->engine == CF_ENGINE_TCGEN05 && tc_can_emit_bits(m->tc.get());
+    // The head thresholds its own probabilities and emits label bits: they reach the interval caller without a round
+    // trip through HBM, and probs_dev (nullptr: not wanted) receives the probabilities themselves.
     LabelBits bits;
     bits.threshold = threshold;
     CF_TRY(k6_bits_prepare(x->k6, plan.total_samples, &bits, stream));
-    float* probs = probs_dev;
-    if (!fused_bits && !probs) {
-        CF_TRY(x->probs_internal.ensure(sizeof(float) * (size_t)plan.total_samples));
-        probs = x->probs_internal.as<float>();
-    }
     StatsScratch sc{&x->wide_flags, &x->wide_scratch, &x->k1_chunked, &x->k1_chunk_tab, &x->pin_chunks, &x->chunks_copied};
     CF_TRY(compute_read_stats(raw0, offsets_host, offsets_dev, n_reads, x->stats.as<double>(), sc, stream, &x->prof));
     {
@@ -511,10 +490,8 @@ static int infer_reads_device(cf_model* m, Exec* x, const int16_t* raw_dev,
         CF_TRY(k1_window_table(offsets_dev, win_off_dev, n_reads, plan.total_windows, plan.n_tiles, tab, stream,
                                bits.bwords, plan.total_samples));
     }
-    CF_TRY(engine_forward(m, x, raw0, x->stats.as<double>(), nullptr, tab, plan.n_tiles, probs, stream, false,
-                          fused_bits ? &bits : nullptr));
-    ProfScope ps(&x->prof, KC_K6_INTERVALS, stream, fused_bits ? 3 : 4);
-    if (!fused_bits) CF_TRY(k6_pack_bits(probs, BITS_FROM_F32, threshold, 1, plan.total_samples, bits, stream));
+    CF_TRY(engine_forward(m, x, raw0, x->stats.as<double>(), nullptr, tab, plan.n_tiles, probs_dev, stream, false, &bits));
+    ProfScope ps(&x->prof, KC_K6_INTERVALS, stream, 3);
     CF_TRY(k6_intervals_from_bits(x->k6, bits, offsets_dev, n_reads, plan.total_samples, intervals_dev,
                                   interval_offsets_dev, nullptr, capacity, min_run, ext_left, ext_right, stream));
     return CF_OK;
@@ -768,10 +745,9 @@ static int reserve(cf_model* m, cf::Exec* x, int64_t max_samples, int32_t max_re
     CF_TRY(x->wide_flags.ensure(sizeof(int32_t) * (size_t)max_reads));
     CF_TRY(x->wide_scratch.ensure(cf::k1_wide_scratch_bytes(cf::kWideSlots)));
     if (cf::stats_may_use_chunks(max_reads)) CF_TRY(x->k1_chunked.ensure(cf::k1_chunked_scratch_bytes(max_reads)));
-    CF_TRY(x->probs_internal.ensure(sizeof(float) * (size_t)max_samples));
     CF_TRY(x->val_sweep.ensure(cf::k11_scratch_bytes(cf::kSweepMaxThresholds)));
-    if (m->engine == CF_ENGINE_TCGEN05) return cf::tc_reserve(m->tc.get(), &x->tc_ws, &x->simt_ws, m->hm, tiles);
-    return cf::simt_reserve(&x->simt_ws, m->hm, tiles);
+    if (m->engine == CF_ENGINE_TCGEN05) return cf::tc_reserve(&x->ws, tiles);
+    return cf::simt_reserve(&x->ws, m->hm, tiles);
 }
 
 int cf_model_reserve(cf_model* m, int64_t max_samples, int32_t max_reads) {
@@ -797,9 +773,7 @@ int cf_infer_windows(cf_model* m, const float* x_dev, int64_t n_windows, float* 
     const int64_t tiles = cf::ceil_div(n_windows, cf::kTileWindows);
     cf::WindowTable tab;
     CF_TRY(cf::ensure_table(x, tiles, &tab));
-    const int64_t slots = tiles * cf::kTileWindows;
-    cf::dense_window_table_kernel<<<(unsigned)cf::ceil_div(slots, 256), 256, 0, st>>>(n_windows, slots, tab.src, tab.valid, tab.read);
-    CF_LAUNCHED();
+    CF_TRY(cf::k1_dense_window_table(n_windows, tiles, tab, st));
     return cf::engine_forward(m, x, nullptr, nullptr, x_dev, tab, tiles, probs_dev, st);
 }
 
@@ -814,9 +788,7 @@ static int validate_forward(cf_model* m, cf::Exec* x, const float* x_dev, const 
     CF_TRY(x->val_partial.ensure(sizeof(long long) * 6 * ((size_t)blocks + 1)));
     cf::WindowTable tab;
     CF_TRY(cf::ensure_table(x, tiles, &tab));
-    const int64_t slots = tiles * cf::kTileWindows;
-    cf::dense_window_table_kernel<<<(unsigned)cf::ceil_div(slots, 256), 256, 0, st>>>(n_windows, slots, tab.src, tab.valid, tab.read);
-    CF_LAUNCHED();
+    CF_TRY(cf::k1_dense_window_table(n_windows, tiles, tab, st));
     CF_TRY(cf::engine_forward(m, x, nullptr, nullptr, x_dev, tab, tiles, x->val_logits.as<float>(), st,
                               /*want_logits=*/true));
     long long* partial = x->val_partial.as<long long>();

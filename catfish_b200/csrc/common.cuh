@@ -182,6 +182,12 @@ int k1_normalize_f64(const int16_t* raw, const int64_t* offsets_dev, int32_t n_r
 int k1_window_table(const int64_t* offsets_dev, const int64_t* win_off_dev, int32_t n_reads,
                     int64_t total_windows, int64_t n_tiles, WindowTable tab, cudaStream_t stream,
                     unsigned* bwords, int64_t total_samples);
+// One launch: the table of n_windows dense windows (window g covers xwin[35 g .. 35 g + 35)) over n_tiles tiles.
+int k1_dense_window_table(int64_t n_windows, int64_t n_tiles, WindowTable tab, cudaStream_t stream);
+// One launch: the normalised samples of the windows of tiles [tile0, tile0 + tiles) (window_input), as fp32 rows
+// x[(tile * 35 + t) * 128 + w] - the input of the first layer of either engine when there are no residual blocks.
+int k1_fill_windows(const int16_t* raw, const double* stats, const float* xwin, WindowTable tab, int64_t tile0,
+                    int64_t tiles, float* x, cudaStream_t stream);
 size_t k1_wide_scratch_bytes(int n_slots);
 constexpr int kK1ChunkSamples = 32768;
 size_t k1_chunked_scratch_bytes(int n_reads);
@@ -202,8 +208,8 @@ enum BitSource { BITS_FROM_F32 = 0, BITS_FROM_F64 = 1, BITS_FROM_I64_EQ = 2 };
 // Label bits and read-start bits over the concatenated sample index space.  k6_bits_prepare sizes and zeroes them; the
 // producers set them; k6_intervals_from_bits turns them into intervals in three launches (count + scan by the last
 // block, emit, per-read offsets).
-//   label bits: the head kernel of the tensor-core engine thresholds its own probabilities and ORs them in (they
-//               never make the HBM round trip); every other caller has the values in memory and calls k6_pack_bits.
+//   label bits: on the inference path the head kernels of both engines threshold their own probabilities and OR
+//               them in (head_output); the model-free entry points have the values in memory and call k6_pack_bits.
 //   read-start bits: k1_window_table on the inference path, k6_read_starts for the model-free entry points.
 struct LabelBits {
     unsigned* lwords = nullptr;     // [n_words + 1] label bits over the concatenated sample index space

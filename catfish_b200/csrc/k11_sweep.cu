@@ -15,7 +15,7 @@
 #include <algorithm>
 #include <cmath>
 
-#include "common.cuh"
+#include "window_io.cuh"
 
 namespace cf {
 
@@ -23,7 +23,7 @@ constexpr int kSweepThreads = 256;
 constexpr int kSweepCountThreads = 1024;
 
 __device__ __forceinline__ int sweep_key(float v, unsigned label, bool logits, const float* th, int T, int top) {
-    const float p = logits ? 1.f / (1.f + expf(-v)) : v;     // K9's and the head kernels' sigmoid
+    const float p = logits ? head_sigmoid(v) : v;
     int k = 0;                                                // thresholds th[0..k) are <= p; NaN: none
     for (int step = top; step > 0; step >>= 1)
         if (k + step <= T && th[k + step - 1] <= p) k += step;

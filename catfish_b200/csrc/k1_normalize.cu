@@ -1,4 +1,5 @@
-// K1: per-read exact median / MAD of the raw int16 signal, and the window table.
+// K1: per-read exact median / MAD of the raw int16 signal, the window tables, and the gathered scalar input of
+// networks without residual blocks.
 //
 // Replaces infer.normalize_raw_signal (catfish/infer.py:96-105):
 //     shift = np.median(raw); scale = np.median(np.abs(raw - shift)); (raw - shift) / scale
@@ -11,7 +12,7 @@
 // One CTA per read; the signal is read twice (min/max, then histogram) with 128-bit loads, the
 // second pass out of L2.  Reads whose value range exceeds the shared-memory histogram take the
 // same algorithm on a 65536-bin histogram in global scratch (k1_stats_wide_kernel).
-#include "common.cuh"
+#include "window_io.cuh"
 
 namespace cf {
 
@@ -373,6 +374,48 @@ int k1_window_table(const int64_t* offsets_dev, const int64_t* win_off_dev, int3
     // every read has at least one window, so slots >= n_reads and thread g < n_reads exists for every read
     k1_window_table_kernel<<<(unsigned)ceil_div(slots, 256), 256, 0, stream>>>(
         offsets_dev, win_off_dev, n_reads, total_windows, slots, tab.src, tab.valid, tab.read, bwords, total_samples);
+    CF_LAUNCHED();
+    return CF_OK;
+}
+
+// dense windows of cf_infer_windows and the validation row: window g covers x[35 g .. 35 g + 35)
+__global__ void k1_dense_window_table_kernel(int64_t n_windows, int64_t n_slots, int64_t* __restrict__ src,
+                                             int32_t* __restrict__ valid, int32_t* __restrict__ read) {
+    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= n_slots) return;
+    const bool real = g < n_windows;
+    src[g] = real ? g * kWindow : -1;
+    valid[g] = real ? kWindow : 0;
+    read[g] = -1;
+}
+
+int k1_dense_window_table(int64_t n_windows, int64_t n_tiles, WindowTable tab, cudaStream_t stream) {
+    const int64_t slots = n_tiles * kTileWindows;
+    k1_dense_window_table_kernel<<<(unsigned)ceil_div(slots, 256), 256, 0, stream>>>(n_windows, slots, tab.src, tab.valid, tab.read);
+    CF_LAUNCHED();
+    return CF_OK;
+}
+
+// ---------------------------------------------------------------- scalar network input
+// x[(tile*35+t)*128+w] = sample t of window (tile0 + tile) * 128 + w (window_input)
+__global__ void k1_fill_windows_kernel(const int16_t* __restrict__ raw, const double* __restrict__ stats,
+                                       const float* __restrict__ xwin, const int64_t* __restrict__ src,
+                                       const int32_t* __restrict__ valid, const int32_t* __restrict__ read,
+                                       int64_t tile0, int64_t n_rows, float* __restrict__ x) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;   // local row
+    if (i >= n_rows) return;
+    const int w = (int)(i % kTileWindows);
+    const int64_t tt = i / kTileWindows;
+    const int t = (int)(tt % kWindow);
+    const int64_t tile = tt / kWindow;
+    x[i] = window_input(raw, stats, xwin, src, valid, read, (tile0 + tile) * kTileWindows + w)(t);
+}
+
+int k1_fill_windows(const int16_t* raw, const double* stats, const float* xwin, WindowTable tab, int64_t tile0,
+                    int64_t tiles, float* x, cudaStream_t stream) {
+    const int64_t rows = tiles * kWindow * kTileWindows;
+    k1_fill_windows_kernel<<<(unsigned)ceil_div(rows, 256), 256, 0, stream>>>(raw, stats, xwin, tab.src, tab.valid, tab.read,
+                                                                               tile0, rows, x);
     CF_LAUNCHED();
     return CF_OK;
 }

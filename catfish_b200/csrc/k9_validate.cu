@@ -9,10 +9,10 @@
 // from the true negatives afterwards, rnn_class.py:247 - the caller of this kernel does the same).
 //
 // Input is the dense layer's output (logits) that the forward pass leaves in HBM when asked to
-// skip the sigmoid; the probability is recomputed here with the head kernels' own formula so that
+// skip the sigmoid; the probability is recomputed here with the heads' own function (head_sigmoid) so that
 // predictions are bit-identical to cf_infer_windows.  HBM-bound: 4 B logit + 1 B label per position.
 // Deterministic: every block reduces in a fixed order into its own slot, one block adds the slots.
-#include "common.cuh"
+#include "window_io.cuh"
 
 namespace cf {
 
@@ -25,7 +25,7 @@ struct ValAcc {
 };
 
 __device__ __forceinline__ void val_accumulate(ValAcc& a, float z, unsigned label, double threshold) {
-    const float p = 1.f / (1.f + expf(-z));
+    const float p = head_sigmoid(z);
     const bool pred = (double)p >= threshold;
     // metrics.confusion_matrix: a predicted 1 is a TP only for label 1, a predicted 0 is a TN only
     // for label 0; any other label value lands in fp / fn

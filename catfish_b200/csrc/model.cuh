@@ -60,19 +60,18 @@ using TcEnginePtr = std::unique_ptr<TcEngine, EngineDelete>;
 // ---------------------------------------------------------------- SIMT (fp32) engine
 // Uploads the weights; CF_ERR_ALLOC / CF_ERR_CUDA when an allocation / a copy fails.
 int simt_create(const HostModel& hm, SimtEnginePtr* out);
-// Forward pass over n_tiles tiles of 128 windows.  Input is either the raw int16 signal with
-// per-read (shift, scale) or already-normalised float windows; output probabilities are
-// scattered to probs[tab.src[g] + t] for t < tab.valid[g].  With want_logits the dense layer's output
+// Both engines' forward passes over n_tiles tiles of 128 windows.  Input is either the raw int16 signal with
+// per-read (shift, scale) or already-normalised float windows.  The head writes every real sample (t < tab.valid[g],
+// window_io.cuh): its probability to probs[tab.src[g] + t] unless probs is nullptr, and with bits its label bit
+// (probability >= bits->threshold) into bits->lwords (k6_bits_prepare).  With want_logits the dense layer's output
 // (rnn_class.py:178-183) is written instead of its sigmoid - the validation row needs it for the loss.
 // ws: the calling context's workspace, grown to the pass's needs.
 int simt_forward(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* raw, const double* stats,
                  const float* xwin, WindowTable tab, int64_t n_tiles, float* probs,
-                 cudaStream_t stream, Profiler* prof, bool want_logits = false);
+                 cudaStream_t stream, Profiler* prof, bool want_logits = false, const LabelBits* bits = nullptr);
 
 // Grow ws to what simt_forward needs for a pass over n_tiles tiles.
 int simt_reserve(DevBuf* ws, const HostModel& hm, int64_t n_tiles);
-// Grow ws to what simt_conv_stack needs for passes of chunk_tiles tiles (the tensor-core engine's RNN-only input).
-int simt_conv_stack_reserve(DevBuf* ws, const HostModel& hm, int64_t chunk_tiles);
 
 // ---------------------------------------------------------------- tcgen05 engine
 bool tc_supported(const HostModel& hm);
@@ -80,17 +79,12 @@ bool tc_supported(const HostModel& hm);
 // fails.
 int tc_create(const HostModel& hm, TcEnginePtr* out);
 int tc_operand_format(const TcEngine* e);    // 0 = split bf16 (3 MMA passes), 1 = fp16 + e5m2 corrections (2 pass-equivalents)
-// bits != nullptr (networks with a GRU head): the head thresholds its own scores and ORs label bits into
-// bits->lwords (k6_bits_prepare) instead of writing probabilities - probs may then be nullptr.
-bool tc_can_emit_bits(const TcEngine* e);
-// ws: the calling context's tensor-core workspace; simt_ws: its CUDA-core workspace (RNN-only networks normalise
-// their scalar input with simt_conv_stack).  Both grow to the pass's needs.
-int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, const int16_t* raw, const double* stats,
-               const float* xwin, WindowTable tab, int64_t n_tiles, float* probs,
-               cudaStream_t stream, Profiler* prof, bool want_logits = false, const LabelBits* bits = nullptr);
+int tc_forward(TcEngine* e, DevBuf* ws, const int16_t* raw, const double* stats, const float* xwin, WindowTable tab,
+               int64_t n_tiles, float* probs, cudaStream_t stream, Profiler* prof, bool want_logits = false,
+               const LabelBits* bits = nullptr);
 
-// Grow ws / simt_ws to what tc_forward needs for a pass over n_tiles tiles.
-int tc_reserve(const TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, int64_t n_tiles);
+// Grow ws to what tc_forward needs for a pass over n_tiles tiles.
+int tc_reserve(DevBuf* ws, int64_t n_tiles);
 
 int tc_selftest_f16e5(const float* a_dev, int K, int N, const float* w_host, int mode, float* out_dev, cudaStream_t stream);
 

@@ -12,6 +12,7 @@
 #include <cmath>
 
 #include "model.cuh"
+#include "window_io.cuh"
 
 namespace cf {
 
@@ -63,32 +64,6 @@ int simt_create(const HostModel& hm, SimtEnginePtr* out) {
     e->head_b = hm.head_b;
     *out = std::move(e);
     return CF_OK;
-}
-
-// ---------------------------------------------------------------- input
-// x[(tile*35+t)*128+w] = t < valid ? float((raw - shift) / scale) : 0   (infer.py:32-38,105; the
-// f64 -> f32 cast is the placeholder feed of rnn_class.py:159)
-__global__ void simt_fill_x_kernel(const int16_t* __restrict__ raw, const double* __restrict__ stats,
-                                   const float* __restrict__ xwin, const int64_t* __restrict__ src,
-                                   const int32_t* __restrict__ valid, const int32_t* __restrict__ read,
-                                   int64_t tile0, int64_t n_rows, float* __restrict__ x) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;   // local row
-    if (i >= n_rows) return;
-    const int w = (int)(i % kTileWindows);
-    const int64_t tt = i / kTileWindows;
-    const int t = (int)(tt % kWindow);
-    const int64_t tile = tt / kWindow;
-    const int64_t g = (tile0 + tile) * kTileWindows + w;
-    float v = 0.f;
-    if (t < valid[g]) {
-        if (raw) {
-            const int r = read[g];
-            v = (float)(((double)raw[src[g] + t] - stats[2 * r]) / stats[2 * r + 1]);
-        } else {
-            v = xwin[src[g] + t];
-        }
-    }
-    x[i] = v;
 }
 
 // ---------------------------------------------------------------- conv1d (+ folded BN, relu, residual)
@@ -233,40 +208,34 @@ simt_gru_kernel(const float* __restrict__ xp, const float* __restrict__ wgh_fw,
 }
 
 // ---------------------------------------------------------------- dense + sigmoid + un-window
-// p = sigmoid(y[row] . w + b), written to probs[src[g] + t] for the real (unpadded) positions
-// (rnn_class.py:178-183,84; the cut of the padding is infer.py:47).
+// p = sigmoid(y[row] . w + b) for the real (unpadded) positions (rnn_class.py:178-183,84), written by head_output.
 __global__ void simt_head_kernel(const float* __restrict__ y, const float* __restrict__ w, float b, int F,
-                                 const int64_t* __restrict__ src, const int32_t* __restrict__ valid,
-                                 const int32_t* __restrict__ read, const double* __restrict__ stats,
-                                 int64_t tile0, int64_t n_rows, float* __restrict__ probs, int want_logits) {
+                                 int64_t tile0, int64_t n_rows, HeadOut out) {
     // thread i handles (window, t) with t fastest so that the scatter is coalesced
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_rows) return;
+    if ((i & ~(int64_t)31) >= n_rows) return;            // whole warps only: head_output needs every lane
     const int t = (int)(i % kWindow);
     const int64_t wi = i / kWindow;                      // tile * 128 + w (local)
     const int w_in = (int)(wi % kTileWindows);
     const int64_t tile = wi / kTileWindows;
     const int64_t g = (tile0 + tile) * kTileWindows + w_in;
-    if (t >= valid[g]) return;
-    const float* yr = y + ((tile * kWindow + t) * kTileWindows + w_in) * (int64_t)F;
+    const bool real = i < n_rows && t < out.valid[g];
     float acc = b;
-    for (int k = 0; k < F; ++k) acc = fmaf(yr[k], w[k], acc);
-    float p = want_logits ? acc : 1.f / (1.f + expf(-acc));
-    if (stats) {                                         // scale == 0 or NaN: the reference divides by it
-        const double sc = stats[2 * read[g] + 1];
-        if (!(sc > 0.0)) p = nanf("");
+    if (real) {
+        const float* yr = y + ((tile * kWindow + t) * kTileWindows + w_in) * (int64_t)F;
+        for (int k = 0; k < F; ++k) acc = fmaf(yr[k], w[k], acc);
     }
-    probs[src[g] + t] = p;
+    head_output(out, g, t, real, acc);
 }
 
 // ---------------------------------------------------------------- forward
 // Carve the workspace for passes of at most `chunk_tiles` tiles.
 struct SimtBufs { float *x, *ca, *cb, *csc, *cout, *xproj, *y0, *y1; };
 
-static int simt_prepare(DevBuf* ws, const HostModel& hm, int64_t chunk_tiles, bool with_rnn, SimtBufs* b) {
+static int simt_prepare(DevBuf* ws, const HostModel& hm, int64_t chunk_tiles, SimtBufs* b) {
     const int64_t rows = chunk_tiles * kWindow * kTileWindows;
     const int C = hm.conv_channels(), H = hm.desc.layer_size;
-    const bool res = hm.n_res() > 0, rnn = with_rnn && hm.n_rnn() > 0;
+    const bool res = hm.n_res() > 0, rnn = hm.n_rnn() > 0;
     size_t fl = (size_t)rows;
     if (res) fl += (size_t)rows * C * 4;
     if (rnn) fl += (size_t)rows * (6 * H + 2 * 2 * H);
@@ -282,72 +251,49 @@ static int simt_prepare(DevBuf* ws, const HostModel& hm, int64_t chunk_tiles, bo
     return CF_OK;
 }
 
-// Normalise + window gather + residual blocks for tiles [tile0, tile0 + tiles): *feat points at
-// fp32 rows [(tile*35+t)*128+w][C] (or [..][1] when the network has no residual blocks).
-static int conv_stack(SimtEngine* e, const HostModel& hm, const SimtBufs& b, const int16_t* raw, const double* stats,
-                      const float* xwin, WindowTable tab, int64_t tile0, int64_t tiles, const float** feat,
-                      cudaStream_t stream, Profiler* prof) {
-    const int64_t rows = tiles * kWindow * kTileWindows;
-    {
-        ProfScope ps(prof, KC_K2_CONV, stream);
-        simt_fill_x_kernel<<<(unsigned)ceil_div(rows, 256), 256, 0, stream>>>(
-            raw, stats, xwin, tab.src, tab.valid, tab.read, tile0, rows, b.x);
-        CF_LAUNCHED();
-    }
-    *feat = b.x;
-    for (int blk = 0; blk < hm.n_res(); ++blk) {
-        auto conv = [&](int i, const float* in, const float* res, float* out, int relu) -> int {
-            const ConvLayer& c = hm.convs[i];
-            const int64_t total = rows * c.cout;
-            ProfScope ps(prof, KC_K2_CONV, stream);
-            simt_conv_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, stream>>>(
-                in, e->conv_w[i].as<float>(), e->conv_b[i].as<float>(), res, out, rows, c.k, c.cin, c.cout, relu);
-            CF_LAUNCHED();
-            return CF_OK;
-        };
-        const int i = 4 * blk;
-        CF_TRY(conv(i, *feat, nullptr, b.csc, 0));          // shortcut: BN(conv k1)
-        CF_TRY(conv(i + 1, *feat, nullptr, b.ca, 1));
-        CF_TRY(conv(i + 2, b.ca, nullptr, b.cb, 1));
-        CF_TRY(conv(i + 3, b.cb, b.csc, b.cout, 1));        // relu(relu(BN(conv)) + shortcut)
-        *feat = b.cout;                                     // conv i+3 no longer reads the block input
-    }
-    return CF_OK;
-}
-
-int simt_conv_stack(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* raw, const double* stats,
-                    const float* xwin, WindowTable tab, int64_t tile0, int64_t tiles, int64_t chunk_tiles,
-                    const float** feat, cudaStream_t stream, Profiler* prof) {
-    SimtBufs b;
-    CF_TRY(simt_prepare(ws, hm, chunk_tiles, false, &b));
-    return conv_stack(e, hm, b, raw, stats, xwin, tab, tile0, tiles, feat, stream, prof);
-}
-
 int simt_reserve(DevBuf* ws, const HostModel& hm, int64_t n_tiles) {
     if (n_tiles <= 0) return CF_OK;
     SimtBufs b;
-    return simt_prepare(ws, hm, n_tiles < kSimtChunkTiles ? n_tiles : kSimtChunkTiles, true, &b);
-}
-
-int simt_conv_stack_reserve(DevBuf* ws, const HostModel& hm, int64_t chunk_tiles) {
-    if (chunk_tiles <= 0) return CF_OK;
-    SimtBufs b;
-    return simt_prepare(ws, hm, chunk_tiles, false, &b);
+    return simt_prepare(ws, hm, n_tiles < kSimtChunkTiles ? n_tiles : kSimtChunkTiles, &b);
 }
 
 int simt_forward(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* raw, const double* stats,
                  const float* xwin, WindowTable tab, int64_t n_tiles, float* probs,
-                 cudaStream_t stream, Profiler* prof, bool want_logits) {
+                 cudaStream_t stream, Profiler* prof, bool want_logits, const LabelBits* bits) {
     if (n_tiles <= 0) return CF_OK;
     const int64_t chunk = n_tiles < kSimtChunkTiles ? n_tiles : kSimtChunkTiles;
     SimtBufs b;
-    CF_TRY(simt_prepare(ws, hm, chunk, true, &b));
+    CF_TRY(simt_prepare(ws, hm, chunk, &b));
+    const HeadOut head{tab.src, tab.valid, tab.read, raw ? stats : nullptr, probs, bits ? bits->lwords : nullptr,
+                      bits ? bits->threshold : 0.0, want_logits ? 1 : 0};
     const int H = hm.desc.layer_size;
     for (int64_t tile0 = 0; tile0 < n_tiles; tile0 += kSimtChunkTiles) {
         const int64_t tiles = (n_tiles - tile0) < kSimtChunkTiles ? (n_tiles - tile0) : kSimtChunkTiles;
         const int64_t rows = tiles * kWindow * kTileWindows;
-        const float* feat = nullptr;
-        CF_TRY(conv_stack(e, hm, b, raw, stats, xwin, tab, tile0, tiles, &feat, stream, prof));
+        // normalise + window gather, then the residual blocks: feat = fp32 rows [(tile*35+t)*128+w][C] (or [..][1]
+        // when the network has no residual blocks)
+        {
+            ProfScope ps(prof, KC_K2_CONV, stream);
+            CF_TRY(k1_fill_windows(raw, stats, xwin, tab, tile0, tiles, b.x, stream));
+        }
+        const float* feat = b.x;
+        for (int blk = 0; blk < hm.n_res(); ++blk) {
+            auto conv = [&](int i, const float* in, const float* res, float* out, int relu) -> int {
+                const ConvLayer& c = hm.convs[i];
+                const int64_t total = rows * c.cout;
+                ProfScope ps(prof, KC_K2_CONV, stream);
+                simt_conv_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, stream>>>(
+                    in, e->conv_w[i].as<float>(), e->conv_b[i].as<float>(), res, out, rows, c.k, c.cin, c.cout, relu);
+                CF_LAUNCHED();
+                return CF_OK;
+            };
+            const int i = 4 * blk;
+            CF_TRY(conv(i, feat, nullptr, b.csc, 0));           // shortcut: BN(conv k1)
+            CF_TRY(conv(i + 1, feat, nullptr, b.ca, 1));
+            CF_TRY(conv(i + 2, b.ca, nullptr, b.cb, 1));
+            CF_TRY(conv(i + 3, b.cb, b.csc, b.cout, 1));        // relu(relu(BN(conv)) + shortcut)
+            feat = b.cout;                                      // conv i+3 no longer reads the block input
+        }
         const int feat_dim = hm.n_res() ? hm.conv_channels() : 1;
         float* yin = nullptr;
         for (int l = 0; l < hm.n_rnn(); ++l) {
@@ -376,8 +322,7 @@ int simt_forward(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* 
         const float* hin = hm.n_rnn() ? yin : feat;
         ProfScope ps(prof, KC_K5_HEAD, stream);
         simt_head_kernel<<<(unsigned)ceil_div(rows, 256), 256, 0, stream>>>(
-            hin, e->head_w.as<float>(), e->head_b, hm.head_features(), tab.src, tab.valid, tab.read, raw ? stats : nullptr,
-            tile0, rows, probs, want_logits ? 1 : 0);
+            hin, e->head_w.as<float>(), e->head_b, hm.head_features(), tile0, rows, head);
         CF_LAUNCHED();
     }
     return CF_OK;

@@ -13,13 +13,15 @@
 // Default path of a pass (at most kTcChunkTiles tiles):
 //   TK2   tc_conv4_kernel        residual conv stack, two chains, operands in tensor memory
 //   TK4G  tc_gru_fused2_kernel   one GRU layer (input projection + recurrence), two tiles per CTA
-//   TK5   tc_head_kernel         dense 128 -> 1 + sigmoid from the partial dots of the last layer
+//   TK5   tc_head_kernel         dense 128 -> 1 + sigmoid from the partial dots of the last layer, then
+//                                probabilities and / or label bits (head_output, window_io.cuh)
 // (the conv stack and the GRU layer it feeds use bf16x3, the 128-wide GRU layers f16e5).
 // Other shapes: tc_conv2_kernel (networks with ONE residual block), tc_conv_block_kernel (every block
 // after the second of deeper stacks, once per block, from and to the K = 32 operand form),
 // tc_head_conv_kernel (ResNet-only networks other than two blocks).  Layer 0 of
 // RNN-only networks, whose input is 1 wide, is the KX = 1 form of TK4G: no x MMAs, the rank-1 update
-// x_t * w_row is added in the epilogue.
+// x_t * w_row is added in the epilogue; k1_fill_windows gathers that input into the conv stack's buffer.
+// The conv kernels gather their input by the same rule (window_input).
 //
 // Data layout: a tile is 128 windows (= 128 TMEM lanes = UMMA M); a block is (tile, t), one of
 // the 35 positions of those windows.  Activations that feed an MMA live in global memory as
@@ -33,6 +35,7 @@
 
 #include "model.cuh"
 #include "tc_ptx.cuh"
+#include "window_io.cuh"
 
 namespace cf {
 
@@ -110,7 +113,6 @@ struct TcLayer {
 };
 
 struct TcEngine {
-    SimtEnginePtr simt;               // RNN-only networks: normalised scalar input (simt_conv_stack without blocks)
     DevBuf conv_params;               // TK2 parameter block (see ConvParams), then [conv_nres - 2] parameter blocks of
                                       // tc_conv_block_kernel (block-1 slots); empty = no residual blocks
     int conv_nres = 0;
@@ -199,7 +201,6 @@ int tc_create(const HostModel& narrow, TcEnginePtr* out) {
     int dev = 0;
     CF_CUDA(cudaGetDevice(&dev));
     CF_CUDA(cudaDeviceGetAttribute(&e->n_sms, cudaDevAttrMultiProcessorCount, dev));
-    if (narrow.n_res() == 0) CF_TRY(simt_create(narrow, &e->simt));
     const HostModel hm = pad_model(narrow);          // everything below, the operand format included, sees C = 32 / H = 64
 #ifdef CF_TRACE_PROBES
     e->trace_path = getenv("CF_TC_TRACE");
@@ -301,7 +302,6 @@ int tc_create(const HostModel& narrow, TcEnginePtr* out) {
 }
 
 int tc_operand_format(const TcEngine* e) { return e ? e->fmt : 0; }
-bool tc_can_emit_bits(const TcEngine* e) { return e && !e->layers.empty(); }
 
 // ====================================================================== TK2: residual conv stack
 // Fuses, per tile of 128 windows: median/MAD normalisation of the raw signal, the 35-sample
@@ -440,17 +440,9 @@ tc_conv2_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
             // ---- gather + normalise (infer.py:101-105, 32-38): the two threads of a window split its 35 samples
             asm volatile("bar.sync 1, 256;" ::: "memory");        // previous tile's readers of xs are done
             {
-                const int64_t g = (tile0 + tile) * kTileWindows + row;
-                const int nv = valid[g];
-                const int64_t s0 = src[g];
-                double shift = 0.0, scale = 1.0;
-                if (raw && nv > 0) { const int r = read[g]; shift = stats[2 * r]; scale = stats[2 * r + 1]; }
+                const WindowInput x = window_input(raw, stats, xwin, src, valid, read, (tile0 + tile) * kTileWindows + row);
                 const int tb = ch ? 18 : 0, te = ch ? kWindow : 18;
-                for (int t = tb; t < te; ++t) {
-                    float v = 0.f;
-                    if (t < nv) v = raw ? (float)(((double)raw[s0 + t] - shift) / scale) : xwin[s0 + t];
-                    xs[t * 128 + row] = v;
-                }
+                for (int t = tb; t < te; ++t) xs[t * 128 + row] = x(t);
             }
             asm volatile("bar.sync 1, 256;" ::: "memory");
             make_o1(0);
@@ -708,17 +700,9 @@ tc_conv4_kernel(const uint8_t* __restrict__ params, const int16_t* __restrict__ 
                 // gather + normalise (infer.py:101-105, 32-38): the two threads of a window split its 35 samples
                 asm volatile("bar.sync 1, 256;" ::: "memory");        // previous tile's readers of xs are done
                 {
-                    const int64_t g = (tile0 + tile) * kTileWindows + row;
-                    const int nv = valid[g];
-                    const int64_t s0 = src[g];
-                    double shift = 0.0, scale = 1.0;
-                    if (raw && nv > 0) { const int r = read[g]; shift = stats[2 * r]; scale = stats[2 * r + 1]; }
+                    const WindowInput x = window_input(raw, stats, xwin, src, valid, read, (tile0 + tile) * kTileWindows + row);
                     const int tb = ch ? 18 : 0, te = ch ? kWindow : 18;
-                    for (int t = tb; t < te; ++t) {
-                        float v = 0.f;
-                        if (t < nv) v = raw ? (float)(((double)raw[s0 + t] - shift) / scale) : xwin[s0 + t];
-                        xs[t * 128 + row] = v;
-                    }
+                    for (int t = tb; t < te; ++t) xs[t * 128 + row] = x(t);
                 }
                 asm volatile("bar.sync 1, 256;" ::: "memory");
                 // the previous tile's last X batch (which read o1 slots) completed before its last epilogue
@@ -1551,14 +1535,11 @@ tc_gru_fused2_kernel(const uint8_t* __restrict__ wpk, const float* __restrict__ 
 
 // ====================================================================== TK5: head
 // p = sigmoid(sum of the partial dots + b), scattered to sample order with the padding cut
-// (infer.py:47).  One CTA per tile: the partials are read window-fastest (coalesced), transposed
+// (head_output).  One CTA per tile: the partials are read window-fastest (coalesced), transposed
 // through shared memory, and the probabilities are written position-fastest, which is contiguous in
 // the read because consecutive windows of a read are consecutive in the signal.
 __global__ void __launch_bounds__(256)
-tc_head_kernel(const float* __restrict__ head_part, int n_parts, float b, const int64_t* __restrict__ src,
-               const int32_t* __restrict__ valid, const int32_t* __restrict__ read,
-               const double* __restrict__ stats, int64_t tile0, int64_t n_rows, float* __restrict__ probs, int want_logits,
-               unsigned* __restrict__ lwords, double threshold) {
+tc_head_kernel(const float* __restrict__ head_part, int n_parts, float b, int64_t tile0, int64_t n_rows, HeadOut out) {
     __shared__ float logit[kWindow][kTileWindows + 1];
     const int64_t tile = blockIdx.x;
     if (tile * kTileWindows * kWindow >= n_rows) return;
@@ -1570,34 +1551,11 @@ tc_head_kernel(const float* __restrict__ head_part, int n_parts, float b, const 
         logit[t][w] = acc;
     }
     __syncthreads();
-    // 4480 = 35 * 128 = 17.5 * 256: the tail iteration runs whole warps, so the warp-level votes below are converged
+    // 4480 = 35 * 128 = 17.5 * 256: the tail iteration runs whole warps, so head_output's lanes are converged
     for (int i = threadIdx.x; i < kWindow * kTileWindows; i += blockDim.x) {
         const int w = i / kWindow, t = i % kWindow;
         const int64_t g = (tile0 + tile) * kTileWindows + w;
-        const bool real = t < valid[g];
-        float p = 0.f;
-        if (real) {
-            p = want_logits ? logit[t][w] : 1.f / (1.f + expf(-logit[t][w]));
-            if (stats) {
-                const double sc = stats[2 * read[g] + 1];
-                if (!(sc > 0.0)) p = nanf("");
-            }
-        }
-        if (!lwords) {
-            if (real) probs[src[g] + t] = p;
-            continue;
-        }
-        // label bits instead of probabilities (class_from_threshold, infer.py:128-138: the f32 score widened to
-        // double, >=): consecutive lanes hold consecutive samples, so a warp touches at most a few label words -
-        // lanes of one word OR their bits together and one of them issues the atomic
-        const bool hit = real && (double)p >= threshold;
-        const unsigned hits = __ballot_sync(0xffffffffu, hit);
-        if (hit) {
-            const int64_t sidx = src[g] + t;
-            const unsigned peers = __match_any_sync(hits, (unsigned long long)(sidx >> 5));
-            const unsigned bits = __reduce_or_sync(peers, 1u << (sidx & 31));
-            if ((threadIdx.x & 31) == __ffs(peers) - 1) atomicOr(&lwords[sidx >> 5], bits);
-        }
+        head_output(out, g, t, t < out.valid[g], logit[t][w]);
     }
 }
 
@@ -1607,10 +1565,8 @@ tc_head_kernel(const float* __restrict__ head_part, int n_parts, float b, const 
 // contiguous bytes per plane and K group), the logits are transposed through shared memory and the
 // probabilities written position-fastest (contiguous in the read).
 __global__ void __launch_bounds__(256)
-tc_head_conv_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ w, float b,
-                    const int64_t* __restrict__ src, const int32_t* __restrict__ valid,
-                    const int32_t* __restrict__ read, const double* __restrict__ stats,
-                    int64_t tile0, int64_t n_rows, float* __restrict__ probs, int want_logits) {
+tc_head_conv_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ w, float b, int64_t tile0, int64_t n_rows,
+                    HeadOut out) {
     __shared__ float logit[kWindow][kTileWindows + 1];
     __shared__ float ws[kC];
     const int64_t tile = blockIdx.x;
@@ -1637,24 +1593,15 @@ tc_head_conv_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict
         logit[t][wr] = acc;
     }
     __syncthreads();
+    // whole warps in the tail iteration, as in tc_head_kernel
     for (int i = threadIdx.x; i < kWindow * kTileWindows; i += blockDim.x) {
         const int wr = i / kWindow, t = i % kWindow;
         const int64_t g = (tile0 + tile) * kTileWindows + wr;
-        if (t >= valid[g]) continue;
-        float p = want_logits ? logit[t][wr] : 1.f / (1.f + expf(-logit[t][wr]));
-        if (stats) {
-            const double sc = stats[2 * read[g] + 1];
-            if (!(sc > 0.0)) p = nanf("");
-        }
-        probs[src[g] + t] = p;
+        head_output(out, g, t, t < out.valid[g], logit[t][wr]);
     }
 }
 
 // ====================================================================== forward
-int simt_conv_stack(SimtEngine* e, DevBuf* ws, const HostModel& hm, const int16_t* raw, const double* stats,
-                    const float* xwin, WindowTable tab, int64_t tile0, int64_t tiles, int64_t chunk_tiles,
-                    const float** feat, cudaStream_t stream, Profiler* prof);
-
 static size_t tc_workspace_bytes(int64_t tiles) {
     const size_t blocks = (size_t)tiles * kWindow;
     size_t b = 0;
@@ -1664,12 +1611,9 @@ static size_t tc_workspace_bytes(int64_t tiles) {
     return b + 4096;
 }
 
-int tc_reserve(const TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, int64_t n_tiles) {
+int tc_reserve(DevBuf* ws, int64_t n_tiles) {
     if (n_tiles <= 0) return CF_OK;
-    const int64_t chunk = n_tiles < kTcChunkTiles ? n_tiles : kTcChunkTiles;
-    CF_TRY(ws->ensure(tc_workspace_bytes(chunk)));
-    if (!e->conv_params.ptr) CF_TRY(simt_conv_stack_reserve(simt_ws, hm, chunk));
-    return CF_OK;
+    return ws->ensure(tc_workspace_bytes(n_tiles < kTcChunkTiles ? n_tiles : kTcChunkTiles));
 }
 
 // Every tensor-core kernel allocates all 512 TMEM columns of its SM.  Calls on different execution contexts may
@@ -1698,11 +1642,11 @@ static int tc_set_attributes() {
     return CF_OK;
 }
 
-int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, const int16_t* raw, const double* stats,
-               const float* xwin, WindowTable tab, int64_t n_tiles, float* probs, cudaStream_t stream, Profiler* prof,
-               bool want_logits, const LabelBits* bits) {
+int tc_forward(TcEngine* e, DevBuf* ws, const int16_t* raw, const double* stats, const float* xwin, WindowTable tab,
+               int64_t n_tiles, float* probs, cudaStream_t stream, Profiler* prof, bool want_logits, const LabelBits* bits) {
     if (n_tiles <= 0) return CF_OK;
-    if (bits && (e->layers.empty() || want_logits)) { set_error("label-bit output needs a GRU head"); return CF_ERR_BAD_ARG; }
+    const HeadOut head{tab.src, tab.valid, tab.read, raw ? stats : nullptr, probs, bits ? bits->lwords : nullptr,
+                      bits ? bits->threshold : 0.0, want_logits ? 1 : 0};
     const int64_t chunk = n_tiles < kTcChunkTiles ? n_tiles : kTcChunkTiles;
     CF_TRY(ws->ensure(tc_workspace_bytes(chunk)));
     const size_t blocks_max = (size_t)chunk * kWindow;
@@ -1721,7 +1665,7 @@ int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, co
         const int64_t tiles = std::min<int64_t>(kTcChunkTiles, n_tiles - tile0);
         const int64_t blocks = tiles * kWindow;
         const int64_t rows = blocks * 128;
-        const float* feat = nullptr;             // RNN-only networks: the normalised scalar input x [rows]
+        float* feat = nullptr;                   // RNN-only networks: the normalised scalar input x [rows]
         const __nv_bfloat16* a_in = nullptr;
         if (e->conv_params.ptr) {
             ProfScope ps(prof, KC_K2_CONV, stream);
@@ -1747,7 +1691,10 @@ int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, co
                 a_in = out;
             }
         } else {
-            CF_TRY(simt_conv_stack(e->simt.get(), simt_ws, hm, raw, stats, xwin, tab, tile0, tiles, chunk, &feat, stream, prof));
+            // no residual blocks: a0, which only the conv stack writes, holds the scalar input (rows * 4 bytes)
+            ProfScope ps(prof, KC_K2_CONV, stream);
+            feat = reinterpret_cast<float*>(a0);
+            CF_TRY(k1_fill_windows(raw, stats, xwin, tab, tile0, tiles, feat, stream));
         }
         for (int l = 0; l < n_layers; ++l) {
             const TcLayer& L = e->layers[l];
@@ -1812,22 +1759,17 @@ int tc_forward(TcEngine* e, DevBuf* ws, DevBuf* simt_ws, const HostModel& hm, co
         if (n_layers == 0 && e->conv_nres == 2) {
             // ResNet-only, two residual blocks: the conv kernel's epilogue already took the dense layer (two partial dots)
             ProfScope ps(prof, KC_K5_HEAD, stream);
-            tc_head_kernel<<<(unsigned)tiles, 256, 0, stream>>>(
-                head_part, 2, e->head_b, tab.src, tab.valid, tab.read, raw ? stats : nullptr, tile0, rows, probs, want_logits ? 1 : 0,
-                nullptr, 0.0);
+            tc_head_kernel<<<(unsigned)tiles, 256, 0, stream>>>(head_part, 2, e->head_b, tile0, rows, head);
             CF_LAUNCHED();
         } else if (n_layers == 0) {
             // ResNet-only: dense on the conv output
             ProfScope ps(prof, KC_K5_HEAD, stream);
-            tc_head_conv_kernel<<<(unsigned)tiles, 256, 0, stream>>>(
-                a_in, e->head_w.as<float>(), e->head_b, tab.src, tab.valid, tab.read, raw ? stats : nullptr, tile0, rows, probs, want_logits ? 1 : 0);
+            tc_head_conv_kernel<<<(unsigned)tiles, 256, 0, stream>>>(a_in, e->head_w.as<float>(), e->head_b, tile0, rows, head);
             CF_LAUNCHED();
         } else {
             // GRU head: the last layer's epilogue wrote eight partial dots per position (2 directions x 4 unit groups)
             ProfScope ps(prof, KC_K5_HEAD, stream);
-            tc_head_kernel<<<(unsigned)tiles, 256, 0, stream>>>(
-                head_part, 8, e->head_b, tab.src, tab.valid, tab.read, raw ? stats : nullptr, tile0, rows, probs, want_logits ? 1 : 0,
-                bits ? bits->lwords : nullptr, bits ? bits->threshold : 0.0);
+            tc_head_kernel<<<(unsigned)tiles, 256, 0, stream>>>(head_part, 8, e->head_b, tile0, rows, head);
             CF_LAUNCHED();
         }
     }

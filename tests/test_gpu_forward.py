@@ -133,18 +133,19 @@ def test_engine_cross_check_large():
 def test_tcgen05_kernel_variants(kind, n_res):
     """Networks off the default path, which run split-bf16 operands in every layer, against the fp32 SIMT engine:
     one residual block (tc_conv2_kernel, then the 32- and 128-wide GRU layers or tc_head_conv_kernel) and three
-    (the CUDA-core conv stack, tc_pack_a_kernel, then the GRU layers).  The longest input spans more tiles than
-    the GPU has SMs, so a CTA of every kernel runs several tiles."""
+    (tc_conv4_kernel for blocks 0 and 1, tc_conv_block_kernel for block 2, then the GRU layers).  The longest input
+    spans more tiles than the GPU has SMs, so a CTA of every kernel runs several tiles."""
     w = weights.random_init(kind, seed=30 + n_res, n_layers_res=n_res)
     m = _model(kind, "auto", w, n_layers_res=n_res)
     assert m.resolved_engine == "tcgen05" and m.operand_format == "bf16x3"
     ref = _model(kind, "simt", w, n_layers_res=n_res)
+    g = golden("forward_resnetrnn_shipped.npz")
+    reads = [g["read%d" % i] for i in range(int(g["n_reads"]))] + synth.synth_reads([30000, 4481, 700000], base_seed=77)
     if kind == "ResNet":
         x = np.random.default_rng(31).normal(0, 1.5, size=(20000, 35, 1)).astype(np.float32)
         assert np.abs(m.infer(x) - ref.infer(x)).max() < PROB_TOL
-        return
-    g = golden("forward_resnetrnn_shipped.npz")
-    reads = [g["read%d" % i] for i in range(int(g["n_reads"]))] + synth.synth_reads([30000, 4481, 700000], base_seed=77)
+        # tc_head_conv_kernel's label bits: the intervals without scores are those with scores
+        assert infer.infer_reads(reads, m)[0] == infer.infer_reads(reads, m, return_scores=True)[0]
     hps, lengths, scores = infer.infer_reads(reads, m, return_scores=True)
     hps2, lengths2, scores2 = infer.infer_reads(reads, ref, return_scores=True)
     assert lengths == lengths2

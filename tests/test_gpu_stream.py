@@ -68,6 +68,7 @@ def test_stream_equals_infer_reads(kind, shipped):
         got = list(infer.infer_stream(iter(reads), model, group_samples=group_samples, depth=depth))
         _assert_same(got, hps, lengths)
     hps_s, lengths_s, scores = infer.infer_reads(reads, model, return_scores=True)
+    assert hps_s == hps and lengths_s == lengths        # the label bits do not depend on writing the scores
     for group_samples, depth in [(1, 3), (300_000, 2)]:
         got = list(infer.infer_stream(reads, model, return_scores=True, group_samples=group_samples, depth=depth))
         _assert_same(got, hps_s, lengths_s, scores)
