@@ -88,6 +88,17 @@ SIGNATURES = {
                                       c_void]),
     "cf_selftest_f16e5": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int32, ctypes.c_int32, c_void, ctypes.c_int32, c_void, c_void]),
     "cf_launch_count": (ctypes.c_int64, []),
+    "cf_trainer_create": (ctypes.c_int, [ctypes.POINTER(ModelDesc), ctypes.POINTER(c_void), c_i64_p, ctypes.c_int32,
+                                         ctypes.POINTER(c_void), ctypes.POINTER(c_void), ctypes.c_int32,
+                                         ctypes.POINTER(c_void)]),
+    "cf_trainer_destroy": (None, [c_void]),
+    "cf_trainer_step": (ctypes.c_int, [c_void, c_void, c_void, ctypes.c_int64, ctypes.c_float, ctypes.c_float,
+                                       ctypes.c_uint64, ctypes.c_int64, ctypes.POINTER(ctypes.c_double),
+                                       ctypes.POINTER(ctypes.c_double), c_void]),
+    "cf_trainer_gradients": (ctypes.c_int, [c_void, c_void, c_void, ctypes.c_int64, ctypes.c_float, ctypes.c_uint64,
+                                            ctypes.c_int64, ctypes.POINTER(c_void), ctypes.POINTER(ctypes.c_double),
+                                            c_void]),
+    "cf_trainer_read": (ctypes.c_int, [c_void, ctypes.POINTER(c_void), ctypes.POINTER(c_void), ctypes.POINTER(c_void)]),
 }
 
 _lib = None

@@ -18,7 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(HERE, "..", "include")
 LIB = os.environ.get("CF_LIB_OUT") or os.path.join(HERE, "libcatfish_b200.so")
-SOURCES = ["api.cu", "k1_normalize.cu", "k6_intervals.cu", "k7_chunks.cu", "k8_split.cu", "k9_validate.cu", "k11_sweep.cu", "simt_engine.cu", "tc_engine.cu"]
+SOURCES = ["api.cu", "k1_normalize.cu", "k6_intervals.cu", "k7_chunks.cu", "k8_split.cu", "k9_validate.cu", "k11_sweep.cu", "k12_train.cu", "simt_engine.cu", "tc_engine.cu"]
 NVCC_FLAGS = (["-DCF_PRECISE_ACT"] if os.environ.get("CF_PRECISE_ACT") else []) + os.environ.get("CF_EXTRA_DEFS", "").split() + ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC,-O2,-Wall", "-Xptxas", "-v"]
 

@@ -1,11 +1,18 @@
-"""Mirror of the reference's ``RNN`` model class, inference only.
+"""Mirror of the reference's ``RNN`` model class: inference and RMSProp training on the device.
 
 Reference: /root/reference/catfish/models/rnn_class.py (``RNN.__init__`` :10-54,
 ``restore_network`` :191-198, ``initialize_network`` :186-188, ``infer`` :213-219).
 Same constructor kwargs, attributes and return types; the TensorFlow graph and
 session are replaced by a handle of the C-ABI CUDA library.  ``test_network``
-follows the validation twin networks/rnn_class.py:222-261.  Training
-(``train_network``, optimizer, TensorBoard) is out of scope and raises.
+follows the validation twin networks/rnn_class.py:222-261.
+
+``train_network`` runs one step of the reference's optimizer (tf.train.RMSPropOptimizer,
+``optimizer_choice: RMSProp``) on a ``cf_trainer`` (csrc/k12_train.cu): output dropout
+on every GRU cell with a Philox mask keyed by ``dropout_seed`` and ``global_step``, mean
+sigmoid cross-entropy, TF 1.x ApplyRMSProp.  Inference after a step sees the trained
+weights; ``save_network`` writes ``ckpnt-<step>.npz`` with the optimizer slots under the
+TF bundle's names, and ``restore_network`` brings them back, so training resumes bit for
+bit.  TensorBoard and log directories (``RNN(save=True)``) are out of scope and raise.
 """
 
 import ctypes
@@ -40,13 +47,21 @@ class RNN(object):
             self.network_type = self.cell_type
         self.model_type = self.network_type
         if save:
-            raise NotImplementedError("training / model saving is out of scope of catfish_b200")
+            raise NotImplementedError("TensorBoard / log directories (save=True) are out of scope of catfish_b200; "
+                                      "use save_network()")
         from . import get_device
         self.device = get_device() if device is None else int(device)
         self.engine = {"auto": _cabi.ENGINE_AUTO, "tcgen05": _cabi.ENGINE_TCGEN05,
                        "simt": _cabi.ENGINE_SIMT}[engine]
         self._handle = None
         self._weights = None
+        # training: the Philox key of the dropout mask, the step counter train_network advances, the cf_trainer
+        # (created by the first step), the optimizer state a restore brought, and whether _handle predates a step
+        self.dropout_seed = 0
+        self.global_step = 0
+        self._trainer = None
+        self._opt_state = None
+        self._trained = False
         self.tp = self.fp = self.tn = self.fn = 0
         self.sweep_counts = None        # test_network_sweep's [T, 4] accumulator (reset_sweep)
         # idle slots (infer._Slot: stream, buffers) of infer_reads / evaluate_reads on the default context; a call
@@ -68,12 +83,20 @@ class RNN(object):
 
     # ------------------------------------------------------------------ weights
     def set_weights(self, weights):
-        """Install a ``{tf_variable_name: array}`` weight set and (re)build the device handle."""
+        """Install a ``{tf_variable_name: array}`` weight set and (re)build the device handle.  Training restarts
+        from these weights with fresh optimizer slots."""
+        self._drop_trainer()
+        self._opt_state = None
+        return self._install(weights)
+
+    def _names(self):
+        return list(_weights.expected_shapes(self.network_type_name, **self._hpm()).keys())
+
+    def _install(self, weights):
         w = _weights.check_weights(weights, self.network_type_name, **self._hpm())
         lib = _cabi.load_library()
         self._release()
-        names = list(_weights.expected_shapes(self.network_type_name, **self._hpm()).keys())
-        arrays = [np.ascontiguousarray(w[n], np.float32) for n in names]
+        arrays = [np.ascontiguousarray(w[n], np.float32) for n in self._names()]
         ptrs = (ctypes.c_void_p * len(arrays))(*[a.ctypes.data for a in arrays])
         sizes = (ctypes.c_int64 * len(arrays))(*[a.size for a in arrays])
         handle = ctypes.c_void_p()
@@ -82,9 +105,11 @@ class RNN(object):
                                         ctypes.byref(handle)))
         self._handle = handle
         self._weights = w
+        self._trained = False
         return self
 
     def get_weights(self):
+        self._sync_trained()
         return dict(self._weights) if self._weights is not None else None
 
     def initialize_network(self, seed=0):
@@ -100,12 +125,17 @@ class RNN(object):
             ckpnt = _latest_checkpoint(path)
         prefix = os.path.join(path, ckpnt)
         if os.path.exists(prefix + ".index"):
-            w = _weights.load_tf_checkpoint(prefix)
+            w, slots = _weights.split_slots(_weights.tf_checkpoint.load_checkpoint(prefix))
         elif os.path.exists(prefix + ".npz"):
-            w = _weights.load_npz(prefix + ".npz")
+            w, slots = _weights.split_slots(_weights.load_npz(prefix + ".npz"))
         else:
             raise ValueError("checkpoint %s not found" % prefix)
         self.set_weights(w)
+        # the optimizer state travels with the checkpoint: the next train_network continues where it stopped
+        self._opt_state = slots or None
+        step = _weights.checkpoint_step(ckpnt)
+        if step is not None:
+            self.global_step = step
         print("Model {} restored\n".format(os.path.normpath(path).split(os.sep)[-2]
                                            if os.sep in os.path.normpath(path) else path))
         return self
@@ -113,6 +143,7 @@ class RNN(object):
     # ------------------------------------------------------------------ inference
     @property
     def handle(self):
+        self._sync_trained()
         if self._handle is None:
             raise RuntimeError("network has no weights: call restore_network() or initialize_network() first")
         return self._handle
@@ -144,9 +175,147 @@ class RNN(object):
             confidences = pd.cpu().numpy()
         return np.reshape(confidences, (-1)).astype(float)
 
-    # ------------------------------------------------------------------ out of scope
-    def train_network(self, *args, **kwargs):
-        raise NotImplementedError("training is out of scope of catfish_b200 (inference hot path only)")
+    # ------------------------------------------------------------------ training
+    def train_network(self, train_x, train_y):
+        """One optimizer step on one batch (rnn_class.py ``train_network``): ``train_x`` [n, 35, 1], ``train_y``
+        n * 35 labels in {0, 1}.  Uses ``self.learning_rate``, ``self.keep_prob`` and the dropout mask of
+        (``self.dropout_seed``, ``self.global_step``), advances ``global_step`` and returns ``(train_acc, train_loss)``
+        of the step's forward pass (dropout applied)."""
+        import torch
+        keep = self._check_train_params(self.keep_prob)
+        lr = float(self.learning_rate)
+        if not (np.isfinite(lr) and lr > 0):
+            raise ValueError("learning_rate must be finite and > 0, got %r" % (self.learning_rate,))
+        x, y8 = self._train_arrays(train_x, train_y)
+        trainer = self._ensure_trainer()
+        acc, loss = ctypes.c_double(), ctypes.c_double()
+        dev = torch.device("cuda", self.device)
+        with torch.cuda.device(dev):
+            xd = torch.from_numpy(x.reshape(x.shape[0], self.window)).to(dev)
+            yd = torch.from_numpy(y8).to(dev)
+            stream = torch.cuda.current_stream(dev)
+            _cabi.check(_cabi.load_library().cf_trainer_step(
+                trainer, xd.data_ptr(), yd.data_ptr(), x.shape[0], lr, keep, self._seed(), int(self.global_step),
+                ctypes.byref(loss), ctypes.byref(acc), stream.cuda_stream))
+        self.global_step += 1
+        self._trained = True
+        return np.float32(acc.value), np.float32(loss.value)
+
+    def compute_gradients(self, train_x, train_y, keep_prob=None, step=None):
+        """``{variable: dL/dvar}`` of the step ``train_network`` would take (no update, ``global_step`` unchanged);
+        ``keep_prob`` / ``step`` default to ``self.keep_prob`` / ``self.global_step``.  Returns (gradients, loss)."""
+        import torch
+        keep = self._check_train_params(self.keep_prob if keep_prob is None else keep_prob)
+        x, y8 = self._train_arrays(train_x, train_y)
+        trainer = self._ensure_trainer()
+        names = self._names()
+        grads = {n: np.zeros(self._weights[n].shape, np.float32) for n in names if _weights.is_trainable(n)}
+        ptrs = (ctypes.c_void_p * len(names))(*[grads[n].ctypes.data if n in grads else None for n in names])
+        loss = ctypes.c_double()
+        dev = torch.device("cuda", self.device)
+        with torch.cuda.device(dev):
+            xd = torch.from_numpy(x.reshape(x.shape[0], self.window)).to(dev)
+            yd = torch.from_numpy(y8).to(dev)
+            stream = torch.cuda.current_stream(dev)
+            _cabi.check(_cabi.load_library().cf_trainer_gradients(
+                trainer, xd.data_ptr(), yd.data_ptr(), x.shape[0], keep, self._seed(),
+                int(self.global_step if step is None else step), ptrs, ctypes.byref(loss), stream.cuda_stream))
+        return grads, float(loss.value)
+
+    def optimizer_state(self):
+        """``{"<var>/RMSProp": ms, "<var>/RMSProp_1": mom}`` of the optimizer (fresh slots before the first step)."""
+        if self._trainer is not None:
+            return self._read_trainer()[1]
+        if self._opt_state is not None:
+            return dict(self._opt_state)
+        return _weights.fresh_slots(self.get_weights())
+
+    def save_network(self, path, step=None):
+        """``tf.train.Saver.save``: ``<path>/ckpnt-<step>.npz`` (``step`` defaults to ``global_step``) holding the
+        inference tensors and the optimizer slots under the TF bundle's names; ``<path>/checkpoint`` points at it.
+        Returns the file's path."""
+        w = self.get_weights()
+        if w is None:
+            raise RuntimeError("network has no weights: call restore_network() or initialize_network() first")
+        return _weights.save_checkpoint(path, self.global_step if step is None else step, w, self.optimizer_state())
+
+    def _check_train_params(self, keep_prob):
+        if self.optimizer_choice != "RMSProp":
+            raise ValueError("optimizer_choice %r is not supported (RMSProp only)" % (self.optimizer_choice,))
+        keep = float(keep_prob)
+        if not (0.0 < keep <= 1.0):
+            raise ValueError("keep_prob must be in (0, 1], got %r" % (keep_prob,))
+        return keep
+
+    def _seed(self):
+        return int(self.dropout_seed) & 0xFFFFFFFFFFFFFFFF
+
+    def _train_arrays(self, train_x, train_y):
+        x, y8 = self._validation_arrays(train_x, train_y)
+        if x.shape[0] < 1:
+            raise ValueError("a training batch needs at least one window")
+        if y8.max() > 1:
+            raise ValueError("training labels must be 0 or 1")
+        return x, np.ascontiguousarray(y8)
+
+    def _ensure_trainer(self):
+        if self._trainer is not None:
+            return self._trainer
+        if self._weights is None:
+            raise RuntimeError("network has no weights: call restore_network() or initialize_network() first")
+        names = self._names()
+        arrays = [np.ascontiguousarray(self._weights[n], np.float32) for n in names]
+        keep_alive = list(arrays)
+        ptrs = (ctypes.c_void_p * len(names))(*[a.ctypes.data for a in arrays])
+        sizes = (ctypes.c_int64 * len(names))(*[a.size for a in arrays])
+        rms = mom = None
+        if self._opt_state:
+            fresh = _weights.fresh_slots(self._weights)
+            slots = {k: np.ascontiguousarray(self._opt_state.get(k, v), np.float32) for k, v in fresh.items()}
+            for k, v in slots.items():
+                if v.shape != fresh[k].shape:
+                    raise ValueError("optimizer slot %s has shape %s, expected %s" % (k, v.shape, fresh[k].shape))
+            keep_alive += list(slots.values())
+            rms = (ctypes.c_void_p * len(names))(*[slots[n + _weights.RMS_SLOT].ctypes.data
+                                                   if _weights.is_trainable(n) else None for n in names])
+            mom = (ctypes.c_void_p * len(names))(*[slots[n + _weights.MOM_SLOT].ctypes.data
+                                                   if _weights.is_trainable(n) else None for n in names])
+        handle = ctypes.c_void_p()
+        desc = self._desc()
+        _cabi.check(_cabi.load_library().cf_trainer_create(ctypes.byref(desc), ptrs, sizes, len(names), rms, mom,
+                                                           self.device, ctypes.byref(handle)))
+        del keep_alive
+        self._trainer = handle
+        return handle
+
+    def _read_trainer(self):
+        """(variables, slots) of the trainer, copied to the host."""
+        names = self._names()
+        w = {n: np.empty(self._weights[n].shape, np.float32) for n in names}
+        trainable = [n for n in names if _weights.is_trainable(n)]
+        slots = {}
+        for n in trainable:
+            slots[n + _weights.RMS_SLOT] = np.empty(w[n].shape, np.float32)
+            slots[n + _weights.MOM_SLOT] = np.empty(w[n].shape, np.float32)
+        ptr = lambda d, suffix: (ctypes.c_void_p * len(names))(*[
+            d[n + suffix].ctypes.data if (n + suffix) in d else None for n in names])
+        _cabi.check(_cabi.load_library().cf_trainer_read(self._trainer, ptr(w, ""), ptr(slots, _weights.RMS_SLOT),
+                                                         ptr(slots, _weights.MOM_SLOT)))
+        return w, slots
+
+    def _sync_trained(self):
+        """Rebuild the inference handle from the trainer's variables once after training steps."""
+        if self._trained and self._trainer is not None:
+            self._install(self._read_trainer()[0])
+
+    def _drop_trainer(self):
+        if getattr(self, "_trainer", None) is not None:
+            try:
+                _cabi.load_library().cf_trainer_destroy(self._trainer)
+            except Exception:
+                pass
+            self._trainer = None
+        self._trained = False
 
     def test_network(self, test_x, test_y, read_name=None, file_path=None, padding_size=0, threshold=0.5):
         """networks/rnn_class.py:222-261 ("next" row N4): forward pass + confusion counts.
@@ -237,9 +406,11 @@ class RNN(object):
 
     def close(self):
         self._release()
+        self._drop_trainer()
 
     def __del__(self):
         self._release()
+        self._drop_trainer()
 
 
 def _latest_checkpoint(path):

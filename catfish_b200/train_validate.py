@@ -1,4 +1,5 @@
-"""Validation driver of the reference over in-memory reads ("next" row N4).
+"""Validation driver of the reference over in-memory reads ("next" row N4).  The training half of
+``train_and_validate`` is ``RNN.train_network`` / ``save_network`` (INTEGRATION.md, "Training loop").
 
 Reference: /root/reference/networks/train_validate.py (``padding`` :51-64, ``reshape_input`` :15-31,
 ``validate`` :188-295).  ``validate`` here takes ``(data, labels)`` arrays instead of ``.npz``

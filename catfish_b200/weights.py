@@ -129,6 +129,53 @@ def save_npz(path, weights):
     np.savez(path, **{k: np.asarray(v, np.float32) for k, v in weights.items()})
 
 
+def is_trainable(name):
+    """Whether the optimizer updates ``name``: every inference variable but the BN moving statistics."""
+    return not (name.endswith("/moving_mean") or name.endswith("/moving_variance"))
+
+
+# the two slots tf.train.RMSPropOptimizer keeps per trainable variable, under the TF bundle's names
+RMS_SLOT, MOM_SLOT = "/RMSProp", "/RMSProp_1"
+
+
+def split_slots(tensors):
+    """``{name: array}`` of a checkpoint -> (inference tensors, RMSProp slots)."""
+    slots = {k: v for k, v in tensors.items() if k.endswith(RMS_SLOT) or k.endswith(MOM_SLOT)}
+    return {k: v for k, v in tensors.items() if tf_checkpoint.is_inference_tensor(k)}, slots
+
+
+def fresh_slots(weights):
+    """Slots of a fresh optimizer: ``<var>/RMSProp`` ones, ``<var>/RMSProp_1`` zeros."""
+    out = {}
+    for k, v in weights.items():
+        if is_trainable(k):
+            out[k + RMS_SLOT] = np.ones(v.shape, np.float32)
+            out[k + MOM_SLOT] = np.zeros(v.shape, np.float32)
+    return out
+
+
+def save_checkpoint(path, step, weights, slots):
+    """Write ``<path>/ckpnt-<step>.npz`` (inference tensors + slots) and point ``<path>/checkpoint`` at it, as
+    tf.train.Saver does for the reference's ``ckpnt-<step>`` bundles.  Returns the .npz path."""
+    os.makedirs(path, exist_ok=True)
+    name = "ckpnt-%d" % int(step)
+    out = os.path.join(path, name + ".npz")
+    tensors = dict(weights)
+    tensors.update(slots)
+    save_npz(out, tensors)
+    with open(os.path.join(path, "checkpoint"), "w") as f:
+        f.write('model_checkpoint_path: "%s"\nall_model_checkpoint_paths: "%s"\n' % (name, name))
+    return out
+
+
+def checkpoint_step(ckpnt):
+    """The global step in a checkpoint name ``ckpnt-<step>``, or None."""
+    try:
+        return int(str(ckpnt).rsplit("-", 1)[1])
+    except (IndexError, ValueError):
+        return None
+
+
 def load_tf_checkpoint(prefix):
     """Inference variables of a TF-V2 bundle (optimizer slots dropped)."""
     return tf_checkpoint.load_checkpoint(prefix, names=tf_checkpoint.is_inference_tensor)

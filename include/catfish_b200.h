@@ -321,6 +321,37 @@ int cf_vote_events(int32_t device, const double* scores_dev, int64_t n_scores, c
 int cf_selftest_f16e5(int32_t device, const float* a_dev, int32_t k, int32_t n, const float* w_host, int32_t mode,
                       float* out_dev, void* stream);
 
+/*
+ * cf_trainer - RMSProp training of the network (rnn_class.py train_network with tf.train.RMSPropOptimizer), fp32 on
+ * CUDA cores.  A trainer owns fp32 variables in TF layout (the tensors of cf_model_create, same order), the optimizer
+ * slots <var>/RMSProp (ms) and <var>/RMSProp_1 (mom), and a workspace that only grows.  One step: the inference
+ * graph with output dropout on every GRU cell, mean sigmoid cross-entropy over all n_windows * 35 positions, and
+ * TF 1.x ApplyRMSProp (decay 0.9, momentum 0, epsilon 1e-10) on every variable but the BN moving statistics.
+ * The dropout mask is Philox4x32-10 with key = seed and counter = (step, 2 * layer + direction, window, t * H + unit):
+ * a unit is kept when the top 24 bits of output word 0 are < round(keep_prob * 2^24); keep_prob = 1 draws nothing.
+ * Calls on one trainer are ordered on the device as calls on one execution context are.  Deterministic: the same
+ * inputs give bit-identical variables and slots.
+ */
+typedef struct cf_trainer cf_trainer;
+/* tensors / sizes as cf_model_create; rms / mom parallel to tensors (NULL = fresh slots: ones / zeros; entries of the
+ * BN moving statistics are ignored).  desc->engine is ignored. */
+int cf_trainer_create(const cf_model_desc* desc, const float* const* tensors, const int64_t* sizes, int32_t n_tensors,
+                      const float* const* rms, const float* const* mom, int32_t device, cf_trainer** out);
+void cf_trainer_destroy(cf_trainer* trainer);
+/* One RMSProp step on x_dev float32 [n_windows][35], labels_dev uint8 [n_windows * 35] in {0, 1}; step in [0, 2^32).
+ * loss / accuracy of the step's forward (either may be NULL; non-NULL synchronises).  CF_ERR_BAD_ARG for NULL
+ * pointers, n_windows < 1, keep_prob outside (0, 1], a learning_rate that is not finite or <= 0. */
+int cf_trainer_step(cf_trainer* trainer, const float* x_dev, const uint8_t* labels_dev, int64_t n_windows,
+                    float learning_rate, float keep_prob, uint64_t seed, int64_t step, double* loss_out,
+                    double* accuracy_out, void* stream);
+/* Gradients of the same step without the update: grads_host parallel to tensors (entries may be NULL; the BN moving
+ * statistics are never written).  Synchronises. */
+int cf_trainer_gradients(cf_trainer* trainer, const float* x_dev, const uint8_t* labels_dev, int64_t n_windows,
+                         float keep_prob, uint64_t seed, int64_t step, float* const* grads_host, double* loss_out,
+                         void* stream);
+/* Copy variables and slots out (any of the three arrays may be NULL, and any entry of them).  Synchronises. */
+int cf_trainer_read(cf_trainer* trainer, float* const* tensors_host, float* const* rms_host, float* const* mom_host);
+
 /* Kernel launches issued by this library since process start (bench.py's gpu_launches). */
 int64_t cf_launch_count(void);
 
