@@ -14,10 +14,34 @@ def hpm_from_golden(g):
     return {k[4:]: int(v) for k, v in g.items() if k.startswith("hpm_")}
 
 
-def random_bn_weights(seed):
-    """Seeded ResNetRNN weights (shipped hyper-parameters) with non-trivial BN gamma/beta/moving stats."""
+# tc_create runs f16e5 only while max |w| * kCandScale * kCorrScale < 60000 (the fp16 weight plane holds S w)
+F16E5_WMAX = 60000.0 / (2.8853900817779268 * 64.0)
+
+
+def hparams(kind, c=32, h=64, n_res=2, n_layers=3):
+    """Hyper-parameters of a `kind` network: conv channels c and blocks n_res, GRU units h and layers n_layers."""
+    hpm = {}
+    if kind != "RNN":
+        hpm.update(layer_size_res=c, n_layers_res=n_res)
+    if kind != "ResNet":
+        hpm.update(layer_size=h, n_layers=n_layers)
+    return hpm
+
+
+def build_model(kind, engine, w, **hpm):
+    """A `kind` model on `engine` with weights w; hyper-parameters not in hpm are the shipped ones."""
+    from catfish_b200 import neural_network, weights
+    full = dict(weights.SHIPPED_HPARAMS)
+    full.update(hpm)
+    m = neural_network.build_model(kind, engine=engine, **full)
+    m.set_weights(w)
+    return m
+
+
+def bn_weights(kind, seed, **hpm):
+    """Seeded weights of any shape with non-trivial BN gamma / beta / moving statistics."""
     from catfish_b200 import weights
-    w = weights.random_init("ResNetRNN", seed=seed, layer_size=64, n_layers=3, layer_size_res=32, n_layers_res=2)
+    w = weights.random_init(kind, seed=seed, **hpm)
     rng = np.random.default_rng(seed + 1000)
     for k in sorted(w):
         if k.endswith("moving_mean"):
@@ -29,6 +53,11 @@ def random_bn_weights(seed):
         elif k.endswith("gamma"):
             w[k] = rng.uniform(0.5, 1.5, size=w[k].shape).astype(np.float32)
     return w
+
+
+def random_bn_weights(seed):
+    """Seeded ResNetRNN weights (shipped hyper-parameters) with non-trivial BN gamma/beta/moving stats."""
+    return bn_weights("ResNetRNN", seed, layer_size=64, n_layers=3, layer_size_res=32, n_layers_res=2)
 
 
 def random_labels(rng, n, p_switch=0.08):

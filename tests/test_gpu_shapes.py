@@ -7,47 +7,14 @@ an explicitly padded network bit for bit, and deep stacks against the fp32 CUDA-
 import numpy as np
 import pytest
 
-from helpers import allowed_label_flips
-from catfish_b200 import infer, neural_network, synth, weights
+from helpers import allowed_label_flips, bn_weights as _bn_weights, build_model as _model, hparams as _hpm
+from catfish_b200 import infer, synth, weights
 from oracle import postprocess, tf_graph
 
 pytestmark = pytest.mark.gpu
 
 PROB_TOL = 1e-3
 PAD_C, PAD_H = 32, 64
-
-
-def _bn_weights(kind, seed, **hpm):
-    """Seeded weights of any shape with non-trivial BN gamma / beta / moving statistics."""
-    w = weights.random_init(kind, seed=seed, **hpm)
-    rng = np.random.default_rng(seed + 1000)
-    for k in sorted(w):
-        if k.endswith("moving_mean"):
-            w[k] = rng.normal(0, 0.3, size=w[k].shape).astype(np.float32)
-        elif k.endswith("moving_variance"):
-            w[k] = rng.uniform(0.3, 2.0, size=w[k].shape).astype(np.float32)
-        elif k.endswith("beta"):
-            w[k] = rng.normal(0, 0.2, size=w[k].shape).astype(np.float32)
-        elif k.endswith("gamma"):
-            w[k] = rng.uniform(0.5, 1.5, size=w[k].shape).astype(np.float32)
-    return w
-
-
-def _hpm(kind, c=32, h=64, n_res=2, n_layers=3):
-    hpm = {}
-    if kind != "RNN":
-        hpm.update(layer_size_res=c, n_layers_res=n_res)
-    if kind != "ResNet":
-        hpm.update(layer_size=h, n_layers=n_layers)
-    return hpm
-
-
-def _model(kind, engine, w, **hpm):
-    full = dict(weights.SHIPPED_HPARAMS)
-    full.update(hpm)
-    m = neural_network.build_model(kind, engine=engine, **full)
-    m.set_weights(w)
-    return m
 
 
 def _check_intervals(got_hps, scores_gpu, p_ref, threshold=0.5):

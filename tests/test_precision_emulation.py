@@ -1,6 +1,7 @@
 """CPU: the operand-format emulation behind DESIGN.md section 4 keeps its ordering on a small sample
 (single 16-bit passes miss the contract's margin, the split formats do not), and the f16e5 budget statistic of
-tests/test_gpu_operand_formats.py tells a lost correction term from the correct scheme."""
+tests/test_gpu_operand_formats.py tells a lost correction term from the correct scheme, as the bf16x3 budget of
+tests/test_gpu_precision_budgets.py tells one convolution tap without a correction pass."""
 import os
 import sys
 
@@ -51,3 +52,23 @@ def test_f16e5_fault_budget(shipped_weights):
     for fault in ("-lo", "-hi", "-both"):
         assert worst[fault] >= 3 * worst[""], (fault, worst)
     assert max_dp["-both"] < 1e-3, max_dp
+
+
+def test_bf16x3_one_tap_fault_budget(shipped_weights):
+    """The shipped network in the engine's formats, two tiles of synthetic-read windows, with one tap of the first
+    32 -> 32 convolution losing a bf16x3 correction pass: max |p - p64| stays inside the 1e-3 contract, while the
+    worst-tile RMS is at least 3x that of the correct scheme - the budget of tests/test_gpu_precision_budgets.py
+    sees such a fault, the contract tolerance does not."""
+    import precision_emulation as pe
+    from oracle import tf_graph
+    x = pe.synthetic_windows(2 * 128)
+    ref = tf_graph.forward_np(shipped_weights, x, np.float64)
+    worst, max_dp = {}, {}
+    for fault in ("", "-lo", "-hi"):
+        bf3 = pe.confine(pe.make_mm("bf16x3" + fault), pe.make_mm("bf16x3"), {1})    # the middle tap
+        p = pe.forward(shipped_weights, x, pe.engine_mm("ResNetRNN", bf16x3=bf3))
+        worst[fault] = float(pe.tile_rms(p, ref).max())
+        max_dp[fault] = float(np.abs(p - ref).max())
+    for fault in ("-lo", "-hi"):
+        assert worst[fault] >= 3 * worst[""], (fault, worst)
+        assert max_dp[fault] < 1e-3, (fault, max_dp)

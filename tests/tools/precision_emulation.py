@@ -8,13 +8,15 @@ a product of ROUNDED operands accumulated in fp64 (the tensor core accumulates i
 difference is below the effects studied here).  The Cin = 1 convolutions, the head and all
 elementwise math stay exact, as in the CUDA engine.  Schemes:
   bf16x3     a_hi w_hi + a_lo w_hi + a_hi w_lo, bf16 pieces              (the shipped scheme, 3 passes)
+  bf16x3 faults, each a correction pass lost:  "-lo" drops a_lo w_hi, "-hi" drops a_hi w_lo, "-both" drops both
   bf16x1     one bf16 pass                          fp16x1   one fp16 pass
   fp16x2     (a_hi + a_lo) w_hi, fp16 pieces                               (2 passes)
   fp16+e5m2  a_hi w_hi in fp16 + [a_lo 2^s | a_hi 2^-s] [w_hi 2^-s ; w_lo 2^s] in e5m2, the a_hi 2^-s byte
              truncated (it is the top byte of the fp16 value, never stored in HBM)
              (1 fp16 pass + 1 fp8 pass with doubled K = 2 pass-equivalents; DESIGN.md section 4)
   fp16+e5m2 faults, each a correction term lost:  "-lo" drops a_lo w_hi, "-hi" drops a_hi w_lo, "-both" drops both
-engine_mm(kind) picks the format per matmul the way the tensor-core engine does.
+engine_mm(kind) picks the format per matmul the way the tensor-core engine does; confine(fault, base, calls) applies
+a fault to chosen matmuls of one forward pass only.
 Test infrastructure only (imports oracle/).
 """
 import os
@@ -54,10 +56,18 @@ def make_mm(scheme, s_corr=6):
             return rnd(a, bf) @ rnd(w, bf)
         if scheme == "fp16x1":
             return rnd(a, hf) @ rnd(w, hf)
-        if scheme == "bf16x3":
+        if scheme.startswith("bf16x3"):
+            fault = scheme[len("bf16x3"):]
+            if fault not in ("", "-lo", "-hi", "-both"):
+                raise ValueError(scheme)
             ah, al = split(a, bf)
             wh, wl = split(w, bf)
-            return ah @ wh + al @ wh + ah @ wl
+            out = ah @ wh
+            if fault not in ("-lo", "-both"):
+                out = out + al @ wh
+            if fault not in ("-hi", "-both"):
+                out = out + ah @ wl
+            return out
         if scheme == "fp16x2":
             ah, al = split(a, hf)
             return (ah + al) @ rnd(w, hf)
@@ -80,14 +90,19 @@ def make_mm(scheme, s_corr=6):
     return mm
 
 
-def engine_mm(kind, f16e5="fp16+e5m2"):
+def engine_mm(kind, f16e5="fp16+e5m2", bf16x3="bf16x3"):
     """Matmul in the operand format the tensor-core engine uses for each product of the H = 64 networks, with
-    `f16e5` (a fp16+e5m2 scheme, possibly a fault) where the engine runs f16e5.  ResNetRNN: the convolutions
-    (K = 32) and GRU layer 0 (K = 32 + 64) are bf16x3, the 128-wide layers (K = 128 + 64) f16e5.  RNN: every layer is
-    f16e5, except that layer 0's scalar input row (K = 1 + 64) is an exact rank-1 update."""
-    if kind not in ("ResNetRNN", "RNN"):
+    `f16e5` (a fp16+e5m2 scheme, possibly a fault) where the engine runs f16e5 and `bf16x3` (a bf16x3 scheme or a
+    matmul, e.g. from confine) where it runs bf16x3.  ResNetRNN: the convolutions (K = 32) and GRU layer 0
+    (K = 32 + 64) are bf16x3, the 128-wide layers (K = 128 + 64) f16e5.  RNN: every layer is f16e5, except that layer
+    0's scalar input row (K = 1 + 64) is an exact rank-1 update.  "bf16x3": a network the engine runs in bf16x3
+    throughout (one or three or more residual blocks, ResNet, or GRU weights beyond f16e5's range)."""
+    if kind not in ("ResNetRNN", "RNN", "bf16x3"):
         raise ValueError(kind)
-    bf3, f16 = make_mm("bf16x3"), make_mm(f16e5)
+    bf3 = make_mm(bf16x3) if isinstance(bf16x3, str) else bf16x3
+    if kind == "bf16x3":
+        return bf3
+    f16 = make_mm(f16e5)
 
     def mm(a, w):
         k = np.shape(a)[1]
@@ -95,6 +110,18 @@ def engine_mm(kind, f16e5="fp16+e5m2"):
             a, w = np.asarray(a, np.float64), np.asarray(w, np.float64)
             return a[:, :1] @ w[:1] + f16(a[:, 1:], w[1:])
         return f16(a, w) if kind == "RNN" or k == 128 + 64 else bf3(a, w)
+    return mm
+
+
+def confine(fault, base, calls):
+    """A matmul that runs `fault` on the calls whose 0-based ordinal is in `calls` and `base` on every other; the
+    ordinals count the calls of one forward pass (so use a fresh one per pass).  forward() calls one conv tap per
+    matmul, first tap first: the three taps of the first 32 -> 32 convolution are calls 0, 1, 2."""
+    n = [0]
+
+    def mm(a, w):
+        n[0] += 1
+        return (fault if n[0] - 1 in calls else base)(a, w)
     return mm
 
 
