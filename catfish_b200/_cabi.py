@@ -83,6 +83,12 @@ SIGNATURES = {
                                                  c_void]),
     "cf_sweep_thresholds": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int32, c_void, ctypes.c_int64, c_void, ctypes.c_int32,
                                            c_i64_p, c_void]),
+    "cf_curve_create": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int32, c_void, ctypes.c_int64, c_void,
+                                       ctypes.POINTER(c_void)]),
+    "cf_curve_summary": (ctypes.c_int, [c_void, c_i64_p, c_i64_p, c_i64_p, c_i64_p, ctypes.POINTER(ctypes.c_double),
+                                        ctypes.POINTER(ctypes.c_double)]),
+    "cf_curve_read": (ctypes.c_int, [c_void, ctypes.c_int64, ctypes.c_int64, c_void, c_void]),
+    "cf_curve_destroy": (None, [c_void]),
     "cf_vote_events": (ctypes.c_int, [ctypes.c_int32, c_void, ctypes.c_int64, c_i64_p, ctypes.c_int64, ctypes.c_int64,
                                       ctypes.c_int64, c_void, c_i64_p, c_i64_p, c_i64_p, ctypes.POINTER(ctypes.c_int32),
                                       c_void]),

@@ -902,6 +902,95 @@ int cf_sweep_thresholds(int32_t device, const float* values_dev, int32_t values_
     return CF_OK;
 }
 
+}  // extern "C"
+
+struct cf_curve {
+    int device = 0;
+    cf::CurveSummary sum;      // n_rows counts the rows after row 0
+    cf::CurveRows rows;
+};
+
+extern "C" {
+
+int cf_curve_create(int32_t device, const float* values_dev, int32_t values_are_logits, const uint8_t* labels_dev,
+                    int64_t n, void* stream, cf_curve** out) {
+    if (!out || n < 0 || n > INT32_MAX || (n > 0 && (!values_dev || !labels_dev))) {
+        cf::set_error("cf_curve_create: bad argument");
+        return CF_ERR_BAD_ARG;
+    }
+    *out = nullptr;
+    std::unique_ptr<cf_curve> c(new cf_curve());
+    c->device = device;
+    c->sum.roc_auc = c->sum.average_precision = NAN;
+    if (n > 0) {
+        cf::DeviceGuard guard;
+        CF_TRY(guard.set(device));
+        cudaStream_t st = static_cast<cudaStream_t>(stream);
+        const int s = cf::k13_curve(values_dev, values_are_logits != 0, labels_dev, n, &c->rows, &c->sum, st);
+        const cudaError_t e = cudaStreamSynchronize(st);    // scratch is freed on return, also after a failed launch
+        CF_TRY(s);
+        if (e != cudaSuccess) {
+            cf::set_error("cf_curve_create: %s", cudaGetErrorString(e));
+            return CF_ERR_CUDA;
+        }
+    }
+    *out = c.release();
+    return CF_OK;
+}
+
+int cf_curve_summary(const cf_curve* c, int64_t* n_points, int64_t* n_neg, int64_t* n_pos, int64_t* n_nan,
+                     double* roc_auc, double* average_precision) {
+    if (!c) { cf::set_error("cf_curve_summary: NULL curve"); return CF_ERR_BAD_ARG; }
+    if (n_points) *n_points = c->sum.n_rows + 1;
+    if (n_neg) *n_neg = c->sum.n_neg;
+    if (n_pos) *n_pos = c->sum.n_pos;
+    if (n_nan) *n_nan = c->sum.n_nan;
+    if (roc_auc) *roc_auc = c->sum.roc_auc;
+    if (average_precision) *average_precision = c->sum.average_precision;
+    return CF_OK;
+}
+
+int cf_curve_read(const cf_curve* c, int64_t first, int64_t count, double* thresholds_host, int64_t* counts_host) {
+    if (!c || first < 0 || count < 0 || first > c->sum.n_rows + 1 || count > c->sum.n_rows + 1 - first) {
+        cf::set_error("cf_curve_read: bad argument (rows [%lld, %lld + %lld) of %lld)", (long long)first,
+                      (long long)first, (long long)count, c ? (long long)(c->sum.n_rows + 1) : 0LL);
+        return CF_ERR_BAD_ARG;
+    }
+    if (count == 0) return CF_OK;
+    const int64_t n0 = c->sum.n_neg, n1 = c->sum.n_pos;
+    if (first == 0) {                                         // threshold +inf: nothing predicted positive
+        if (thresholds_host) thresholds_host[0] = INFINITY;
+        if (counts_host) { counts_host[0] = 0; counts_host[1] = 0; counts_host[2] = n0; counts_host[3] = n1; }
+    }
+    const int64_t r0 = first == 0 ? 0 : first - 1, m = first + count - 1 - r0, skip = first == 0 ? 1 : 0;
+    if (m == 0) return CF_OK;
+    cf::DeviceGuard guard;
+    CF_TRY(guard.set(c->device));
+    std::vector<float> thr((size_t)m);
+    std::vector<uint32_t> tp((size_t)m), fp((size_t)m);
+    CF_CUDA(cudaMemcpy(thr.data(), c->rows.thr.as<float>() + r0, sizeof(float) * (size_t)m, cudaMemcpyDeviceToHost));
+    CF_CUDA(cudaMemcpy(tp.data(), c->rows.tp.as<uint32_t>() + r0, sizeof(uint32_t) * (size_t)m, cudaMemcpyDeviceToHost));
+    CF_CUDA(cudaMemcpy(fp.data(), c->rows.fp.as<uint32_t>() + r0, sizeof(uint32_t) * (size_t)m, cudaMemcpyDeviceToHost));
+    for (int64_t i = 0; i < m; ++i) {
+        if (thresholds_host) thresholds_host[skip + i] = (double)thr[(size_t)i];
+        if (counts_host) {
+            int64_t* o = counts_host + 4 * (skip + i);
+            o[0] = tp[(size_t)i];
+            o[1] = fp[(size_t)i];
+            o[2] = n0 - (int64_t)fp[(size_t)i];
+            o[3] = n1 - (int64_t)tp[(size_t)i];
+        }
+    }
+    return CF_OK;
+}
+
+void cf_curve_destroy(cf_curve* c) {
+    if (!c) return;
+    cf::DeviceGuard guard;
+    if (c->rows.thr.ptr) guard.set(c->device);               // the rows are freed on their device
+    delete c;
+}
+
 int cf_vote_events(int32_t device, const double* scores_dev, int64_t n_scores, const int64_t* event_lengths_host,
                    int64_t n_events, int64_t start, int64_t length, int32_t* classes_dev, int64_t* n_voted_out,
                    int64_t* start_event_out, int64_t* final_event_out, int32_t* empty_event_out, void* stream) {

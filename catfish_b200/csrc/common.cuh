@@ -262,6 +262,23 @@ size_t k11_scratch_bytes(int n_thresholds);
 int k11_sweep(const float* values, bool values_are_logits, const uint8_t* labels, int64_t n,
               const std::vector<float>& sorted, void* scratch, long long* counts_host, cudaStream_t stream);
 
+// ---------------------------------------------------------------- k13: exact score curves
+// The rows after row 0 (threshold +inf): one per distinct non-NaN score, in descending score order.
+struct CurveRows {
+    DevBuf thr;    // float [n_rows]: the score
+    DevBuf tp;     // uint32 [n_rows]: positives with a score >= thr
+    DevBuf fp;     // uint32 [n_rows]: negatives with a score >= thr
+};
+struct CurveSummary {
+    int64_t n_rows = 0, n_neg = 0, n_pos = 0, n_nan = 0;
+    double roc_auc = 0.0, average_precision = 0.0;
+};
+// Sorts and counts 1 <= n < 2^31 positions (scores, or logits with values_are_logits; labels 0 / 1); fills rows and
+// sum.  CF_ERR_BAD_ARG naming the first bad position when a label is not 0 / 1 or a score is neither NaN nor in [0, 1].
+// Scratch (8.5 B per position) is allocated and freed inside; synchronises the stream.
+int k13_curve(const float* values, bool values_are_logits, const uint8_t* labels, int64_t n, CurveRows* rows,
+              CurveSummary* sum, cudaStream_t stream);
+
 // ---------------------------------------------------------------- k10: event voting (next row N3)
 int k10_vote_events(const double* scores, int64_t n_scores, const int64_t* ev_begin, int64_t first_event,
                     int64_t n_voted, int32_t* classes, int32_t* empty_flag, cudaStream_t stream);

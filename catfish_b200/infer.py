@@ -11,6 +11,7 @@ infer_class_from_signal :12   infer_class_from_signal     cf_infer_reads
                               infer_reads
 (the CLI's per-file loop)     infer_stream                cf_exec_infer_reads
 (precision_recall_ROC.py)     evaluate_reads              cf_infer_reads + cf_sweep_thresholds
+(metrics.py, sklearn curves)  evaluate_reads_curve        cf_infer_reads + cf_curve_create
 process_signal :77            process_signal (h5py)       cf_normalize_reads
 normalize_raw_signal :96      normalize_raw_signal        cf_normalize_reads
 reshape_input :108            reshape_input               (pure reshape, host)
@@ -214,6 +215,55 @@ def evaluate_reads(raws, labels, model, thresholds, window_size=35):
     Row i equals ``metrics.confusion_matrix`` of the labels against ``scores >= thresholds[i]`` for the scores
     ``infer_reads(..., return_scores=True)`` gives; reads with MAD = 0 have NaN scores, predicted 0 everywhere.
     Batches are processed in groups of about one engine pass; no probability travels to the host."""
+    arrays, labs = _labelled_reads(raws, labels, model, window_size)
+    th = np.ascontiguousarray(np.asarray(thresholds, dtype=np.float64).reshape(-1))
+    counts = np.zeros((th.size, 4), np.int64)
+    # no positions: checks the thresholds on the host, before any device work, and leaves the counts at zero
+    _cabi.check(_cabi.load_library().cf_sweep_thresholds(0, None, 0, None, 0, th.ctypes.data, min(th.size, 2 ** 31 - 1),
+                                                         counts.ctypes.data_as(_cabi.c_i64_p), None))
+    if not arrays:
+        return counts
+    offsets = np.zeros(len(arrays) + 1, np.int64)
+    np.cumsum([a.size for a in arrays], out=offsets[1:])
+    params = (0.5, 15, 11, 16)                                 # only the probabilities are used
+    for part in _run_on_model(model, [(arrays[lo:hi], params, False, labs[lo:hi], th)
+                                      for lo, hi in _cut_groups(offsets, _GROUP_SAMPLES, _GROUP_SAMPLES)]):
+        counts += part
+    return counts
+
+
+def evaluate_reads_curve(raws, labels, model, window_size=35, points=True):
+    """The exact curve of labelled raw reads at every distinct score: ``metrics.score_curve`` of the scores
+    ``infer_reads(..., return_scores=True)`` gives and the labels (0 / 1 only, one per sample), as a
+    ``metrics.ScoreCurve``; reads with MAD = 0 have NaN scores, never positive.
+
+    The reads take ``evaluate_reads``' production path, in groups of about one engine pass; each group's network
+    writes its probabilities straight into one device tensor for the whole read set, at the group's offset, and its
+    labels go to one uint8 tensor beside it.  One ``cf_curve_create`` then sorts and counts both.  No probability
+    travels to the host.  Device memory: 5 B per sample for the probabilities and labels, 8.5 B per sample of sort
+    scratch during the count, and 12 B per row of the curve while it is read."""
+    from . import metrics
+    arrays, labs = _labelled_reads(raws, labels, model, window_size)
+    for r, y in enumerate(labs):
+        if y.size and int(y.max()) > 1:
+            raise ValueError("score curve: read %d has a label other than 0 / 1" % r)
+    offsets = np.zeros(len(arrays) + 1, np.int64)
+    np.cumsum([a.size for a in arrays], out=offsets[1:])
+    total = int(offsets[-1])
+    if total == 0:
+        return metrics.score_curve(np.zeros(0, np.float32), np.zeros(0, np.uint8), points=points)
+    torch = _torch()
+    with torch.cuda.device(model.device):
+        probs = torch.empty(total, dtype=torch.float32, device="cuda:%d" % model.device)
+        labs_dev = torch.empty(total, dtype=torch.uint8, device="cuda:%d" % model.device)
+    params = (0.5, 15, 11, 16)                                 # only the probabilities are used
+    _run_on_model(model, [(arrays[lo:hi], params, False, labs[lo:hi], None, (probs, labs_dev, int(offsets[lo])))
+                          for lo, hi in _cut_groups(offsets, _GROUP_SAMPLES, _GROUP_SAMPLES)])
+    return metrics.score_curve(probs, labs_dev, points=points)
+
+
+def _labelled_reads(raws, labels, model, window_size):
+    """The int16 reads and their uint8 labels (one per sample) of ``evaluate_reads`` and ``evaluate_reads_curve``."""
     if window_size != model.window:
         raise ValueError("window_size must equal the model's window (%d)" % model.window)
     arrays = [_as_int16(r) for r in raws]
@@ -231,20 +281,7 @@ def evaluate_reads(raws, labels, model, thresholds, window_size=35):
         if not np.array_equal(y8, y):
             raise ValueError("labels must be small non-negative integers")
         labs.append(y8)
-    th = np.ascontiguousarray(np.asarray(thresholds, dtype=np.float64).reshape(-1))
-    counts = np.zeros((th.size, 4), np.int64)
-    # no positions: checks the thresholds on the host, before any device work, and leaves the counts at zero
-    _cabi.check(_cabi.load_library().cf_sweep_thresholds(0, None, 0, None, 0, th.ctypes.data, min(th.size, 2 ** 31 - 1),
-                                                         counts.ctypes.data_as(_cabi.c_i64_p), None))
-    if not arrays:
-        return counts
-    offsets = np.zeros(len(arrays) + 1, np.int64)
-    np.cumsum([a.size for a in arrays], out=offsets[1:])
-    params = (0.5, 15, 11, 16)                                 # only the probabilities are used
-    for part in _run_on_model(model, [(arrays[lo:hi], params, False, labs[lo:hi], th)
-                                      for lo, hi in _cut_groups(offsets, _GROUP_SAMPLES, _GROUP_SAMPLES)]):
-        counts += part
-    return counts
+    return arrays, labs
 
 
 _STREAM_DEPTH = 2                       # groups in flight in infer_stream
@@ -313,9 +350,11 @@ class _Slot(object):
             self.buf[name] = t
         return t
 
-    def submit(self, arrays, params, return_scores, labels=None, thresholds=None):
+    def submit(self, arrays, params, return_scores, labels=None, thresholds=None, dest=None):
         """Stage, copy and enqueue one group on this slot's stream (returns without waiting for the device).  With
-        ``labels`` (one uint8 array per read) the group is counted at ``thresholds`` instead of returning intervals."""
+        ``labels`` (one uint8 array per read) the group is counted at ``thresholds`` instead of returning intervals,
+        or, with ``dest = (probs, labels, offset)``, its probabilities and labels go to those device tensors at
+        ``offset`` and nothing comes back."""
         torch = self.torch
         threshold, min_run, ext_left, ext_right = params
         n = len(arrays)
@@ -329,13 +368,19 @@ class _Slot(object):
             # the intervals [cap, 2], then the n + 1 interval offsets: one copy brings both back
             m = 2 * cap + n + 1
             out = self._ensure("out", m, torch.int64)
-            probs = self._ensure("probs", total, torch.float32) if return_scores or labels is not None else None
+            if dest is not None:
+                probs, lab_dev = dest[0][dest[2]:dest[2] + total], dest[1][dest[2]:dest[2] + total]
+            elif return_scores or labels is not None:
+                probs = self._ensure("probs", total, torch.float32)
+                lab_dev = self._ensure("lab", total, torch.uint8) if labels is not None else None
+            else:
+                probs = None
             _concat_into(stage.numpy()[:total], arrays, offsets)
             raw[:total].copy_(stage[:total], non_blocking=True)
             if labels is not None:
                 lab_pin = self._ensure("lab_pin", total, torch.uint8, pinned=True)
                 np.concatenate(labels, out=lab_pin.numpy()[:total])
-                self._ensure("lab", total, torch.uint8)[:total].copy_(lab_pin[:total], non_blocking=True)
+                lab_dev[:total].copy_(lab_pin[:total], non_blocking=True)
             _cabi.check(self.infer(
                 self.target, raw.data_ptr(), _offsets_ptr(offsets), n, probs.data_ptr() if probs is not None else None,
                 out.data_ptr(), out.data_ptr() + 16 * cap, cap, threshold, min_run, ext_left, ext_right,
@@ -345,17 +390,21 @@ class _Slot(object):
                 probs_pin = self._ensure("probs_pin", total, torch.float32, pinned=True)
                 probs_pin[:total].copy_(probs[:total], non_blocking=True)
             self.event.record(self.stream)
-        self.group = (offsets, cap, return_scores, thresholds if labels is not None else None)
+        self.group = (offsets, cap, return_scores, thresholds if labels is not None else None, dest is not None)
 
     def done(self):
         return self.event.query()
 
     def results(self):
         """Wait for the group and return ``(offsets, intervals, interval_offsets, scores or None)`` of its reads - or,
-        for a group submitted with labels, its int64 ``[T, 4]`` confusion counts.  The slot is then free."""
-        offsets, cap, return_scores, thresholds = self.group
+        for a group submitted with labels, its int64 ``[T, 4]`` confusion counts (None with ``dest``).  The slot is
+        then free."""
+        offsets, cap, return_scores, thresholds, to_dest = self.group
         self.group = None
         n, total = len(offsets) - 1, int(offsets[-1])
+        if to_dest:
+            self.event.synchronize()
+            return None
         if thresholds is not None:
             counts = np.zeros((thresholds.size, 4), np.int64)
             # queued behind the group on the slot's stream; synchronises

@@ -6,7 +6,10 @@ The per-position counting for a forward pass runs on the GPU inside ``RNN.test_n
 (C ABI ``cf_validate_windows``); ``confusion_matrix`` here is the array-level twin for label
 lists that already live on the host.  ``confusion_curve`` counts at many thresholds at once on the GPU (K11,
 ``cf_sweep_thresholds``); ``precision_recall_curve`` / ``roc_curve`` turn those counts into the rates of the
-reference's networks/precision_recall_ROC.py.  Plotting helpers are out of scope.
+reference's networks/precision_recall_ROC.py.  ``score_curve`` gives the exact curve at every distinct score with its
+ROC AUC and average precision (K13, ``cf_curve_create``: a radix sort on the GPU), the numbers sklearn's
+``roc_auc_score`` / ``average_precision_score`` give in the reference's networks/metrics.py.  Plotting helpers are out
+of scope.
 """
 
 import collections
@@ -172,3 +175,84 @@ def roc_curve(counts):
     tp, fp, tn, fn = _counts_rows(counts)
     fpr, tpr = _rates(fp, fp + tn), _rates(tp, tp + fn)
     return RocCurve(fpr, tpr, _trapezoid(fpr, tpr))
+
+
+def average_precision(counts):
+    """sklearn's ``average_precision_score`` over the rows of ``confusion_curve`` (or ``score_curve``): the step sum
+    ``sum (R_i - R_{i-1}) P_i`` with the rows taken in increasing number of predicted positives (tp + fp) from recall
+    0; precision is 0 where nothing is predicted positive.  NaN when no row has a positive label.  Over a sweep it
+    covers only the given thresholds; over every row of a ``score_curve`` without NaN scores it is that curve's
+    ``average_precision``."""
+    tp, fp, tn, fn = _counts_rows(counts)
+    positives = tp + fn
+    if not positives.size or not positives.any():
+        return float("nan")
+    order = np.lexsort((tp, tp + fp))
+    tp, predicted, positives = tp[order], (tp + fp)[order], positives[order]
+    recall = _rates(tp, positives)
+    return float(np.sum(np.diff(recall, prepend=0.0) * _rates(tp, predicted)))
+
+
+# ------------------------------------------------------------------------------ exact curves
+ScoreCurve = collections.namedtuple("ScoreCurve", "thresholds counts roc_auc average_precision")
+
+
+def score_curve(scores, labels, logits=False, points=True):
+    """The exact curve at every distinct score (K13, ``cf_curve_create``): ``ScoreCurve(thresholds, counts, roc_auc,
+    average_precision)``.
+
+    ``thresholds`` float64 ``[P]`` holds +inf and then every distinct non-NaN score in decreasing order; row i of
+    ``counts`` (int64 ``[P, 4]``, tp, fp, tn, fn) is ``confusion_curve(scores, labels, [thresholds[i]])``, so
+    ``roc_curve`` and ``precision_recall_curve`` apply to it unchanged - these are the points of sklearn's
+    ``roc_curve`` without ``drop_intermediate``.  ``roc_auc`` and ``average_precision`` are sklearn's
+    ``roc_auc_score`` and ``average_precision_score``, with NaN scores taken as one tie below every number (they
+    close the curve at (1, 1)); NaN when a class they divide by is empty.  Deterministic.
+
+    Labels must be 0 or 1 and scores NaN or in [0, 1] (``logits=True``: logits, mapped as the network's head does).
+    Inputs are staged as ``confusion_curve`` stages them: numpy arrays are checked on the host and uploaded, CUDA
+    float32 / uint8 tensors are used in place and checked on the device.  The GPU sorts every score; with
+    ``points=False`` only the areas come back (``thresholds`` and ``counts`` are None), which saves the copy of a
+    curve that can hold as many rows as positions."""
+    from . import _cabi
+    import ctypes
+    n = _length(scores)
+    if _length(labels) != n:
+        raise ValueError("Length of labels to compare is not equal.")
+    lib = _cabi.load_library()
+    if not _is_cuda_tensor(labels):
+        y = np.asarray(labels).reshape(-1)
+        bad = np.flatnonzero((y != 0) & (y != 1))
+        if bad.size:
+            raise ValueError("score curve: label %r at position %d is not 0 or 1" % (y[bad[0]], bad[0]))
+    if not logits and not _is_cuda_tensor(scores):
+        s = np.asarray(scores).reshape(-1)
+        bad = np.flatnonzero(~np.isnan(s) & ((s < 0) | (s > 1)))
+        if bad.size:
+            raise ValueError("score curve: score %r at position %d is neither NaN nor in [0, 1]" % (s[bad[0]], bad[0]))
+    handle = ctypes.c_void_p()
+    if n == 0:
+        _cabi.check(lib.cf_curve_create(0, None, int(bool(logits)), None, 0, None, ctypes.byref(handle)))
+    else:
+        import torch
+        dev = next((x.device.index for x in (scores, labels) if _is_cuda_tensor(x)), None)
+        if dev is None:
+            from . import get_device
+            dev = get_device()
+        with torch.cuda.device(dev):
+            s = _device_scores(torch, scores, dev)
+            y = _device_labels(torch, labels, dev)
+            _cabi.check(lib.cf_curve_create(dev, s.data_ptr(), int(bool(logits)), y.data_ptr(), n,
+                                            torch.cuda.current_stream(dev).cuda_stream, ctypes.byref(handle)))
+    try:
+        rows = ctypes.c_int64()
+        auc, ap = ctypes.c_double(), ctypes.c_double()
+        _cabi.check(lib.cf_curve_summary(handle, ctypes.byref(rows), None, None, None, ctypes.byref(auc),
+                                         ctypes.byref(ap)))
+        thresholds = counts = None
+        if points:
+            thresholds = np.empty(rows.value, np.float64)
+            counts = np.empty((rows.value, 4), np.int64)
+            _cabi.check(lib.cf_curve_read(handle, 0, rows.value, thresholds.ctypes.data, counts.ctypes.data))
+        return ScoreCurve(thresholds, counts, auc.value, ap.value)
+    finally:
+        lib.cf_curve_destroy(handle)

@@ -295,6 +295,33 @@ int cf_validate_windows_sweep(cf_model* model, const float* x_dev, const uint8_t
                               int64_t* counts_out_host, double* accuracy_out, double* loss_out, void* stream);
 
 /*
+ * Exact score curves (K13; the reference's networks/metrics.py: sklearn's roc_curve, precision_recall_curve,
+ * roc_auc_score and average_precision_score over validation outputs): confusion counts at every distinct score.
+ * Labels must be 0 or 1 and scores NaN or in [0, 1] (after the logit mapping with values_are_logits), else
+ * CF_ERR_BAD_ARG naming the first bad position.  -0.0 and +0.0 are one score.  With s_1 > ... > s_{P-1} the distinct
+ * non-NaN scores, row 0 is at threshold +inf and row i at s_i; each row holds (tp, fp, tn, fn) for "predicted
+ * positive <=> (double)p >= threshold", as cf_sweep_thresholds at that threshold (NaN scores are never positive).
+ * roc_auc is the trapezoid over the rows and the closing point (1, 1) - NaN scores form one tie below every number -
+ * summed exactly in int64 and divided once; average_precision is sum (R_i - R_{i-1}) P_i over the same points in
+ * float64, in a fixed order.  Both are deterministic; roc_auc is NaN without positives or negatives, average_precision
+ * NaN without positives.  n = 0 gives one row (+inf, all zeros) and needs no device.  1 <= n <= 2^31 - 1 positions
+ * per call.
+ */
+typedef struct cf_curve cf_curve;
+/* Sorts and counts; synchronises.  values_dev float32 [n], labels_dev uint8 [n] on `device`.  During the call the
+ * library holds 8.5 B of scratch per position; the curve keeps 12 B per row on the device until destroyed. */
+int cf_curve_create(int32_t device, const float* values_dev, int32_t values_are_logits, const uint8_t* labels_dev,
+                    int64_t n, void* stream, cf_curve** out);
+/* P, N0, N1, number of NaN scores, roc_auc, average_precision (any pointer may be NULL). */
+int cf_curve_summary(const cf_curve* curve, int64_t* n_points, int64_t* n_neg, int64_t* n_pos, int64_t* n_nan,
+                     double* roc_auc, double* average_precision);
+/* Rows [first, first + count) to the host: thresholds float64 [count] (row 0 = +inf), counts int64 [count][4] =
+ * tp, fp, tn, fn (either pointer may be NULL).  CF_ERR_BAD_ARG unless 0 <= first <= first + count <= P.
+ * Synchronises. */
+int cf_curve_read(const cf_curve* curve, int64_t first, int64_t count, double* thresholds_host, int64_t* counts_host);
+void cf_curve_destroy(cf_curve* curve);
+
+/*
  * cf_vote_events - "next" row N3: the arithmetic of correct_events (networks/correct_output.py:38-61,
  * unfinished in the reference): walk the events as the reference's loop does (start found at the
  * first event whose first measurement is >= start; stop before the event that would pass `length`,
